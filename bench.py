@@ -2,6 +2,7 @@
 """bench.py -- aggregate MCMC sweeps/s across chains (BASELINE.json's metric).
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun)
+    python bench.py ... --dump-outputs DIR                   (+ the last timed step's results as DIR/*.npy)
     python bench.py --impl reference --steps K --warmup W    (the reference's CPU path)
 
 Workload = BASELINE.json config 4: g2s2 (526 x 296, the largest NOW subset), 16 384 chains IN TOTAL, sharded over the
@@ -31,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 # algorithmic work per sweep (SURVEY.md section 8d closed forms): canonical cells C, smem bytes B = C/8,
 # fp64 candidate weights F = M(N+2) -> 10 F flops, HBM bytes per thinned sample
@@ -83,7 +85,12 @@ def parse_args():
     ap.add_argument("--stationary-chains", type=int, default=4096)
     ap.add_argument("--cpu-calls", type=int, default=0, help="mcmc_sample() calls per CPU process (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                    "(float64; rank 0: the global cross-chain result and its own shard's per-chain arrays)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 # ------------------------------------------------------------------ CPU reference arm
@@ -107,7 +114,7 @@ def cpu_reference_run(dataset, calls, procs):
             raise RuntimeError("reference binary failed: %r" % rcs)
         return procs * calls * 10 / dt, "reference"
     # no prebuilt reference binary: time the restatement (one process per core)
-    code = ("import sys; sys.path.insert(0, %r); from oracle import oracle as O; import bench;"
+    code = ("import sys; sys.dont_write_bytecode = True; sys.path.insert(0, %r); from oracle import oracle as O; import bench;"
             "X,h=bench.load_dataset(%r); o=O.Oracle(X,h).source_mt(int(sys.argv[1])); o.randomize();"
             "[o.sample() for _ in range(%d)]" % (ROOT, dataset, calls))
     O.build()
@@ -230,6 +237,35 @@ class Job:
         return h2d, d2h
 
 
+def _seeded_rows(n, cap):
+    """all of range(n), or a fixed sorted sample of `cap` of them"""
+    import numpy as np
+    return np.arange(n) if n <= cap else np.sort(np.random.default_rng(20060206).choice(n, cap, replace=False))
+
+
+def dump_outputs(out_dir, job, run):
+    """What a caller of the timed path receives from its last step, so that two builds can be compared output for output (the
+    inputs -- dataset, seed, chain ids -- are fixed by the arguments): the cross-chain result (chosen global chain ids, the
+    E[-logL] minimum and sigma, the chosen chains' pair-order counts), E[-logL], E[c], E[d] of every chain of this rank, and
+    the final state and stored pi samples of a fixed sample of 64 chains.  float64 holds every integer here exactly; per-chain
+    arrays beyond 262 144 chains are sampled the same way, which keeps the dump under 64 MB for every dataset."""
+    import numpy as np
+    res = run.cross_chain_result()
+    stats = run.chain_stats()
+    rows = _seeded_rows(job.n_local, 1 << 18)
+    some = _seeded_rows(job.n_local, 64)
+    states = [run.state(int(i)) for i in some]
+    out = {"chosen": res["chosen"], "min_sigma": [res["min"], res["sigma"]], "po_counts": res["counts"][:len(res["chosen"])],
+           "chain_ids": rows + job.rank * job.n_local, "e_negloglik": stats["e_negloglik"][rows], "e_c": stats["e_c"][rows],
+           "e_d": stats["e_d"][rows], "sample_chain_ids": some + job.rank * job.n_local,
+           "sample_pi_history": np.stack([run.fetch_samples(int(i), full=False)["pi"] for i in some])}
+    for k in ("a", "b", "pi", "c", "d", "loglik"):
+        out["sample_" + k] = np.stack([s[k] for s in states])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def main():
     args = parse_args()
     if args.impl == "reference":
@@ -310,6 +346,8 @@ def main():
         clocks.start()
     dt, launches, sweep_ms, dev_ms = timed(job, run, args.steps, 0, True)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, job, run)
     run.close()
     dt_e2e, _, _, _ = timed(job, None, args.steps, args.warmup, False)
 

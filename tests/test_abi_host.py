@@ -82,18 +82,6 @@ def test_genus_and_sites_readers(S, tmp_path):
         ds.read_names(str(g), None)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Dataset"), reason="reference tree not present")
-@pytest.mark.parametrize("name", NOW)
-def test_readers_on_the_reference_files(S, name):
-    ds = S.Dataset.read_txt(f"/root/reference/Dataset/{name}.txt")
-    X, hard = load_hex_dataset(name)
-    X2, h2 = ds.arrays()
-    assert np.array_equal(X, X2) and np.array_equal(hard, h2)
-    ds.read_names(f"/root/reference/Dataset/{name}.genus", f"/root/reference/Dataset/{name}.sites")
-    stars = [ds.site_age(n)[2] for n in range(ds.N)]
-    assert np.array_equal(np.array(stars, np.uint8), hard)  # '*' in .sites == '*' in .txt
-
-
 def test_synthetic_generator(S):
     ds = S.Dataset.synthetic(1024, 4096, 16)
     X, hard = ds.arrays()

@@ -237,31 +237,35 @@ def test_reference_file_writers(S, oracle_mod, tmp_path):
 
 
 def test_cli_drop_in_full_length_vs_reference_cli(S, oracle_mod, tmp_path):
-    """`mcmc 7 < g10s10.txt`, the call script.py:44-45 makes: the UNMODIFIED reference main()
-    (1000 + 1000 calls = 20 000 sweeps, files under Chains/chain_07/) against this repo's `mcmc`
-    replaying the tape the reference recorded.  All five files are byte-identical."""
+    """`mcmc 7 < g10s10.txt`, the call script.py:44-45 makes: the UNMODIFIED reference main() with GSL_RNG_SEED=7
+    (1000 + 1000 calls = 20 000 sweeps, files under Chains/chain_07/) left E[-logL] = tests/golden/ref_free_g10s10.npz's
+    e_negloglik[7] in its exp_data.csv (tools/make_golden_free.py).  This repo's `mcmc` replays the shim's MT19937 stream of
+    that seed (regenerated by the oracle, tests/test_oracle_vs_ref.py) and must print the same number; its chain_data.csv
+    carries the oracle's 1000 samples."""
     import subprocess
     from tools.datasets import write_txt
-    if not oracle_mod.ref_available():
-        pytest.skip("oracle/_ref/ref_mcmc not built")
+    g = np.load(os.path.join(GOLDEN, "ref_free_g10s10.npz"))
     X, hard = load_hex_dataset("g10s10")
     ds = tmp_path / "g10s10.txt"
     write_txt(str(ds), X, hard)
-    ref_dir, our_dir, tape = tmp_path / "ref", tmp_path / "ours", tmp_path / "tape.bin"
-    (ref_dir / "Chains" / "chain_07").mkdir(parents=True)
-    our_dir.mkdir()
-    env = dict(os.environ, GSL_RNG_SEED="5", SER_TAPE_OUT=str(tape))
-    with open(ds) as f:
-        subprocess.run([oracle_mod.REF_BIN, "cli", "7"], stdin=f, cwd=ref_dir, env=env, check=True,
-                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-    env = dict(os.environ, SER_TAPE_IN=str(tape))
+    o, init, res, final, tape = _oracle_chain(oracle_mod, X, hard, 7, 1000, 1000)
+    tape_path = tmp_path / "tape.bin"
+    tape.tofile(str(tape_path))
+    env = dict(os.environ, SER_TAPE_IN=str(tape_path))
     env.pop("GSL_RNG_SEED", None)
     with open(ds) as f:
-        subprocess.run([os.path.join(S.PKG_DIR, "mcmc"), "7"], stdin=f, cwd=our_dir, env=env, check=True)
-    r, o = ref_dir / "Chains" / "chain_07", our_dir / "Chains" / "chain_07"
-    assert len((r / "chain_data.csv").read_text().split("\n")) == 1001
-    for name in ("chain_data.csv", "exp_data.csv", "taxa.csv", "sites.csv", "hard_sites.csv"):
-        assert (r / name).read_bytes() == (o / name).read_bytes(), name
+        subprocess.run([os.path.join(S.PKG_DIR, "mcmc"), "7"], stdin=f, cwd=tmp_path, env=env, check=True)
+    out = tmp_path / "Chains" / "chain_07"
+    exp = (out / "exp_data.csv").read_text().split("\n")
+    assert exp[0] == "exp_loglik,exp_c,exp_d"
+    assert float(exp[1].split(",")[0]) == g["e_negloglik"][7]
+    lines = (out / "chain_data.csv").read_text().split("\n")
+    assert len(lines) == 1001
+    for s in (0, 499, 999):
+        f = lines[s].split(",")
+        assert [int(v) for v in f[0].split()] == res["a"][s].tolist() and [int(v) for v in f[1].split()] == res["b"][s].tolist()
+        assert [int(v.strip()) for v in f[2].split(" ")[:X.shape[0]]] == res["pi"][s].tolist()
+    assert [int(v) for v in (out / "sites.csv").read_text().split("\n")[1:X.shape[0] + 1]] == final.pi.tolist()
 
 
 def test_cli_batch_mode(S, tmp_path):
@@ -840,27 +844,35 @@ def test_config5_replay_vs_unmodified_reference_golden(S, oracle_mod):
     the states oracle/_ref/ref_mcmc_big (mcmc.c with MAXS raised, nothing else) went through for 8 seeds x 10
     mcmc_sample() calls = 100 sweeps.  The tapes (53 MB) are regenerated from the seeds by the oracle's MT19937 --
     length and CRC must equal the reference's recorded tapes -- and replayed through the large-shape kernel:
-    a, b, pi, c, d and the saved log-likelihood bits of every call, totals and cursor at the end."""
+    a, b, pi (the first seed's in full, every seed's by CRC32), c, d and the saved log-likelihood bits of every call,
+    totals and cursor at the end."""
     import zlib
     g = np.load(os.path.join(GOLDEN, "ref_synthetic_1024x4096.npz"))
     X, hard = S.Dataset.synthetic(1024, 4096, 16).arrays()
     assert [zlib.crc32(X.tobytes()), zlib.crc32(hard.tobytes())] == g["x_crc"].tolist()
-    seeds, calls = [int(s) for s in g["seeds"]], g["a"].shape[1] - 1
+    seeds, calls = [int(s) for s in g["seeds"]], g["a_crc"].shape[1] - 1
     chains = _oracle_chains_parallel(oracle_mod, X, hard, seeds, 0, calls)
     for i, c in enumerate(chains):
         assert c[4].size == int(g["tape_len"][i]) and zlib.crc32(c[4].tobytes()) == int(g["tape_crc"][i]), i
+
+    def same_states(i, k, got, recs):
+        """got[j]: chain i's `k` after record recs[j] of the reference"""
+        assert [zlib.crc32(v.astype(np.int16).tobytes()) for v in got] == g[k + "_crc"][i][recs].tolist(), (i, k)
+        if i < len(g[k]):
+            assert np.array_equal(got, g[k][i][recs].astype(np.int32)), (i, k)
+
     run = S.Run(S.Dataset.from_bits(X, hard), len(seeds), mode=S.MODE_REPLAY, store=S.STORE_FULL, max_samples=calls)
     run.set_tapes([c[4] for c in chains]).init().sync()
     for i in range(len(seeds)):
         st = run.state(i)
         for k in ("a", "b", "pi"):
-            assert np.array_equal(st[k], g[k][i][0].astype(np.int32)), ("init", i, k)
+            same_states(i, k, st[k][None], [0])
     run.advance(calls, True).sync()
     assert run.check() == 0
     for i in range(len(seeds)):
         got, st = run.fetch_samples(i), run.state(i)
         for k in ("a", "b", "pi"):
-            assert np.array_equal(got[k], g[k][i][1:].astype(np.int32)), (i, k)
+            same_states(i, k, got[k], list(range(1, calls + 1)))
         assert np.array_equal(got["c"], g["cdl"][i][1:, 0]) and np.array_equal(got["d"], g["cdl"][i][1:, 1]), i
         assert np.array_equal(got["loglik"], g["cdl"][i][1:, 2]), (i, np.max(np.abs(got["loglik"] - g["cdl"][i][1:, 2])))
         assert np.array_equal(st["tot"], g["tot"][i][-1]) and st["slots"] == int(g["slots"][i][-1]), i
