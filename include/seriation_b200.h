@@ -100,6 +100,12 @@ int ser_dataset_synthetic(int32_t N, int32_t M, int32_t n_hard, uint64_t seed, s
 
 /* ---------------------------------------------------------------- runs (device) */
 int ser_run_create(const ser_dataset *ds, const ser_run_config *cfg, ser_run **out);
+/* A run whose local chain c is GLOBAL chain chain_ids[c] (distinct, >= 0, any order; cfg->n_chains == n, cfg->chain_offset == 0):
+ * free-running chains are keyed by (seed, global id), so the chosen chains of an earlier run are re-simulated alone, bit-identical
+ * to their first run (replay mode: one tape per local chain, as ever).  The cross-chain getters take global ids; local-index
+ * entry points (ser_run_get_state, ser_write_chain_files, ...) keep indexing local chains.  The arguments are checked before
+ * any CUDA call. */
+int ser_run_create_chains(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chain_ids, int32_t n, ser_run **out);
 void ser_run_destroy(ser_run *run);
 /* replay mode: all chains' tapes concatenated; offsets has n_chains+1 entries (in doubles) */
 int ser_run_set_tapes(ser_run *run, const double *flat, const uint64_t *offsets);
@@ -200,6 +206,23 @@ int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t k, int32_t
  * positive, like the report), corr_mn: x = the integer MN unit.  Host doubles; needs SER_STORE_PI. */
 int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *chosen, int32_t k, double *corr_age,
                           double *corr_mn, int32_t *n_sites_used);
+
+/* ---------------------------------------------------------------- streaming summaries
+ * Flags of ser_run_accumulate and the per-local-chain device accumulators they allocate: */
+#define SER_ACC_PO 1    /* pair-order counts            [n][N][N] int32                                   */
+#define SER_ACC_SUMS 2  /* pi_sum [n][N] int32 (corr_num is derived from it on the way out)                */
+#define SER_ACC_AB 4    /* a_sum, b_sum                 [n][M] int32 each   (needs SER_STORE_FULL)           */
+#define SER_ACC_ALIVE 8 /* alive difference slab        [n][N][M] int32     (needs SER_STORE_FULL)           */
+/* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
+ * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
+ * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),
+ * ser_run_posterior_sums, ser_run_alive_counts and ser_run_site_age_corr then return totals over EVERY sample taken since
+ * (T = the chain's sample count), with the usual global ids and slab convention; ser_run_fetch_samples /
+ * ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does ser_run_cross_chain_async.
+ * Call it before the first sampling call (ser_run_init zeroes the accumulators).  Errors: SER_E_STATE on a run that has
+ * already sampled, on a store below what the flags need, or a second time; SER_E_ARG for max_samples < 1; SER_E_CUDA with
+ * the byte count when an accumulator does not fit (the alive slab at 2048 x 8192 is 64 MB per chain). */
+int ser_run_accumulate(ser_run *run, int32_t what);
 
 /* ---------------------------------------------------------------- cross-chain step, one call
  * E[-logL] of every chain -> (all-gather) -> choose_chains(k) -> pair-order counts of the chosen chains

@@ -18,6 +18,7 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
+ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE = 1, 2, 4, 8
 
 _i32p, _dp, _u8p = C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_uint8)
 _i64p, _u64p = C.POINTER(C.c_int64), C.POINTER(C.c_uint64)
@@ -50,6 +51,8 @@ SYMBOLS = [
     ("ser_dataset_site_age", C.c_int, [_vp, C.c_int32, _i32p, _dp, _i32p]),
     ("ser_dataset_synthetic", C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_uint64, C.POINTER(_vp)]),
     ("ser_run_create", C.c_int, [_vp, C.POINTER(RunConfig), C.POINTER(_vp)]),
+    ("ser_run_create_chains", C.c_int, [_vp, C.POINTER(RunConfig), _i32p, C.c_int32, C.POINTER(_vp)]),
+    ("ser_run_accumulate", C.c_int, [_vp, C.c_int32]),
     ("ser_run_destroy", None, [_vp]),
     ("ser_run_set_tapes", C.c_int, [_vp, _dp, _u64p]),
     ("ser_run_init", C.c_int, [_vp]),
@@ -205,18 +208,32 @@ class Dataset:
 
 
 class Run:
-    """A batch of independent chains on one GPU (replaces script.py's Pool of `mcmc` processes)."""
+    """A batch of independent chains on one GPU (replaces script.py's Pool of `mcmc` processes).  ``chain_ids``: the global
+    ids of the local chains (a subset run, ser_run_create_chains; ``n_chains`` is then ignored)."""
 
     def __init__(self, ds: Dataset, n_chains: int, *, mode=MODE_FREE, seed=0, chain_offset=0, sweeps_per_call=10,
-                 store=STORE_NONE, max_samples=0, device=0, manycd=False):
+                 store=STORE_NONE, max_samples=0, device=0, manycd=False, chain_ids=None):
         self.ds = ds
+        ids = None if chain_ids is None else np.ascontiguousarray(chain_ids, dtype=np.int32)
+        if ids is not None:
+            n_chains = ids.size
         self.N, self.M, self.n_chains = ds.N, ds.M, n_chains
         self.manycd = bool(manycd)
         self.cfg = RunConfig(C.sizeof(RunConfig), n_chains, chain_offset, sweeps_per_call, mode, seed, store, max_samples, device,
                              int(self.manycd))
         h = _vp()
-        _check(lib().ser_run_create(ds._h, C.byref(self.cfg), C.byref(h)))
+        if ids is None:
+            _check(lib().ser_run_create(ds._h, C.byref(self.cfg), C.byref(h)))
+        else:
+            _check(lib().ser_run_create_chains(ds._h, C.byref(self.cfg), _p(ids, C.c_int32), ids.size, C.byref(h)))
         self._h = h
+
+    def accumulate(self, po=True, sums=True, ab=False, alive=False):
+        """from now on the sample store is a window of max_samples rows and the summaries sum over every sample taken
+        afterwards (ser_run_accumulate); call before the first sampling call"""
+        what = (ACC_PO if po else 0) | (ACC_SUMS if sums else 0) | (ACC_AB if ab else 0) | (ACC_ALIVE if alive else 0)
+        _check(lib().ser_run_accumulate(self._h, what))
+        return self
 
     def close(self):
         if getattr(self, "_h", None) and _lib is not None:
@@ -535,8 +552,10 @@ class ChainBatch:
     """What ``run_all_chains(dataset)`` leaves behind in the reference -- 100 ``Chains/chain_XX/``
     directories -- kept on the GPU instead: E[-logL] per chain and the pi history."""
 
-    def __init__(self, run: Run, burn_calls: int, sample_calls: int):
+    def __init__(self, run: Run, burn_calls: int, sample_calls: int, *, seed: int = 0, sweeps_per_call: int = 10,
+                 manycd: bool = False):
         self.run, self.burn_calls, self.sample_calls = run, burn_calls, sample_calls
+        self.seed, self.sweeps_per_call, self.manycd = seed, sweeps_per_call, manycd   # what replay_chosen rebuilds the chains from
         self._stats = None
 
     def stats(self):
@@ -555,7 +574,7 @@ def run_all_chains(dataset, n_chains: int = 100, burn_calls: int = 1000, sample_
         store = STORE_FULL
     run = Run(ds, n_chains, mode=MODE_FREE, seed=seed, store=store, max_samples=sample_calls, device=device)
     run.init().advance(burn_calls, False).advance(sample_calls, True).sync()
-    batch = ChainBatch(run, burn_calls, sample_calls)
+    batch = ChainBatch(run, burn_calls, sample_calls, seed=seed, sweeps_per_call=run.cfg.sweeps_per_call, manycd=run.manycd)
     if chains_dir is not None:
         for i in range(min(n_chains, 100)):
             d = os.path.join(chains_dir, "chain_%02d" % i)
@@ -568,6 +587,29 @@ def choose_chains(batch: ChainBatch, chains_selected: int):
     """script.py:70-99 over the batch's E[-logL]."""
     chosen, _, _ = select_chains(batch.stats()["e_negloglik"], chains_selected)
     return [int(c) for c in chosen]
+
+
+def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, device=None) -> ChainBatch:
+    """The second phase of select-then-replay: re-simulate the chosen chains of a batch (typically one run with
+    ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
+    ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
+    run's, so compute_pair_order_matrix, compute_exp_* and the probability maps work on it unchanged.  ``with_ab``
+    also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  Raises SeriationError when
+    a replayed chain's E[-logL] differs from its first run in any bit."""
+    ids = np.ascontiguousarray(chains, dtype=np.int32)
+    run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
+              store=STORE_FULL if with_ab else STORE_PI, max_samples=window,
+              device=batch.run.cfg.device if device is None else device, chain_ids=ids)
+    run.init().accumulate(po=True, sums=True, ab=with_ab, alive=with_ab)
+    run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
+    want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
+    if want.tobytes() != got.tobytes():
+        raise SeriationError(f"replay_chosen: the replayed chains {ids.tolist()} do not reproduce their first run "
+                             f"(E[-logL] {got.tolist()} vs {want.tolist()})")
+    out = ChainBatch(run, batch.burn_calls, batch.sample_calls, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call,
+                     manycd=batch.manycd)
+    out._stats = batch.stats()
+    return out
 
 
 def compute_pair_order_matrix(batch: ChainBatch, chains, chains_selected: int, sites: int | None = None, faithful=True):

@@ -16,7 +16,11 @@
  * Batch mode (replaces script.py's Pool over 100 processes by one call over all the chains, on one GPU or
  * sharded over the GPUs of the box -- ser_multi_*):
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
- *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1]
+ *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
+ * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
+ * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
+ * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
+ * lines and po.csv as the one-shot step, with device memory for K chains' window instead of every chain's history.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -39,7 +43,8 @@ static void usage(const char *argv0)
           "usage: %s <chain_index> < dataset.txt          (reference-compatible single chain)\n"
           "       %s [manycd Tburnin T] < dataset.txt      (manycd 1: per-taxon c, d; chain 0)\n"
           "       %s --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset F]\n"
-          "              [--chains-dir DIR] [--select K] [--po out.csv] [--device D] [--manycd 0|1]\n",
+          "              [--chains-dir DIR] [--select K] [--po out.csv] [--device D] [--manycd 0|1]\n"
+          "              [--replay-selected --window W]   (with --select: keep no sample history, replay the chosen chains)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -63,6 +68,7 @@ static double *read_tape(const char *path, uint64_t *len)
 int main(int argc, char **argv)
 {
   int n_chains = 1, first = 0, burn = 1000, samples = 1000, select_k = 0, device = 0, batch = 0, manycd = 0, gpus = 1, i;
+  int replay_selected = 0, window = 64;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN");
   const char *env_seed = getenv("GSL_RNG_SEED");
@@ -81,6 +87,7 @@ int main(int argc, char **argv)
     batch = 1;
     for (i = 1; i < argc; i++) {
       const char *a = argv[i], *v = (i + 1 < argc) ? argv[i + 1] : NULL;
+      if (!strcmp(a, "--replay-selected")) { replay_selected = 1; continue; }
       if (!v) usage(argv[0]);
       if (!strcmp(a, "--chains")) n_chains = atoi(v);
       else if (!strcmp(a, "--gpus")) gpus = atoi(v);
@@ -94,10 +101,12 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--po")) po_path = v;
       else if (!strcmp(a, "--device")) device = atoi(v);
       else if (!strcmp(a, "--manycd")) manycd = atoi(v) != 0;
+      else if (!strcmp(a, "--window")) window = atoi(v);
       else usage(argv[0]);
       i++;
     }
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
+    if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
   } else if (argc == 2) {
     char *end = NULL;
     const long idx = strtol(argv[1], &end, 10); /* mcmc.c:115,153 */
@@ -127,7 +136,7 @@ int main(int argc, char **argv)
   cfg.sweeps_per_call = 10;
   cfg.mode = tape_path ? SER_MODE_REPLAY : SER_MODE_FREE;
   cfg.seed = (uint32_t)seed;
-  cfg.store = (n_chains <= 100) ? SER_STORE_FULL : SER_STORE_PI;
+  cfg.store = replay_selected ? SER_STORE_NONE : (n_chains <= 100) ? SER_STORE_FULL : SER_STORE_PI;
   cfg.max_samples = samples;
   cfg.device = device;
   cfg.manycd = manycd;
@@ -190,8 +199,26 @@ int main(int argc, char **argv)
       int32_t *counts = po_path ? (int32_t *)calloc((size_t)select_k * N * N, sizeof(int32_t)) : NULL;
       double mn, sd;
       if (!chosen || (po_path && !counts)) { fprintf(stderr, "mcmc: out of memory\n"); return 1; }
-      /* E[-logL] -> selection -> pair-order counts in one step on the device(s) (script.py:70-99, :155-189) */
-      if (ser_multi_cross_chain(multi, select_k, chosen, &nchosen, &mn, &sd, counts)) die("ser_multi_cross_chain");
+      if (!replay_selected) {
+        /* E[-logL] -> selection -> pair-order counts in one step on the device(s) (script.py:70-99, :155-189) */
+        if (ser_multi_cross_chain(multi, select_k, chosen, &nchosen, &mn, &sd, counts)) die("ser_multi_cross_chain");
+      } else {
+        /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
+        if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
+        for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
+        if (counts && nchosen > 0) {
+          ser_run_config c2 = cfg;
+          ser_run *sub = NULL;
+          c2.n_chains = nchosen;
+          c2.chain_offset = 0;
+          c2.store = SER_STORE_PI;
+          c2.max_samples = window;
+          if (ser_run_create_chains(ds, &c2, chosen, nchosen, &sub)) die("ser_run_create_chains");
+          if (ser_run_init(sub) || ser_run_accumulate(sub, SER_ACC_PO)) die("ser_run_accumulate");
+          if (ser_run_advance_both(sub, burn, samples) || ser_run_po_counts(sub, chosen, nchosen, counts)) die("replay of the chosen chains");
+          ser_run_destroy(sub);
+        }
+      }
       printf("selection: min E[-logL] %.6f  sigma %.6f  chosen", mn, sd);
       for (i = 0; i < nchosen; i++) printf(" %d", chosen[i]);
       printf("\n");

@@ -188,22 +188,24 @@ __device__ __forceinline__ int stored_samples(const ChainScalars *scal, int loca
   return n < max_samples ? n : max_samples;
 }
 
-/* pair-order counts (script.py:178-189) for one chosen chain per blockIdx.z: a 32 x 32 tile of (i, j) per
- * block, the positions of the tile's 64 sites staged through shared memory 32 samples at a time (coalesced
- * rows of the sample store).  T = the CHOSEN chain's own sample count.  Only the owner of a chosen chain
- * writes its slab -- to every destination (peer stores: the slabs are disjoint, so no reduction is needed). */
-#define SER_PO_TS 32
-__global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples,
-                                                      const int *chosen, int chain_offset, int n_local, PeerPtrs dst)
+/* Local index of GLOBAL chain g on a run whose local chain c is id_base + c (ids == nullptr), or ids[c] (subset runs,
+ * ser_run_create_chains: a handful of chosen chains, so a scan); -1 when the run does not hold g. */
+__device__ __forceinline__ int local_chain(int g, int id_base, int n_local, const int *ids)
 {
-  const int g = chosen[blockIdx.z];
-  if (g < chain_offset || g >= chain_offset + n_local) return;
-  const int T = stored_samples(scal, g - chain_offset, max_samples);
+  if (!ids) return (g >= id_base && g < id_base + n_local) ? g - id_base : -1;
+  for (int c = 0; c < n_local; c++)
+    if (ids[c] == g) return c;
+  return -1;
+}
+
+/* pair-order counts of a 32 x 32 tile of (i, j) over rows [0, T) of one chain's samples `pi` ([row][N]): the positions of the
+ * tile's 64 sites staged through shared memory 32 samples at a time (coalesced rows).  256 threads; thread (tx, ty) adds
+ * #{t : pi_t(i0+ty+8r) < pi_t(j0+tx)} to c[r].  Every thread of the block calls it (barriers inside). */
+#define SER_PO_TS 32
+__device__ __forceinline__ void po_tile(const uint16_t *pi, int N, int T, int i0, int j0, int c[4])
+{
   __shared__ uint16_t si[SER_PO_TS][32], sj[SER_PO_TS][32];
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5; /* 32 x 8 threads; thread (tx, ty) owns j = j0+tx, i = i0+ty+8r */
-  const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
-  const uint16_t *pi = samp_pi + (size_t)(g - chain_offset) * max_samples * N;
-  int c[4] = {0, 0, 0, 0};
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   for (int t0 = 0; t0 < T; t0 += SER_PO_TS) {
     const int nt = min(SER_PO_TS, T - t0);
     __syncthreads();
@@ -219,6 +221,21 @@ __global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, co
       for (int r = 0; r < 4; r++) c[r] += (int)si[t][ty + 8 * r] < pj;
     }
   }
+}
+
+/* pair-order counts (script.py:178-189) for one chosen chain per blockIdx.z, one 32 x 32 tile per block.  T = the CHOSEN
+ * chain's own sample count.  Only the owner of a chosen chain writes its slab -- to every destination (peer stores: the
+ * slabs are disjoint, so no reduction is needed). */
+__global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples,
+                                                      const int *chosen, int chain_offset, int n_local, const int *ids, PeerPtrs dst)
+{
+  const int local = local_chain(chosen[blockIdx.z], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int T = stored_samples(scal, local, max_samples);
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5; /* 32 x 8 threads; thread (tx, ty) owns j = j0+tx, i = i0+ty+8r */
+  const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
+  int c[4] = {0, 0, 0, 0};
+  po_tile(samp_pi + (size_t)local * max_samples * N, N, T, i0, j0, c);
   const int j = j0 + tx;
   if (j >= N) return;
 #pragma unroll
@@ -232,14 +249,14 @@ __global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, co
 
 /* posterior sums over the stored samples of one chosen chain per block (script.py:129-152, :230-276) */
 __global__ void ser_posterior_kernel(const uint16_t *samp_pi, const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal,
-                                     int N, int M, int max_samples, const int *chosen, int chain_offset, int n_local,
+                                     int N, int M, int max_samples, const int *chosen, int chain_offset, int n_local, const int *ids,
                                      long long *corr_num, int *pi_sum, int *a_sum, int *b_sum, int *n_out)
 {
-  const int g = chosen[blockIdx.x];
-  if (g < chain_offset || g >= chain_offset + n_local) return;
-  const int n_samples = stored_samples(scal, g - chain_offset, max_samples);
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int n_samples = stored_samples(scal, local, max_samples);
   if (threadIdx.x == 0 && n_out) n_out[blockIdx.x] = n_samples;
-  const size_t base = (size_t)(g - chain_offset) * max_samples;
+  const size_t base = (size_t)local * max_samples;
   long long s = 0;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     int acc = 0;
@@ -261,15 +278,15 @@ __global__ void ser_posterior_kernel(const uint16_t *samp_pi, const uint16_t *sa
  * (script.py:321-329; closed at b, as the reference tests it).  One thread per taxon: +1 / -1
  * marks at a and b+1 in its own column of the slab, then a running sum down the positions. */
 __global__ void ser_alive_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
-                                 const int *chosen, int chain_offset, int n_local, int *alive, int *n_out)
+                                 const int *chosen, int chain_offset, int n_local, const int *ids, int *alive, int *n_out)
 {
-  const int g = chosen[blockIdx.x];
-  if (g < chain_offset || g >= chain_offset + n_local) return;
-  const int n_samples = stored_samples(scal, g - chain_offset, max_samples);
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int n_samples = stored_samples(scal, local, max_samples);
   if (blockIdx.y == 0 && threadIdx.x == 0 && n_out) n_out[blockIdx.x] = n_samples;
   const int m = blockIdx.y * blockDim.x + threadIdx.x;
   if (m >= M) return;
-  const size_t base = (size_t)(g - chain_offset) * max_samples;
+  const size_t base = (size_t)local * max_samples;
   int *col = alive + (size_t)blockIdx.x * N * M + m;
   for (int j = 0; j < N; j++) col[(size_t)j * M] = 0;
   for (int t = 0; t < n_samples; t++) {
@@ -279,6 +296,124 @@ __global__ void ser_alive_kernel(const uint16_t *samp_a, const uint16_t *samp_b,
   }
   int acc = 0;
   for (int j = 0; j < N; j++) { acc += col[(size_t)j * M]; col[(size_t)j * M] = acc; }
+}
+
+/* ------------------------------------------------------------------ streaming accumulators (ser_run_accumulate)
+ * On an accumulating run the sample store is a window of max_samples rows per chain.  After every sweep launch of w
+ * sampling calls these kernels add rows [0, w) of EVERY local chain's window into per-chain totals; the getters below
+ * turn the totals into what the one-shot kernels above compute from a store that holds all samples. */
+
+/* rows of the window a chain filled in the last launch (fewer than w only when its replay tape ran out) */
+__device__ __forceinline__ int window_rows(const ChainScalars *scal, int local, int sample_base, int w)
+{
+  const int n = scal[local].n_samples - sample_base;
+  return n < 0 ? 0 : n < w ? n : w;
+}
+
+/* pair-order tiles of every local chain (blockIdx.z) added into acc [n_local][N][N]; the diagonal stays 0 */
+__global__ void __launch_bounds__(256) ser_po_accum_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples,
+                                                            int sample_base, int w, int *acc)
+{
+  const int local = blockIdx.z;
+  const int T = window_rows(scal, local, sample_base, w);
+  if (T == 0) return;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
+  int c[4] = {0, 0, 0, 0};
+  po_tile(samp_pi + (size_t)local * max_samples * N, N, T, i0, j0, c);
+  const int j = j0 + tx;
+  if (j >= N) return;
+  int *slab = acc + (size_t)local * N * N;
+#pragma unroll
+  for (int r = 0; r < 4; r++) {
+    const int i = i0 + ty + 8 * r;
+    if (i < N) slab[(size_t)i * N + j] += c[r];
+  }
+}
+
+/* sum_t pi_t into pi_acc [n_local][N], and sum_t a_t / b_t into a_acc / b_acc [n_local][M] when given; one chain per block */
+__global__ void ser_posterior_accum_kernel(const uint16_t *samp_pi, const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal,
+                                           int N, int M, int max_samples, int sample_base, int w, int *pi_acc, int *a_acc, int *b_acc)
+{
+  const int local = blockIdx.x;
+  const int T = window_rows(scal, local, sample_base, w);
+  const size_t base = (size_t)local * max_samples;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    int acc = 0;
+    for (int t = 0; t < T; t++) acc += samp_pi[(base + t) * N + i];
+    pi_acc[(size_t)local * N + i] += acc;
+  }
+  if (a_acc)
+    for (int m = threadIdx.x; m < M; m += blockDim.x) {
+      int sa = 0, sb = 0;
+      for (int t = 0; t < T; t++) { sa += samp_a[(base + t) * M + m]; sb += samp_b[(base + t) * M + m]; }
+      a_acc[(size_t)local * M + m] += sa;
+      b_acc[(size_t)local * M + m] += sb;
+    }
+}
+
+/* +1 at a, -1 at b+1 of every window row into the difference slab diff [n_local][N][M]; one thread per taxon */
+__global__ void ser_alive_accum_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
+                                       int sample_base, int w, int *diff)
+{
+  const int local = blockIdx.x, m = blockIdx.y * blockDim.x + threadIdx.x;
+  if (m >= M) return;
+  const int T = window_rows(scal, local, sample_base, w);
+  const size_t base = (size_t)local * max_samples;
+  int *col = diff + (size_t)local * N * M + m;
+  for (int t = 0; t < T; t++) {
+    const int a = samp_a[(base + t) * M + m], b = samp_b[(base + t) * M + m];
+    if (a < N) col[(size_t)a * M] += 1;
+    if (b + 1 < N) col[(size_t)(b + 1) * M] -= 1;
+  }
+}
+
+/* getters of an accumulating run: the slab of every chosen chain the run holds, T = all samples taken since accumulation began */
+__global__ void ser_po_acc_out_kernel(const int *acc, const ChainScalars *scal, int N, const int *chosen, int chain_offset, int n_local,
+                                      const int *ids, int *counts)
+{
+  const int local = local_chain(chosen[blockIdx.y], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int T = scal[local].n_samples;
+  const size_t nn = (size_t)N * N;
+  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < nn; q += (size_t)gridDim.x * blockDim.x)
+    counts[blockIdx.y * nn + q] = (q / N == q % N) ? -T : acc[local * nn + q];
+}
+
+__global__ void ser_posterior_acc_out_kernel(const int *pi_acc, const int *a_acc, const int *b_acc, const ChainScalars *scal, int N, int M,
+                                             const int *chosen, int chain_offset, int n_local, const int *ids,
+                                             long long *corr_num, int *pi_sum, int *a_sum, int *b_sum, int *n_out)
+{
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  if (threadIdx.x == 0) n_out[blockIdx.x] = scal[local].n_samples;
+  long long s = 0;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    const int v = pi_acc[(size_t)local * N + i];
+    pi_sum[(size_t)blockIdx.x * N + i] = v;
+    s += (long long)i * v;
+  }
+  if (a_sum)
+    for (int m = threadIdx.x; m < M; m += blockDim.x) {
+      a_sum[(size_t)blockIdx.x * M + m] = a_acc[(size_t)local * M + m];
+      if (b_sum) b_sum[(size_t)blockIdx.x * M + m] = b_acc[(size_t)local * M + m];
+    }
+  atomicAdd((unsigned long long *)&corr_num[blockIdx.x], (unsigned long long)s);
+}
+
+/* running sum of the difference slab down the positions */
+__global__ void ser_alive_acc_out_kernel(const int *diff, const ChainScalars *scal, int N, int M, const int *chosen, int chain_offset,
+                                         int n_local, const int *ids, int *alive, int *n_out)
+{
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = scal[local].n_samples;
+  const int m = blockIdx.y * blockDim.x + threadIdx.x;
+  if (m >= M) return;
+  const int *src = diff + (size_t)local * N * M + m;
+  int *col = alive + (size_t)blockIdx.x * N * M + m;
+  int acc = 0;
+  for (int j = 0; j < N; j++) { acc += src[(size_t)j * M]; col[(size_t)j * M] = acc; }
 }
 
 /* ------------------------------------------------------------------ micro-benchmarks */

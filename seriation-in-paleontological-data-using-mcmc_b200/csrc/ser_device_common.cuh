@@ -69,6 +69,7 @@ struct KParams {
   uint16_t *rpi;       /* [chain][Npad] */
   ChainScalars *scal;  /* [chain] */
   int mode, chain_offset;
+  const int *chain_ids;     /* [n_chains] global id of each local chain (ser_run_create_chains), else nullptr: chain_offset + chain */
   unsigned int seed;
   const double *tape;
   const unsigned long long *tape_off;
@@ -81,6 +82,7 @@ struct KParams {
   unsigned int *queue;      /* next item */
   unsigned int *done;       /* [chain] items completed since init */
   int store, max_samples;
+  int sample_base;          /* samples taken before the store's row 0: 0, or on an accumulating run those already summarised */
   uint16_t *samp_a, *samp_b, *samp_pi;
   double *samp_cdl;
   double c0, cc0, d0, dd0, eps;
@@ -105,6 +107,12 @@ struct KParams {
   int n_units;
   int grp_u[SER_MAX_GROUPS + 1]; /* units of column group g = [grp_u[g], grp_u[g+1]) */
 };
+
+/* the global chain id that keys local chain `chain`'s Philox stream */
+__device__ __forceinline__ unsigned int global_chain(const KParams &p, int chain)
+{
+  return (unsigned int)(p.chain_ids ? p.chain_ids[chain] : p.chain_offset + chain);
+}
 
 /* ------------------------------------------------------------------ shared-memory carve-up */
 struct Smem {
@@ -283,16 +291,16 @@ __global__ void ser_init_kernel(KParams p)
   uint16_t *rest16 = pi16 + p.N, *chosen16 = rest16 + p.N;
 
   const int chain = blockIdx.x, tid = threadIdx.x, N = p.N, M = p.M, C = blockDim.x, nh = p.nh;
-  const unsigned int gchain = (unsigned int)(p.chain_offset + chain);
   const double *tape = nullptr;
   long long tape_len = 0;
   if (p.mode == SER_MODE_REPLAY) {
     tape = p.tape + p.tape_off[chain];
     tape_len = (long long)(p.tape_off[chain + 1] - p.tape_off[chain]);
   }
+  /* the global id is formed where it is used: held across the kernel it costs 8 registers, a resident block per SM at 320 threads */
   for (int t = tid; t < 2 * N; t += C) {
     if (p.mode == SER_MODE_REPLAY) stage[t] = (t < tape_len) ? tape[t] : 0.0;
-    else stage[t] = ser_stream_uniform(p.seed, gchain, SER_SWEEP_INIT, SER_BLK_INIT, (uint32_t)t);
+    else stage[t] = ser_stream_uniform(p.seed, global_chain(p, chain), SER_SWEEP_INIT, SER_BLK_INIT, (uint32_t)t);
   }
   for (int n = tid; n < N; n += C) sm.rpi[n] = (uint16_t)n;
   __syncthreads();

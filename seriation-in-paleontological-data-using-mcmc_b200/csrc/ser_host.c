@@ -487,10 +487,9 @@ int ser_write_labelled_files(ser_run *run, int32_t chain, const ser_dataset *ds,
 int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *chosen, int32_t k, double *corr_age, double *corr_mn,
                           int32_t *n_sites_used)
 {
-  int32_t N, M, nh, nc, T = 0, first;
+  int32_t N, M, nh, nc, T = 0;
   if (!run || !ds || !chosen || k < 1) { ser_set_error("ser_run_site_age_corr: bad argument"); return SER_E_ARG; }
   ser_run_dims(run, &N, &M, &nh, &nc);
-  first = ser_run_chain_offset(run);
   if (ds->N != N) { ser_set_error("ser_run_site_age_corr: dataset does not match the run"); return SER_E_ARG; }
   if (!ds->site_age || !ds->site_mn) { ser_set_error("ser_run_site_age_corr: no site ages loaded (ser_dataset_read_names with a .sites file)"); return SER_E_STATE; }
   for (int32_t n = 0; n < N; n++)
@@ -512,7 +511,7 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
     }
     var_age /= N; var_mn /= N;
     for (int32_t c = 0; c < k; c++) {
-      if (chosen[c] < first || chosen[c] >= first + nc) continue; /* owned by another rank, or -1 */
+      if (ser_run_local_chain(run, chosen[c]) < 0) continue; /* owned by another rank, or -1 */
       owned++;
       for (int32_t n = 0; n < N; n++) {
         const double dp = (double)pis[(size_t)c * N + n] / T - mean_pi;

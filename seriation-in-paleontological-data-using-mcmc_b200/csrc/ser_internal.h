@@ -26,7 +26,8 @@ int ser_run_chain_sums(ser_run *run, int32_t chain, double sums[3], int32_t *n_s
 int ser_run_dims(const ser_run *run, int32_t *N, int32_t *M, int32_t *nh, int32_t *n_chains);
 const uint8_t *ser_run_hard_flags(const ser_run *run);
 int ser_run_is_manycd(const ser_run *run);
-int ser_run_chain_offset(const ser_run *run);
+/* local index of GLOBAL chain id g on this run, -1 when the run does not hold it */
+int ser_run_local_chain(const ser_run *run, int32_t g);
 
 #ifdef __cplusplus
 }

@@ -102,6 +102,11 @@ struct ser_run {
    * timing the dominant kernel does not put a host synchronisation into the timed region */
   std::vector<cudaEvent_t> *sweep_ev;
   size_t sweep_ev_used;
+  /* subset runs (ser_run_create_chains): global id of every local chain, device copy in kp.chain_ids */
+  int *h_chain_ids, *d_chain_ids;
+  /* streaming accumulators (ser_run_accumulate): SER_ACC_* flags, per local chain totals */
+  int acc_what, sampled;
+  int *d_acc_po, *d_acc_pi, *d_acc_a, *d_acc_b, *d_acc_alive;
 };
 
 /* multi-GPU pieces (ser_multi.cuh): NCCL entry points resolved at run time */
@@ -685,6 +690,86 @@ extern "C" int ser_run_create(const ser_dataset *ds, const ser_run_config *cfg, 
   return SER_OK;
 }
 
+extern "C" int ser_run_create_chains(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chain_ids, int32_t n, ser_run **out)
+{
+  if (!ds || !cfg || !chain_ids || !out) { ser_set_error("ser_run_create_chains: null argument"); return SER_E_ARG; }
+  *out = nullptr;
+  if (n < 1 || n != cfg->n_chains) { ser_set_error("ser_run_create_chains: %d chain ids for cfg->n_chains = %d", n, cfg->n_chains); return SER_E_ARG; }
+  if (cfg->chain_offset != 0) { ser_set_error("ser_run_create_chains: cfg->chain_offset is %d; it must be 0 (chain_ids are the global ids)", cfg->chain_offset); return SER_E_ARG; }
+  std::vector<int> sorted(chain_ids, chain_ids + n);
+  std::sort(sorted.begin(), sorted.end());
+  if (sorted[0] < 0) { ser_set_error("ser_run_create_chains: chain id %d is negative", sorted[0]); return SER_E_ARG; }
+  for (int c = 1; c < n; c++)
+    if (sorted[c] == sorted[c - 1]) { ser_set_error("ser_run_create_chains: chain id %d is listed twice", sorted[c]); return SER_E_ARG; }
+  ser_run *run = nullptr;
+  int rc = ser_run_create(ds, cfg, &run);
+  if (rc != SER_OK) return rc;
+  auto attach = [&]() -> int {
+    run->h_chain_ids = (int *)malloc((size_t)n * sizeof(int));
+    if (!run->h_chain_ids) { ser_set_error("ser_run_create_chains: out of memory"); return SER_E_ARG; }
+    memcpy(run->h_chain_ids, chain_ids, (size_t)n * sizeof(int));
+    CUDA_TRY(POOL_ALLOC(&run->d_chain_ids, (size_t)n * sizeof(int)));
+    CUDA_TRY(cudaMemcpyAsync(run->d_chain_ids, chain_ids, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    run->kp.chain_ids = run->d_chain_ids;
+    return SER_OK;
+  };
+  if ((rc = attach()) != SER_OK) { ser_run_destroy(run); return rc; }
+  *out = run;
+  return SER_OK;
+}
+
+/* zero the accumulators of an accumulating run (start of ser_run_init) */
+static int acc_zero(ser_run *run)
+{
+  const size_t nc = (size_t)run->cfg.n_chains, N = run->N, M = run->M;
+  if (run->d_acc_po) CUDA_TRY(cudaMemsetAsync(run->d_acc_po, 0, nc * N * N * sizeof(int), run->stream));
+  if (run->d_acc_pi) CUDA_TRY(cudaMemsetAsync(run->d_acc_pi, 0, nc * N * sizeof(int), run->stream));
+  if (run->d_acc_a) CUDA_TRY(cudaMemsetAsync(run->d_acc_a, 0, nc * M * sizeof(int), run->stream));
+  if (run->d_acc_b) CUDA_TRY(cudaMemsetAsync(run->d_acc_b, 0, nc * M * sizeof(int), run->stream));
+  if (run->d_acc_alive) CUDA_TRY(cudaMemsetAsync(run->d_acc_alive, 0, nc * N * M * sizeof(int), run->stream));
+  return SER_OK;
+}
+
+extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
+{
+  if (!run) { ser_set_error("ser_run_accumulate: null run"); return SER_E_ARG; }
+  if (what < 1 || (what & ~(SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE))) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
+  if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
+  if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
+  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE)) ? SER_STORE_FULL : SER_STORE_PI;
+  if (run->cfg.store < need) {
+    ser_set_error("ser_run_accumulate: these summaries need %s", need == SER_STORE_FULL ? "SER_STORE_FULL (a, b samples)" : "SER_STORE_PI or more");
+    return SER_E_STATE;
+  }
+  if (run->cfg.max_samples < 1) { ser_set_error("ser_run_accumulate: the window needs max_samples >= 1"); return SER_E_ARG; }
+  if (set_device(run)) return SER_E_CUDA;
+  const size_t nc = (size_t)run->cfg.n_chains, N = run->N, M = run->M;
+  auto alloc = [&](int **p, size_t bytes) -> int {
+    const cudaError_t e = POOL_ALLOC(p, bytes);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      ser_set_error("ser_run_accumulate: cannot allocate %zu bytes of accumulators: %s", bytes, cudaGetErrorString(e));
+      return SER_E_CUDA;
+    }
+    return SER_OK;
+  };
+  int rc = SER_OK;
+  if (rc == SER_OK && (what & SER_ACC_PO)) rc = alloc(&run->d_acc_po, nc * N * N * sizeof(int));
+  if (rc == SER_OK && (what & (SER_ACC_SUMS | SER_ACC_AB))) rc = alloc(&run->d_acc_pi, nc * N * sizeof(int));
+  if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_a, nc * M * sizeof(int));
+  if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_b, nc * M * sizeof(int));
+  if (rc == SER_OK && (what & SER_ACC_ALIVE)) rc = alloc(&run->d_acc_alive, nc * N * M * sizeof(int));
+  if (rc == SER_OK) rc = acc_zero(run);
+  if (rc != SER_OK) {
+    int **bufs[] = {&run->d_acc_po, &run->d_acc_pi, &run->d_acc_a, &run->d_acc_b, &run->d_acc_alive};
+    for (int **b : bufs) if (*b) { cudaFreeAsync(*b, run->stream); *b = nullptr; }
+    return rc;
+  }
+  run->acc_what = what;
+  return SER_OK;
+}
+
 extern "C" void ser_run_destroy(ser_run *run)
 {
   if (!run) return;
@@ -692,7 +777,8 @@ extern "C" void ser_run_destroy(ser_run *run)
   void *bufs[] = {run->d_Xs, run->d_hard, run->d_ones, run->d_off, run->d_order, run->d_item_col, run->d_ab, run->d_rpi,
                   run->d_scal, run->d_tape, run->d_tape_off, run->d_samp_a, run->d_samp_b, run->d_samp_pi, run->d_samp_cdl,
                   run->d_scratch_i, run->d_bad, run->d_cd4, run->d_samp_cd_all, run->d_gV, run->d_gpre, run->d_bgrp, run->d_bbat,
-                  run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites, run->d_cl_off, run->d_cl_item, run->d_cl_grp};
+                  run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites, run->d_cl_off, run->d_cl_item, run->d_cl_grp,
+                  run->d_chain_ids, run->d_acc_po, run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_acc_alive};
   for (void *b : bufs) if (b) cudaFreeAsync(b, run->stream);
   if (run->stream) cudaStreamSynchronize(run->stream);
   if (run->sweep_ev) {
@@ -703,6 +789,7 @@ extern "C" void ser_run_destroy(ser_run *run)
   if (run->ev_stop) cudaEventDestroy(run->ev_stop);
   if (run->stream) cudaStreamDestroy(run->stream);
   free(run->h_hard);
+  free(run->h_chain_ids);
   free(run);
 }
 
@@ -717,7 +804,17 @@ extern "C" int ser_run_dims(const ser_run *run, int32_t *N, int32_t *M, int32_t 
 }
 extern "C" const uint8_t *ser_run_hard_flags(const ser_run *run) { return run ? run->h_hard : nullptr; }
 extern "C" int ser_run_is_manycd(const ser_run *run) { return run ? run->cfg.manycd : 0; }
-extern "C" int ser_run_chain_offset(const ser_run *run) { return run ? run->cfg.chain_offset : 0; }
+extern "C" int ser_run_local_chain(const ser_run *run, int32_t g)
+{
+  if (!run) return -1;
+  if (run->h_chain_ids) {
+    for (int c = 0; c < run->cfg.n_chains; c++)
+      if (run->h_chain_ids[c] == g) return c;
+    return -1;
+  }
+  const int l = g - run->cfg.chain_offset;
+  return (l >= 0 && l < run->cfg.n_chains) ? l : -1;
+}
 
 extern "C" int ser_run_set_tapes(ser_run *run, const double *flat, const uint64_t *offsets)
 {
@@ -745,6 +842,9 @@ extern "C" int ser_run_init(ser_run *run)
   if (set_device(run)) return SER_E_CUDA;
   if (run->d_done) CUDA_TRY(cudaMemsetAsync(run->d_done, 0, (size_t)run->cfg.n_chains * sizeof(unsigned int), run->stream));
   run->chunks_done = 0;
+  if (acc_zero(run)) return SER_E_CUDA;
+  run->kp.sample_base = 0;
+  run->sampled = 0;
   mark_launch(run);
   ser_init_kernel<<<run->cfg.n_chains, run->Caux, run->smem_init, run->stream>>>(run->kp);
   CUDA_TRY(cudaGetLastError());
@@ -758,14 +858,9 @@ extern "C" int ser_run_init(ser_run *run)
  * one item whatever the number of chains; chunks are as long as the balance allows (>= 32 items per
  * resident CTA when the launch has that much work), because an item boundary costs one state
  * round trip through HBM. */
-extern "C" int ser_run_advance_both(ser_run *run, int32_t burn_calls, int32_t sample_calls)
+static int launch_sweeps(ser_run *run, int burn_calls, int sample_calls)
 {
-  if (!run) return SER_E_ARG;
-  if (!run->initialized) { ser_set_error("ser_run_advance: call ser_run_init first"); return SER_E_STATE; }
-  if (burn_calls < 0 || sample_calls < 0) { ser_set_error("ser_run_advance: negative call count"); return SER_E_ARG; }
   const int n_calls = burn_calls + sample_calls;
-  if (n_calls <= 0) return SER_OK;
-  if (set_device(run)) return SER_E_CUDA;
   KParams kp = run->kp;
   kp.n_calls = n_calls; kp.burn_calls = burn_calls;
   mark_launch(run);
@@ -825,6 +920,53 @@ extern "C" int ser_run_advance_both(ser_run *run, int32_t burn_calls, int32_t sa
   else ser_sweep_kernel<1024, 1, false><<<grid, run->C, run->smem_sweep, run->stream>>>(kp);
   CUDA_TRY(cudaGetLastError());
   if (rec) CUDA_TRY(cudaEventRecord(ev1, run->stream));
+  return SER_OK;
+}
+
+/* rows [0, w) of every chain's window into the accumulators (ser_run_accumulate), on the run's stream */
+static int accumulate_window(ser_run *run, int w)
+{
+  const int N = run->N, M = run->M, nc = run->cfg.n_chains, W = run->cfg.max_samples, base = run->kp.sample_base;
+  if (run->acc_what & SER_ACC_PO) {
+    mark_launch(run);
+    ser_po_accum_kernel<<<dim3((N + 31) / 32, (N + 31) / 32, nc), 256, 0, run->stream>>>(run->d_samp_pi, run->d_scal, N, W, base, w, run->d_acc_po);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (run->acc_what & (SER_ACC_SUMS | SER_ACC_AB)) {
+    mark_launch(run);
+    ser_posterior_accum_kernel<<<nc, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w,
+                                                             run->d_acc_pi, run->d_acc_a, run->d_acc_b);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (run->acc_what & SER_ACC_ALIVE) {
+    mark_launch(run);
+    ser_alive_accum_kernel<<<dim3(nc, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w,
+                                                                               run->d_acc_alive);
+    CUDA_TRY(cudaGetLastError());
+  }
+  return SER_OK;
+}
+
+extern "C" int ser_run_advance_both(ser_run *run, int32_t burn_calls, int32_t sample_calls)
+{
+  if (!run) return SER_E_ARG;
+  if (!run->initialized) { ser_set_error("ser_run_advance: call ser_run_init first"); return SER_E_STATE; }
+  if (burn_calls < 0 || sample_calls < 0) { ser_set_error("ser_run_advance: negative call count"); return SER_E_ARG; }
+  if (burn_calls + sample_calls <= 0) return SER_OK;
+  if (set_device(run)) return SER_E_CUDA;
+  if (sample_calls > 0) run->sampled = 1;
+  if (!run->acc_what) return launch_sweeps(run, burn_calls, sample_calls);
+  /* accumulating run: launches of at most one window of sampling calls (the burn-in rides on the first), each followed by the
+   * accumulation of the rows it wrote; splitting a launch changes no chain */
+  do {
+    const int w = std::min(sample_calls, run->cfg.max_samples);
+    int rc = launch_sweeps(run, burn_calls, w);
+    if (rc == SER_OK && w > 0) rc = accumulate_window(run, w);
+    if (rc != SER_OK) return rc;
+    run->kp.sample_base += w;
+    burn_calls = 0;
+    sample_calls -= w;
+  } while (sample_calls > 0);
   return SER_OK;
 }
 
@@ -1025,7 +1167,7 @@ static int run_po_to(ser_run *run, const int32_t *d_chosen, int k, const PeerPtr
   dim3 grd((run->N + 31) / 32, (run->N + 31) / 32, k);
   mark_launch(run);
   ser_po_kernel<<<grd, 256, 0, run->stream>>>(run->d_samp_pi, run->d_scal, run->N, run->cfg.max_samples, d_chosen, id_base,
-                                              run->cfg.n_chains, dst);
+                                              run->cfg.n_chains, run->d_chain_ids, dst);
   CUDA_TRY(cudaGetLastError());
   return SER_OK;
 }
@@ -1041,6 +1183,7 @@ extern "C" int ser_run_fetch_samples(ser_run *run, int32_t chain, int32_t *a, in
                                      double *loglik, int32_t *n)
 {
   if (!chain_ok(run, chain)) return SER_E_ARG;
+  if (run->acc_what) { ser_set_error("ser_run_fetch_samples: the store of an accumulating run is a transient window; read the summaries"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   ChainScalars sc;
   CUDA_TRY(cudaMemcpyAsync(&sc, run->d_scal + chain, sizeof(sc), cudaMemcpyDeviceToHost, run->stream));
@@ -1102,6 +1245,7 @@ extern "C" int ser_run_fetch_cd_samples(ser_run *run, int32_t chain, double *c, 
 {
   if (!chain_ok(run, chain)) return SER_E_ARG;
   if (!run->cfg.manycd || !run->d_samp_cd_all) { ser_set_error("ser_run_fetch_cd_samples: needs manycd = 1 and SER_STORE_FULL"); return SER_E_STATE; }
+  if (run->acc_what) { ser_set_error("ser_run_fetch_cd_samples: the store of an accumulating run is a transient window"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   ChainScalars sc;
   CUDA_TRY(cudaMemcpyAsync(&sc, run->d_scal + chain, sizeof(sc), cudaMemcpyDeviceToHost, run->stream));
@@ -1136,6 +1280,15 @@ extern "C" int ser_run_po_counts_device(ser_run *run, const int32_t *d_chosen, i
   if (!run || !d_chosen || !d_counts || k < 1) return SER_E_ARG;
   if (run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_po_counts: run has no pi sample store"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
+  if (run->acc_what) {
+    if (!(run->acc_what & SER_ACC_PO)) { ser_set_error("ser_run_po_counts: the run accumulates without SER_ACC_PO"); return SER_E_STATE; }
+    const int N = run->N, nb = (int)std::min<long long>(((long long)N * N + 255) / 256, 1024);
+    mark_launch(run);
+    ser_po_acc_out_kernel<<<dim3(nb, k), 256, 0, run->stream>>>(run->d_acc_po, run->d_scal, N, d_chosen, run->cfg.chain_offset, run->cfg.n_chains,
+                                                                run->d_chain_ids, d_counts);
+    CUDA_TRY(cudaGetLastError());
+    return SER_OK;
+  }
   return run_po_to(run, d_chosen, k, one_dest(d_counts), run->cfg.chain_offset); /* T is read per chosen chain on the device: no host round trip */
 }
 
@@ -1177,6 +1330,8 @@ extern "C" int ser_run_posterior_sums(ser_run *run, const int32_t *chosen, int32
   if (!run || !chosen || !corr_num || !pi_sum || k < 1) { ser_set_error("ser_run_posterior_sums: bad argument"); return SER_E_ARG; }
   if (run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_posterior_sums: run has no pi sample store"); return SER_E_STATE; }
   if ((a_sum || b_sum) && run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_posterior_sums: a/b sums need SER_STORE_FULL"); return SER_E_STATE; }
+  if (run->acc_what && !(run->acc_what & SER_ACC_SUMS)) { ser_set_error("ser_run_posterior_sums: the run accumulates without SER_ACC_SUMS"); return SER_E_STATE; }
+  if (run->acc_what && (a_sum || b_sum) && !(run->acc_what & SER_ACC_AB)) { ser_set_error("ser_run_posterior_sums: the run accumulates without SER_ACC_AB"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   const int N = run->N, M = run->M;
   int *d_ch = nullptr, *d_pi = nullptr, *d_a = nullptr, *d_b = nullptr, *d_n = nullptr;
@@ -1198,8 +1353,13 @@ extern "C" int ser_run_posterior_sums(ser_run *run, const int32_t *chosen, int32
       if (b_sum) CUDA_TRY(cudaMemcpyAsync(d_b, b_sum, (size_t)k * M * sizeof(int), cudaMemcpyHostToDevice, run->stream));
     }
     mark_launch(run);
-    ser_posterior_kernel<<<k, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
-                                                     run->cfg.chain_offset, run->cfg.n_chains, d_corr, d_pi, d_a, b_sum ? d_b : nullptr, d_n);
+    if (run->acc_what)
+      ser_posterior_acc_out_kernel<<<k, 256, 0, run->stream>>>(run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_scal, N, M, d_ch, run->cfg.chain_offset,
+                                                               run->cfg.n_chains, run->d_chain_ids, d_corr, d_pi, d_a, b_sum ? d_b : nullptr, d_n);
+    else
+      ser_posterior_kernel<<<k, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
+                                                       run->cfg.chain_offset, run->cfg.n_chains, run->d_chain_ids, d_corr, d_pi, d_a,
+                                                       b_sum ? d_b : nullptr, d_n);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(corr_num, d_corr, k * sizeof(long long), cudaMemcpyDeviceToHost, run->stream));
     CUDA_TRY(cudaMemcpyAsync(pi_sum, d_pi, (size_t)k * N * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
@@ -1222,6 +1382,7 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
 {
   if (!run || !chosen || !alive || k < 1) { ser_set_error("ser_run_alive_counts: bad argument"); return SER_E_ARG; }
   if (run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_alive_counts: needs SER_STORE_FULL (a, b samples)"); return SER_E_STATE; }
+  if (run->acc_what && !(run->acc_what & SER_ACC_ALIVE)) { ser_set_error("ser_run_alive_counts: the run accumulates without SER_ACC_ALIVE"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   const int N = run->N, M = run->M;
   const size_t cells = (size_t)k * N * M;
@@ -1235,8 +1396,12 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
     CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
     CUDA_TRY(cudaMemcpyAsync(d_alive, alive, cells * sizeof(int), cudaMemcpyHostToDevice, run->stream));
     mark_launch(run);
-    ser_alive_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
-                                                                       run->cfg.chain_offset, run->cfg.n_chains, d_alive, d_n);
+    if (run->acc_what)
+      ser_alive_acc_out_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_acc_alive, run->d_scal, N, M, d_ch, run->cfg.chain_offset,
+                                                                                   run->cfg.n_chains, run->d_chain_ids, d_alive, d_n);
+    else
+      ser_alive_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
+                                                                         run->cfg.chain_offset, run->cfg.n_chains, run->d_chain_ids, d_alive, d_n);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(alive, d_alive, cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
     CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
@@ -1257,6 +1422,10 @@ extern "C" int ser_run_cross_chain_async(ser_run *run, ser_comm *comm, int32_t k
 {
   if (!run || k < 1) { ser_set_error("ser_run_cross_chain: bad argument"); return SER_E_ARG; }
   if (run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_cross_chain: run has no pi sample store"); return SER_E_STATE; }
+  if (run->acc_what || run->h_chain_ids) {
+    ser_set_error("ser_run_cross_chain: needs a contiguous block of chains that stores all its samples (not a subset or accumulating run)");
+    return SER_E_STATE;
+  }
   if (set_device(run)) return SER_E_CUDA;
   int ranks = 1, rank = 0;
   if (comm && comm_ranks(comm, &ranks, &rank)) return SER_E_ARG;

@@ -132,7 +132,7 @@ __global__ void __launch_bounds__(MAXT, MINB) ser_sweep_kernel(KParams p)
   uint32_t *col = sm.V + tid;
   uint16_t *pre = sm.pre + tid;
   const bool is_taxon = tid < M, is_col = tid <= M;
-  __shared__ unsigned int s_item;
+  __shared__ unsigned int s_item, s_gchain;
 
   /* static per column (the same for every chain this CTA serves) */
   int taxon = 0, off_c = 0, ones_c = 0;
@@ -165,7 +165,10 @@ __global__ void __launch_bounds__(MAXT, MINB) ser_sweep_kernel(KParams p)
     }
     __syncthreads();
   }
-  const unsigned int gchain = (unsigned int)(p.chain_offset + chain);
+  /* the global id lives in shared memory, read at the draws: held in a register across the sweep loop it costs this
+   * register-capped kernel 0.5 % (B200, g2s2) */
+  if (tid == 0) s_gchain = global_chain(p, chain); /* visible after the barrier below the state loads */
+  const unsigned int &gchain = s_gchain;
 
   /* ---- load chain state (L1-bypassing loads: another SM may have written it a moment ago) */
   ChainScalars sc;
@@ -645,7 +648,7 @@ __global__ void __launch_bounds__(MAXT, MINB) ser_sweep_kernel(KParams p)
     /* ================= thinned sample (mcmc_save_chain + compute_exp_data) ================= */
     if constexpr (MANY) {
       if (sampling) {
-        const int sidx = sc.n_samples;
+        const int sidx = sc.n_samples - p.sample_base;
         const double c_first = sm.draws_cd[0], d_first = sm.draws_cd[1]; /* taxon 0's c, d (compute_exp_data, mcmc.c:56-57) */
         if (sidx < p.max_samples) {
           const size_t row = (size_t)chain * p.max_samples + sidx;
@@ -667,7 +670,7 @@ __global__ void __launch_bounds__(MAXT, MINB) ser_sweep_kernel(KParams p)
       }
     } else {
       if (sampling) {
-        const int sidx = sc.n_samples;
+        const int sidx = sc.n_samples - p.sample_base;
         if (sidx < p.max_samples) {
           const size_t row = (size_t)chain * p.max_samples + sidx;
           if (p.store >= SER_STORE_PI)

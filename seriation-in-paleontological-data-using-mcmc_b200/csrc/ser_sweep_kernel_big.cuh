@@ -134,6 +134,7 @@ __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_big(KParams p)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   BigSmem sm;
+  __shared__ unsigned int s_gchain;
   big_layout(&sm, smem_raw, p.N, p.M, p.big_icap, p.big_gcap, MANY ? 1 : 0, WB ? (int)blockDim.x : p.big_gcap);
   const int tid = threadIdx.x, N = p.N, M = p.M, C = blockDim.x, W = p.W, Cs = p.Cs;
   constexpr int BG = SER_BIG_G;
@@ -143,9 +144,10 @@ __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_big(KParams p)
   if (WB && tid == 0) *sm.bctr = 0;
 
   for (int chain = blockIdx.x; chain < p.n_chains; chain += gridDim.x) {
-    const unsigned int gchain = (unsigned int)(p.chain_offset + chain);
+    const unsigned int &gchain = s_gchain; /* in shared memory, like ser_sweep_kernel's */
     double *cd4 = MANY ? p.cd4 + (size_t)chain * 4 * p.Mpad : nullptr;
     __syncthreads(); /* previous chain's state fully saved before the scratch is reused */
+    if (threadIdx.x == 0) s_gchain = global_chain(p, chain); /* visible after the next barrier */
     ChainScalars sc = p.scal[chain];
     for (int n = tid; n < N; n += C) sm.rpi[n] = p.rpi[(size_t)chain * p.Npad + n];
     for (int c = tid; c < M; c += C) {
@@ -730,7 +732,7 @@ __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_big(KParams p)
       if (sc.flags & 1) break;
 
       if (sampling) {
-        const int sidx = sc.n_samples;
+        const int sidx = sc.n_samples - p.sample_base;
         if (sidx < p.max_samples) {
           const size_t row = (size_t)chain * p.max_samples + sidx;
           if (p.store >= SER_STORE_PI)

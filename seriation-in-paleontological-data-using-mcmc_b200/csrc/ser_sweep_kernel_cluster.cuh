@@ -152,6 +152,7 @@ __device__ __forceinline__ void cl_rebuild_hard(const ClSmem &sm, int N, int Mc,
 __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_cl(KParams p)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ unsigned int s_gchain;
   cg::cluster_group cluster = cg::this_cluster();
   const int R = p.cl_R, rank = (int)cluster.block_rank(), n_clusters = (int)gridDim.x / R, cid = (int)blockIdx.x / R;
   const int tid = threadIdx.x, N = p.N, M = p.M, C = blockDim.x, W = p.W, Mc = p.cl_Mc, Cs = Mc + 1;
@@ -168,8 +169,9 @@ __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_cl(KParams p)
   for (int lc = tid; lc < nloc; lc += C) sm.hb32[lc] = p.hbits[lc * R + rank];
 
   for (int chain = cid; chain < p.n_chains; chain += n_clusters) {
-    const unsigned int gchain = (unsigned int)(p.chain_offset + chain);
+    const unsigned int &gchain = s_gchain; /* in shared memory, like ser_sweep_kernel's */
     __syncthreads(); /* the previous chain is done with this CTA's shared memory */
+    if (threadIdx.x == 0) s_gchain = global_chain(p, chain); /* visible after the next barrier */
     ChainScalars sc = p.scal[chain];
     for (int n = tid; n < N; n += C) sm.rpi[n] = p.rpi[(size_t)chain * p.Npad + n];
     for (int lc = tid; lc < nloc; lc += C) {
@@ -510,7 +512,7 @@ __global__ void __launch_bounds__(1024, 1) ser_sweep_kernel_cl(KParams p)
       if (sc.flags & 1) break;
 
       if (sampling) { /* thinned sample: the site order by rank 0, a / b by the columns' owners */
-        const int sidx = sc.n_samples;
+        const int sidx = sc.n_samples - p.sample_base;
         if (sidx < p.max_samples) {
           const size_t row = (size_t)chain * p.max_samples + sidx;
           if (p.store >= SER_STORE_PI && rank == 0)
