@@ -277,6 +277,33 @@ int ser_multi_chain_stats(ser_multi *m, double *e_negloglik, double *e_c, double
 int ser_multi_cross_chain(ser_multi *m, int32_t k, int32_t *chosen, int32_t *n_chosen, double *min_out, double *sigma_out,
                           int32_t *counts);
 
+/* ---------------------------------------------------------------- checkpoints
+ * Every chain of a run written to one file and read back into another run, in another process, on any number of devices:
+ * the chains continue bit for bit.  The file is keyed by global chain id, so a file saved from a ser_multi over 8 GPUs
+ * loads into a ser_multi over 1, 2 or 4, into a ser_run, or into a subset run (ser_run_create_chains), each reading only the
+ * records of its own chains.  Format, size and what is validated: DESIGN.md section 3.6.
+ *
+ * Save waits for the run's stream, writes path.tmp, syncs it to disk and renames it over path (a crash mid-write keeps the
+ * previous file).  The same chains in the same state give a byte-identical file whatever the sharding or the sweep path.
+ *
+ * Load stands in for the init call on a created run, fresh or initialised.  In replay mode set the tapes first; a run that
+ * is to accumulate calls ser_run_accumulate first with the flags it was saved with.  On any error the run is left
+ * uninitialised (advance returns SER_E_STATE); nothing is swept on a state that failed a check:
+ *   SER_E_IO     missing or truncated file, bad magic or version, checksum mismatch
+ *   SER_E_ARG    another dataset (fingerprint of X and the hard flags, or N / M), or a local chain's global id not in the file
+ *   SER_E_STATE  mode, seed, sweeps_per_call, manycd, store, max_samples or accumulate flags differ from the run's
+ *   SER_E_TAPE   a replay cursor beyond the chain's tape
+ *   SER_E_CHECK  a record out of range (a <= b <= N, rpi a permutation) or failing the consistency check (ser_run_check's)
+ * One process per GPU: each rank saves and loads its own file with the ser_run_* pair. */
+int ser_run_save_checkpoint(ser_run *run, const char *path);
+int ser_run_load_checkpoint(ser_run *run, const char *path);
+int ser_multi_save_checkpoint(ser_multi *m, const char *path);
+int ser_multi_load_checkpoint(ser_multi *m, const char *path);
+/* header only, host only, no CUDA call: what a resume needs to plan the remaining calls.  calls_done counts the calls
+ * advanced since init (burn-in and sampling), n_samples the sampling calls.  Any pointer may be NULL. */
+int ser_checkpoint_info(const char *path, int32_t *N, int32_t *M, int32_t *n_chains, int64_t *calls_done,
+                        int32_t *n_samples, uint32_t *seed, int32_t *mode, int32_t *manycd);
+
 /* ---------------------------------------------------------------- reference-compatible files */
 /* Writes Chains-style files for one local chain into `dir` (which must exist, like the
  * reference): chain_data.csv, exp_data.csv, taxa.csv, sites.csv, hard_sites.csv. */

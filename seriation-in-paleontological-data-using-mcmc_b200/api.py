@@ -103,6 +103,11 @@ SYMBOLS = [
     ("ser_multi_check", C.c_int, [_vp, _i32p]),
     ("ser_multi_chain_stats", C.c_int, [_vp, _dp, _dp, _dp, _i32p]),
     ("ser_multi_cross_chain", C.c_int, [_vp, C.c_int32, _i32p, _i32p, _dp, _dp, _i32p]),
+    ("ser_run_save_checkpoint", C.c_int, [_vp, C.c_char_p]),
+    ("ser_run_load_checkpoint", C.c_int, [_vp, C.c_char_p]),
+    ("ser_multi_save_checkpoint", C.c_int, [_vp, C.c_char_p]),
+    ("ser_multi_load_checkpoint", C.c_int, [_vp, C.c_char_p]),
+    ("ser_checkpoint_info", C.c_int, [C.c_char_p, _i32p, _i32p, _i32p, _i64p, _i32p, C.POINTER(C.c_uint32), _i32p, _i32p]),
 ]
 COMM_ID_BYTES = 128
 
@@ -252,6 +257,16 @@ class Run:
 
     def init(self):
         _check(lib().ser_run_init(self._h))
+        return self
+
+    def save_checkpoint(self, path):
+        """every chain's state (and stored samples, accumulators) to ``path``, written atomically (ser_run_save_checkpoint)"""
+        _check(lib().ser_run_save_checkpoint(self._h, os.fsencode(path)))
+        return self
+
+    def load_checkpoint(self, path):
+        """in place of init(): continue the chains saved in ``path`` bit for bit (set_tapes / accumulate come first)"""
+        _check(lib().ser_run_load_checkpoint(self._h, os.fsencode(path)))
         return self
 
     def advance(self, n_calls: int, sampling: bool):
@@ -478,6 +493,16 @@ class Multi:
         _check(lib().ser_multi_advance(self._h, burn_calls, sample_calls))
         return self
 
+    def save_checkpoint(self, path):
+        """every device's chains to one file, in global order (ser_multi_save_checkpoint)"""
+        _check(lib().ser_multi_save_checkpoint(self._h, os.fsencode(path)))
+        return self
+
+    def load_checkpoint(self, path):
+        """in place of init(): each device reads its own chains' records from ``path``"""
+        _check(lib().ser_multi_load_checkpoint(self._h, os.fsencode(path)))
+        return self
+
     def sync(self):
         _check(lib().ser_multi_sync(self._h))
         return self
@@ -526,6 +551,16 @@ def select_chains(e_negloglik, k: int):
     mn, sd = C.c_double(), C.c_double()
     _check(lib().ser_select_chains(_p(e, C.c_double), e.size, k, _p(chosen, C.c_int32), C.byref(n), C.byref(mn), C.byref(sd)))
     return chosen[:n.value].copy(), mn.value, sd.value
+
+
+def checkpoint_info(path) -> dict:
+    """the header of a checkpoint file (host only, no CUDA call): what a resume needs to plan the remaining calls"""
+    n, m, nc, ns, mode, many = (C.c_int32() for _ in range(6))
+    calls, seed = C.c_int64(), C.c_uint32()
+    _check(lib().ser_checkpoint_info(os.fsencode(path), C.byref(n), C.byref(m), C.byref(nc), C.byref(calls), C.byref(ns), C.byref(seed),
+                                     C.byref(mode), C.byref(many)))
+    return dict(N=n.value, M=m.value, n_chains=nc.value, calls_done=calls.value, n_samples=ns.value, seed=seed.value, mode=mode.value,
+                manycd=bool(many.value))
 
 
 def select_chains_device(e_ptr: int, n: int, k: int, chosen_ptr: int, info_ptr: int, device=0, stream=None):

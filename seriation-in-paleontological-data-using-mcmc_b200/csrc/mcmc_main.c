@@ -17,10 +17,17 @@
  * sharded over the GPUs of the box -- ser_multi_*):
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
+ *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
  * lines and po.csv as the one-shot step, with device memory for K chains' window instead of every chain's history.
+ * --checkpoint FILE writes every chain's state to FILE at the end of the sweeps (ser_multi_save_checkpoint), and every C calls
+ * with --checkpoint-every C (the advance runs in segments of at most C calls; splitting a launch changes no chain).  --resume
+ * loads FILE when it exists in place of the random start and runs the calls of the --burn B --samples S schedule that are left
+ * (it refuses a file that has advanced past B + S calls, or whose sample count is not max(0, calls - B)).  --stop-after C
+ * advances at most C calls in this invocation, writes FILE and exits 0 with one line saying where it stopped, before any
+ * summary or Chains/ file: a long run split into slices gives the same output as the run done in one piece.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -44,7 +51,10 @@ static void usage(const char *argv0)
           "       %s [manycd Tburnin T] < dataset.txt      (manycd 1: per-taxon c, d; chain 0)\n"
           "       %s --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset F]\n"
           "              [--chains-dir DIR] [--select K] [--po out.csv] [--device D] [--manycd 0|1]\n"
-          "              [--replay-selected --window W]   (with --select: keep no sample history, replay the chosen chains)\n",
+          "              [--replay-selected --window W]   (with --select: keep no sample history, replay the chosen chains)\n"
+          "              [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]]\n"
+          "                  (save every chain to FILE at the end and every C calls; --resume continues FILE's run; --stop-after C\n"
+          "                   advances at most C calls, saves and exits)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -68,9 +78,10 @@ static double *read_tape(const char *path, uint64_t *len)
 int main(int argc, char **argv)
 {
   int n_chains = 1, first = 0, burn = 1000, samples = 1000, select_k = 0, device = 0, batch = 0, manycd = 0, gpus = 1, i;
-  int replay_selected = 0, window = 64;
+  int replay_selected = 0, window = 64, resume = 0, ckpt_every = 0, stop_after = -1;
+  int64_t done = 0, total;
   unsigned long seed = 0;
-  const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN");
+  const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -88,6 +99,7 @@ int main(int argc, char **argv)
     for (i = 1; i < argc; i++) {
       const char *a = argv[i], *v = (i + 1 < argc) ? argv[i + 1] : NULL;
       if (!strcmp(a, "--replay-selected")) { replay_selected = 1; continue; }
+      if (!strcmp(a, "--resume")) { resume = 1; continue; }
       if (!v) usage(argv[0]);
       if (!strcmp(a, "--chains")) n_chains = atoi(v);
       else if (!strcmp(a, "--gpus")) gpus = atoi(v);
@@ -102,11 +114,15 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--device")) device = atoi(v);
       else if (!strcmp(a, "--manycd")) manycd = atoi(v) != 0;
       else if (!strcmp(a, "--window")) window = atoi(v);
+      else if (!strcmp(a, "--checkpoint")) ckpt_path = v;
+      else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
+      else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
       i++;
     }
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
+    if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
     const long idx = strtol(argv[1], &end, 10); /* mcmc.c:115,153 */
@@ -142,6 +158,8 @@ int main(int argc, char **argv)
   cfg.manycd = manycd;
   for (i = 0; i < 8; i++) devs[i] = device + i;
 
+  if (tape_path && ckpt_path) { fprintf(stderr, "mcmc: --checkpoint drives the free-running batch mode, not SER_TAPE_IN\n"); return 1; }
+  total = (int64_t)burn + samples;
   if (tape_path) { /* replay of one recorded chain (validation against the reference) */
     uint64_t offs[2] = {0, 0};
     double *tape;
@@ -155,9 +173,37 @@ int main(int argc, char **argv)
     if (ser_run_sync(run)) die("ser_run_sync");
     if (ser_run_check(run, &bad)) { fprintf(stderr, "main: error. (%s)\n", ser_last_error()); return 1; } /* mcmc.c:199-204 */
   } else {
+    struct stat sb;
+    int64_t end;
     if (ser_multi_create(ds, &cfg, gpus, devs, &multi)) die("ser_multi_create");
-    if (ser_multi_init(multi)) die("ser_multi_init");
-    if (ser_multi_advance(multi, burn, samples)) die("sweeps"); /* mcmc.c:140-143, :180-185 */
+    if (resume && stat(ckpt_path, &sb) == 0) {
+      int32_t ns = 0;
+      if (ser_checkpoint_info(ckpt_path, NULL, NULL, NULL, &done, &ns, NULL, NULL, NULL)) die("ser_checkpoint_info");
+      if (done > total || ns != (done > burn ? done - burn : 0)) {
+        fprintf(stderr, "mcmc: %s holds %lld calls and %d samples: not a point of the --burn %d --samples %d schedule\n", ckpt_path,
+                (long long)done, ns, burn, samples);
+        return 1;
+      }
+      if (ser_multi_load_checkpoint(multi, ckpt_path)) die("ser_multi_load_checkpoint");
+    } else if (ser_multi_init(multi)) {
+      die("ser_multi_init");
+    }
+    end = (stop_after >= 0 && done + stop_after < total) ? done + stop_after : total;
+    while (done < end) { /* mcmc.c:140-143, :180-185, in segments of at most --checkpoint-every calls */
+      const int64_t seg = (ckpt_every > 0 && end - done > ckpt_every) ? ckpt_every : end - done;
+      const int64_t b = done < burn ? (seg < burn - done ? seg : burn - done) : 0;
+      if (ser_multi_advance(multi, (int32_t)b, (int32_t)(seg - b))) die("sweeps");
+      done += seg;
+      if (ckpt_every > 0 && done < end && ser_multi_save_checkpoint(multi, ckpt_path)) die("ser_multi_save_checkpoint");
+    }
+    if (ckpt_path && ser_multi_save_checkpoint(multi, ckpt_path)) die("ser_multi_save_checkpoint");
+    if (done < total) {
+      printf("stopped after call %lld of %lld; %s holds every chain; run again with --checkpoint %s --resume to continue\n", (long long)done,
+             (long long)total, ckpt_path, ckpt_path);
+      ser_multi_destroy(multi);
+      ser_dataset_free(ds);
+      return 0;
+    }
     if (ser_multi_sync(multi)) die("ser_multi_sync");
     if (ser_multi_check(multi, &bad)) { fprintf(stderr, "main: error. (%s)\n", ser_last_error()); return 1; }
   }

@@ -107,6 +107,10 @@ struct ser_run {
   /* streaming accumulators (ser_run_accumulate): SER_ACC_* flags, per local chain totals */
   int acc_what, sampled;
   int *d_acc_po, *d_acc_pi, *d_acc_a, *d_acc_b, *d_acc_alive;
+  /* checkpoints (ser_ckpt.cuh): calls and sampling calls advanced since init, and the fingerprint of the run's dataset */
+  long long calls_done;
+  int samples_done;
+  uint64_t ds_fp;
 };
 
 /* multi-GPU pieces (ser_multi.cuh): NCCL entry points resolved at run time */
@@ -114,6 +118,7 @@ struct ser_comm;
 static int comm_all_gather_e(ser_comm *comm, double *d_e_all, int n_local, cudaStream_t stream);
 static int comm_all_reduce_counts(ser_comm *comm, int *d_counts, size_t n, cudaStream_t stream);
 static int comm_ranks(const ser_comm *comm, int *n_ranks, int *rank);
+static uint64_t ckpt_dataset_fingerprint(const ser_dataset *ds); /* ser_ckpt.cuh */
 
 /* Stream-ordered pool allocation: cudaMalloc/cudaFree are synchronous driver calls with erratic
  * latency (tens to hundreds of ms on shared hosts).  The library allocates from its OWN memory pool per
@@ -356,6 +361,7 @@ static int run_create_impl(const ser_dataset *ds, const ser_run_config *cfg, ser
   run->h_hard = (uint8_t *)malloc(N);
   if (!run->h_hard) { ser_set_error("ser_run_create: out of memory"); return SER_E_ARG; }
   memcpy(run->h_hard, ds->hard, N);
+  run->ds_fp = ckpt_dataset_fingerprint(ds);
 
   const size_t nc = (size_t)cfg->n_chains;
   CUDA_TRY(POOL_ALLOC(&run->d_Xs, Xs.size() * 4));
@@ -845,6 +851,8 @@ extern "C" int ser_run_init(ser_run *run)
   if (acc_zero(run)) return SER_E_CUDA;
   run->kp.sample_base = 0;
   run->sampled = 0;
+  run->calls_done = 0;
+  run->samples_done = 0;
   mark_launch(run);
   ser_init_kernel<<<run->cfg.n_chains, run->Caux, run->smem_init, run->stream>>>(run->kp);
   CUDA_TRY(cudaGetLastError());
@@ -955,6 +963,8 @@ extern "C" int ser_run_advance_both(ser_run *run, int32_t burn_calls, int32_t sa
   if (burn_calls + sample_calls <= 0) return SER_OK;
   if (set_device(run)) return SER_E_CUDA;
   if (sample_calls > 0) run->sampled = 1;
+  run->calls_done += burn_calls + sample_calls;
+  run->samples_done += sample_calls;
   if (!run->acc_what) return launch_sweeps(run, burn_calls, sample_calls);
   /* accumulating run: launches of at most one window of sampling calls (the burn-in rides on the first), each followed by the
    * accumulation of the rows it wrote; splitting a launch changes no chain */
@@ -1542,3 +1552,4 @@ extern "C" int ser_microbench(int32_t device, double out[3])
 }
 
 #include "ser_multi.cuh"
+#include "ser_ckpt.cuh"
