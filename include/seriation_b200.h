@@ -191,6 +191,25 @@ int ser_po_finalize(const int32_t *counts, int32_t k, int32_t N, int32_t chains_
 int ser_run_posterior_sums(ser_run *run, const int32_t *chosen, int32_t k, int64_t *corr_num, int32_t *pi_sum,
                            int32_t *a_sum, int32_t *b_sum, int32_t *n_samples);
 
+/* Convergence diagnostics over the stored samples (DESIGN.md section 3.7).  Quantity q of sample t:
+ *   q = 0 -loglik, q = 1 exp(c), q = 2 exp(d) (a manycd run: taxon 0's c, d, as in the exp_data sums); q = 3 + i pi_t(i) */
+#define SER_DIAG_SCALARS 1 /* q = 0..2: -loglik, exp(c), exp(d)   (needs SER_STORE_FULL) */
+#define SER_DIAG_SITES 2   /* q = 3+i: pi(i)                       (needs SER_STORE_PI)   */
+/* per chosen chain (GLOBAL ids; -1 / not held: slab untouched) and quantity, over its T stored samples:
+ * stats [k][3+N][4] = mean, var, ess, lags;  halves [k][3+N][4] = mean1, var1, mean2, var2;  n_samples [k] = T.
+ * var has divisor T-1; the halves are the first and last floor(T/2) samples (divisor n-1).  ess is Geyer's initial monotone
+ * sequence estimate of one chain (no rank normalisation) over lags below min(T, max_lag) (max_lag 0 = no cap); lags = the number
+ * of autocorrelations summed -- when it reaches 2 floor(L/2) the cap cut the sequence and ess is an upper bound.  A quantity
+ * constant in a chain has var 0, ess NaN, lags 0.  Host memory; quantities `what` does not request keep their slab.
+ * SER_E_ARG: k < 1, what not in 1..3, max_lag < 0.  SER_E_STATE: a store below what `what` needs, an accumulating run, a run
+ * not initialised, or a chosen chain this run holds with T < 4 (the outputs are then left as they were). */
+int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, int32_t max_lag, double *stats, double *halves,
+                        int32_t *n_samples);
+/* split-R-hat per quantity from the halves of k chains (BDA3 section 11.4; host only, no CUDA call): W = mean of the 2k half
+ * variances, B/n = variance of the 2k half means (divisor 2k-1), R-hat = sqrt(((n-1)/n W + B/n) / W); NaN where W = 0.
+ * SER_E_ARG when the chains' T differ or T < 4. */
+int ser_split_rhat(const double *halves, const int32_t *n_samples, int32_t k, int32_t Q, double *rhat);
+
 /* alive[c][j][m] = #{t : a_t(m) <= j <= b_t(m)} over the stored samples of the chosen chains owned by
  * this run (same slab convention as above; int32 [k][N][M], host memory; needs SER_STORE_FULL).
  * The counts behind plot_taxa_occurence_probability_matrix, plot_false_taxa_occurence_probability

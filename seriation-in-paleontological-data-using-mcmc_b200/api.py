@@ -19,6 +19,7 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
 ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE = 1, 2, 4, 8
+DIAG_SCALARS, DIAG_SITES = 1, 2
 
 _i32p, _dp, _u8p = C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_uint8)
 _i64p, _u64p = C.POINTER(C.c_int64), C.POINTER(C.c_uint64)
@@ -79,6 +80,8 @@ SYMBOLS = [
     ("ser_run_po_counts", C.c_int, [_vp, _i32p, C.c_int32, _i32p]),
     ("ser_po_finalize", C.c_int, [_i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _dp]),
     ("ser_run_posterior_sums", C.c_int, [_vp, _i32p, C.c_int32, _i64p, _i32p, _i32p, _i32p, _i32p]),
+    ("ser_run_diagnostics", C.c_int, [_vp, _i32p, C.c_int32, C.c_int32, C.c_int32, _dp, _dp, _i32p]),
+    ("ser_split_rhat", C.c_int, [_dp, _i32p, C.c_int32, C.c_int32, _dp]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
     ("ser_write_labelled_files", C.c_int, [_vp, C.c_int32, _vp, C.c_char_p]),
     ("ser_microbench", C.c_int, [C.c_int32, _dp]),
@@ -391,6 +394,22 @@ class Run:
         _check(lib().ser_run_alive_counts(self._h, _p(chosen, C.c_int32), len(chosen), _p(out, C.c_int32), C.byref(n)))
         return out, n.value
 
+    def diagnostics(self, chosen, scalars: bool = True, sites: bool = True, max_lag: int = 0) -> dict:
+        """convergence diagnostics of the chosen chains (global ids) over their stored samples (ser_run_diagnostics): per chain and
+        quantity (Q = 3 + N: -loglik, exp(c), exp(d), then pi of every site) ``mean``, ``var``, ``ess``, ``lags`` [k][Q], ``halves``
+        [k][Q][4] (mean1, var1, mean2, var2), ``n_samples`` [k] and the split ``rhat`` [Q] over the chains this run holds (None when
+        their sample counts differ).  Slabs the run does not fill stay NaN (n_samples 0)."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        k, Q = len(chosen), 3 + self.N
+        stats, halves = np.full((k, Q, 4), np.nan), np.full((k, Q, 4), np.nan)
+        n = np.zeros(k, np.int32)
+        what = (DIAG_SCALARS if scalars else 0) | (DIAG_SITES if sites else 0)
+        _check(lib().ser_run_diagnostics(self._h, _p(chosen, C.c_int32), k, what, int(max_lag), _p(stats, C.c_double),
+                                         _p(halves, C.c_double), _p(n, C.c_int32)))
+        held = n > 0
+        rhat = split_rhat(halves[held], n[held]) if held.any() and np.all(n[held] == n[held][0]) else None
+        return dict(mean=stats[..., 0], var=stats[..., 1], ess=stats[..., 2], lags=stats[..., 3], halves=halves, n_samples=n, rhat=rhat)
+
     def po_counts_device(self, chosen_ptr: int, k: int, counts_ptr: int):
         _check(lib().ser_run_po_counts_device(self._h, chosen_ptr, k, counts_ptr))
 
@@ -563,6 +582,16 @@ def checkpoint_info(path) -> dict:
                 manycd=bool(many.value))
 
 
+def split_rhat(halves, n_samples) -> np.ndarray:
+    """split-R-hat per quantity from the [k][Q][4] halves of k chains with equal sample counts (ser_split_rhat, host only)"""
+    halves = np.ascontiguousarray(halves, dtype=np.float64)
+    n = np.ascontiguousarray(n_samples, dtype=np.int32)
+    k, Q = halves.shape[0], halves.shape[1]
+    out = np.empty(Q)
+    _check(lib().ser_split_rhat(_p(halves, C.c_double), _p(n, C.c_int32), k, Q, _p(out, C.c_double)))
+    return out
+
+
 def select_chains_device(e_ptr: int, n: int, k: int, chosen_ptr: int, info_ptr: int, device=0, stream=None):
     _check(lib().ser_select_chains_device(e_ptr, n, k, chosen_ptr, info_ptr, device, stream))
 
@@ -629,13 +658,17 @@ def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool 
     ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
     ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
     run's, so compute_pair_order_matrix, compute_exp_* and the probability maps work on it unchanged.  ``with_ab``
-    also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  Raises SeriationError when
-    a replayed chain's E[-logL] differs from its first run in any bit."""
+    also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  ``window=0`` keeps every
+    sample instead (``STORE_FULL``, no accumulators): the summaries take the one-shot path and ``diagnostics`` works on
+    the result.  Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
     ids = np.ascontiguousarray(chains, dtype=np.int32)
+    keep_all = window == 0
     run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
-              store=STORE_FULL if with_ab else STORE_PI, max_samples=window,
+              store=STORE_FULL if (with_ab or keep_all) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
               device=batch.run.cfg.device if device is None else device, chain_ids=ids)
-    run.init().accumulate(po=True, sums=True, ab=with_ab, alive=with_ab)
+    run.init()
+    if not keep_all:
+        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab)
     run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
     want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
     if want.tobytes() != got.tobytes():
@@ -652,6 +685,13 @@ def compute_pair_order_matrix(batch: ChainBatch, chains, chains_selected: int, s
     the host.  ``sites`` is accepted for signature compatibility."""
     counts = batch.run.po_counts(np.asarray(chains, dtype=np.int32))
     return po_finalize(counts, chains_selected, faithful)
+
+
+def diagnostics(batch: ChainBatch, chains, max_lag: int = 0) -> dict:
+    """Run.diagnostics over the chosen chains of a batch: every site's pi, and -loglik, exp(c), exp(d) when the batch keeps the
+    full sample store (their rows stay NaN otherwise).  A batch from replay_chosen(..., window=0) keeps it."""
+    run = batch.run
+    return run.diagnostics(np.asarray(chains, dtype=np.int32), scalars=run.cfg.store >= STORE_FULL, max_lag=max_lag)
 
 
 def compute_exp_cd(batch: ChainBatch, chains, chains_selected: int, faithful: bool = True):

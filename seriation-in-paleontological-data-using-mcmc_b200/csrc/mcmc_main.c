@@ -17,7 +17,7 @@
  * sharded over the GPUs of the box -- ser_multi_*):
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
- *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]]
+ *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
@@ -28,9 +28,13 @@
  * (it refuses a file that has advanced past B + S calls, or whose sample count is not max(0, calls - B)).  --stop-after C
  * advances at most C calls in this invocation, writes FILE and exits 0 with one line saying where it stopped, before any
  * summary or Chains/ file: a long run split into slices gives the same output as the run done in one piece.
+ * --diagnostics FILE (with --select) re-simulates the chosen chains alone keeping every sample (SER_STORE_FULL, bit-identical to
+ * their first run, which is checked), writes per-quantity split-R-hat and effective sample sizes to FILE and prints one summary
+ * line; under --replay-selected --po the same run supplies the pair-order counts.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
+#include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -54,9 +58,78 @@ static void usage(const char *argv0)
           "              [--replay-selected --window W]   (with --select: keep no sample history, replay the chosen chains)\n"
           "              [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]]\n"
           "                  (save every chain to FILE at the end and every C calls; --resume continues FILE's run; --stop-after C\n"
-          "                   advances at most C calls, saves and exits)\n",
+          "                   advances at most C calls, saves and exits)\n"
+          "              [--diagnostics FILE]   (with --select: split-R-hat and ESS of the chosen chains to FILE)\n",
           argv0, argv0, argv0);
   exit(1);
+}
+
+/* --diagnostics: the chosen chains re-simulated alone with every sample kept (bit-identical to their first run, whose E[-logL]
+ * per global id - first is e[]; any difference exits 1), their split-R-hat and ESS written to `path` as CSV and summarised in one
+ * line.  `counts` (NULL: not wanted) receives their pair-order counts from the same run. */
+static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
+                               int burn, int samples, int32_t *counts, const char *path)
+{
+  ser_run_config c2 = *cfg;
+  ser_run *sub = NULL;
+  int32_t N, M, nh, ns = 0, i, q, c;
+  double *e2, *stats, *halves, *rhat;
+  int32_t *n;
+  FILE *f;
+  int s_max = -1, s_min = -1, constant = 0;
+  double r_max = NAN, ess_min_site = NAN, ess_min[3];
+  ser_dataset_dims(ds, &N, &M, &nh);
+  const int Q = 3 + N;
+  c2.n_chains = k;
+  c2.chain_offset = 0;
+  c2.store = SER_STORE_FULL;
+  c2.max_samples = samples;
+  e2 = (double *)malloc(sizeof(double) * (size_t)k);
+  stats = (double *)malloc(sizeof(double) * (size_t)k * Q * 4);
+  halves = (double *)malloc(sizeof(double) * (size_t)k * Q * 4);
+  rhat = (double *)malloc(sizeof(double) * (size_t)Q);
+  n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k);
+  if (!e2 || !stats || !halves || !rhat || !n) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
+  if (ser_run_init(sub) || ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
+  if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
+  for (i = 0; i < k; i++)
+    if (memcmp(&e2[i], &e[chosen[i] - first], sizeof(double))) {
+      fprintf(stderr, "mcmc: the replayed chain %d does not reproduce its first run (E[-logL] %.17g vs %.17g)\n", chosen[i], e2[i],
+              e[chosen[i] - first]);
+      exit(1);
+    }
+  if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
+  if (ser_run_diagnostics(sub, chosen, k, SER_DIAG_SCALARS | SER_DIAG_SITES, 0, stats, halves, n)) die("ser_run_diagnostics");
+  if (ser_split_rhat(halves, n, k, Q, rhat)) die("ser_split_rhat");
+  ser_run_destroy(sub);
+  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  fprintf(f, "quantity,mean,rhat,ess_min,ess_sum\n");
+  for (q = 0; q < Q; q++) {
+    double mean = 0.0, emin = NAN, esum = NAN;
+    for (c = 0; c < k; c++) {
+      const double *st = stats + ((size_t)c * Q + q) * 4;
+      mean += st[0];
+      if (isnan(st[2])) continue;
+      emin = isnan(emin) || st[2] < emin ? st[2] : emin;
+      esum = isnan(esum) ? st[2] : esum + st[2];
+    }
+    mean /= k;
+    if (q < 3) fprintf(f, "%s,", q == 0 ? "-logL" : q == 1 ? "c" : "d");
+    else fprintf(f, "site_%d,", q - 3);
+    fprintf(f, "%.17g,%.17g,%.17g,%.17g\n", mean, rhat[q], emin, esum);
+    if (q < 3) ess_min[q] = emin;
+    else {
+      if (isnan(emin)) constant++; /* constant in every chosen chain */
+      if (!isnan(rhat[q]) && (s_max < 0 || rhat[q] > r_max)) { r_max = rhat[q]; s_max = q - 3; }
+      if (!isnan(emin) && (s_min < 0 || emin < ess_min_site)) { ess_min_site = emin; s_min = q - 3; }
+    }
+  }
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  for (q = 0; q < 3; q++) constant += isnan(ess_min[q]);
+  printf("diagnostics: R-hat -logL %.4f  c %.4f  d %.4f  sites max %.4f (site %d)  ESS -logL min %.1f  sites min %.1f (site %d)  "
+         "constant %d\n", rhat[0], rhat[1], rhat[2], r_max, s_max, ess_min[0], ess_min_site, s_min, constant);
+  free(e2); free(stats); free(halves); free(rhat); free(n);
 }
 
 static double *read_tape(const char *path, uint64_t *len)
@@ -82,6 +155,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
+  const char *diag_path = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -115,6 +189,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--manycd")) manycd = atoi(v) != 0;
       else if (!strcmp(a, "--window")) window = atoi(v);
       else if (!strcmp(a, "--checkpoint")) ckpt_path = v;
+      else if (!strcmp(a, "--diagnostics")) diag_path = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
@@ -122,6 +197,7 @@ int main(int argc, char **argv)
     }
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
+    if (diag_path && select_k < 1) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
@@ -252,7 +328,7 @@ int main(int argc, char **argv)
         /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0) {
+        if (counts && nchosen > 0 && !diag_path) {
           ser_run_config c2 = cfg;
           ser_run *sub = NULL;
           c2.n_chains = nchosen;
@@ -273,6 +349,8 @@ int main(int argc, char **argv)
         for (i = 0; i < nchosen; i++) { sc += ec[chosen[i] - first]; sdd += ed[chosen[i] - first]; }
         printf("E[c] %.6f  E[d] %.6f over the chosen chains\n", sc / nchosen, sdd / nchosen);
       }
+      if (diag_path && nchosen > 0)
+        replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path);
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);
         FILE *f;

@@ -298,6 +298,155 @@ __global__ void ser_alive_kernel(const uint16_t *samp_a, const uint16_t *samp_b,
   for (int j = 0; j < N; j++) { acc += col[(size_t)j * M]; col[(size_t)j * M] = acc; }
 }
 
+/* ------------------------------------------------------------------ convergence diagnostics (ser_run_diagnostics, DESIGN.md 3.7)
+ * Quantity q of a chain's stored sample t: 0 = -loglik, 1 = exp(c), 2 = exp(d) (samp_cdl; taxon 0's c, d on a manycd run),
+ * 3 + i = pi_t(i), the position of site i.  One block of 32 warps per (chosen chain, 32 consecutive quantities).  The moments
+ * read the store with lane = quantity and warp = t mod 32 (coalesced rows), then reduce the 32 partials in warp order.  The
+ * autocovariances run one warp per quantity, lane l summing lag k0 + l in t order over centred traces staged 64 samples at a
+ * time; a warp stops after the lag block in which a Geyer pair sum turns non-positive.  No sum depends on the grid. */
+#define SER_DIAG_TC 64             /* samples per staged chunk */
+#define SER_DIAG_SA (SER_DIAG_TC + 1)  /* odd row strides: the staging stores hit distinct banks */
+#define SER_DIAG_SB (SER_DIAG_TC + 33)
+
+__device__ __forceinline__ double diag_value(const uint16_t *pi, const double *cdl, int N, int q, int t)
+{
+  if (q >= 3) return (double)pi[(size_t)t * N + q - 3];
+  if (q == 0) return -cdl[(size_t)t * 3 + 2];
+  return exp(cdl[(size_t)t * 3 + q - 1]);
+}
+
+/* stats [k][3+N][4] = mean, var, ess, lags; halves [k][3+N][4] = mean1, var1, mean2, var2 for quantities [qlo, qhi); n_out[c] = T */
+__global__ void __launch_bounds__(1024, 1) ser_diag_kernel(const uint16_t *samp_pi, const double *samp_cdl, const ChainScalars *scal, int N,
+                                                           int max_samples, const int *chosen, int chain_offset, int n_local, const int *ids,
+                                                           int qlo, int qhi, int max_lag, double *stats, double *halves, int *n_out)
+{
+  __shared__ double sbuf[32 * (SER_DIAG_SA + SER_DIAG_SB)]; /* moment partials [5][32 warps][32 lanes], then the staged chunks */
+  __shared__ double s_mean[32], s_m1[32], s_m2[32];
+  __shared__ int s_on[32];  /* quantity requested, and not constant in this chain */
+  __shared__ int s_act[32]; /* its warp is still summing lags: only these traces are staged */
+  __shared__ int s_eq1[32], s_eq2[32]; /* every sample of the first / last half equals that half's first one */
+  const int c = blockIdx.x;
+  const int local = local_chain(chosen[c], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int T = stored_samples(scal, local, max_samples);
+  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[c] = T;
+  if (T < 4) return; /* the host refuses the call */
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, Q = 3 + N, n = T / 2;
+  const int q0 = (qlo / 32 + blockIdx.y) * 32;
+  const size_t row0 = (size_t)local * max_samples;
+  const uint16_t *pi = samp_pi ? samp_pi + row0 * N : nullptr;
+  const double *cdl = samp_cdl ? samp_cdl + row0 * 3 : nullptr;
+  const double NaN = __longlong_as_double(0x7ff8000000000000LL);
+  const int q = q0 + lane;
+  const bool valid = q >= qlo && q < qhi;
+  double *out = stats + ((size_t)c * Q + q) * 4, *hv = halves + ((size_t)c * Q + q) * 4;
+  if (w == 0) { s_eq1[lane] = 1; s_eq2[lane] = 1; }
+  __syncthreads();
+
+  /* pass 1: sums over the trace and its halves (the middle sample of an odd T is in neither), min and max, and whether each half
+   * is constant -- then its mean is its value and its variance 0 exactly, not the rounding residue of S / n */
+  double s = 0.0, s1 = 0.0, s2 = 0.0, lo = INFINITY, hi = -INFINITY;
+  const double f1 = valid ? diag_value(pi, cdl, N, q, 0) : 0.0, f2 = valid ? diag_value(pi, cdl, N, q, T - n) : 0.0;
+  bool eq1 = true, eq2 = true;
+  if (valid)
+    for (int t = w; t < T; t += 32) {
+      const double x = diag_value(pi, cdl, N, q, t);
+      s += x;
+      if (t < n) { s1 += x; eq1 = eq1 && x == f1; }
+      if (t >= T - n) { s2 += x; eq2 = eq2 && x == f2; }
+      lo = fmin(lo, x); hi = fmax(hi, x);
+    }
+  if (!eq1) atomicAnd(&s_eq1[lane], 0); /* an AND: the same result in any order */
+  if (!eq2) atomicAnd(&s_eq2[lane], 0);
+  double *ps = sbuf + threadIdx.x; /* partial [r][w][lane] at ps[r * 1024] */
+  ps[0] = s; ps[1024] = s1; ps[2048] = s2; ps[3072] = lo; ps[4096] = hi;
+  __syncthreads();
+  if (w == 0) {
+    double S = 0.0, S1 = 0.0, S2 = 0.0, L0 = INFINITY, H0 = -INFINITY;
+    for (int u = 0; u < 32; u++) {
+      const double *p = sbuf + u * 32 + lane;
+      S += p[0]; S1 += p[1024]; S2 += p[2048]; L0 = fmin(L0, p[3072]); H0 = fmax(H0, p[4096]);
+    }
+    const bool constant = L0 == H0; /* gamma_0 = 0: the mean is the value itself, exactly */
+    s_mean[lane] = constant ? L0 : S / T;
+    s_m1[lane] = s_eq1[lane] ? f1 : S1 / n;
+    s_m2[lane] = s_eq2[lane] ? f2 : S2 / n;
+    s_on[lane] = valid && !constant;
+  }
+  __syncthreads();
+  /* pass 2: centred squares about each part's own mean (zero for a constant quantity or half) */
+  const double m = s_mean[lane], m1 = s_m1[lane], m2 = s_m2[lane];
+  const bool var1 = !s_eq1[lane], var2 = !s_eq2[lane];
+  double v = 0.0, v1 = 0.0, v2 = 0.0;
+  if (s_on[lane])
+    for (int t = w; t < T; t += 32) {
+      const double x = diag_value(pi, cdl, N, q, t);
+      v += (x - m) * (x - m);
+      if (t < n && var1) v1 += (x - m1) * (x - m1);
+      if (t >= T - n && var2) v2 += (x - m2) * (x - m2);
+    }
+  ps[0] = v; ps[1024] = v1; ps[2048] = v2;
+  __syncthreads();
+  if (w == 0 && valid) {
+    double V = 0.0, V1 = 0.0, V2 = 0.0;
+    for (int u = 0; u < 32; u++) {
+      const double *p = sbuf + u * 32 + lane;
+      V += p[0]; V1 += p[1024]; V2 += p[2048];
+    }
+    out[0] = m; out[1] = V / (T - 1);
+    hv[0] = m1; hv[1] = V1 / (n - 1); hv[2] = m2; hv[3] = V2 / (n - 1);
+  }
+
+  /* autocovariances: warp w owns quantity q0 + w; lane l sums (x_t - m)(x_{t+k} - m) for k = k0 + l over t < T - k0 in t order */
+  const int L = (max_lag > 0 && max_lag < T) ? max_lag : T;
+  const int qw = q0 + w;
+  bool on = s_on[w] != 0;
+  double g0 = 0.0, psum = 0.0, pprev = INFINITY;
+  int lags = 0;
+  double *sA = sbuf, *sB = sbuf + 32 * SER_DIAG_SA;
+  for (int k0 = 0;; k0 += 32) {
+    if (lane == 0) s_act[w] = on;
+    if (!__syncthreads_or(on)) break;
+    double acc = 0.0;
+    const int span = T - k0;
+    for (int t0 = 0; t0 < span; t0 += SER_DIAG_TC) {
+      __syncthreads();
+      for (int e = threadIdx.x; e < 32 * SER_DIAG_TC; e += 1024) {
+        const int t = t0 + (e >> 5), j = e & 31;
+        sA[j * SER_DIAG_SA + (e >> 5)] = (s_act[j] && t < T) ? diag_value(pi, cdl, N, q0 + j, t) - s_mean[j] : 0.0;
+      }
+      for (int e = threadIdx.x; e < 32 * (SER_DIAG_TC + 32); e += 1024) {
+        const int t = t0 + k0 + (e >> 5), j = e & 31;
+        sB[j * SER_DIAG_SB + (e >> 5)] = (s_act[j] && t < T) ? diag_value(pi, cdl, N, q0 + j, t) - s_mean[j] : 0.0;
+      }
+      __syncthreads();
+      if (on) {
+        const double *a = sA + w * SER_DIAG_SA, *b = sB + w * SER_DIAG_SB + lane;
+        const int nt = min(SER_DIAG_TC, span - t0);
+        for (int t = 0; t < nt; t++) acc = fma(a[t], b[t], acc);
+      }
+    }
+    if (on) { /* Geyer's initial monotone sequence over this block's 16 pairs; every lane follows it, so `on` stays warp-uniform */
+      if (k0 == 0) g0 = __shfl_sync(0xffffffffu, acc, 0) / T;
+      for (int i = 0; i < 16; i++) {
+        const double r0 = __shfl_sync(0xffffffffu, acc, 2 * i) / T / g0, r1 = __shfl_sync(0xffffffffu, acc, 2 * i + 1) / T / g0;
+        if (k0 + 2 * i + 1 >= L) { on = false; break; } /* the pair needs both lags below L */
+        double P = r0 + r1;
+        if (!(P > 0.0)) { on = false; break; }
+        P = fmin(P, pprev);
+        pprev = P; psum += P; lags += 2;
+      }
+      if (k0 + 33 >= L) on = false;
+    }
+  }
+  if (lane == 0 && qw >= qlo && qw < qhi) {
+    double *o = stats + ((size_t)c * Q + qw) * 4;
+    const bool defined = s_on[w] != 0;
+    o[2] = defined ? T / fmax(-1.0 + 2.0 * psum, 1.0 / log10((double)T)) : NaN;
+    o[3] = defined ? (double)lags : 0.0;
+  }
+}
+
 /* ------------------------------------------------------------------ streaming accumulators (ser_run_accumulate)
  * On an accumulating run the sample store is a window of max_samples rows per chain.  After every sweep launch of w
  * sampling calls these kernels add rows [0, w) of EVERY local chain's window into per-chain totals; the getters below

@@ -358,6 +358,36 @@ int ser_po_finalize(const int32_t *counts, int32_t k, int32_t N, int32_t chains_
   return SER_OK;
 }
 
+/* split-R-hat (BDA3 section 11.4) from the half-sequences ser_run_diagnostics reports: halves [k][Q][4] = mean1, var1, mean2, var2 */
+int ser_split_rhat(const double *halves, const int32_t *n_samples, int32_t k, int32_t Q, double *rhat)
+{
+  if (!halves || !n_samples || !rhat || k < 1 || Q < 1) { ser_set_error("ser_split_rhat: bad argument (k = %d, Q = %d)", k, Q); return SER_E_ARG; }
+  for (int32_t c = 1; c < k; c++)
+    if (n_samples[c] != n_samples[0]) {
+      ser_set_error("ser_split_rhat: the chains hold different numbers of samples (%d vs %d)", n_samples[0], n_samples[c]);
+      return SER_E_ARG;
+    }
+  if (n_samples[0] < 4) { ser_set_error("ser_split_rhat: %d samples per chain (at least 4 are needed)", n_samples[0]); return SER_E_ARG; }
+  const double n = (double)(n_samples[0] / 2), m = 2.0 * k;
+  for (int32_t q = 0; q < Q; q++) {
+    double W = 0.0, mean = 0.0, B = 0.0;
+    for (int32_t c = 0; c < k; c++) {
+      const double *h = halves + ((size_t)c * Q + q) * 4;
+      W += h[1] + h[3];
+      mean += h[0] + h[2];
+    }
+    W /= m;
+    mean /= m;
+    for (int32_t c = 0; c < k; c++) {
+      const double *h = halves + ((size_t)c * Q + q) * 4;
+      B += (h[0] - mean) * (h[0] - mean) + (h[2] - mean) * (h[2] - mean);
+    }
+    B /= m - 1.0; /* B / n */
+    rhat[q] = W > 0.0 ? sqrt(((n - 1.0) / n * W + B) / W) : NAN;
+  }
+  return SER_OK;
+}
+
 /* ------------------------------------------------------------------ Chains/chain_XX writers */
 int ser_write_chain_files(ser_run *run, int32_t chain, const char *dir)
 {

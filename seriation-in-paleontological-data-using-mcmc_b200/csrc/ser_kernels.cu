@@ -1425,6 +1425,60 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
   return common_samples(n_out, n_samples, "ser_run_alive_counts");
 }
 
+extern "C" int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, int32_t max_lag, double *stats,
+                                   double *halves, int32_t *n_samples)
+{
+  if (!run || !chosen || !stats || !halves || !n_samples || k < 1 || what < 1 || what > 3 || max_lag < 0) {
+    ser_set_error("ser_run_diagnostics: bad argument (k = %d, what = %d, max_lag = %d)", k, what, max_lag);
+    return SER_E_ARG;
+  }
+  if (!run->initialized) { ser_set_error("ser_run_diagnostics: run not initialised"); return SER_E_STATE; }
+  if (run->acc_what) { ser_set_error("ser_run_diagnostics: the store of an accumulating run is a transient window"); return SER_E_STATE; }
+  if ((what & SER_DIAG_SCALARS) && run->cfg.store < SER_STORE_FULL) {
+    ser_set_error("ser_run_diagnostics: -loglik, exp(c), exp(d) need SER_STORE_FULL");
+    return SER_E_STATE;
+  }
+  if ((what & SER_DIAG_SITES) && run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_diagnostics: pi needs SER_STORE_PI"); return SER_E_STATE; }
+  if (set_device(run)) return SER_E_CUDA;
+  const int Q = 3 + run->N, qlo = (what & SER_DIAG_SCALARS) ? 0 : 3, qhi = (what & SER_DIAG_SITES) ? Q : 3;
+  const size_t cells = (size_t)k * Q * 4;
+  int *d_ch = nullptr, *d_n = nullptr;
+  double *d_stats = nullptr, *d_halves = nullptr;
+  std::vector<int> n_out(k);
+  auto body = [&]() -> int {
+    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
+    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
+    CUDA_TRY(POOL_ALLOC(&d_stats, cells * sizeof(double)));
+    CUDA_TRY(POOL_ALLOC(&d_halves, cells * sizeof(double)));
+    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_stats, stats, cells * sizeof(double), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_halves, halves, cells * sizeof(double), cudaMemcpyHostToDevice, run->stream));
+    mark_launch(run);
+    ser_diag_kernel<<<dim3(k, (qhi - 1) / 32 - qlo / 32 + 1), 1024, 0, run->stream>>>(
+        run->d_samp_pi, run->d_samp_cdl, run->d_scal, run->N, run->cfg.max_samples, d_ch, run->cfg.chain_offset, run->cfg.n_chains,
+        run->d_chain_ids, qlo, qhi, max_lag, d_stats, d_halves, d_n);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    for (int c = 0; c < k; c++)
+      if (n_out[c] >= 0 && n_out[c] < 4) {
+        ser_set_error("ser_run_diagnostics: chain %d holds %d stored samples (at least 4 are needed)", chosen[c], n_out[c]);
+        return SER_E_STATE;
+      }
+    CUDA_TRY(cudaMemcpyAsync(stats, d_stats, cells * sizeof(double), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaMemcpyAsync(halves, d_halves, cells * sizeof(double), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    for (int c = 0; c < k; c++)
+      if (n_out[c] >= 0) n_samples[c] = n_out[c];
+    return SER_OK;
+  };
+  const int rc = body();
+  void *tmp[] = {d_ch, d_n, d_stats, d_halves};
+  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
+  return rc;
+}
+
 /* ------------------------------------------------------------------ the cross-chain step on one stream
  * stats -> (all-gather) -> selection -> zero counts -> pair-order slabs -> (all-reduce): six enqueues, no host
  * synchronisation (script.py:70-99 + :155-189 over run_all_chains' chains, :48-67). */
