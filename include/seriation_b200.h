@@ -216,6 +216,23 @@ int ser_split_rhat(const double *halves, const int32_t *n_samples, int32_t k, in
  * and plot_false_ones_probability (script.py:306-448): alive, T - alive, X * (T - alive). */
 int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t k, int32_t *alive, int32_t *n_samples);
 
+/* Posterior marginals (DESIGN.md section 3.8).  For chosen chain c over its T samples t (T = that chain's own count):
+ *   pos[c][i][p]    = #{t : pi_t(i) = p}   site i in file order, position p in [0, N); every row sums to T    (needs SER_STORE_PI)
+ *   a_hist[c][m][j] = #{t : a_t(m) = j}    taxon m in file order, j in [0, N] (N + 1 bins); b_hist likewise (need SER_STORE_FULL)
+ * a and b are the sampler's half-open range: taxon m is alive at positions a <= pos < b.  Exact integer identities:
+ *   sum_p p * pos[c][i][p] == pi_sum[c][i] and sum_j j * a_hist[c][m][j] == a_sum[c][m] (b alike) of ser_run_posterior_sums.
+ * Counts add over windows, chains and devices.  Chosen ids are GLOBAL; -1 or a chain this run does not hold leaves its slabs untouched
+ * and n_samples[c] = 0; a held chain's slabs are written in full.  Host memory: pos [k][N][N], a_hist / b_hist [k][M][N+1] int32, any
+ * of the three may be NULL.  On an accumulating run (SER_ACC_POS / SER_ACC_RANGE) T counts every sample taken since accumulation began.
+ * Checked before any CUDA call: SER_E_ARG for k < 1, a NULL chosen or n_samples, or all three outputs NULL; SER_E_STATE for a store
+ * below what a requested output needs, an accumulating run without the flag of a requested output, or a run not initialised. */
+int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k, int32_t *pos, int32_t *a_hist, int32_t *b_hist,
+                      int32_t *n_samples);
+/* Quantiles of histograms (host only, no CUDA call): out[r][q] = the smallest bin b with sum_{j <= b} hist[r][j] >= probs[q] * total_r
+ * (the inverse of the empirical CDF, numpy's "inverted_cdf"), -1 for a row whose total is 0.  hist [rows][bins], out [rows][n_probs].
+ * SER_E_ARG: rows < 1, bins < 1, n_probs < 1, a NULL pointer, or a probability outside (0, 1] (NaN included). */
+int ser_hist_quantiles(const int32_t *hist, int32_t rows, int32_t bins, const double *probs, int32_t n_probs, int32_t *out);
+
 /* CORR_MN (Docs/Report.pdf Table 1; SURVEY section 8f #3): Pearson correlation of the posterior mean
  * position E[pi(site)] over the stored samples of the chosen chains owned by this run with the MN age
  * of the site read from the .sites file (ser_dataset_read_names): the mean over the stored samples of
@@ -232,15 +249,17 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
 #define SER_ACC_SUMS 2  /* pi_sum [n][N] int32 (corr_num is derived from it on the way out)                */
 #define SER_ACC_AB 4    /* a_sum, b_sum                 [n][M] int32 each   (needs SER_STORE_FULL)           */
 #define SER_ACC_ALIVE 8 /* alive difference slab        [n][N][M] int32     (needs SER_STORE_FULL)           */
+#define SER_ACC_POS 16  /* position histograms          [n][N][N] int32     (ser_run_marginals' pos)          */
+#define SER_ACC_RANGE 32 /* a and b histograms          [n][2][M][N+1] int32 (needs SER_STORE_FULL)           */
 /* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
  * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
  * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),
- * ser_run_posterior_sums, ser_run_alive_counts and ser_run_site_age_corr then return totals over EVERY sample taken since
+ * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals and ser_run_site_age_corr then return totals over EVERY sample taken since
  * (T = the chain's sample count), with the usual global ids and slab convention; ser_run_fetch_samples /
  * ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does ser_run_cross_chain_async.
  * Call it before the first sampling call (ser_run_init zeroes the accumulators).  Errors: SER_E_STATE on a run that has
  * already sampled, on a store below what the flags need, or a second time; SER_E_ARG for max_samples < 1; SER_E_CUDA with
- * the byte count when an accumulator does not fit (the alive slab at 2048 x 8192 is 64 MB per chain). */
+ * the byte count when an accumulator does not fit (per chain at 2048 x 8192: the alive slab is 64 MB, the a / b histograms 134 MB). */
 int ser_run_accumulate(ser_run *run, int32_t what);
 
 /* ---------------------------------------------------------------- cross-chain step, one call

@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
-ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE = 1, 2, 4, 8
+ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE = 1, 2, 4, 8, 16, 32
 DIAG_SCALARS, DIAG_SITES = 1, 2
 
 _i32p, _dp, _u8p = C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_uint8)
@@ -82,6 +82,8 @@ SYMBOLS = [
     ("ser_run_posterior_sums", C.c_int, [_vp, _i32p, C.c_int32, _i64p, _i32p, _i32p, _i32p, _i32p]),
     ("ser_run_diagnostics", C.c_int, [_vp, _i32p, C.c_int32, C.c_int32, C.c_int32, _dp, _dp, _i32p]),
     ("ser_split_rhat", C.c_int, [_dp, _i32p, C.c_int32, C.c_int32, _dp]),
+    ("ser_run_marginals", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p]),
+    ("ser_hist_quantiles", C.c_int, [_i32p, C.c_int32, C.c_int32, _dp, C.c_int32, _i32p]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
     ("ser_write_labelled_files", C.c_int, [_vp, C.c_int32, _vp, C.c_char_p]),
     ("ser_microbench", C.c_int, [C.c_int32, _dp]),
@@ -236,10 +238,12 @@ class Run:
             _check(lib().ser_run_create_chains(ds._h, C.byref(self.cfg), _p(ids, C.c_int32), ids.size, C.byref(h)))
         self._h = h
 
-    def accumulate(self, po=True, sums=True, ab=False, alive=False):
+    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False):
         """from now on the sample store is a window of max_samples rows and the summaries sum over every sample taken
-        afterwards (ser_run_accumulate); call before the first sampling call"""
+        afterwards (ser_run_accumulate); call before the first sampling call.  ``positions`` / ``ranges`` accumulate the
+        histograms of marginals()"""
         what = (ACC_PO if po else 0) | (ACC_SUMS if sums else 0) | (ACC_AB if ab else 0) | (ACC_ALIVE if alive else 0)
+        what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0)
         _check(lib().ser_run_accumulate(self._h, what))
         return self
 
@@ -409,6 +413,20 @@ class Run:
         held = n > 0
         rhat = split_rhat(halves[held], n[held]) if held.any() and np.all(n[held] == n[held][0]) else None
         return dict(mean=stats[..., 0], var=stats[..., 1], ess=stats[..., 2], lags=stats[..., 3], halves=halves, n_samples=n, rhat=rhat)
+
+    def marginals(self, chosen, ranges: bool = False, positions: bool = True) -> dict:
+        """histograms of the chosen chains (global ids) over their samples (ser_run_marginals): ``pos`` [k][N][N] = #{t: pi_t(i) = p},
+        and with ``ranges`` ``a`` / ``b`` [k][M][N+1] = #{t: a_t(m) = j}; ``n_samples`` [k] = T.  Slabs the run does not fill stay 0
+        (n_samples 0)."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        k, N, M = len(chosen), self.N, self.M
+        pos = np.zeros((k, N, N), np.int32) if positions else None
+        a = np.zeros((k, M, N + 1), np.int32) if ranges else None
+        b = np.zeros((k, M, N + 1), np.int32) if ranges else None
+        n = np.zeros(k, np.int32)
+        _check(lib().ser_run_marginals(self._h, _p(chosen, C.c_int32), k, _p(pos, C.c_int32), _p(a, C.c_int32), _p(b, C.c_int32),
+                                       _p(n, C.c_int32)))
+        return dict(pos=pos, a=a, b=b, n_samples=n)
 
     def po_counts_device(self, chosen_ptr: int, k: int, counts_ptr: int):
         _check(lib().ser_run_po_counts_device(self._h, chosen_ptr, k, counts_ptr))
@@ -592,6 +610,18 @@ def split_rhat(halves, n_samples) -> np.ndarray:
     return out
 
 
+def hist_quantiles(hist, probs) -> np.ndarray:
+    """per row of ``hist`` [..., bins] the smallest bin whose cumulative count reaches p * total for each p in ``probs``
+    (numpy's "inverted_cdf"; -1 for an empty row), [..., len(probs)] (ser_hist_quantiles, host only)"""
+    h = np.ascontiguousarray(hist, dtype=np.int32)
+    p = np.ascontiguousarray(np.atleast_1d(probs), dtype=np.float64)
+    bins = h.shape[-1]
+    rows = h.size // bins if bins else 0
+    out = np.empty(h.shape[:-1] + (p.size,), np.int32)
+    _check(lib().ser_hist_quantiles(_p(h, C.c_int32), rows, bins, _p(p, C.c_double), p.size, _p(out, C.c_int32)))
+    return out
+
+
 def select_chains_device(e_ptr: int, n: int, k: int, chosen_ptr: int, info_ptr: int, device=0, stream=None):
     _check(lib().ser_select_chains_device(e_ptr, n, k, chosen_ptr, info_ptr, device, stream))
 
@@ -653,22 +683,24 @@ def choose_chains(batch: ChainBatch, chains_selected: int):
     return [int(c) for c in chosen]
 
 
-def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, device=None) -> ChainBatch:
+def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, marginals: bool = False,
+                  device=None) -> ChainBatch:
     """The second phase of select-then-replay: re-simulate the chosen chains of a batch (typically one run with
     ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
     ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
     run's, so compute_pair_order_matrix, compute_exp_* and the probability maps work on it unchanged.  ``with_ab``
     also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  ``window=0`` keeps every
     sample instead (``STORE_FULL``, no accumulators): the summaries take the one-shot path and ``diagnostics`` works on
-    the result.  Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
+    the result.  ``marginals`` also accumulates the position and a/b histograms of marginals() (the window then keeps a and b).
+    Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
     ids = np.ascontiguousarray(chains, dtype=np.int32)
     keep_all = window == 0
     run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
-              store=STORE_FULL if (with_ab or keep_all) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
+              store=STORE_FULL if (with_ab or keep_all or marginals) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
               device=batch.run.cfg.device if device is None else device, chain_ids=ids)
     run.init()
     if not keep_all:
-        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab)
+        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals)
     run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
     want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
     if want.tobytes() != got.tobytes():
@@ -692,6 +724,29 @@ def diagnostics(batch: ChainBatch, chains, max_lag: int = 0) -> dict:
     full sample store (their rows stay NaN otherwise).  A batch from replay_chosen(..., window=0) keeps it."""
     run = batch.run
     return run.diagnostics(np.asarray(chains, dtype=np.int32), scalars=run.cfg.store >= STORE_FULL, max_lag=max_lag)
+
+
+def _marginal_summary(hist, probs):
+    """mean, quantiles [rows][len(probs)], mode and P(mode) of every row of pooled counts [rows][bins]"""
+    total = hist.sum(axis=1, dtype=np.int64)
+    mean = (hist.astype(np.int64) @ np.arange(hist.shape[1], dtype=np.int64)) / total
+    mode = hist.argmax(axis=1)
+    return dict(mean=mean, quantiles=hist_quantiles(hist, probs), mode=mode, p_mode=hist[np.arange(len(hist)), mode] / total)
+
+
+def marginals(batch: ChainBatch, chains, probs=(0.025, 0.5, 0.975)) -> dict:
+    """Posterior marginals pooled over the chosen chains by summing their counts: per site (file order) the position's ``mean``,
+    ``quantiles`` [N][len(probs)], ``mode`` and ``p_mode``, in ``sites``; per taxon the same for a and for b, in ``a`` and ``b``
+    (None unless the batch keeps a and b: the full sample store, or replay_chosen(..., marginals=True)).  ``probs`` are inverse-CDF
+    quantiles (hist_quantiles); ``counts`` holds the pooled histograms and ``n_samples`` the pooled sample count."""
+    run = batch.run
+    ranges = run.cfg.store >= STORE_FULL
+    m = run.marginals(np.asarray(chains, dtype=np.int32), ranges=ranges)
+    pooled = {key: (m[key].sum(axis=0, dtype=np.int64).astype(np.int32) if m[key] is not None else None) for key in ("pos", "a", "b")}
+    return dict(sites=_marginal_summary(pooled["pos"], probs),
+                a=_marginal_summary(pooled["a"], probs) if ranges else None,
+                b=_marginal_summary(pooled["b"], probs) if ranges else None,
+                counts=pooled, n_samples=int(m["n_samples"].sum()), probs=tuple(probs))
 
 
 def compute_exp_cd(batch: ChainBatch, chains, chains_selected: int, faithful: bool = True):

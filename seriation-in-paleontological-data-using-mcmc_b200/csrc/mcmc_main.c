@@ -17,7 +17,7 @@
  * sharded over the GPUs of the box -- ser_multi_*):
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
- *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE]
+ *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--marginals PREFIX]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
@@ -31,6 +31,11 @@
  * --diagnostics FILE (with --select) re-simulates the chosen chains alone keeping every sample (SER_STORE_FULL, bit-identical to
  * their first run, which is checked), writes per-quantity split-R-hat and effective sample sizes to FILE and prints one summary
  * line; under --replay-selected --po the same run supplies the pair-order counts.
+ * --marginals PREFIX (with --select) re-simulates the chosen chains alone through a window of W samples (--window, default 64) while
+ * their position and a / b histograms accumulate (bit-identical to their first run, which is checked), pools the counts over the
+ * chains and writes PREFIX.sites.csv "site,hard,mean,q025,median,q975,mode,p_mode" (file order, 0-based positions) and
+ * PREFIX.taxa.csv "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975", and prints one summary line; under
+ * --replay-selected --po (without --diagnostics) the same run supplies the pair-order counts, so the chains are replayed once.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -59,7 +64,9 @@ static void usage(const char *argv0)
           "              [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]]\n"
           "                  (save every chain to FILE at the end and every C calls; --resume continues FILE's run; --stop-after C\n"
           "                   advances at most C calls, saves and exits)\n"
-          "              [--diagnostics FILE]   (with --select: split-R-hat and ESS of the chosen chains to FILE)\n",
+          "              [--diagnostics FILE]   (with --select: split-R-hat and ESS of the chosen chains to FILE)\n"
+          "              [--marginals PREFIX]   (with --select: position and a / b credible intervals of the chosen chains to\n"
+          "                                      PREFIX.sites.csv and PREFIX.taxa.csv; the replay uses --window W)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -132,6 +139,107 @@ static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg,
   free(e2); free(stats); free(halves); free(rhat); free(n);
 }
 
+/* mean, 2.5 / 50 / 97.5 % quantiles, mode and P(mode) of one row of pooled counts */
+struct marginal {
+  double mean, p_mode;
+  int32_t q[3], mode;
+};
+static void summarise(const int32_t *h, int32_t bins, struct marginal *out)
+{
+  static const double probs[3] = {0.025, 0.5, 0.975};
+  int64_t total = 0, num = 0;
+  int32_t j;
+  out->mode = 0;
+  for (j = 0; j < bins; j++) {
+    total += h[j];
+    num += (int64_t)j * h[j];
+    if (h[j] > h[out->mode]) out->mode = j;
+  }
+  out->mean = (double)num / (double)total;
+  out->p_mode = (double)h[out->mode] / (double)total;
+  if (ser_hist_quantiles(h, 1, bins, probs, 3, out->q)) die("ser_hist_quantiles");
+}
+
+static int cmp_double(const void *x, const void *y)
+{
+  const double a = *(const double *)x, b = *(const double *)y;
+  return a < b ? -1 : a > b;
+}
+
+/* median width q97.5 - q2.5 of n marginals (sorts w) */
+static double median_width(const struct marginal *m, int32_t n, double *w)
+{
+  int32_t i;
+  for (i = 0; i < n; i++) w[i] = m[i].q[2] - m[i].q[0];
+  qsort(w, (size_t)n, sizeof(double), cmp_double);
+  return n % 2 ? w[n / 2] : 0.5 * (w[n / 2 - 1] + w[n / 2]);
+}
+
+/* --marginals: the chosen chains re-simulated alone through a window of W samples while their position and a / b histograms accumulate
+ * (bit-identical to their first run, whose E[-logL] per global id - first is e[]; any difference exits 1), the counts pooled over the
+ * chains, PREFIX.sites.csv and PREFIX.taxa.csv written and one summary line printed.  `counts` (NULL: not wanted) receives their
+ * pair-order counts from the same run. */
+static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
+                             int burn, int samples, int window, int32_t *counts, const char *prefix)
+{
+  ser_run_config c2 = *cfg;
+  ser_run *sub = NULL;
+  int32_t N, M, nh, ns = 0, i, c, tot = 0;
+  size_t j;
+  char path[4096];
+  FILE *f;
+  ser_dataset_dims(ds, &N, &M, &nh);
+  const size_t NN = (size_t)N * N, MB = (size_t)M * (N + 1);
+  int32_t *pos = (int32_t *)malloc(sizeof(int32_t) * k * NN), *ah = (int32_t *)malloc(sizeof(int32_t) * k * MB);
+  int32_t *bh = (int32_t *)malloc(sizeof(int32_t) * k * MB), *n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k);
+  double *e2 = (double *)malloc(sizeof(double) * (size_t)k), *w = (double *)malloc(sizeof(double) * (size_t)(N > M ? N : M));
+  struct marginal *ms = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)N);
+  struct marginal *ma = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)M), *mb = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)M);
+  uint8_t *hard = (uint8_t *)malloc((size_t)N);
+  if (!pos || !ah || !bh || !n || !e2 || !w || !ms || !ma || !mb || !hard) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  c2.n_chains = k;
+  c2.chain_offset = 0;
+  c2.store = SER_STORE_FULL;
+  c2.max_samples = window;
+  if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
+  if (ser_run_init(sub) || ser_run_accumulate(sub, SER_ACC_POS | SER_ACC_RANGE | (counts ? SER_ACC_PO : 0))) die("ser_run_accumulate");
+  if (ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
+  if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
+  for (i = 0; i < k; i++)
+    if (memcmp(&e2[i], &e[chosen[i] - first], sizeof(double))) {
+      fprintf(stderr, "mcmc: the replayed chain %d does not reproduce its first run (E[-logL] %.17g vs %.17g)\n", chosen[i], e2[i],
+              e[chosen[i] - first]);
+      exit(1);
+    }
+  if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
+  if (ser_run_marginals(sub, chosen, k, pos, ah, bh, n)) die("ser_run_marginals");
+  ser_run_destroy(sub);
+  for (c = 1; c < k; c++) { /* pool the chains' counts into chain 0's slabs */
+    for (j = 0; j < NN; j++) pos[j] += pos[c * NN + j];
+    for (j = 0; j < MB; j++) { ah[j] += ah[c * MB + j]; bh[j] += bh[c * MB + j]; }
+  }
+  for (c = 0; c < k; c++) tot += n[c];
+  for (i = 0; i < N; i++) summarise(pos + (size_t)i * N, N, &ms[i]);
+  for (i = 0; i < M; i++) { summarise(ah + (size_t)i * (N + 1), N + 1, &ma[i]); summarise(bh + (size_t)i * (N + 1), N + 1, &mb[i]); }
+  ser_dataset_get(ds, NULL, hard);
+  snprintf(path, sizeof(path), "%s.sites.csv", prefix);
+  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  fprintf(f, "site,hard,mean,q025,median,q975,mode,p_mode\n");
+  for (i = 0; i < N; i++)
+    fprintf(f, "%d,%d,%.6f,%d,%d,%d,%d,%.6f\n", i, hard[i] != 0, ms[i].mean, ms[i].q[0], ms[i].q[1], ms[i].q[2], ms[i].mode, ms[i].p_mode);
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  snprintf(path, sizeof(path), "%s.taxa.csv", prefix);
+  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  fprintf(f, "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975\n");
+  for (i = 0; i < M; i++)
+    fprintf(f, "%d,%.6f,%d,%d,%d,%.6f,%d,%d,%d\n", i, ma[i].mean, ma[i].q[0], ma[i].q[1], ma[i].q[2], mb[i].mean, mb[i].q[0], mb[i].q[1],
+            mb[i].q[2]);
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  printf("marginals: %d chains  %d samples  median width of the 95%% intervals: sites %.1f  a %.1f  b %.1f positions\n", k, tot,
+         median_width(ms, N, w), median_width(ma, M, w), median_width(mb, M, w));
+  free(pos); free(ah); free(bh); free(n); free(e2); free(w); free(ms); free(ma); free(mb); free(hard);
+}
+
 static double *read_tape(const char *path, uint64_t *len)
 {
   FILE *f = fopen(path, "rb");
@@ -155,7 +263,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
-  const char *diag_path = NULL;
+  const char *diag_path = NULL, *marg_prefix = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -190,6 +298,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--window")) window = atoi(v);
       else if (!strcmp(a, "--checkpoint")) ckpt_path = v;
       else if (!strcmp(a, "--diagnostics")) diag_path = v;
+      else if (!strcmp(a, "--marginals")) marg_prefix = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
@@ -198,6 +307,7 @@ int main(int argc, char **argv)
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
     if (diag_path && select_k < 1) usage(argv[0]);
+    if (marg_prefix && (select_k < 1 || window < 1)) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
@@ -328,7 +438,7 @@ int main(int argc, char **argv)
         /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0 && !diag_path) {
+        if (counts && nchosen > 0 && !diag_path && !marg_prefix) {
           ser_run_config c2 = cfg;
           ser_run *sub = NULL;
           c2.n_chains = nchosen;
@@ -351,6 +461,9 @@ int main(int argc, char **argv)
       }
       if (diag_path && nchosen > 0)
         replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path);
+      if (marg_prefix && nchosen > 0)
+        replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window, (replay_selected && !diag_path) ? counts : NULL,
+                         marg_prefix);
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);
         FILE *f;

@@ -447,6 +447,62 @@ __global__ void __launch_bounds__(1024, 1) ser_diag_kernel(const uint16_t *samp_
   }
 }
 
+/* ------------------------------------------------------------------ posterior marginals (ser_run_marginals, DESIGN.md 3.8)
+ * Histogram of item r over T samples: h[r][v] = #{t : x[t * stride + r] = v}, v in [0, bins).  pi: items = sites, stride N, N bins;
+ * a, b: items = taxa (file order, as stored), stride M, N + 1 bins.  One thread owns one item's row, so no atomics are needed; the
+ * loads of a sample row are coalesced (consecutive items are consecutive uint16_t).  The block's rows [r0, r0 + blockDim.x) are
+ * contiguous in a [items][bins] slab: they are zeroed and written out as one coalesced span.  With s_rows (blockDim.x * bins ints
+ * of dynamic shared memory) the counts are kept there; without, in the slab itself. */
+__device__ void hist_tile(const uint16_t *x, int stride, int items, int bins, int T, int r0, int *slab, int *s_rows, bool add)
+{
+  const int nt = blockDim.x, n = min(nt, items - r0);
+  const size_t cells = (size_t)n * bins;
+  int *dst = slab + (size_t)r0 * bins, *h = s_rows ? s_rows : dst;
+  if (s_rows || !add) {
+    for (size_t e = threadIdx.x; e < cells; e += nt) h[e] = 0;
+    __syncthreads();
+  }
+  if ((int)threadIdx.x < n) {
+    int *row = h + (size_t)threadIdx.x * bins;
+    const uint16_t *col = x + r0 + threadIdx.x;
+    for (int t = 0; t < T; t++) row[col[(size_t)t * stride]]++;
+  }
+  if (s_rows) {
+    __syncthreads();
+    for (size_t e = threadIdx.x; e < cells; e += nt) dst[e] = add ? dst[e] + h[e] : h[e];
+  }
+}
+
+/* pos [k][N][N]: per chosen chain (blockIdx.x) the position histogram of every site over its stored samples; a chain this run does
+ * not hold (or -1) leaves its slab untouched, a held chain's slab is written in full.  n_out[c] = T of a held chain. */
+__global__ void ser_pos_hist_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, const int *chosen,
+                                    int chain_offset, int n_local, const int *ids, int use_smem, int *pos, int *n_out)
+{
+  extern __shared__ int s_hist[];
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int T = stored_samples(scal, local, max_samples);
+  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = T;
+  hist_tile(samp_pi + (size_t)local * max_samples * N, N, N, N, T, blockIdx.y * blockDim.x, pos + (size_t)blockIdx.x * N * N,
+            use_smem ? s_hist : nullptr, false);
+}
+
+/* a_hist / b_hist [k][M][N+1] (blockIdx.z = 0 / 1; either may be nullptr): per chosen chain the histograms of every taxon's a and b */
+__global__ void ser_range_hist_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
+                                      const int *chosen, int chain_offset, int n_local, const int *ids, int use_smem, int *a_hist,
+                                      int *b_hist, int *n_out)
+{
+  extern __shared__ int s_hist[];
+  int *out = blockIdx.z ? b_hist : a_hist;
+  if (!out) return;
+  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  if (local < 0) return;
+  const int T = stored_samples(scal, local, max_samples);
+  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = T;
+  const uint16_t *x = (blockIdx.z ? samp_b : samp_a) + (size_t)local * max_samples * M;
+  hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, out + (size_t)blockIdx.x * M * (N + 1), use_smem ? s_hist : nullptr, false);
+}
+
 /* ------------------------------------------------------------------ streaming accumulators (ser_run_accumulate)
  * On an accumulating run the sample store is a window of max_samples rows per chain.  After every sweep launch of w
  * sampling calls these kernels add rows [0, w) of EVERY local chain's window into per-chain totals; the getters below
@@ -517,7 +573,47 @@ __global__ void ser_alive_accum_kernel(const uint16_t *samp_a, const uint16_t *s
   }
 }
 
+/* position histograms of the window's rows of every local chain (blockIdx.x) added into acc [n_local][N][N] */
+__global__ void ser_pos_hist_accum_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, int sample_base, int w,
+                                          int use_smem, int *acc)
+{
+  extern __shared__ int s_hist[];
+  const int local = blockIdx.x;
+  const int T = window_rows(scal, local, sample_base, w);
+  if (T == 0) return;
+  hist_tile(samp_pi + (size_t)local * max_samples * N, N, N, N, T, blockIdx.y * blockDim.x, acc + (size_t)local * N * N,
+            use_smem ? s_hist : nullptr, true);
+}
+
+/* a (blockIdx.z = 0) and b (1) histograms of the window's rows added into acc [n_local][2][M][N+1] */
+__global__ void ser_range_hist_accum_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M,
+                                            int max_samples, int sample_base, int w, int use_smem, int *acc)
+{
+  extern __shared__ int s_hist[];
+  const int local = blockIdx.x;
+  const int T = window_rows(scal, local, sample_base, w);
+  if (T == 0) return;
+  const size_t slab = (size_t)M * (N + 1);
+  const uint16_t *x = (blockIdx.z ? samp_b : samp_a) + (size_t)local * max_samples * M;
+  hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, acc + ((size_t)local * 2 + blockIdx.z) * slab, use_smem ? s_hist : nullptr, true);
+}
+
 /* getters of an accumulating run: the slab of every chosen chain the run holds, T = all samples taken since accumulation began */
+/* slab part [part * cells, (part + 1) * cells) of a local chain's accumulator of `per_chain` ints into out [k][cells] (nullptr: not
+ * wanted); blockIdx.y = chosen chain, blockIdx.z = part */
+__global__ void ser_hist_acc_out_kernel(const int *acc, size_t per_chain, size_t cells, const ChainScalars *scal, const int *chosen,
+                                        int chain_offset, int n_local, const int *ids, int *out0, int *out1, int *n_out)
+{
+  int *out = blockIdx.z ? out1 : out0;
+  if (!out) return;
+  const int local = local_chain(chosen[blockIdx.y], chain_offset, n_local, ids);
+  if (local < 0) return;
+  if (blockIdx.x == 0 && threadIdx.x == 0) n_out[blockIdx.y] = scal[local].n_samples;
+  const int *src = acc + local * per_chain + blockIdx.z * cells;
+  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < cells; q += (size_t)gridDim.x * blockDim.x)
+    out[blockIdx.y * cells + q] = src[q];
+}
+
 __global__ void ser_po_acc_out_kernel(const int *acc, const ChainScalars *scal, int N, const int *chosen, int chain_offset, int n_local,
                                       const int *ids, int *counts)
 {

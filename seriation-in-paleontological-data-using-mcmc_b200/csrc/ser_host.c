@@ -359,6 +359,36 @@ int ser_po_finalize(const int32_t *counts, int32_t k, int32_t N, int32_t chains_
 }
 
 /* split-R-hat (BDA3 section 11.4) from the half-sequences ser_run_diagnostics reports: halves [k][Q][4] = mean1, var1, mean2, var2 */
+/* inverse-CDF quantiles of integer histograms (ser_run_marginals' rows): the comparison is made in double, p * total against the
+ * running count, as numpy's searchsorted(cumsum(h), p * total) makes it */
+int ser_hist_quantiles(const int32_t *hist, int32_t rows, int32_t bins, const double *probs, int32_t n_probs, int32_t *out)
+{
+  if (!hist || !probs || !out || rows < 1 || bins < 1 || n_probs < 1) {
+    ser_set_error("ser_hist_quantiles: bad argument (rows = %d, bins = %d, n_probs = %d)", rows, bins, n_probs);
+    return SER_E_ARG;
+  }
+  for (int32_t q = 0; q < n_probs; q++)
+    if (!(probs[q] > 0.0 && probs[q] <= 1.0)) { ser_set_error("ser_hist_quantiles: probability %g is not in (0, 1]", probs[q]); return SER_E_ARG; }
+  for (int32_t r = 0; r < rows; r++) {
+    const int32_t *h = hist + (size_t)r * bins;
+    int64_t total = 0;
+    for (int32_t j = 0; j < bins; j++) total += h[j];
+    for (int32_t q = 0; q < n_probs; q++) {
+      int32_t b = -1;
+      if (total > 0) {
+        const double target = probs[q] * (double)total;
+        int64_t cum = 0;
+        for (b = 0; b < bins - 1; b++) {
+          cum += h[b];
+          if ((double)cum >= target) break;
+        }
+      }
+      out[(size_t)r * n_probs + q] = b;
+    }
+  }
+  return SER_OK;
+}
+
 int ser_split_rhat(const double *halves, const int32_t *n_samples, int32_t k, int32_t Q, double *rhat)
 {
   if (!halves || !n_samples || !rhat || k < 1 || Q < 1) { ser_set_error("ser_split_rhat: bad argument (k = %d, Q = %d)", k, Q); return SER_E_ARG; }

@@ -107,6 +107,7 @@ struct ser_run {
   /* streaming accumulators (ser_run_accumulate): SER_ACC_* flags, per local chain totals */
   int acc_what, sampled;
   int *d_acc_po, *d_acc_pi, *d_acc_a, *d_acc_b, *d_acc_alive;
+  int *d_acc_pos, *d_acc_range; /* [n][N][N] position and [n][2][M][N+1] a / b histograms */
   /* checkpoints (ser_ckpt.cuh): calls and sampling calls advanced since init, and the fingerprint of the run's dataset */
   long long calls_done;
   int samples_done;
@@ -734,16 +735,18 @@ static int acc_zero(ser_run *run)
   if (run->d_acc_a) CUDA_TRY(cudaMemsetAsync(run->d_acc_a, 0, nc * M * sizeof(int), run->stream));
   if (run->d_acc_b) CUDA_TRY(cudaMemsetAsync(run->d_acc_b, 0, nc * M * sizeof(int), run->stream));
   if (run->d_acc_alive) CUDA_TRY(cudaMemsetAsync(run->d_acc_alive, 0, nc * N * M * sizeof(int), run->stream));
+  if (run->d_acc_pos) CUDA_TRY(cudaMemsetAsync(run->d_acc_pos, 0, nc * N * N * sizeof(int), run->stream));
+  if (run->d_acc_range) CUDA_TRY(cudaMemsetAsync(run->d_acc_range, 0, nc * 2 * M * (N + 1) * sizeof(int), run->stream));
   return SER_OK;
 }
 
 extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
 {
   if (!run) { ser_set_error("ser_run_accumulate: null run"); return SER_E_ARG; }
-  if (what < 1 || (what & ~(SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE))) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
+  if (what < 1 || (what & ~(SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE))) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
   if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
   if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
-  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE)) ? SER_STORE_FULL : SER_STORE_PI;
+  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE)) ? SER_STORE_FULL : SER_STORE_PI;
   if (run->cfg.store < need) {
     ser_set_error("ser_run_accumulate: these summaries need %s", need == SER_STORE_FULL ? "SER_STORE_FULL (a, b samples)" : "SER_STORE_PI or more");
     return SER_E_STATE;
@@ -766,9 +769,11 @@ extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
   if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_a, nc * M * sizeof(int));
   if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_b, nc * M * sizeof(int));
   if (rc == SER_OK && (what & SER_ACC_ALIVE)) rc = alloc(&run->d_acc_alive, nc * N * M * sizeof(int));
+  if (rc == SER_OK && (what & SER_ACC_POS)) rc = alloc(&run->d_acc_pos, nc * N * N * sizeof(int));
+  if (rc == SER_OK && (what & SER_ACC_RANGE)) rc = alloc(&run->d_acc_range, nc * 2 * M * (N + 1) * sizeof(int));
   if (rc == SER_OK) rc = acc_zero(run);
   if (rc != SER_OK) {
-    int **bufs[] = {&run->d_acc_po, &run->d_acc_pi, &run->d_acc_a, &run->d_acc_b, &run->d_acc_alive};
+    int **bufs[] = {&run->d_acc_po, &run->d_acc_pi, &run->d_acc_a, &run->d_acc_b, &run->d_acc_alive, &run->d_acc_pos, &run->d_acc_range};
     for (int **b : bufs) if (*b) { cudaFreeAsync(*b, run->stream); *b = nullptr; }
     return rc;
   }
@@ -784,7 +789,8 @@ extern "C" void ser_run_destroy(ser_run *run)
                   run->d_scal, run->d_tape, run->d_tape_off, run->d_samp_a, run->d_samp_b, run->d_samp_pi, run->d_samp_cdl,
                   run->d_scratch_i, run->d_bad, run->d_cd4, run->d_samp_cd_all, run->d_gV, run->d_gpre, run->d_bgrp, run->d_bbat,
                   run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites, run->d_cl_off, run->d_cl_item, run->d_cl_grp,
-                  run->d_chain_ids, run->d_acc_po, run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_acc_alive};
+                  run->d_chain_ids, run->d_acc_po, run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_acc_alive, run->d_acc_pos,
+                  run->d_acc_range};
   for (void *b : bufs) if (b) cudaFreeAsync(b, run->stream);
   if (run->stream) cudaStreamSynchronize(run->stream);
   if (run->sweep_ev) {
@@ -931,6 +937,23 @@ static int launch_sweeps(ser_run *run, int burn_calls, int sample_calls)
   return SER_OK;
 }
 
+/* Block shape of a histogram kernel whose threads own rows of `bins` ints (hist_tile): 128 threads, halved down to 32 while their rows
+ * do not fit SER_HIST_SMEM bytes of shared memory; rows that do not fit even then are counted in global memory (smem = 0). */
+#define SER_HIST_SMEM (96 * 1024)
+struct HistShape {
+  int threads;
+  size_t smem;
+};
+static cudaError_t hist_shape(const void *kernel, int bins, HistShape *h)
+{
+  h->threads = 128;
+  h->smem = 0;
+  while (h->threads > 32 && (size_t)h->threads * bins * sizeof(int) > SER_HIST_SMEM) h->threads >>= 1;
+  const size_t bytes = (size_t)h->threads * bins * sizeof(int);
+  if (bytes <= SER_HIST_SMEM) h->smem = bytes;
+  return h->smem > 48 * 1024 ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SER_HIST_SMEM) : cudaSuccess;
+}
+
 /* rows [0, w) of every chain's window into the accumulators (ser_run_accumulate), on the run's stream */
 static int accumulate_window(ser_run *run, int w)
 {
@@ -950,6 +973,22 @@ static int accumulate_window(ser_run *run, int w)
     mark_launch(run);
     ser_alive_accum_kernel<<<dim3(nc, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w,
                                                                                run->d_acc_alive);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (run->acc_what & SER_ACC_POS) {
+    HistShape hs;
+    CUDA_TRY(hist_shape((const void *)ser_pos_hist_accum_kernel, N, &hs));
+    mark_launch(run);
+    ser_pos_hist_accum_kernel<<<dim3(nc, (N + hs.threads - 1) / hs.threads), hs.threads, hs.smem, run->stream>>>(
+        run->d_samp_pi, run->d_scal, N, W, base, w, hs.smem > 0, run->d_acc_pos);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (run->acc_what & SER_ACC_RANGE) {
+    HistShape hs;
+    CUDA_TRY(hist_shape((const void *)ser_range_hist_accum_kernel, N + 1, &hs));
+    mark_launch(run);
+    ser_range_hist_accum_kernel<<<dim3(nc, (M + hs.threads - 1) / hs.threads, 2), hs.threads, hs.smem, run->stream>>>(
+        run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w, hs.smem > 0, run->d_acc_range);
     CUDA_TRY(cudaGetLastError());
   }
   return SER_OK;
@@ -1423,6 +1462,89 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
   for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
   if (rc != SER_OK) return rc;
   return common_samples(n_out, n_samples, "ser_run_alive_counts");
+}
+
+extern "C" int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k, int32_t *pos, int32_t *a_hist, int32_t *b_hist,
+                                 int32_t *n_samples)
+{
+  if (!run || !chosen || !n_samples || k < 1 || (!pos && !a_hist && !b_hist)) {
+    ser_set_error("ser_run_marginals: bad argument (k = %d; chosen, n_samples and at least one of pos, a_hist, b_hist are needed)", k);
+    return SER_E_ARG;
+  }
+  if (!run->initialized) { ser_set_error("ser_run_marginals: run not initialised"); return SER_E_STATE; }
+  const bool ranges = a_hist || b_hist;
+  if (pos && run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_marginals: positions need SER_STORE_PI"); return SER_E_STATE; }
+  if (ranges && run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_marginals: a / b histograms need SER_STORE_FULL"); return SER_E_STATE; }
+  if (run->acc_what && pos && !(run->acc_what & SER_ACC_POS)) { ser_set_error("ser_run_marginals: the run accumulates without SER_ACC_POS"); return SER_E_STATE; }
+  if (run->acc_what && ranges && !(run->acc_what & SER_ACC_RANGE)) {
+    ser_set_error("ser_run_marginals: the run accumulates without SER_ACC_RANGE");
+    return SER_E_STATE;
+  }
+  if (set_device(run)) return SER_E_CUDA;
+  const int N = run->N, M = run->M;
+  const size_t pos_cells = (size_t)N * N, range_cells = (size_t)M * (N + 1);
+  int *d_ch = nullptr, *d_n = nullptr, *d_pos = nullptr, *d_a = nullptr, *d_b = nullptr;
+  std::vector<int> n_out(k);
+  auto body = [&]() -> int {
+    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
+    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
+    if (pos) CUDA_TRY(POOL_ALLOC(&d_pos, k * pos_cells * sizeof(int)));
+    if (a_hist) CUDA_TRY(POOL_ALLOC(&d_a, k * range_cells * sizeof(int)));
+    if (b_hist) CUDA_TRY(POOL_ALLOC(&d_b, k * range_cells * sizeof(int)));
+    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
+    const int *ids = run->d_chain_ids;
+    const int off = run->cfg.chain_offset, nl = run->cfg.n_chains;
+    if (run->acc_what) {
+      const int nb = 256;
+      if (pos) {
+        mark_launch(run);
+        ser_hist_acc_out_kernel<<<dim3(nb, k, 1), 256, 0, run->stream>>>(run->d_acc_pos, pos_cells, pos_cells, run->d_scal, d_ch, off, nl, ids,
+                                                                         d_pos, nullptr, d_n);
+        CUDA_TRY(cudaGetLastError());
+      }
+      if (ranges) {
+        mark_launch(run);
+        ser_hist_acc_out_kernel<<<dim3(nb, k, 2), 256, 0, run->stream>>>(run->d_acc_range, 2 * range_cells, range_cells, run->d_scal, d_ch, off,
+                                                                         nl, ids, d_a, d_b, d_n);
+        CUDA_TRY(cudaGetLastError());
+      }
+    } else {
+      const int W = run->cfg.max_samples;
+      if (pos) {
+        HistShape hs;
+        CUDA_TRY(hist_shape((const void *)ser_pos_hist_kernel, N, &hs));
+        mark_launch(run);
+        ser_pos_hist_kernel<<<dim3(k, (N + hs.threads - 1) / hs.threads), hs.threads, hs.smem, run->stream>>>(
+            run->d_samp_pi, run->d_scal, N, W, d_ch, off, nl, ids, hs.smem > 0, d_pos, d_n);
+        CUDA_TRY(cudaGetLastError());
+      }
+      if (ranges) {
+        HistShape hs;
+        CUDA_TRY(hist_shape((const void *)ser_range_hist_kernel, N + 1, &hs));
+        mark_launch(run);
+        ser_range_hist_kernel<<<dim3(k, (M + hs.threads - 1) / hs.threads, 2), hs.threads, hs.smem, run->stream>>>(
+            run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, d_ch, off, nl, ids, hs.smem > 0, d_a, d_b, d_n);
+        CUDA_TRY(cudaGetLastError());
+      }
+    }
+    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    /* only the slabs of held chains come back: the others stay as the caller left them */
+    for (int c = 0; c < k; c++) {
+      if (n_out[c] < 0) continue;
+      if (pos) CUDA_TRY(cudaMemcpyAsync(pos + c * pos_cells, d_pos + c * pos_cells, pos_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+      if (a_hist) CUDA_TRY(cudaMemcpyAsync(a_hist + c * range_cells, d_a + c * range_cells, range_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+      if (b_hist) CUDA_TRY(cudaMemcpyAsync(b_hist + c * range_cells, d_b + c * range_cells, range_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    for (int c = 0; c < k; c++) n_samples[c] = n_out[c] < 0 ? 0 : n_out[c];
+    return SER_OK;
+  };
+  const int rc = body();
+  void *tmp[] = {d_ch, d_n, d_pos, d_a, d_b};
+  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
+  return rc;
 }
 
 extern "C" int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, int32_t max_lag, double *stats,
