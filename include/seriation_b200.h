@@ -331,7 +331,8 @@ int ser_multi_cross_chain(ser_multi *m, int32_t k, int32_t *chosen, int32_t *n_c
  *   SER_E_ARG    another dataset (fingerprint of X and the hard flags, or N / M), or a local chain's global id not in the file
  *   SER_E_STATE  mode, seed, sweeps_per_call, manycd, store, max_samples or accumulate flags differ from the run's
  *   SER_E_TAPE   a replay cursor beyond the chain's tape
- *   SER_E_CHECK  a record out of range (a <= b <= N, rpi a permutation) or failing the consistency check (ser_run_check's)
+ *   SER_E_CHECK  a record out of range (a <= b <= N, rpi a permutation; the same for each stored sample row the chain holds)
+ *                or failing the consistency check (ser_run_check's)
  * One process per GPU: each rank saves and loads its own file with the ser_run_* pair. */
 int ser_run_save_checkpoint(ser_run *run, const char *path);
 int ser_run_load_checkpoint(ser_run *run, const char *path);

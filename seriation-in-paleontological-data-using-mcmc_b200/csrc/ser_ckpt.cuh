@@ -460,8 +460,39 @@ static int ckpt_save(ser_run *const *runs, int n_runs, const char *path, const c
   return rc;
 }
 
-/* What a record may hold before it goes near a sweep kernel, which indexes shared memory with rpi and a/b, the tape with the
- * cursor and the sample store with n_samples - sample_base.  Checked on the host, from the file's bytes. */
+/* One permutation row (u16 [N] at perm) and, with ab, one a/b row (u16 [M] a at ab, u16 [M] b at ab + b_off) of chain g: the
+ * permutation holds each of 0..N-1 once, and every taxon has a <= b <= N.  `row` < 0 names the live state, else a stored row. */
+static int ckpt_check_rows(const unsigned char *perm, const char *perm_name, const unsigned char *ab, long long b_off, const char *ab_name,
+                           int N, int M, std::vector<unsigned char> &seen, int g, long long row, const char *who)
+{
+  char where[40] = "";
+  auto name_row = [&]() { if (row >= 0) snprintf(where, sizeof(where), "stored row %lld: ", row); };
+  std::fill(seen.begin(), seen.end(), 0);
+  for (int n = 0; n < N; n++) {
+    const int s = (int)get_le(perm + 2 * n, 2);
+    if (s >= N || seen[s]) {
+      name_row();
+      ser_set_error("%s: chain %d: %s%s is not a permutation of 0..%d (entry %d holds %d)", who, g, where, perm_name, N - 1, n, s);
+      return SER_E_CHECK;
+    }
+    seen[s] = 1;
+  }
+  if (ab)
+    for (int m = 0; m < M; m++) {
+      const int a = (int)get_le(ab + 2 * m, 2), b = (int)get_le(ab + b_off + 2 * m, 2);
+      if (!(a <= b && b <= N)) {
+        name_row();
+        ser_set_error("%s: chain %d: %s%s of taxon %d has a = %d, b = %d (needs a <= b <= %d)", who, g, where, ab_name, m, a, b, N);
+        return SER_E_CHECK;
+      }
+    }
+  return SER_OK;
+}
+
+/* What a record may hold before it goes near a kernel.  The sweep kernels index shared memory with rpi and a/b, the tape with
+ * the cursor and the sample store with n_samples - sample_base.  The histogram kernels (ser_run_marginals and the SER_ACC_POS /
+ * SER_ACC_RANGE accumulators) index their rows with the stored pi, a and b, so the chain's own stored rows obey the rules of the
+ * state; rows past its own count are never read and stay unchecked.  Checked on the host, from the file's bytes. */
 static int ckpt_check_record(const unsigned char *rec, const CkptLayout &L, const CkptHeader &h, long long tape_len, int g, const char *who)
 {
   const int N = h.N, M = h.M;
@@ -469,26 +500,25 @@ static int ckpt_check_record(const unsigned char *rec, const CkptLayout &L, cons
   const int n_samples = (int32_t)get_le(rec + 156, 4);
   const uint32_t flags = (uint32_t)get_le(rec + 160, 4);
   if (flags > 1) { ser_set_error("%s: chain %d: flags %u (only bit 0, tape exhausted, is stored)", who, g, flags); return SER_E_CHECK; }
-  std::vector<unsigned char> seen(N, 0);
-  for (int n = 0; n < N; n++) {
-    const int s = (int)get_le(rec + L.rpi + 2 * n, 2);
-    if (s >= N || seen[s]) { ser_set_error("%s: chain %d: rpi is not a permutation of 0..%d (position %d holds %d)", who, g, N - 1, n, s); return SER_E_CHECK; }
-    seen[s] = 1;
-  }
-  for (int m = 0; m < M; m++) {
-    const int a = (int)get_le(rec + L.ab + 2 * m, 2), b = (int)get_le(rec + L.ab + 2 * (M + m), 2);
-    if (!(a <= b && b <= N)) { ser_set_error("%s: chain %d: taxon %d has a = %d, b = %d (needs a <= b <= %d)", who, g, m, a, b, N); return SER_E_CHECK; }
-  }
+  std::vector<unsigned char> seen(N);
+  int rc = ckpt_check_rows(rec + L.rpi, "rpi", rec + L.ab, 2ll * M, "a/b", N, M, seen, g, -1, who);
+  if (rc) return rc;
   if (cursor < 0) { ser_set_error("%s: chain %d: negative tape cursor %lld", who, g, cursor); return SER_E_CHECK; }
-  if (!(flags & 1)) { /* a chain whose tape ran out never sweeps again */
-    if (h.mode == SER_MODE_REPLAY && cursor > tape_len) {
-      ser_set_error("%s: chain %d: replay cursor %lld is beyond its tape of %lld draws", who, g, cursor, tape_len);
-      return SER_E_TAPE;
-    }
-    if (n_samples < h.sample_base || n_samples > h.n_samples) {
-      ser_set_error("%s: chain %d: n_samples %d outside [sample_base %d, %d]", who, g, n_samples, h.sample_base, h.n_samples);
-      return SER_E_CHECK;
-    }
+  if (!(flags & 1) && h.mode == SER_MODE_REPLAY && cursor > tape_len) { /* a chain whose tape ran out never sweeps again */
+    ser_set_error("%s: chain %d: replay cursor %lld is beyond its tape of %lld draws", who, g, cursor, tape_len);
+    return SER_E_TAPE;
+  }
+  /* an exhausted chain may hold fewer samples than sample_base, never more than the run: the reductions read
+   * min(n_samples, max_samples) of its rows */
+  if (n_samples > h.n_samples || (!(flags & 1) && n_samples < h.sample_base)) {
+    ser_set_error("%s: chain %d: n_samples %d outside [sample_base %d, %d]", who, g, n_samples, h.sample_base, h.n_samples);
+    return SER_E_CHECK;
+  }
+  const bool full = h.store >= SER_STORE_FULL;
+  const long long own = std::max(0ll, std::min((long long)n_samples - h.sample_base, (long long)L.rows));
+  for (long long t = 0; t < own; t++) {
+    rc = ckpt_check_rows(rec + L.spi + 2 * N * t, "spi", full ? rec + L.sa + 2 * M * t : nullptr, L.sb - L.sa, "sa/sb", N, M, seen, g, t, who);
+    if (rc) return rc;
   }
   return SER_OK;
 }

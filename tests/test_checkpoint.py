@@ -361,7 +361,14 @@ def test_refusals_leave_the_run_unusable_and_sweep_nothing(S, tmp_path):
     def loglik(rec, L):                                               # in range, but the totals no longer match: ser_check_kernel
         struct.pack_into("<d", rec, 32, struct.unpack_from("<d", rec, 32)[0] + 1.0)
 
-    for name, edit, text in (("pi", dup_rpi, "not a permutation"), ("ab", a_after_b, "a = 7, b = 3"), ("ll", loglik, "consistency check")):
+    def stored_pi(rec, L):                                            # the histogram kernels index their rows with these
+        struct.pack_into("<H", rec, L["spi"] + 2 * (ds.N + 3), ds.N)
+
+    def stored_b(rec, L):
+        struct.pack_into("<H", rec, L["sb"] + 2 * (ds.M + 5), ds.N + 1)
+
+    for name, edit, text in (("pi", dup_rpi, "not a permutation"), ("ab", a_after_b, "a = 7, b = 3"), ("ll", loglik, "consistency check"),
+                             ("spi", stored_pi, "stored row 1: spi is not a permutation"), ("sb", stored_b, "stored row 1: sa/sb of taxon 5")):
         open(f + name, "wb").write(_patch_record(f, 2, edit))
         refused(E_CHECK, S.Run(ds, 4, **base), f + name, text)
     refused(E_IO, S.Run(ds, 4, **base), str(tmp_path / "missing"))
