@@ -175,14 +175,14 @@ int ser_select_chains_device(const double *d_e, int32_t n, int32_t k, int32_t *d
  * entries owned by other ranks (or -1) leave their slab untouched.  d_counts: [k][N][N] int32
  * in DEVICE memory (zero it first; all-reduce it across ranks afterwards). */
 int ser_run_po_counts_device(ser_run *run, const int32_t *d_chosen, int32_t k, int32_t *d_counts);
-/* host convenience wrapper: chosen / counts in host memory */
+/* host convenience wrapper: chosen / counts in host memory; only the slabs of held chains are written */
 int ser_run_po_counts(ser_run *run, const int32_t *chosen, int32_t k, int32_t *counts);
 /* script.py:155-175 finalisation incl. the reference's carry-over between chains when faithful != 0 */
 int ser_po_finalize(const int32_t *counts, int32_t k, int32_t N, int32_t chains_selected, int32_t faithful,
                     double *po);
 
 /* per-chain sums over the stored thinned samples of the chosen chains owned by this run
- * (GLOBAL ids; others / -1 leave their slab untouched; zero the buffers first; host memory):
+ * (GLOBAL ids; others / -1 leave their slab untouched, a held chain's slab is written in full, corr_num included; host memory):
  *   corr_num[c]  = sum_t sum_i i * pi_t(i)   -> mean Pearson r of pi with 0..N-1 (script.py:129-152):
  *                  r = (corr_num/(T*N) - ((N-1)/2)^2) / ((N^2-1)/12), exact because pi_t is a permutation
  *   pi_sum[c][i] = sum_t pi_t(i)   (script.py:230-252)      needs SER_STORE_PI
@@ -244,13 +244,13 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
                           double *corr_mn, int32_t *n_sites_used);
 
 /* ---------------------------------------------------------------- streaming summaries
- * Flags of ser_run_accumulate and the per-local-chain device accumulators they allocate: */
-#define SER_ACC_PO 1    /* pair-order counts            [n][N][N] int32                                   */
-#define SER_ACC_SUMS 2  /* pi_sum [n][N] int32 (corr_num is derived from it on the way out)                */
-#define SER_ACC_AB 4    /* a_sum, b_sum                 [n][M] int32 each   (needs SER_STORE_FULL)           */
-#define SER_ACC_ALIVE 8 /* alive difference slab        [n][N][M] int32     (needs SER_STORE_FULL)           */
-#define SER_ACC_POS 16  /* position histograms          [n][N][N] int32     (ser_run_marginals' pos)          */
-#define SER_ACC_RANGE 32 /* a and b histograms          [n][2][M][N+1] int32 (needs SER_STORE_FULL)           */
+ * Flags of ser_run_accumulate and the parts of the one int32 device record per local chain they allocate, in this order: */
+#define SER_ACC_PO 1    /* pair-order counts            [N][N]                                            */
+#define SER_ACC_SUMS 2  /* pi_sum [N] (corr_num is derived from it on the way out)                          */
+#define SER_ACC_AB 4    /* pi_sum [N], then a_sum, b_sum [M] each   (needs SER_STORE_FULL)                  */
+#define SER_ACC_ALIVE 8 /* alive difference slab        [N][M]      (needs SER_STORE_FULL)                  */
+#define SER_ACC_POS 16  /* position histograms          [N][N]      (ser_run_marginals' pos)                */
+#define SER_ACC_RANGE 32 /* a and b histograms          [2][M][N+1] (needs SER_STORE_FULL)                  */
 /* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
  * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
  * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),

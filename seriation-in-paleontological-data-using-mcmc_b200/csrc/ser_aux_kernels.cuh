@@ -198,6 +198,38 @@ __device__ __forceinline__ int local_chain(int g, int id_base, int n_local, cons
   return -1;
 }
 
+/* rows [0, T) of a chain's store taken since sample_base, at most w (fewer only when its replay tape ran out) */
+__device__ __forceinline__ int window_rows(const ChainScalars *scal, int local, int sample_base, int w)
+{
+  const int n = scal[local].n_samples - sample_base;
+  return n < 0 ? 0 : n < w ? n : w;
+}
+
+/* Which chain block b of a summary kernel reads, and how many rows of its store:
+ *   one-shot (chosen != nullptr): the local chain holding global id chosen[b] (none: the block does nothing), sample_base 0 and
+ *     rows = max_samples, i.e. every stored sample (the copy-out kernels of an accumulating run pass rows = INT_MAX: T = every
+ *     sample taken since accumulation began);
+ *   streaming (chosen == nullptr): local chain b, the rows of the window its last sweep launch of w sampling calls filled
+ *     (sample_base, rows = w).
+ * The chain's T goes to n_out[b] when n_out is given. */
+struct SumSel {
+  const int *chosen;
+  int id_base, n_local;
+  const int *ids;
+  int sample_base, rows;
+  int *n_out;
+};
+
+/* local chain of block b (-1: not held) and its T; `lead` = the one thread of the block's chain that writes n_out */
+__device__ __forceinline__ int sel_chain(const SumSel &s, const ChainScalars *scal, int b, bool lead, int *T)
+{
+  const int local = s.chosen ? local_chain(s.chosen[b], s.id_base, s.n_local, s.ids) : b;
+  if (local < 0) return -1;
+  *T = window_rows(scal, local, s.sample_base, s.rows);
+  if (lead && s.n_out) s.n_out[b] = *T;
+  return local;
+}
+
 /* pair-order counts of a 32 x 32 tile of (i, j) over rows [0, T) of one chain's samples `pi` ([row][N]): the positions of the
  * tile's 64 sites staged through shared memory 32 samples at a time (coalesced rows).  256 threads; thread (tx, ty) adds
  * #{t : pi_t(i0+ty+8r) < pi_t(j0+tx)} to c[r].  Every thread of the block calls it (barriers inside). */
@@ -223,15 +255,18 @@ __device__ __forceinline__ void po_tile(const uint16_t *pi, int N, int T, int i0
   }
 }
 
-/* pair-order counts (script.py:178-189) for one chosen chain per blockIdx.z, one 32 x 32 tile per block.  T = the CHOSEN
- * chain's own sample count.  Only the owner of a chosen chain writes its slab -- to every destination (peer stores: the
- * slabs are disjoint, so no reduction is needed). */
-__global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples,
-                                                      const int *chosen, int chain_offset, int n_local, const int *ids, PeerPtrs dst)
+/* Summary kernels: every one serves both the one-shot getters and the streaming accumulators.  Block b reads the chain and rows
+ * sel_chain gives it and writes slab b of its output (out + b * stride: a [k][..] output, or the part of a chain's accumulator record,
+ * stride acc_layout().ints); add = 0 stores the slab, add = 1 adds into it.  A chain the run does not hold leaves its slab untouched. */
+
+/* pair-order counts (script.py:178-189), one 32 x 32 tile per block, slab blockIdx.z into every destination (peer stores: the slabs
+ * are disjoint, so no reduction is needed).  Stored: diagonal -T; added: the diagonal stays 0 (a site is never before itself). */
+__global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, SumSel sel,
+                                                      PeerPtrs dst, size_t stride, int add)
 {
-  const int local = local_chain(chosen[blockIdx.z], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.z, blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  const int T = stored_samples(scal, local, max_samples);
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5; /* 32 x 8 threads; thread (tx, ty) owns j = j0+tx, i = i0+ty+8r */
   const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
   int c[4] = {0, 0, 0, 0};
@@ -242,58 +277,72 @@ __global__ void __launch_bounds__(256) ser_po_kernel(const uint16_t *samp_pi, co
   for (int r = 0; r < 4; r++) {
     const int i = i0 + ty + 8 * r;
     if (i >= N) continue;
-    const int v = (i == j) ? -T : c[r];
-    for (int q = 0; q < dst.n; q++) ((int *)dst.p[q])[((size_t)blockIdx.z * N + i) * N + j] = v;
+    const size_t e = (size_t)blockIdx.z * stride + (size_t)i * N + j;
+#pragma unroll
+    for (int q = 0; q < SER_MAX_PEERS; q++) /* constant indices: a loop to dst.n would copy the destinations to the stack */
+      if (q < dst.n) {
+        int *d = (int *)dst.p[q] + e;
+        *d = add ? *d + c[r] : (i == j ? -T : c[r]);
+      }
   }
 }
 
-/* posterior sums over the stored samples of one chosen chain per block (script.py:129-152, :230-276) */
+/* posterior sums (script.py:129-152, :230-276), one chain per block: sum_t pi_t into pi_sum, sum_t a_t / b_t into a_sum / b_sum when
+ * given; corr_num[b] = sum_i i * (this block's sum_t pi_t(i)) when given (the one-shot getter) */
 __global__ void ser_posterior_kernel(const uint16_t *samp_pi, const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal,
-                                     int N, int M, int max_samples, const int *chosen, int chain_offset, int n_local, const int *ids,
-                                     long long *corr_num, int *pi_sum, int *a_sum, int *b_sum, int *n_out)
+                                     int N, int M, int max_samples, SumSel sel, int *pi_sum, size_t pi_stride, int *a_sum, int *b_sum,
+                                     size_t ab_stride, long long *corr_num, int add)
 {
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  __shared__ unsigned long long s_corr;
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, threadIdx.x == 0, &T);
   if (local < 0) return;
-  const int n_samples = stored_samples(scal, local, max_samples);
-  if (threadIdx.x == 0 && n_out) n_out[blockIdx.x] = n_samples;
+  if (threadIdx.x == 0) s_corr = 0;
   const size_t base = (size_t)local * max_samples;
+  int *ps = pi_sum + blockIdx.x * pi_stride;
   long long s = 0;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     int acc = 0;
-    for (int t = 0; t < n_samples; t++) acc += samp_pi[(base + t) * N + i];
-    pi_sum[(size_t)blockIdx.x * N + i] = acc;
+    for (int t = 0; t < T; t++) acc += samp_pi[(base + t) * N + i];
+    ps[i] = add ? ps[i] + acc : acc;
     s += (long long)i * acc;
   }
-  if (a_sum && samp_a)
+  if (a_sum || b_sum)
     for (int m = threadIdx.x; m < M; m += blockDim.x) {
       int sa = 0, sb = 0;
-      for (int t = 0; t < n_samples; t++) { sa += samp_a[(base + t) * M + m]; sb += samp_b[(base + t) * M + m]; }
-      a_sum[(size_t)blockIdx.x * M + m] = sa;
-      if (b_sum) b_sum[(size_t)blockIdx.x * M + m] = sb;
+      for (int t = 0; t < T; t++) { sa += samp_a[(base + t) * M + m]; sb += samp_b[(base + t) * M + m]; }
+      const size_t e = blockIdx.x * ab_stride + m;
+      if (a_sum) a_sum[e] = add ? a_sum[e] + sa : sa;
+      if (b_sum) b_sum[e] = add ? b_sum[e] + sb : sb;
     }
-  atomicAdd((unsigned long long *)&corr_num[blockIdx.x], (unsigned long long)s);
+  if (!corr_num) return;
+  __syncthreads();
+  atomicAdd(&s_corr, (unsigned long long)s); /* an integer sum: the same in any order */
+  __syncthreads();
+  if (threadIdx.x == 0) corr_num[blockIdx.x] = (long long)s_corr;
 }
 
-/* alive[c][j][m] = #{t : a_t(m) <= j <= b_t(m)} over the stored samples of chosen chain c
- * (script.py:321-329; closed at b, as the reference tests it).  One thread per taxon: +1 / -1
- * marks at a and b+1 in its own column of the slab, then a running sum down the positions. */
+/* alive[j][m] = #{t : a_t(m) <= j <= b_t(m)} (script.py:321-329; closed at b, as the reference tests it).  One thread per taxon: +1 / -1
+ * marks at a and b+1 in its own column of the slab.  Stored: the column is zeroed first and the marks are summed down the positions;
+ * added: the marks alone go into a difference slab, whose running sum the accumulating getter takes. */
 __global__ void ser_alive_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
-                                 const int *chosen, int chain_offset, int n_local, const int *ids, int *alive, int *n_out)
+                                 SumSel sel, int *alive, size_t stride, int add)
 {
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, blockIdx.y == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  const int n_samples = stored_samples(scal, local, max_samples);
-  if (blockIdx.y == 0 && threadIdx.x == 0 && n_out) n_out[blockIdx.x] = n_samples;
   const int m = blockIdx.y * blockDim.x + threadIdx.x;
   if (m >= M) return;
   const size_t base = (size_t)local * max_samples;
-  int *col = alive + (size_t)blockIdx.x * N * M + m;
-  for (int j = 0; j < N; j++) col[(size_t)j * M] = 0;
-  for (int t = 0; t < n_samples; t++) {
+  int *col = alive + blockIdx.x * stride + m;
+  if (!add)
+    for (int j = 0; j < N; j++) col[(size_t)j * M] = 0;
+  for (int t = 0; t < T; t++) {
     const int a = samp_a[(base + t) * M + m], b = samp_b[(base + t) * M + m];
     if (a < N) col[(size_t)a * M] += 1;
     if (b + 1 < N) col[(size_t)(b + 1) * M] -= 1;
   }
+  if (add) return;
   int acc = 0;
   for (int j = 0; j < N; j++) { acc += col[(size_t)j * M]; col[(size_t)j * M] = acc; }
 }
@@ -473,192 +522,128 @@ __device__ void hist_tile(const uint16_t *x, int stride, int items, int bins, in
   }
 }
 
-/* pos [k][N][N]: per chosen chain (blockIdx.x) the position histogram of every site over its stored samples; a chain this run does
- * not hold (or -1) leaves its slab untouched, a held chain's slab is written in full.  n_out[c] = T of a held chain. */
-__global__ void ser_pos_hist_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, const int *chosen,
-                                    int chain_offset, int n_local, const int *ids, int use_smem, int *pos, int *n_out)
+/* pos [N][N]: the position histogram of every site over the chain's rows */
+__global__ void ser_pos_hist_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, SumSel sel, int use_smem,
+                                    int *pos, size_t stride, int add)
 {
   extern __shared__ int s_hist[];
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, blockIdx.y == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  const int T = stored_samples(scal, local, max_samples);
-  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = T;
-  hist_tile(samp_pi + (size_t)local * max_samples * N, N, N, N, T, blockIdx.y * blockDim.x, pos + (size_t)blockIdx.x * N * N,
-            use_smem ? s_hist : nullptr, false);
+  hist_tile(samp_pi + (size_t)local * max_samples * N, N, N, N, T, blockIdx.y * blockDim.x, pos + blockIdx.x * stride,
+            use_smem ? s_hist : nullptr, add);
 }
 
-/* a_hist / b_hist [k][M][N+1] (blockIdx.z = 0 / 1; either may be nullptr): per chosen chain the histograms of every taxon's a and b */
+/* a_hist / b_hist [M][N+1] (blockIdx.z = 0 / 1; either may be nullptr): the histograms of every taxon's a and b over the chain's rows */
 __global__ void ser_range_hist_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
-                                      const int *chosen, int chain_offset, int n_local, const int *ids, int use_smem, int *a_hist,
-                                      int *b_hist, int *n_out)
+                                      SumSel sel, int use_smem, int *a_hist, int *b_hist, size_t stride, int add)
 {
   extern __shared__ int s_hist[];
   int *out = blockIdx.z ? b_hist : a_hist;
   if (!out) return;
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, blockIdx.y == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  const int T = stored_samples(scal, local, max_samples);
-  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = T;
   const uint16_t *x = (blockIdx.z ? samp_b : samp_a) + (size_t)local * max_samples * M;
-  hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, out + (size_t)blockIdx.x * M * (N + 1), use_smem ? s_hist : nullptr, false);
+  hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, out + blockIdx.x * stride, use_smem ? s_hist : nullptr, add);
 }
 
 /* ------------------------------------------------------------------ streaming accumulators (ser_run_accumulate)
- * On an accumulating run the sample store is a window of max_samples rows per chain.  After every sweep launch of w
- * sampling calls these kernels add rows [0, w) of EVERY local chain's window into per-chain totals; the getters below
- * turn the totals into what the one-shot kernels above compute from a store that holds all samples. */
+ * On an accumulating run the sample store is a window of max_samples rows per chain.  After every sweep launch of w sampling calls
+ * the summary kernels above add the window's rows of EVERY local chain into that chain's accumulator record; the getters turn the
+ * records into what the one-shot kernels compute from a store that holds all samples, with the kernels below. */
 
-/* rows of the window a chain filled in the last launch (fewer than w only when its replay tape ran out) */
-__device__ __forceinline__ int window_rows(const ChainScalars *scal, int local, int sample_base, int w)
+#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE)
+
+/* One local chain's accumulator record: int32 offsets of the parts the flags `what` select, in this order, and the record's length.
+ * The run holds [n_local][ints]; a checkpoint record holds the same ints in the same order.
+ *   po [N][N] (SER_ACC_PO; diagonal 0), pi [N] (SER_ACC_SUMS or SER_ACC_AB), asum [M], bsum [M] (SER_ACC_AB),
+ *   alive [N][M] (SER_ACC_ALIVE; the difference slab), pos [N][N] (SER_ACC_POS), range [2][M][N+1] (SER_ACC_RANGE; a, then b) */
+struct AccLayout {
+  size_t po, pi, asum, bsum, alive, pos, range, ints;
+};
+__host__ __device__ inline AccLayout acc_layout(int N, int M, int what)
 {
-  const int n = scal[local].n_samples - sample_base;
-  return n < 0 ? 0 : n < w ? n : w;
+  AccLayout L;
+  const size_t n = N, m = M;
+  size_t o = 0;
+  L.po = o; o += (what & SER_ACC_PO) ? n * n : 0;
+  L.pi = o; o += (what & (SER_ACC_SUMS | SER_ACC_AB)) ? n : 0;
+  L.asum = o; o += (what & SER_ACC_AB) ? m : 0;
+  L.bsum = o; o += (what & SER_ACC_AB) ? m : 0;
+  L.alive = o; o += (what & SER_ACC_ALIVE) ? n * m : 0;
+  L.pos = o; o += (what & SER_ACC_POS) ? n * n : 0;
+  L.range = o; o += (what & SER_ACC_RANGE) ? 2 * m * (n + 1) : 0;
+  L.ints = o;
+  return L;
 }
 
-/* pair-order tiles of every local chain (blockIdx.z) added into acc [n_local][N][N]; the diagonal stays 0 */
-__global__ void __launch_bounds__(256) ser_po_accum_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples,
-                                                            int sample_base, int w, int *acc)
-{
-  const int local = blockIdx.z;
-  const int T = window_rows(scal, local, sample_base, w);
-  if (T == 0) return;
-  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-  const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
-  int c[4] = {0, 0, 0, 0};
-  po_tile(samp_pi + (size_t)local * max_samples * N, N, T, i0, j0, c);
-  const int j = j0 + tx;
-  if (j >= N) return;
-  int *slab = acc + (size_t)local * N * N;
-#pragma unroll
-  for (int r = 0; r < 4; r++) {
-    const int i = i0 + ty + 8 * r;
-    if (i < N) slab[(size_t)i * N + j] += c[r];
-  }
-}
+/* The getters of an accumulating run read the records of the chosen chains the run holds (sel: rows = INT_MAX, so T = all samples
+ * taken since accumulation began); `acc` points at the part in local chain 0's record, records are `per_chain` ints apart. */
 
-/* sum_t pi_t into pi_acc [n_local][N], and sum_t a_t / b_t into a_acc / b_acc [n_local][M] when given; one chain per block */
-__global__ void ser_posterior_accum_kernel(const uint16_t *samp_pi, const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal,
-                                           int N, int M, int max_samples, int sample_base, int w, int *pi_acc, int *a_acc, int *b_acc)
+/* counts [k][N][N]: the pair-order part with the diagonal -T */
+__global__ void ser_po_acc_out_kernel(const int *acc, size_t per_chain, const ChainScalars *scal, int N, SumSel sel, int *counts)
 {
-  const int local = blockIdx.x;
-  const int T = window_rows(scal, local, sample_base, w);
-  const size_t base = (size_t)local * max_samples;
-  for (int i = threadIdx.x; i < N; i += blockDim.x) {
-    int acc = 0;
-    for (int t = 0; t < T; t++) acc += samp_pi[(base + t) * N + i];
-    pi_acc[(size_t)local * N + i] += acc;
-  }
-  if (a_acc)
-    for (int m = threadIdx.x; m < M; m += blockDim.x) {
-      int sa = 0, sb = 0;
-      for (int t = 0; t < T; t++) { sa += samp_a[(base + t) * M + m]; sb += samp_b[(base + t) * M + m]; }
-      a_acc[(size_t)local * M + m] += sa;
-      b_acc[(size_t)local * M + m] += sb;
-    }
-}
-
-/* +1 at a, -1 at b+1 of every window row into the difference slab diff [n_local][N][M]; one thread per taxon */
-__global__ void ser_alive_accum_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M, int max_samples,
-                                       int sample_base, int w, int *diff)
-{
-  const int local = blockIdx.x, m = blockIdx.y * blockDim.x + threadIdx.x;
-  if (m >= M) return;
-  const int T = window_rows(scal, local, sample_base, w);
-  const size_t base = (size_t)local * max_samples;
-  int *col = diff + (size_t)local * N * M + m;
-  for (int t = 0; t < T; t++) {
-    const int a = samp_a[(base + t) * M + m], b = samp_b[(base + t) * M + m];
-    if (a < N) col[(size_t)a * M] += 1;
-    if (b + 1 < N) col[(size_t)(b + 1) * M] -= 1;
-  }
-}
-
-/* position histograms of the window's rows of every local chain (blockIdx.x) added into acc [n_local][N][N] */
-__global__ void ser_pos_hist_accum_kernel(const uint16_t *samp_pi, const ChainScalars *scal, int N, int max_samples, int sample_base, int w,
-                                          int use_smem, int *acc)
-{
-  extern __shared__ int s_hist[];
-  const int local = blockIdx.x;
-  const int T = window_rows(scal, local, sample_base, w);
-  if (T == 0) return;
-  hist_tile(samp_pi + (size_t)local * max_samples * N, N, N, N, T, blockIdx.y * blockDim.x, acc + (size_t)local * N * N,
-            use_smem ? s_hist : nullptr, true);
-}
-
-/* a (blockIdx.z = 0) and b (1) histograms of the window's rows added into acc [n_local][2][M][N+1] */
-__global__ void ser_range_hist_accum_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int N, int M,
-                                            int max_samples, int sample_base, int w, int use_smem, int *acc)
-{
-  extern __shared__ int s_hist[];
-  const int local = blockIdx.x;
-  const int T = window_rows(scal, local, sample_base, w);
-  if (T == 0) return;
-  const size_t slab = (size_t)M * (N + 1);
-  const uint16_t *x = (blockIdx.z ? samp_b : samp_a) + (size_t)local * max_samples * M;
-  hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, acc + ((size_t)local * 2 + blockIdx.z) * slab, use_smem ? s_hist : nullptr, true);
-}
-
-/* getters of an accumulating run: the slab of every chosen chain the run holds, T = all samples taken since accumulation began */
-/* slab part [part * cells, (part + 1) * cells) of a local chain's accumulator of `per_chain` ints into out [k][cells] (nullptr: not
- * wanted); blockIdx.y = chosen chain, blockIdx.z = part */
-__global__ void ser_hist_acc_out_kernel(const int *acc, size_t per_chain, size_t cells, const ChainScalars *scal, const int *chosen,
-                                        int chain_offset, int n_local, const int *ids, int *out0, int *out1, int *n_out)
-{
-  int *out = blockIdx.z ? out1 : out0;
-  if (!out) return;
-  const int local = local_chain(chosen[blockIdx.y], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.y, blockIdx.x == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  if (blockIdx.x == 0 && threadIdx.x == 0) n_out[blockIdx.y] = scal[local].n_samples;
-  const int *src = acc + local * per_chain + blockIdx.z * cells;
-  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < cells; q += (size_t)gridDim.x * blockDim.x)
-    out[blockIdx.y * cells + q] = src[q];
-}
-
-__global__ void ser_po_acc_out_kernel(const int *acc, const ChainScalars *scal, int N, const int *chosen, int chain_offset, int n_local,
-                                      const int *ids, int *counts)
-{
-  const int local = local_chain(chosen[blockIdx.y], chain_offset, n_local, ids);
-  if (local < 0) return;
-  const int T = scal[local].n_samples;
   const size_t nn = (size_t)N * N;
   for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < nn; q += (size_t)gridDim.x * blockDim.x)
-    counts[blockIdx.y * nn + q] = (q / N == q % N) ? -T : acc[local * nn + q];
+    counts[blockIdx.y * nn + q] = (q / N == q % N) ? -T : acc[local * per_chain + q];
 }
 
-__global__ void ser_posterior_acc_out_kernel(const int *pi_acc, const int *a_acc, const int *b_acc, const ChainScalars *scal, int N, int M,
-                                             const int *chosen, int chain_offset, int n_local, const int *ids,
-                                             long long *corr_num, int *pi_sum, int *a_sum, int *b_sum, int *n_out)
+/* the pi, a and b sums (a_sum / b_sum may be nullptr) and corr_num[c] = sum_i i * pi_sum[c][i] */
+__global__ void ser_posterior_acc_out_kernel(const int *pi_acc, const int *a_acc, const int *b_acc, size_t per_chain, const ChainScalars *scal,
+                                             int N, int M, SumSel sel, long long *corr_num, int *pi_sum, int *a_sum, int *b_sum)
 {
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  __shared__ unsigned long long s_corr;
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, threadIdx.x == 0, &T);
   if (local < 0) return;
-  if (threadIdx.x == 0) n_out[blockIdx.x] = scal[local].n_samples;
+  if (threadIdx.x == 0) s_corr = 0;
+  __syncthreads();
+  const size_t src = local * per_chain;
   long long s = 0;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
-    const int v = pi_acc[(size_t)local * N + i];
+    const int v = pi_acc[src + i];
     pi_sum[(size_t)blockIdx.x * N + i] = v;
     s += (long long)i * v;
   }
-  if (a_sum)
-    for (int m = threadIdx.x; m < M; m += blockDim.x) {
-      a_sum[(size_t)blockIdx.x * M + m] = a_acc[(size_t)local * M + m];
-      if (b_sum) b_sum[(size_t)blockIdx.x * M + m] = b_acc[(size_t)local * M + m];
-    }
-  atomicAdd((unsigned long long *)&corr_num[blockIdx.x], (unsigned long long)s);
+  for (int m = threadIdx.x; m < M; m += blockDim.x) {
+    if (a_sum) a_sum[(size_t)blockIdx.x * M + m] = a_acc[src + m];
+    if (b_sum) b_sum[(size_t)blockIdx.x * M + m] = b_acc[src + m];
+  }
+  atomicAdd(&s_corr, (unsigned long long)s); /* an integer sum: the same in any order */
+  __syncthreads();
+  if (threadIdx.x == 0) corr_num[blockIdx.x] = (long long)s_corr;
 }
 
-/* running sum of the difference slab down the positions */
-__global__ void ser_alive_acc_out_kernel(const int *diff, const ChainScalars *scal, int N, int M, const int *chosen, int chain_offset,
-                                         int n_local, const int *ids, int *alive, int *n_out)
+/* alive [k][N][M]: the running sum of the difference slab down the positions */
+__global__ void ser_alive_acc_out_kernel(const int *diff, size_t per_chain, const ChainScalars *scal, int N, int M, SumSel sel, int *alive)
 {
-  const int local = local_chain(chosen[blockIdx.x], chain_offset, n_local, ids);
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, blockIdx.y == 0 && threadIdx.x == 0, &T);
   if (local < 0) return;
-  if (blockIdx.y == 0 && threadIdx.x == 0) n_out[blockIdx.x] = scal[local].n_samples;
   const int m = blockIdx.y * blockDim.x + threadIdx.x;
   if (m >= M) return;
-  const int *src = diff + (size_t)local * N * M + m;
+  const int *src = diff + local * per_chain + m;
   int *col = alive + (size_t)blockIdx.x * N * M + m;
   int acc = 0;
   for (int j = 0; j < N; j++) { acc += src[(size_t)j * M]; col[(size_t)j * M] = acc; }
+}
+
+/* histogram part z (blockIdx.z) of `cells` ints into out_z [k][cells] (nullptr: not wanted), chosen chain blockIdx.y */
+__global__ void ser_hist_acc_out_kernel(const int *acc, size_t per_chain, size_t cells, const ChainScalars *scal, SumSel sel, int *out0,
+                                        int *out1)
+{
+  int *out = blockIdx.z ? out1 : out0;
+  if (!out) return;
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.y, blockIdx.x == 0 && threadIdx.x == 0, &T);
+  if (local < 0) return;
+  const int *src = acc + local * per_chain + blockIdx.z * cells;
+  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < cells; q += (size_t)gridDim.x * blockDim.x)
+    out[blockIdx.y * cells + q] = src[q];
 }
 
 /* ------------------------------------------------------------------ micro-benchmarks */

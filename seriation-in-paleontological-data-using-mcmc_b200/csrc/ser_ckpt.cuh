@@ -105,13 +105,7 @@ struct CkptLayout {
   long long cd;      /* f64 [4][M] c, log(1-e^c), d, log(1-e^d) per taxon (manycd)                */
   long long cdl;     /* f64 [rows][3] c, d, loglik of every stored row (SER_STORE_FULL)           */
   long long cd_all;  /* f64 [rows][2][M] per-taxon c, d of every stored row (FULL + manycd)       */
-  long long po;      /* i32 [N][N] pair-order totals (SER_ACC_PO)                                 */
-  long long pi;      /* i32 [N] pi sums (SER_ACC_SUMS or SER_ACC_AB)                              */
-  long long asum;    /* i32 [M] a sums, then bsum (SER_ACC_AB)                                    */
-  long long bsum;
-  long long alive;   /* i32 [N][M] alive difference slab (SER_ACC_ALIVE)                          */
-  long long pos;     /* i32 [N][N] position histograms (SER_ACC_POS)                              */
-  long long range;   /* i32 [2][M][N+1] a, then b histograms (SER_ACC_RANGE)                      */
+  long long acc;     /* i32 [acc_layout().ints] the chain's accumulator record (SER_ACC_*), up to rpi */
   long long rpi;     /* u16 [N] site at each position                                             */
   long long ab;      /* u16 [M] a, then u16 [M] b, per taxon                                       */
   long long spi;     /* u16 [rows][N] stored pi rows (SER_STORE_PI)                                */
@@ -131,13 +125,7 @@ __host__ __device__ inline CkptLayout ckpt_layout(int N, int M, int manycd, int 
   L.cd = o; o += manycd ? 8 * 4 * m : 0;
   L.cdl = o; o += full ? 8 * 3 * r : 0;
   L.cd_all = o; o += (full && manycd) ? 8 * 2 * m * r : 0;
-  L.po = o; o += (acc & SER_ACC_PO) ? 4 * n * n : 0;
-  L.pi = o; o += (acc & (SER_ACC_SUMS | SER_ACC_AB)) ? 4 * n : 0;
-  L.asum = o; o += (acc & SER_ACC_AB) ? 4 * m : 0;
-  L.bsum = o; o += (acc & SER_ACC_AB) ? 4 * m : 0;
-  L.alive = o; o += (acc & SER_ACC_ALIVE) ? 4 * n * m : 0;
-  L.pos = o; o += (acc & SER_ACC_POS) ? 4 * n * n : 0;
-  L.range = o; o += (acc & SER_ACC_RANGE) ? 8 * m * (n + 1) : 0;
+  L.acc = o; o += 4 * (long long)acc_layout(N, M, acc).ints;
   L.rpi = o; o += 2 * n;
   L.ab = o; o += 4 * m;
   L.spi = o; o += store >= SER_STORE_PI ? 2 * n * r : 0;
@@ -148,11 +136,6 @@ __host__ __device__ inline CkptLayout ckpt_layout(int N, int M, int manycd, int 
   return L;
 }
 
-/* the run's accumulators (ser_run_accumulate), nullptr where the run has none */
-struct CkptAcc {
-  int *po, *pi, *a, *b, *alive, *pos, *range;
-};
-
 /* dst[0, total) = src[0, valid), then zeros: rows past a chain's own count (a replay chain whose tape ran out) are written as
  * zeros so that a file never holds uninitialised bytes */
 template <typename T>
@@ -162,7 +145,7 @@ __device__ __forceinline__ void ckpt_copy(T *dst, const T *src, long long valid,
 }
 
 /* one record per block: local chain locals[blockIdx.x] into out + blockIdx.x * L.size (the checksum slot is left zero) */
-__global__ void ser_ckpt_pack_kernel(KParams p, CkptLayout L, CkptAcc acc, const int *locals, unsigned char *out)
+__global__ void ser_ckpt_pack_kernel(KParams p, CkptLayout L, const int *acc, const int *locals, unsigned char *out)
 {
   const int chain = locals[blockIdx.x], tid = threadIdx.x, nt = blockDim.x, N = p.N, M = p.M;
   unsigned char *rec = out + (size_t)blockIdx.x * L.size;
@@ -201,20 +184,14 @@ __global__ void ser_ckpt_pack_kernel(KParams p, CkptLayout L, CkptAcc acc, const
       if (p.manycd) ckpt_copy((double *)(rec + L.cd_all), p.samp_cd_all + row0 * 2 * M, own * 2 * M, R * 2 * M);
     }
   }
-  const long long nn = (long long)N * N, nm = (long long)N * M, nr = 2ll * M * (N + 1);
-  if (acc.po) ckpt_copy((int *)(rec + L.po), acc.po + chain * nn, nn, nn);
-  if (acc.pi) ckpt_copy((int *)(rec + L.pi), acc.pi + (long long)chain * N, N, N);
-  if (acc.a) ckpt_copy((int *)(rec + L.asum), acc.a + (long long)chain * M, M, M);
-  if (acc.b) ckpt_copy((int *)(rec + L.bsum), acc.b + (long long)chain * M, M, M);
-  if (acc.alive) ckpt_copy((int *)(rec + L.alive), acc.alive + chain * nm, nm, nm);
-  if (acc.pos) ckpt_copy((int *)(rec + L.pos), acc.pos + chain * nn, nn, nn);
-  if (acc.range) ckpt_copy((int *)(rec + L.range), acc.range + chain * nr, nr, nr);
+  const long long na = (L.rpi - L.acc) / 4;
+  if (acc) ckpt_copy((int *)(rec + L.acc), acc + chain * na, na, na);
   for (long long o = L.end + tid; o < L.size; o += nt) rec[o] = 0;
 }
 
 /* the mirror: record blockIdx.x of `in` into local chain locals[blockIdx.x].  The flags keep bit 0 alone: the bit columns
  * (SER_FLAG_COLUMNS) are rebuilt from rpi by the next sweep, and bits 1-4 are ser_check_kernel's to set. */
-__global__ void ser_ckpt_unpack_kernel(KParams p, CkptLayout L, CkptAcc acc, const int *locals, const unsigned char *in)
+__global__ void ser_ckpt_unpack_kernel(KParams p, CkptLayout L, int *acc, const int *locals, const unsigned char *in)
 {
   const int chain = locals[blockIdx.x], tid = threadIdx.x, nt = blockDim.x, N = p.N, M = p.M;
   const unsigned char *rec = in + (size_t)blockIdx.x * L.size;
@@ -255,14 +232,8 @@ __global__ void ser_ckpt_unpack_kernel(KParams p, CkptLayout L, CkptAcc acc, con
       if (p.manycd) ckpt_copy(p.samp_cd_all + row0 * 2 * M, (const double *)(rec + L.cd_all), R * 2 * M, R * 2 * M);
     }
   }
-  const long long nn = (long long)N * N, nm = (long long)N * M, nr = 2ll * M * (N + 1);
-  if (acc.po) ckpt_copy(acc.po + chain * nn, (const int *)(rec + L.po), nn, nn);
-  if (acc.pi) ckpt_copy(acc.pi + (long long)chain * N, (const int *)(rec + L.pi), N, N);
-  if (acc.a) ckpt_copy(acc.a + (long long)chain * M, (const int *)(rec + L.asum), M, M);
-  if (acc.b) ckpt_copy(acc.b + (long long)chain * M, (const int *)(rec + L.bsum), M, M);
-  if (acc.alive) ckpt_copy(acc.alive + chain * nm, (const int *)(rec + L.alive), nm, nm);
-  if (acc.pos) ckpt_copy(acc.pos + chain * nn, (const int *)(rec + L.pos), nn, nn);
-  if (acc.range) ckpt_copy(acc.range + chain * nr, (const int *)(rec + L.range), nr, nr);
+  const long long na = (L.rpi - L.acc) / 4;
+  if (acc) ckpt_copy(acc + chain * na, (const int *)(rec + L.acc), na, na);
 }
 
 /* ------------------------------------------------------------------ host side */
@@ -276,8 +247,6 @@ static int ckpt_rows(int store, int max_samples, int n_samples, int sample_base)
 }
 
 static CkptLayout ckpt_layout_of(const CkptHeader &h) { return ckpt_layout(h.N, h.M, h.manycd, h.store, h.rows, h.acc); }
-
-static CkptAcc ckpt_acc_of(const ser_run *run) { return CkptAcc{run->d_acc_po, run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_acc_alive, run->d_acc_pos, run->d_acc_range}; }
 
 static long long ckpt_table_bytes(int n) { return ((long long)n * 4 + 7) / 8 * 8 + 8; }
 
@@ -324,7 +293,7 @@ static int ckpt_read_head(int fd, const char *path, CkptHeader *h, std::vector<i
   const bool sane = h->N >= 2 && h->N <= SER_MAX_SITES && h->M >= 1 && h->M <= SER_MAX_TAXA && h->n_chains >= 1 && h->max_samples >= 0 &&
                     h->store >= SER_STORE_NONE && h->store <= SER_STORE_FULL && (h->manycd == 0 || h->manycd == 1) && h->n_samples >= 0 &&
                     h->sample_base >= 0 && h->sample_base <= h->n_samples && h->calls_done >= h->n_samples &&
-                    h->rows == ckpt_rows(h->store, h->max_samples, h->n_samples, h->sample_base) && (h->acc & ~(SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE)) == 0;
+                    h->rows == ckpt_rows(h->store, h->max_samples, h->n_samples, h->sample_base) && (h->acc & ~SER_ACC_ALL) == 0;
   if (!sane) { ser_set_error("checkpoint %s: inconsistent header fields", path); return SER_E_IO; }
   if (h->record_size != (uint64_t)ckpt_layout_of(*h).size) {
     ser_set_error("checkpoint %s: record size %llu does not match the layout of its header (%lld)", path, (unsigned long long)h->record_size,
@@ -425,7 +394,7 @@ static int ckpt_save(ser_run *const *runs, int n_runs, const char *path, const c
           const int nb = (int)std::min<size_t>(stage.per_block, pos.size() - i0);
           CUDA_TRY(cudaMemcpyAsync(d_loc, loc.data() + i0, (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, run->stream));
           mark_launch(run);
-          ser_ckpt_pack_kernel<<<nb, 256, 0, run->stream>>>(run->kp, L, ckpt_acc_of(run), d_loc, d_stage);
+          ser_ckpt_pack_kernel<<<nb, 256, 0, run->stream>>>(run->kp, L, run->d_acc, d_loc, d_stage);
           CUDA_TRY(cudaGetLastError());
           CUDA_TRY(cudaMemcpyAsync(stage.host, d_stage, (size_t)nb * L.size, cudaMemcpyDeviceToHost, run->stream));
           CUDA_TRY(cudaStreamSynchronize(run->stream));
@@ -574,7 +543,7 @@ static int ckpt_load_run(ser_run *run, int fd, const char *path, const CkptHeade
       CUDA_TRY(cudaMemcpyAsync(d_stage, stage.host, (size_t)nb * L.size, cudaMemcpyHostToDevice, run->stream));
       CUDA_TRY(cudaMemcpyAsync(d_loc, loc.data(), (size_t)nb * sizeof(int), cudaMemcpyHostToDevice, run->stream));
       mark_launch(run);
-      ser_ckpt_unpack_kernel<<<nb, 256, 0, run->stream>>>(run->kp, L, ckpt_acc_of(run), d_loc, d_stage);
+      ser_ckpt_unpack_kernel<<<nb, 256, 0, run->stream>>>(run->kp, L, run->d_acc, d_loc, d_stage);
       CUDA_TRY(cudaGetLastError());
       CUDA_TRY(cudaStreamSynchronize(run->stream)); /* the pinned buffer and loc are refilled by the next block */
     }

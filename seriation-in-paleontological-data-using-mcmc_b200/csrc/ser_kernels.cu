@@ -17,6 +17,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
+#include <climits>
 #include <cstring>
 #include <vector>
 
@@ -104,10 +105,9 @@ struct ser_run {
   size_t sweep_ev_used;
   /* subset runs (ser_run_create_chains): global id of every local chain, device copy in kp.chain_ids */
   int *h_chain_ids, *d_chain_ids;
-  /* streaming accumulators (ser_run_accumulate): SER_ACC_* flags, per local chain totals */
+  /* streaming accumulators (ser_run_accumulate): SER_ACC_* flags, one record per local chain [n][acc_layout().ints] */
   int acc_what, sampled;
-  int *d_acc_po, *d_acc_pi, *d_acc_a, *d_acc_b, *d_acc_alive;
-  int *d_acc_pos, *d_acc_range; /* [n][N][N] position and [n][2][M][N+1] a / b histograms */
+  int *d_acc;
   /* checkpoints (ser_ckpt.cuh): calls and sampling calls advanced since init, and the fingerprint of the run's dataset */
   long long calls_done;
   int samples_done;
@@ -726,24 +726,19 @@ extern "C" int ser_run_create_chains(const ser_dataset *ds, const ser_run_config
   return SER_OK;
 }
 
+static size_t acc_bytes(const ser_run *run) { return (size_t)run->cfg.n_chains * acc_layout(run->N, run->M, run->acc_what).ints * sizeof(int); }
+
 /* zero the accumulators of an accumulating run (start of ser_run_init) */
 static int acc_zero(ser_run *run)
 {
-  const size_t nc = (size_t)run->cfg.n_chains, N = run->N, M = run->M;
-  if (run->d_acc_po) CUDA_TRY(cudaMemsetAsync(run->d_acc_po, 0, nc * N * N * sizeof(int), run->stream));
-  if (run->d_acc_pi) CUDA_TRY(cudaMemsetAsync(run->d_acc_pi, 0, nc * N * sizeof(int), run->stream));
-  if (run->d_acc_a) CUDA_TRY(cudaMemsetAsync(run->d_acc_a, 0, nc * M * sizeof(int), run->stream));
-  if (run->d_acc_b) CUDA_TRY(cudaMemsetAsync(run->d_acc_b, 0, nc * M * sizeof(int), run->stream));
-  if (run->d_acc_alive) CUDA_TRY(cudaMemsetAsync(run->d_acc_alive, 0, nc * N * M * sizeof(int), run->stream));
-  if (run->d_acc_pos) CUDA_TRY(cudaMemsetAsync(run->d_acc_pos, 0, nc * N * N * sizeof(int), run->stream));
-  if (run->d_acc_range) CUDA_TRY(cudaMemsetAsync(run->d_acc_range, 0, nc * 2 * M * (N + 1) * sizeof(int), run->stream));
+  if (run->d_acc) CUDA_TRY(cudaMemsetAsync(run->d_acc, 0, acc_bytes(run), run->stream));
   return SER_OK;
 }
 
 extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
 {
   if (!run) { ser_set_error("ser_run_accumulate: null run"); return SER_E_ARG; }
-  if (what < 1 || (what & ~(SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE))) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
+  if (what < 1 || (what & ~SER_ACC_ALL)) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
   if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
   if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
   const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE)) ? SER_STORE_FULL : SER_STORE_PI;
@@ -753,31 +748,17 @@ extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
   }
   if (run->cfg.max_samples < 1) { ser_set_error("ser_run_accumulate: the window needs max_samples >= 1"); return SER_E_ARG; }
   if (set_device(run)) return SER_E_CUDA;
-  const size_t nc = (size_t)run->cfg.n_chains, N = run->N, M = run->M;
-  auto alloc = [&](int **p, size_t bytes) -> int {
-    const cudaError_t e = POOL_ALLOC(p, bytes);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      ser_set_error("ser_run_accumulate: cannot allocate %zu bytes of accumulators: %s", bytes, cudaGetErrorString(e));
-      return SER_E_CUDA;
-    }
-    return SER_OK;
-  };
-  int rc = SER_OK;
-  if (rc == SER_OK && (what & SER_ACC_PO)) rc = alloc(&run->d_acc_po, nc * N * N * sizeof(int));
-  if (rc == SER_OK && (what & (SER_ACC_SUMS | SER_ACC_AB))) rc = alloc(&run->d_acc_pi, nc * N * sizeof(int));
-  if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_a, nc * M * sizeof(int));
-  if (rc == SER_OK && (what & SER_ACC_AB)) rc = alloc(&run->d_acc_b, nc * M * sizeof(int));
-  if (rc == SER_OK && (what & SER_ACC_ALIVE)) rc = alloc(&run->d_acc_alive, nc * N * M * sizeof(int));
-  if (rc == SER_OK && (what & SER_ACC_POS)) rc = alloc(&run->d_acc_pos, nc * N * N * sizeof(int));
-  if (rc == SER_OK && (what & SER_ACC_RANGE)) rc = alloc(&run->d_acc_range, nc * 2 * M * (N + 1) * sizeof(int));
-  if (rc == SER_OK) rc = acc_zero(run);
-  if (rc != SER_OK) {
-    int **bufs[] = {&run->d_acc_po, &run->d_acc_pi, &run->d_acc_a, &run->d_acc_b, &run->d_acc_alive, &run->d_acc_pos, &run->d_acc_range};
-    for (int **b : bufs) if (*b) { cudaFreeAsync(*b, run->stream); *b = nullptr; }
-    return rc;
-  }
   run->acc_what = what;
+  cudaError_t e = POOL_ALLOC(&run->d_acc, acc_bytes(run));
+  if (e == cudaSuccess) e = cudaMemsetAsync(run->d_acc, 0, acc_bytes(run), run->stream);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    ser_set_error("ser_run_accumulate: cannot allocate %zu bytes of accumulators: %s", acc_bytes(run), cudaGetErrorString(e));
+    if (run->d_acc) cudaFreeAsync(run->d_acc, run->stream);
+    run->d_acc = nullptr;
+    run->acc_what = 0;
+    return SER_E_CUDA;
+  }
   return SER_OK;
 }
 
@@ -789,8 +770,7 @@ extern "C" void ser_run_destroy(ser_run *run)
                   run->d_scal, run->d_tape, run->d_tape_off, run->d_samp_a, run->d_samp_b, run->d_samp_pi, run->d_samp_cdl,
                   run->d_scratch_i, run->d_bad, run->d_cd4, run->d_samp_cd_all, run->d_gV, run->d_gpre, run->d_bgrp, run->d_bbat,
                   run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites, run->d_cl_off, run->d_cl_item, run->d_cl_grp,
-                  run->d_chain_ids, run->d_acc_po, run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_acc_alive, run->d_acc_pos,
-                  run->d_acc_range};
+                  run->d_chain_ids, run->d_acc};
   for (void *b : bufs) if (b) cudaFreeAsync(b, run->stream);
   if (run->stream) cudaStreamSynchronize(run->stream);
   if (run->sweep_ev) {
@@ -954,44 +934,91 @@ static cudaError_t hist_shape(const void *kernel, int bins, HistShape *h)
   return h->smem > 48 * 1024 ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SER_HIST_SMEM) : cudaSuccess;
 }
 
-/* rows [0, w) of every chain's window into the accumulators (ser_run_accumulate), on the run's stream */
+static PeerPtrs one_dest(void *ptr)
+{
+  PeerPtrs d;
+  memset(&d, 0, sizeof(d));
+  d.p[0] = ptr; d.n = 1;
+  return d;
+}
+
+/* the chosen chains of a getter (d_chosen in the numbering where local chain 0 is id_base); rows as SumSel describes */
+static SumSel sel_chosen(const ser_run *run, const int *d_chosen, int id_base, int rows, int *d_n)
+{
+  return SumSel{d_chosen, id_base, run->cfg.n_chains, run->d_chain_ids, 0, rows, d_n};
+}
+
+/* Launches of the summary kernels over k slabs, on the run's stream: the one-shot getters (add = 0) and accumulate_window (add = 1) */
+static int launch_po(ser_run *run, const SumSel &sel, int k, const PeerPtrs &dst, size_t stride, int add)
+{
+  const int N = run->N;
+  mark_launch(run);
+  ser_po_kernel<<<dim3((N + 31) / 32, (N + 31) / 32, k), 256, 0, run->stream>>>(run->d_samp_pi, run->d_scal, N, run->cfg.max_samples, sel,
+                                                                                 dst, stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
+static int launch_posterior(ser_run *run, const SumSel &sel, int k, int *pi, size_t pi_stride, int *a, int *b, size_t ab_stride,
+                            long long *corr_num, int add)
+{
+  mark_launch(run);
+  ser_posterior_kernel<<<k, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, run->N, run->M,
+                                                   run->cfg.max_samples, sel, pi, pi_stride, a, b, ab_stride, corr_num, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
+static int launch_alive(ser_run *run, const SumSel &sel, int k, int *alive, size_t stride, int add)
+{
+  mark_launch(run);
+  ser_alive_kernel<<<dim3(k, (run->M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, run->N, run->M,
+                                                                            run->cfg.max_samples, sel, alive, stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
+static int launch_pos_hist(ser_run *run, const SumSel &sel, int k, int *pos, size_t stride, int add)
+{
+  const int N = run->N;
+  HistShape hs;
+  CUDA_TRY(hist_shape((const void *)ser_pos_hist_kernel, N, &hs));
+  mark_launch(run);
+  ser_pos_hist_kernel<<<dim3(k, (N + hs.threads - 1) / hs.threads), hs.threads, hs.smem, run->stream>>>(
+      run->d_samp_pi, run->d_scal, N, run->cfg.max_samples, sel, hs.smem > 0, pos, stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
+static int launch_range_hist(ser_run *run, const SumSel &sel, int k, int *a_hist, int *b_hist, size_t stride, int add)
+{
+  const int N = run->N, M = run->M;
+  HistShape hs;
+  CUDA_TRY(hist_shape((const void *)ser_range_hist_kernel, N + 1, &hs));
+  mark_launch(run);
+  ser_range_hist_kernel<<<dim3(k, (M + hs.threads - 1) / hs.threads, 2), hs.threads, hs.smem, run->stream>>>(
+      run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, sel, hs.smem > 0, a_hist, b_hist, stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
+/* rows [0, w) of every chain's window added into its accumulator record (ser_run_accumulate), on the run's stream */
 static int accumulate_window(ser_run *run, int w)
 {
-  const int N = run->N, M = run->M, nc = run->cfg.n_chains, W = run->cfg.max_samples, base = run->kp.sample_base;
-  if (run->acc_what & SER_ACC_PO) {
-    mark_launch(run);
-    ser_po_accum_kernel<<<dim3((N + 31) / 32, (N + 31) / 32, nc), 256, 0, run->stream>>>(run->d_samp_pi, run->d_scal, N, W, base, w, run->d_acc_po);
-    CUDA_TRY(cudaGetLastError());
+  const int what = run->acc_what, nc = run->cfg.n_chains;
+  const AccLayout L = acc_layout(run->N, run->M, what);
+  const SumSel sel = {nullptr, 0, 0, nullptr, run->kp.sample_base, w, nullptr};
+  int *acc = run->d_acc;
+  int rc = SER_OK;
+  if (what & SER_ACC_PO) rc = launch_po(run, sel, nc, one_dest(acc + L.po), L.ints, 1);
+  if (!rc && (what & (SER_ACC_SUMS | SER_ACC_AB))) {
+    const bool ab = what & SER_ACC_AB;
+    rc = launch_posterior(run, sel, nc, acc + L.pi, L.ints, ab ? acc + L.asum : nullptr, ab ? acc + L.bsum : nullptr, L.ints, nullptr, 1);
   }
-  if (run->acc_what & (SER_ACC_SUMS | SER_ACC_AB)) {
-    mark_launch(run);
-    ser_posterior_accum_kernel<<<nc, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w,
-                                                             run->d_acc_pi, run->d_acc_a, run->d_acc_b);
-    CUDA_TRY(cudaGetLastError());
-  }
-  if (run->acc_what & SER_ACC_ALIVE) {
-    mark_launch(run);
-    ser_alive_accum_kernel<<<dim3(nc, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w,
-                                                                               run->d_acc_alive);
-    CUDA_TRY(cudaGetLastError());
-  }
-  if (run->acc_what & SER_ACC_POS) {
-    HistShape hs;
-    CUDA_TRY(hist_shape((const void *)ser_pos_hist_accum_kernel, N, &hs));
-    mark_launch(run);
-    ser_pos_hist_accum_kernel<<<dim3(nc, (N + hs.threads - 1) / hs.threads), hs.threads, hs.smem, run->stream>>>(
-        run->d_samp_pi, run->d_scal, N, W, base, w, hs.smem > 0, run->d_acc_pos);
-    CUDA_TRY(cudaGetLastError());
-  }
-  if (run->acc_what & SER_ACC_RANGE) {
-    HistShape hs;
-    CUDA_TRY(hist_shape((const void *)ser_range_hist_accum_kernel, N + 1, &hs));
-    mark_launch(run);
-    ser_range_hist_accum_kernel<<<dim3(nc, (M + hs.threads - 1) / hs.threads, 2), hs.threads, hs.smem, run->stream>>>(
-        run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, base, w, hs.smem > 0, run->d_acc_range);
-    CUDA_TRY(cudaGetLastError());
-  }
-  return SER_OK;
+  if (!rc && (what & SER_ACC_ALIVE)) rc = launch_alive(run, sel, nc, acc + L.alive, L.ints, 1);
+  if (!rc && (what & SER_ACC_POS)) rc = launch_pos_hist(run, sel, nc, acc + L.pos, L.ints, 1);
+  if (!rc && (what & SER_ACC_RANGE)) rc = launch_range_hist(run, sel, nc, acc + L.range, acc + L.range + (size_t)run->M * (run->N + 1), L.ints, 1);
+  return rc;
 }
 
 extern "C" int ser_run_advance_both(ser_run *run, int32_t burn_calls, int32_t sample_calls)
@@ -1191,14 +1218,6 @@ extern "C" int ser_run_chain_stats(ser_run *run, double *e_negloglik, double *e_
   return SER_OK;
 }
 
-static PeerPtrs one_dest(void *ptr)
-{
-  PeerPtrs d;
-  memset(&d, 0, sizeof(d));
-  d.p[0] = ptr; d.n = 1;
-  return d;
-}
-
 /* E[-logL] of the local chains at dst[offset + chain] of every destination, on the run's stream */
 static int run_stats_to(ser_run *run, const PeerPtrs &dst, int offset)
 {
@@ -1213,12 +1232,7 @@ static int run_stats_to(ser_run *run, const PeerPtrs &dst, int offset)
 /* id_base = the id local chain 0 has in the numbering `d_chosen` uses */
 static int run_po_to(ser_run *run, const int32_t *d_chosen, int k, const PeerPtrs &dst, int id_base)
 {
-  dim3 grd((run->N + 31) / 32, (run->N + 31) / 32, k);
-  mark_launch(run);
-  ser_po_kernel<<<grd, 256, 0, run->stream>>>(run->d_samp_pi, run->d_scal, run->N, run->cfg.max_samples, d_chosen, id_base,
-                                              run->cfg.n_chains, run->d_chain_ids, dst);
-  CUDA_TRY(cudaGetLastError());
-  return SER_OK;
+  return launch_po(run, sel_chosen(run, d_chosen, id_base, run->cfg.max_samples, nullptr), k, dst, (size_t)run->N * run->N, 0);
 }
 
 extern "C" int ser_run_chain_stats_device(ser_run *run, double *d_e_negloglik)
@@ -1324,40 +1338,79 @@ extern "C" int ser_select_chains_device(const double *d_e, int32_t n, int32_t k,
   return SER_OK;
 }
 
+/* d_counts [k][N][N]; n_out[c] = T of a held chain when d_n is given */
+static int po_counts_to(ser_run *run, const int32_t *d_chosen, int k, int32_t *d_counts, int *d_n)
+{
+  if (run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_po_counts: run has no pi sample store"); return SER_E_STATE; }
+  if (!run->acc_what) /* T is read per chosen chain on the device: no host round trip */
+    return launch_po(run, sel_chosen(run, d_chosen, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, one_dest(d_counts),
+                     (size_t)run->N * run->N, 0);
+  if (!(run->acc_what & SER_ACC_PO)) { ser_set_error("ser_run_po_counts: the run accumulates without SER_ACC_PO"); return SER_E_STATE; }
+  const int N = run->N, nb = (int)std::min<long long>(((long long)N * N + 255) / 256, 1024);
+  const AccLayout L = acc_layout(N, run->M, run->acc_what);
+  mark_launch(run);
+  ser_po_acc_out_kernel<<<dim3(nb, k), 256, 0, run->stream>>>(run->d_acc + L.po, L.ints, run->d_scal, N,
+                                                              sel_chosen(run, d_chosen, run->cfg.chain_offset, INT_MAX, d_n), d_counts);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
 extern "C" int ser_run_po_counts_device(ser_run *run, const int32_t *d_chosen, int32_t k, int32_t *d_counts)
 {
   if (!run || !d_chosen || !d_counts || k < 1) return SER_E_ARG;
-  if (run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_po_counts: run has no pi sample store"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
-  if (run->acc_what) {
-    if (!(run->acc_what & SER_ACC_PO)) { ser_set_error("ser_run_po_counts: the run accumulates without SER_ACC_PO"); return SER_E_STATE; }
-    const int N = run->N, nb = (int)std::min<long long>(((long long)N * N + 255) / 256, 1024);
-    mark_launch(run);
-    ser_po_acc_out_kernel<<<dim3(nb, k), 256, 0, run->stream>>>(run->d_acc_po, run->d_scal, N, d_chosen, run->cfg.chain_offset, run->cfg.n_chains,
-                                                                run->d_chain_ids, d_counts);
-    CUDA_TRY(cudaGetLastError());
+  return po_counts_to(run, d_chosen, k, d_counts, nullptr);
+}
+
+/* One host output of a getter: k slabs of `bytes` each at `host` (nullptr: not wanted), staged through `dev`. */
+struct GetterOut {
+  void *host;
+  size_t bytes;
+  void *dev;
+};
+
+/* The shared part of the host getters over k chosen global ids: the ids go up, n_out[c] starts at -1 and `launch` (given the device
+ * ids and n_out) enqueues kernels that write T and the slabs of every chosen chain the run holds; those slabs come back to the host,
+ * the others stay as the caller passed them.  Every temporary is freed on every path. */
+template <class Launch>
+static int run_getter(ser_run *run, const int32_t *chosen, int k, std::vector<int> &n_out, std::initializer_list<GetterOut *> outs,
+                      Launch launch)
+{
+  int *d_ch = nullptr, *d_n = nullptr;
+  n_out.assign(k, -1);
+  auto body = [&]() -> int {
+    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
+    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
+    for (GetterOut *o : outs)
+      if (o->host) CUDA_TRY(POOL_ALLOC(&o->dev, k * o->bytes));
+    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
+    const int rc = launch(d_ch, d_n);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    for (int c = 0; c < k; c++)
+      for (GetterOut *o : outs)
+        if (o->host && n_out[c] >= 0)
+          CUDA_TRY(cudaMemcpyAsync((char *)o->host + c * o->bytes, (char *)o->dev + c * o->bytes, o->bytes, cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
     return SER_OK;
-  }
-  return run_po_to(run, d_chosen, k, one_dest(d_counts), run->cfg.chain_offset); /* T is read per chosen chain on the device: no host round trip */
+  };
+  const int rc = body();
+  if (d_ch) cudaFreeAsync(d_ch, run->stream);
+  if (d_n) cudaFreeAsync(d_n, run->stream);
+  for (GetterOut *o : outs)
+    if (o->dev) { cudaFreeAsync(o->dev, run->stream); o->dev = nullptr; }
+  return rc;
 }
 
 extern "C" int ser_run_po_counts(ser_run *run, const int32_t *chosen, int32_t k, int32_t *counts)
 {
   if (!run || !chosen || !counts || k < 1) return SER_E_ARG;
   if (set_device(run)) return SER_E_CUDA;
-  int *d_ch = nullptr, *d_cnt = nullptr;
-  const size_t nn = (size_t)k * run->N * run->N;
-  CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
-  CUDA_TRY(POOL_ALLOC(&d_cnt, nn * sizeof(int)));
-  CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, nn * sizeof(int), run->stream));
-  int rc = ser_run_po_counts_device(run, d_ch, k, d_cnt);
-  if (rc == SER_OK) {
-    if (cudaMemcpyAsync(counts, d_cnt, nn * sizeof(int), cudaMemcpyDeviceToHost, run->stream) != cudaSuccess ||
-        cudaStreamSynchronize(run->stream) != cudaSuccess) { ser_set_error("ser_run_po_counts: copy back failed"); rc = SER_E_CUDA; }
-  }
-  cudaFreeAsync(d_ch, run->stream); cudaFreeAsync(d_cnt, run->stream);
-  return rc;
+  GetterOut cnt = {counts, (size_t)run->N * run->N * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  return run_getter(run, chosen, k, n_out, {&cnt}, [&](const int *d_ch, int *d_n) { return po_counts_to(run, d_ch, k, (int *)cnt.dev, d_n); });
 }
 
 /* common sample count of the chosen chains this run owns (n_out[c] < 0: not owned) */
@@ -1383,46 +1436,21 @@ extern "C" int ser_run_posterior_sums(ser_run *run, const int32_t *chosen, int32
   if (run->acc_what && (a_sum || b_sum) && !(run->acc_what & SER_ACC_AB)) { ser_set_error("ser_run_posterior_sums: the run accumulates without SER_ACC_AB"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   const int N = run->N, M = run->M;
-  int *d_ch = nullptr, *d_pi = nullptr, *d_a = nullptr, *d_b = nullptr, *d_n = nullptr;
-  long long *d_corr = nullptr;
-  std::vector<int> n_out(k, -1);
-  int rc = SER_OK;
-  auto body = [&]() -> int {
-    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
-    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
-    CUDA_TRY(POOL_ALLOC(&d_corr, k * sizeof(long long)));
-    CUDA_TRY(POOL_ALLOC(&d_pi, (size_t)k * N * sizeof(int)));
-    if (a_sum) { CUDA_TRY(POOL_ALLOC(&d_a, (size_t)k * M * sizeof(int))); CUDA_TRY(POOL_ALLOC(&d_b, (size_t)k * M * sizeof(int))); }
-    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
-    CUDA_TRY(cudaMemcpyAsync(d_corr, corr_num, k * sizeof(long long), cudaMemcpyHostToDevice, run->stream));
-    CUDA_TRY(cudaMemcpyAsync(d_pi, pi_sum, (size_t)k * N * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-    if (a_sum) {
-      CUDA_TRY(cudaMemcpyAsync(d_a, a_sum, (size_t)k * M * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-      if (b_sum) CUDA_TRY(cudaMemcpyAsync(d_b, b_sum, (size_t)k * M * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-    }
+  GetterOut corr = {corr_num, sizeof(long long), nullptr}, pi = {pi_sum, N * sizeof(int), nullptr};
+  GetterOut a = {a_sum, M * sizeof(int), nullptr}, b = {b_sum, M * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&corr, &pi, &a, &b}, [&](const int *d_ch, int *d_n) -> int {
+    if (!run->acc_what)
+      return launch_posterior(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, (int *)pi.dev, N,
+                              (int *)a.dev, (int *)b.dev, M, (long long *)corr.dev, 0);
+    const AccLayout L = acc_layout(N, M, run->acc_what);
     mark_launch(run);
-    if (run->acc_what)
-      ser_posterior_acc_out_kernel<<<k, 256, 0, run->stream>>>(run->d_acc_pi, run->d_acc_a, run->d_acc_b, run->d_scal, N, M, d_ch, run->cfg.chain_offset,
-                                                               run->cfg.n_chains, run->d_chain_ids, d_corr, d_pi, d_a, b_sum ? d_b : nullptr, d_n);
-    else
-      ser_posterior_kernel<<<k, 256, 0, run->stream>>>(run->d_samp_pi, run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
-                                                       run->cfg.chain_offset, run->cfg.n_chains, run->d_chain_ids, d_corr, d_pi, d_a,
-                                                       b_sum ? d_b : nullptr, d_n);
+    ser_posterior_acc_out_kernel<<<k, 256, 0, run->stream>>>(run->d_acc + L.pi, run->d_acc + L.asum, run->d_acc + L.bsum, L.ints, run->d_scal,
+                                                             N, M, sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n),
+                                                             (long long *)corr.dev, (int *)pi.dev, (int *)a.dev, (int *)b.dev);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(corr_num, d_corr, k * sizeof(long long), cudaMemcpyDeviceToHost, run->stream));
-    CUDA_TRY(cudaMemcpyAsync(pi_sum, d_pi, (size_t)k * N * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    if (a_sum) {
-      CUDA_TRY(cudaMemcpyAsync(a_sum, d_a, (size_t)k * M * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-      if (b_sum) CUDA_TRY(cudaMemcpyAsync(b_sum, d_b, (size_t)k * M * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(run->stream));
     return SER_OK;
-  };
-  rc = body();
-  void *tmp[] = {d_ch, d_n, d_corr, d_pi, d_a, d_b};
-  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
+  });
   if (rc != SER_OK) return rc;
   return common_samples(n_out, n_samples, "ser_run_posterior_sums");
 }
@@ -1434,32 +1462,19 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
   if (run->acc_what && !(run->acc_what & SER_ACC_ALIVE)) { ser_set_error("ser_run_alive_counts: the run accumulates without SER_ACC_ALIVE"); return SER_E_STATE; }
   if (set_device(run)) return SER_E_CUDA;
   const int N = run->N, M = run->M;
-  const size_t cells = (size_t)k * N * M;
-  int *d_ch = nullptr, *d_alive = nullptr, *d_n = nullptr;
-  std::vector<int> n_out(k, -1);
-  auto body = [&]() -> int {
-    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
-    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
-    CUDA_TRY(POOL_ALLOC(&d_alive, cells * sizeof(int)));
-    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
-    CUDA_TRY(cudaMemcpyAsync(d_alive, alive, cells * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+  GetterOut out = {alive, (size_t)N * M * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&out}, [&](const int *d_ch, int *d_n) -> int {
+    if (!run->acc_what)
+      return launch_alive(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, (int *)out.dev, (size_t)N * M, 0);
+    const AccLayout L = acc_layout(N, M, run->acc_what);
     mark_launch(run);
-    if (run->acc_what)
-      ser_alive_acc_out_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_acc_alive, run->d_scal, N, M, d_ch, run->cfg.chain_offset,
-                                                                                   run->cfg.n_chains, run->d_chain_ids, d_alive, d_n);
-    else
-      ser_alive_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, N, M, run->cfg.max_samples, d_ch,
-                                                                         run->cfg.chain_offset, run->cfg.n_chains, run->d_chain_ids, d_alive, d_n);
+    ser_alive_acc_out_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_acc + L.alive, L.ints, run->d_scal, N, M,
+                                                                                 sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n),
+                                                                                 (int *)out.dev);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(alive, d_alive, cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    CUDA_TRY(cudaStreamSynchronize(run->stream));
     return SER_OK;
-  };
-  const int rc = body();
-  void *tmp[] = {d_ch, d_n, d_alive};
-  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
+  });
   if (rc != SER_OK) return rc;
   return common_samples(n_out, n_samples, "ser_run_alive_counts");
 }
@@ -1483,68 +1498,33 @@ extern "C" int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k,
   if (set_device(run)) return SER_E_CUDA;
   const int N = run->N, M = run->M;
   const size_t pos_cells = (size_t)N * N, range_cells = (size_t)M * (N + 1);
-  int *d_ch = nullptr, *d_n = nullptr, *d_pos = nullptr, *d_a = nullptr, *d_b = nullptr;
-  std::vector<int> n_out(k);
-  auto body = [&]() -> int {
-    CUDA_TRY(POOL_ALLOC(&d_ch, k * sizeof(int)));
-    CUDA_TRY(POOL_ALLOC(&d_n, k * sizeof(int)));
-    if (pos) CUDA_TRY(POOL_ALLOC(&d_pos, k * pos_cells * sizeof(int)));
-    if (a_hist) CUDA_TRY(POOL_ALLOC(&d_a, k * range_cells * sizeof(int)));
-    if (b_hist) CUDA_TRY(POOL_ALLOC(&d_b, k * range_cells * sizeof(int)));
-    CUDA_TRY(cudaMemcpyAsync(d_ch, chosen, k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-    CUDA_TRY(cudaMemsetAsync(d_n, 0xff, k * sizeof(int), run->stream));
-    const int *ids = run->d_chain_ids;
-    const int off = run->cfg.chain_offset, nl = run->cfg.n_chains;
-    if (run->acc_what) {
-      const int nb = 256;
-      if (pos) {
-        mark_launch(run);
-        ser_hist_acc_out_kernel<<<dim3(nb, k, 1), 256, 0, run->stream>>>(run->d_acc_pos, pos_cells, pos_cells, run->d_scal, d_ch, off, nl, ids,
-                                                                         d_pos, nullptr, d_n);
-        CUDA_TRY(cudaGetLastError());
-      }
-      if (ranges) {
-        mark_launch(run);
-        ser_hist_acc_out_kernel<<<dim3(nb, k, 2), 256, 0, run->stream>>>(run->d_acc_range, 2 * range_cells, range_cells, run->d_scal, d_ch, off,
-                                                                         nl, ids, d_a, d_b, d_n);
-        CUDA_TRY(cudaGetLastError());
-      }
-    } else {
-      const int W = run->cfg.max_samples;
-      if (pos) {
-        HistShape hs;
-        CUDA_TRY(hist_shape((const void *)ser_pos_hist_kernel, N, &hs));
-        mark_launch(run);
-        ser_pos_hist_kernel<<<dim3(k, (N + hs.threads - 1) / hs.threads), hs.threads, hs.smem, run->stream>>>(
-            run->d_samp_pi, run->d_scal, N, W, d_ch, off, nl, ids, hs.smem > 0, d_pos, d_n);
-        CUDA_TRY(cudaGetLastError());
-      }
-      if (ranges) {
-        HistShape hs;
-        CUDA_TRY(hist_shape((const void *)ser_range_hist_kernel, N + 1, &hs));
-        mark_launch(run);
-        ser_range_hist_kernel<<<dim3(k, (M + hs.threads - 1) / hs.threads, 2), hs.threads, hs.smem, run->stream>>>(
-            run->d_samp_a, run->d_samp_b, run->d_scal, N, M, W, d_ch, off, nl, ids, hs.smem > 0, d_a, d_b, d_n);
-        CUDA_TRY(cudaGetLastError());
-      }
+  GetterOut p = {pos, pos_cells * sizeof(int), nullptr}, a = {a_hist, range_cells * sizeof(int), nullptr}, b = {b_hist, range_cells * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&p, &a, &b}, [&](const int *d_ch, int *d_n) -> int {
+    if (!run->acc_what) {
+      const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n);
+      int rc = pos ? launch_pos_hist(run, sel, k, (int *)p.dev, pos_cells, 0) : SER_OK;
+      if (!rc && ranges) rc = launch_range_hist(run, sel, k, (int *)a.dev, (int *)b.dev, range_cells, 0);
+      return rc;
     }
-    CUDA_TRY(cudaMemcpyAsync(n_out.data(), d_n, k * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-    CUDA_TRY(cudaStreamSynchronize(run->stream));
-    /* only the slabs of held chains come back: the others stay as the caller left them */
-    for (int c = 0; c < k; c++) {
-      if (n_out[c] < 0) continue;
-      if (pos) CUDA_TRY(cudaMemcpyAsync(pos + c * pos_cells, d_pos + c * pos_cells, pos_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-      if (a_hist) CUDA_TRY(cudaMemcpyAsync(a_hist + c * range_cells, d_a + c * range_cells, range_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
-      if (b_hist) CUDA_TRY(cudaMemcpyAsync(b_hist + c * range_cells, d_b + c * range_cells, range_cells * sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+    const AccLayout L = acc_layout(N, M, run->acc_what);
+    const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
+    if (pos) {
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3(256, k, 1), 256, 0, run->stream>>>(run->d_acc + L.pos, L.ints, pos_cells, run->d_scal, sel, (int *)p.dev, nullptr);
+      CUDA_TRY(cudaGetLastError());
     }
-    CUDA_TRY(cudaStreamSynchronize(run->stream));
-    for (int c = 0; c < k; c++) n_samples[c] = n_out[c] < 0 ? 0 : n_out[c];
+    if (ranges) {
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.range, L.ints, range_cells, run->d_scal, sel, (int *)a.dev,
+                                                                        (int *)b.dev);
+      CUDA_TRY(cudaGetLastError());
+    }
     return SER_OK;
-  };
-  const int rc = body();
-  void *tmp[] = {d_ch, d_n, d_pos, d_a, d_b};
-  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
-  return rc;
+  });
+  if (rc != SER_OK) return rc;
+  for (int c = 0; c < k; c++) n_samples[c] = n_out[c] < 0 ? 0 : n_out[c];
+  return SER_OK;
 }
 
 extern "C" int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, int32_t max_lag, double *stats,

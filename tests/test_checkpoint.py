@@ -56,6 +56,8 @@ def _layout(N, M, manycd, store, rows, acc):
     take("asum", 4 * M if acc & 4 else 0)
     take("bsum", 4 * M if acc & 4 else 0)
     take("alive", 4 * N * M if acc & 8 else 0)
+    take("pos", 4 * N * N if acc & 16 else 0)
+    take("range", 8 * M * (N + 1) if acc & 32 else 0)
     take("rpi", 2 * N)
     take("ab", 4 * M)
     take("spi", 2 * N * rows if store >= 1 else 0)
@@ -235,6 +237,39 @@ def test_accumulating_run_resumes_mid_window(S, tmp_path):
     for k in want:
         assert np.array_equal(np.asarray(got[k]), np.asarray(want[k])), k
     _same_stats(rest, whole)
+
+
+@pytest.mark.gpu
+def test_accumulator_parts_sit_where_the_layout_puts_them(S, tmp_path):
+    ds = S.Dataset.from_bits(*load_hex_dataset("g10s10"))
+    N, M, n, T = ds.N, ds.M, 3, 23
+    flags = dict(po=True, sums=True, ab=True, alive=True, positions=True, ranges=True)
+    run = S.Run(ds, n, seed=9, store=S.STORE_FULL, max_samples=16).init().accumulate(**flags).advance(4, False).advance(T, True).sync()
+    f = tmp_path / "ck"
+    run.save_checkpoint(f)                                              # mid-window: 23 samples through a window of 16
+    data = f.read_bytes()
+    acc, rows, size = struct.unpack_from("<i", data, 60)[0], struct.unpack_from("<i", data, 80)[0], struct.unpack_from("<Q", data, 88)[0]
+    assert acc == 63
+    L = _layout(N, M, 0, S.STORE_FULL, rows, acc)
+    assert L["size"] == size
+    chosen = list(range(n))
+    po, ps, (alive, t), m = run.po_counts(chosen), run.posterior_sums(chosen, with_ab=True), run.alive_counts(chosen), run.marginals(chosen, ranges=True)
+    assert t == ps["n_samples"] == T
+    first = HEADER + (4 * n + 7) // 8 * 8 + 8
+    for c in range(n):
+        rec = data[first + c * size:first + (c + 1) * size]
+
+        def part(name, *shape):
+            return np.frombuffer(rec, np.int32, int(np.prod(shape)), L[name]).reshape(shape)
+        want_po = po[c].copy()
+        np.fill_diagonal(want_po, 0)
+        assert np.array_equal(part("po", N, N), want_po), c
+        assert np.array_equal(part("pi", N), ps["pi_sum"][c]), c
+        assert np.array_equal(part("asum", M), ps["a_sum"][c]) and np.array_equal(part("bsum", M), ps["b_sum"][c]), c
+        assert np.array_equal(np.cumsum(part("alive", N, M), axis=0), alive[c]), c
+        assert np.array_equal(part("pos", N, N), m["pos"][c]), c
+        ab = part("range", 2, M, N + 1)
+        assert np.array_equal(ab[0], m["a"][c]) and np.array_equal(ab[1], m["b"][c]), c
 
 
 @pytest.mark.gpu

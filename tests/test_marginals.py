@@ -88,14 +88,14 @@ def test_marginals_argument_checks_without_a_device(S):
     assert L.ser_run_accumulate(None, 16 | 32) == E_ARG
 
 
-def test_histogram_kernels_are_built_for_sm100a_without_spills(S):
+def test_summary_kernels_are_built_for_sm100a_without_stack_or_spills(S):
     exe = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
     if not os.path.exists(exe):
         pytest.skip("cuobjdump is not installed")
     out = subprocess.run([exe, "-res-usage", S.LIB_PATH], check=True, capture_output=True, text=True).stdout
     assert "sm_100a" in out
-    names = ("ser_pos_hist_kernel", "ser_range_hist_kernel", "ser_pos_hist_accum_kernel", "ser_range_hist_accum_kernel",
-             "ser_hist_acc_out_kernel")
+    names = ("ser_po_kernel", "ser_posterior_kernel", "ser_alive_kernel", "ser_pos_hist_kernel", "ser_range_hist_kernel",
+             "ser_po_acc_out_kernel", "ser_posterior_acc_out_kernel", "ser_alive_acc_out_kernel", "ser_hist_acc_out_kernel")
     lines = out.splitlines()
     for name in names:
         idx = [i for i, ln in enumerate(lines) if "Function" in ln and name in ln]

@@ -139,18 +139,36 @@ def test_streaming_summaries_equal_the_one_shot_store(S, tmp_path):
 @pytest.mark.gpu
 def test_a_chosen_id_the_run_does_not_hold_leaves_its_slab_untouched(S):
     ds = S.Dataset.from_bits(*load_hex_dataset("g10s10"))
-    sub = S.Run(ds, 0, seed=2, store=S.STORE_FULL, max_samples=3, chain_ids=[7, 30]).init().accumulate(ab=True, alive=True)
-    sub.advance(2, False).advance(5, True).sync()
+    kw = dict(seed=2, store=S.STORE_FULL, chain_ids=[7, 30])
+    streaming = S.Run(ds, 0, max_samples=3, **kw).init().accumulate(ab=True, alive=True, positions=True, ranges=True)
+    one_shot = S.Run(ds, 0, max_samples=5, **kw).init()
     chosen = np.array([30, 8, 7], np.int32)
     k, N, M = 3, ds.N, ds.M
-    corr, pi = np.full(k, 7, np.int64), np.full((k, N), 7, np.int32)
-    alive, n = np.full((k, N, M), 7, np.int32), C.c_int32()
     i32 = C.POINTER(C.c_int32)
-    assert S.lib().ser_run_posterior_sums(sub._h, chosen.ctypes.data_as(i32), k, corr.ctypes.data_as(C.POINTER(C.c_int64)),
-                                          pi.ctypes.data_as(i32), None, None, C.byref(n)) == 0
-    assert S.lib().ser_run_alive_counts(sub._h, chosen.ctypes.data_as(i32), k, alive.ctypes.data_as(i32), C.byref(n)) == 0
-    assert n.value == 5 and corr[1] == 7 and np.all(pi[1] == 7) and np.all(alive[1] == 7)
-    assert np.all(pi[[0, 2]].sum(axis=1) == 5 * N * (N - 1) // 2) and np.all(alive[[0, 2]] != 7)
+    for what, run in (("streaming", streaming), ("one-shot", one_shot)):
+        run.advance(2, False).advance(5, True).sync()
+        corr, pi = np.full(k, 7, np.int64), np.full((k, N), 7, np.int32)
+        alive, n = np.full((k, N, M), 7, np.int32), C.c_int32()
+        po, pos, nm = np.full((k, N, N), 7, np.int32), np.full((k, N, N), 7, np.int32), np.full(k, 7, np.int32)
+        ah, bh = np.full((k, M, N + 1), 7, np.int32), np.full((k, M, N + 1), 7, np.int32)
+        assert S.lib().ser_run_posterior_sums(run._h, chosen.ctypes.data_as(i32), k, corr.ctypes.data_as(C.POINTER(C.c_int64)),
+                                              pi.ctypes.data_as(i32), None, None, C.byref(n)) == 0
+        assert S.lib().ser_run_alive_counts(run._h, chosen.ctypes.data_as(i32), k, alive.ctypes.data_as(i32), C.byref(n)) == 0
+        assert S.lib().ser_run_po_counts(run._h, chosen.ctypes.data_as(i32), k, po.ctypes.data_as(i32)) == 0
+        assert S.lib().ser_run_marginals(run._h, chosen.ctypes.data_as(i32), k, pos.ctypes.data_as(i32), ah.ctypes.data_as(i32),
+                                         bh.ctypes.data_as(i32), nm.ctypes.data_as(i32)) == 0
+        assert n.value == 5 and corr[1] == 7 and np.all(pi[1] == 7) and np.all(alive[1] == 7), what
+        assert np.all(po[1] == 7) and np.all(pos[1] == 7) and np.all(ah[1] == 7) and np.all(bh[1] == 7) and nm.tolist() == [5, 0, 5], what
+        assert np.all(pi[[0, 2]].sum(axis=1) == 5 * N * (N - 1) // 2) and np.all(alive[[0, 2]] != 7), what
+        # a held slab is written in full, whatever the caller preset: corr_num included
+        assert np.array_equal(corr[[0, 2]], pi[[0, 2]].astype(np.int64) @ np.arange(N)), what
+        for c, g in ((0, 30), (2, 7)):
+            m = run.marginals([g], ranges=True)
+            assert np.array_equal(po[c], run.po_counts([g])[0]) and np.all(np.diagonal(po[c]) == -5), (what, g)
+            assert np.array_equal(pos[c], m["pos"][0]) and np.array_equal(ah[c], m["a"][0]) and np.array_equal(bh[c], m["b"][0]), (what, g)
+    for c, local in ((0, 1), (2, 0)):
+        rows = one_shot.fetch_samples(local)["pi"].astype(np.int64)
+        assert corr[c] == (rows @ np.arange(N)).sum()
 
 
 @pytest.mark.gpu

@@ -11,7 +11,8 @@ the slabs back and synchronises), taken in the same loop.
 Phase 2 of select-then-replay (the k chosen chains of a 65 536-chain phase 1 re-simulated alone at 1000 + 1000 calls through a
 window of W samples), without the marginals (SER_STORE_PI, SER_ACC_PO | SER_ACC_SUMS, as replay_selected_time.py) and with them
 (SER_STORE_FULL, + SER_ACC_POS | SER_ACC_RANGE): wall time, CUDA-event time of the sweep launches, and in a separate profiled
-pass the summed device time of the accumulation kernels.  The card's name and power limit are read in the same process.
+pass the summed device time of the accumulation kernels: the summary kernels serve both paths, so in a pass that only advances
+the run every launch of them is an accumulation.  The card's name and power limit are read in the same process.
 --quick shrinks everything to a rehearsal.
 """
 import argparse
@@ -29,7 +30,7 @@ import seriation_b200 as S  # noqa: E402
 from tools.datasets import load_hex_dataset  # noqa: E402
 
 ONE_SHOT = ("ser_pos_hist_kernel", "ser_range_hist_kernel")
-ACC = ("ser_po_accum_kernel", "ser_posterior_accum_kernel", "ser_pos_hist_accum_kernel", "ser_range_hist_accum_kernel")
+ACC = ("ser_po_kernel", "ser_posterior_kernel", "ser_pos_hist_kernel", "ser_range_hist_kernel")
 
 
 def kernel_ms(prof, names):

@@ -6,7 +6,8 @@ of W samples (ser_run_accumulate), at the reference's 1000 + 1000 schedule.
 
 Per case and window: phase-2 wall time (host clock around the launches and a final synchronise), the CUDA-event time of the
 sweep launches alone, and the summed kernel time of the accumulation kernels (torch.profiler, in a separate profiled pass
-so the wall time is taken without tracing).  Device memory of each phase = memory in use (cudaMemGetInfo) after the phase's
+so the wall time is taken without tracing; that pass only advances the run, so every launch of a summary kernel in it is an
+accumulation).  Device memory of each phase = memory in use (cudaMemGetInfo) after the phase's
 run is created, initialised and has taken a sample, minus what was in use before; the library's pool keeps no freed blocks
 (SER_POOL_KEEP_MB=0).  Phase 1 runs only 1 + 1 calls: it is here for its memory and to choose the chains, whose phase-2
 cost does not depend on which chains they are.  --quick shortens everything to a rehearsal.
@@ -24,7 +25,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import seriation_b200 as S  # noqa: E402
 from tools.datasets import load_hex_dataset  # noqa: E402
 
-ACC_KERNELS = ("ser_po_accum_kernel", "ser_posterior_accum_kernel")
+ACC_KERNELS = ("ser_po_kernel", "ser_posterior_kernel")
 
 
 def used_bytes(torch):
