@@ -122,7 +122,7 @@ int ser_run_sync(ser_run *run);
 int ser_run_elapsed_ms(ser_run *run, double *ms, int32_t reset);
 int ser_run_kernel_launches(const ser_run *run, int64_t *n);
 /* which sweep kernel serves this run's shape: 0 = one thread per taxon (ser_sweep_kernel), 1 = large-shape kernel with
- * CTA-wide column groups, 2 = large-shape kernel with warp batches, 3 = cluster kernel */
+ * CTA-wide column groups, 2 = large-shape kernel with warp batches */
 int ser_run_kernel_path(const ser_run *run, int32_t *path);
 /* The warp batches the large-shape kernel's Gibbs phase would use for a matrix whose sorted columns hold ones_sorted[c] ones, with
  * slices of `wcap` items per warp (host only; no device needed): batches[4 b ..] = {first column, columns | lane shift << 16,

@@ -306,8 +306,7 @@ class Run:
         return n.value
 
     def kernel_path(self) -> int:
-        """0 = one thread per taxon, 1 = large-shape kernel (CTA-wide column groups), 2 = large-shape kernel (warp batches),
-        3 = cluster kernel"""
+        """0 = one thread per taxon, 1 = large-shape kernel (CTA-wide column groups), 2 = large-shape kernel (warp batches)"""
         n = C.c_int32()
         _check(lib().ser_run_kernel_path(self._h, C.byref(n)))
         return n.value

@@ -96,12 +96,6 @@ struct KParams {
    * Ival doubles: a smaller buffer = more resident chains per SM */
   int n_groups, Ival;
   int grp_c[SER_MAX_GROUPS + 1], grp_e[SER_MAX_GROUPS + 1];
-  /* cluster path (ser_sweep_kernel_cl): one chain per cluster of cl_R CTAs, sorted column gc owned by rank gc % cl_R */
-  int cl_R, cl_Mc, cl_icap, cl_gcap;
-  const int *cl_off;        /* [M] first item of column gc inside its rank's item numbering */
-  const uint32_t *cl_item;  /* per rank, concatenated: item -> (local column << 16) | index inside the column */
-  const int *cl_grp;        /* per rank, concatenated: column groups as {first local column, first item} pairs */
-  int cl_item_base[9], cl_grp_base[9]; /* [rank] first entry of the rank's part (cl_grp_base in pairs) */
   /* units of the Gibbs phase: heavy columns are served by 2, 4, .. 32 adjacent lanes (ser_sweep_kernel.cuh) */
   const uint2 *unit_tab; /* [n_units] = {column | sub << 16 | lsh << 24, first item of the column} */
   int n_units;

@@ -36,10 +36,19 @@
 #include "ser_device_common.cuh"
 #include "ser_sweep_kernel.cuh"
 #include "ser_sweep_kernel_big.cuh"
-#include "ser_sweep_kernel_cluster.cuh"
 #include "ser_aux_kernels.cuh"
 
 /* ================================================================== host side: the run object */
+/* The sweep kernel instantiations a run can launch.  One thread per taxon, [manycd][variant]: variant 0 = 64 registers, any
+ * block size; variant 1 = 80 registers, blocks of <= 384 threads, two of them resident.  Large shapes, [warp][manycd]: the Gibbs
+ * phase in CTA-wide column groups (warp = 0) or in warp batches (1).  The entries' order is the order the instantiations are
+ * compiled in, and it matters: with <false, true> listed before <true, false>, those two get another register allocation. */
+typedef void (*SweepFn)(KParams);
+static const SweepFn SWEEP_SMALL[2][2] = {{ser_sweep_kernel<1024, 1, false>, ser_sweep_kernel<384, 2, false>},
+                                          {ser_sweep_kernel<1024, 1, true>, ser_sweep_kernel<384, 2, true>}};
+static const SweepFn SWEEP_BIG[2][2] = {{ser_sweep_kernel_big<false, false>, ser_sweep_kernel_big<true, false>},
+                                        {ser_sweep_kernel_big<false, true>, ser_sweep_kernel_big<true, true>}};
+
 #define CUDA_TRY(expr)                                                                          \
   do {                                                                                          \
     cudaError_t e__ = (expr);                                                                   \
@@ -68,7 +77,6 @@ struct ser_run {
   unsigned long long *d_tape_off;
   uint16_t *d_samp_a, *d_samp_b, *d_samp_pi;
   double *d_samp_cdl, *d_cd4, *d_samp_cd_all;
-  size_t smem_many;
   int *d_scratch_i; /* export buffers: a,b,pi,rpi,cnt[4M] */
   int *d_bad;
   cudaStream_t stream;
@@ -76,25 +84,24 @@ struct ser_run {
   int timing_open;
   double elapsed_ms;
   long long launches;
-  size_t smem_sweep, smem_init, smem_small, smem_big;
-  int Caux, big, big_threads, big_slots, variant, variant_many;
+  size_t smem_init, smem_small;
+  int Caux, big, big_threads;
   uint32_t *d_gV;
   uint16_t *d_gpre;
   int *d_bgrp;
   int4 *d_bbat;
   int big_warp; /* the Gibbs phase of the large-shape kernel runs warp batches (else CTA-wide column groups) */
-  /* cluster path of the large shapes */
-  int cl_mode, cl_R, cl_clusters;
-  size_t smem_cl;
-  int *d_cl_off, *d_cl_grp;
-  uint32_t *d_cl_item;
+  /* the sweep kernel instantiation the run launches (SWEEP_SMALL / SWEEP_BIG), its block size and dynamic shared memory */
+  SweepFn sweep_fn;
+  int sweep_block;
+  size_t sweep_smem;
+  int sweep_slots; /* resident CTAs of sweep_fn on the whole device; on the large-shape path no more than chains (one gV slot each) */
   int initialized, have_tapes;
   /* persistent work-queue grid of ser_sweep_kernel: (chain, chunk of calls) items, see ser_run_advance_both */
   uint32_t *d_V;            /* [chain][W][C] bit columns carried between work items */
   unsigned int *d_queue;    /* next work item of the running launch */
   unsigned int *d_done;     /* [chain] work items completed since init (monotonic) */
   unsigned int chunks_done; /* host mirror: items every chain has completed before the next launch */
-  int sweep_slots;          /* resident CTAs of the chosen sweep instantiation on the whole device */
   /* cross-chain step on the run's stream (ser_run_cross_chain_async) */
   double *d_e_all, *d_info;
   int *d_chosen, *d_counts;
@@ -177,7 +184,7 @@ static void mark_launch(ser_run *run)
 #define SER_SMEM_DYN_MAX (SER_SMEM_OPTIN - 1024) /* the sweep kernels hold 1 KB of static shared memory */
 static cudaError_t allow_max_dynamic_smem(void)
 {
-  /* once per device: seven driver calls that run creation (the e2e path creates a run per job) need not repeat */
+  /* once per device: driver calls that run creation (the e2e path creates a run per job) need not repeat */
   static std::mutex mu;
   static bool done[64] = {false};
   int dev = 0;
@@ -191,15 +198,11 @@ static cudaError_t allow_max_dynamic_smem(void)
     if (e == cudaSuccess) e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SER_SMEM_OPTIN - (int)fa.sharedSizeBytes);
   };
   allow((const void *)ser_init_kernel);
-  allow((const void *)ser_sweep_kernel<1024, 1, false>);
-  allow((const void *)ser_sweep_kernel<384, 2, false>);
-  allow((const void *)ser_sweep_kernel<1024, 1, true>);
-  allow((const void *)ser_sweep_kernel<384, 2, true>);
-  allow((const void *)ser_sweep_kernel_big<false, false>);
-  allow((const void *)ser_sweep_kernel_big<true, false>);
-  allow((const void *)ser_sweep_kernel_big<false, true>);
-  allow((const void *)ser_sweep_kernel_big<true, true>);
-  allow((const void *)ser_sweep_kernel_cl);
+  for (int m = 0; m < 2; m++)
+    for (int v = 0; v < 2; v++) {
+      allow((const void *)SWEEP_SMALL[m][v]);
+      allow((const void *)SWEEP_BIG[m][v]);
+    }
   if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
   return e;
 }
@@ -411,118 +414,27 @@ static int run_create_impl(const ser_dataset *ds, const ser_run_config *cfg, ser
   run->smem_small = aux_layout(nullptr, nullptr, N);
   run->smem_init = run->smem_small + sizeof(double) * 2 * N + sizeof(uint16_t) * 3 * N + 64;
   CUDA_TRY(allow_max_dynamic_smem());
-  if (cfg->manycd) {
-    /* per-taxon c, d: one thread per taxon while the chain's columns and postings fit shared memory, else (or with
-     * SER_FORCE_BIG) the large-shape slot kernel's per-taxon instantiation.  The one-thread-per-taxon kernel needs its 80
-     * registers (2.7 M vs 2.5 M sweeps/s on g2s2 with 64): the groups are sized for the instantiation that will run. */
-    int rc = SER_E_ARG;
-    if (!run->big)
-      rc = run->C <= 384 ? choose_groups(kp, off, M, N, run->W, run->C, 1, ser_sweep_kernel<384, 2, true>, &run->smem_many)
-                         : choose_groups(kp, off, M, N, run->W, run->C, 1, ser_sweep_kernel<1024, 1, true>, &run->smem_many);
+  const int manycd = cfg->manycd;
+  if (!run->big) {
+    /* one thread per column while the columns, postings and one group's item weights fit shared memory, else (or with
+     * SER_FORCE_BIG) the large-shape kernel.  The groups are sized on the 80-register variant for per-taxon c, d in blocks of
+     * up to 384 threads, which needs those registers (2.7 M vs 2.5 M sweeps/s on g2s2 with 64), else on the 64-register one.
+     * Then the variant with more resident CTAs runs, the roomier one on a tie; SER_SWEEP_VARIANT forces it. */
+    const bool fits85 = run->C <= 384;
+    const int rc = choose_groups(kp, off, M, N, run->W, run->C, manycd, SWEEP_SMALL[manycd][manycd && fits85], &run->sweep_smem);
     if (rc == SER_E_CUDA) return rc;
     if (rc != SER_OK) run->big = 1;
     else {
       int occ64 = 0, occ85 = 0;
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ64, ser_sweep_kernel<1024, 1, true>, run->C, run->smem_many));
-      if (run->C <= 384) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ85, ser_sweep_kernel<384, 2, true>, run->C, run->smem_many));
-      run->variant_many = (occ85 >= occ64 && occ85 > 0) ? 1 : 0;
-    }
-  } else if (!run->big) {
-    /* one thread per column while the columns, postings and one group's item weights fit shared memory
-     * (SER_PREFER_BIG=1: only while ALL item weights fit, the pre-grouping rule); else the large-shape kernel */
-    const bool prefer_big = getenv("SER_PREFER_BIG") && atoi(getenv("SER_PREFER_BIG")) != 0;
-    int rc = SER_E_ARG;
-    if (!prefer_big || smem_layout(nullptr, nullptr, N, run->W, run->C, run->kp.I) <= SER_SMEM_DYN_MAX)
-      rc = choose_groups(kp, off, M, N, run->W, run->C, 0, ser_sweep_kernel<1024, 1, false>, &run->smem_sweep);
-    if (rc == SER_E_CUDA) return rc;
-    if (rc != SER_OK) run->big = 1;
-    else {
-      /* two register budgets: 64 regs (any block size) and 80 regs (blocks <= 384 threads, two of
-       * them resident); take the one with more resident CTAs, the roomier one on a tie */
-      int occ64 = 0, occ85 = 0;
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ64, ser_sweep_kernel<1024, 1, false>, run->C, run->smem_sweep));
-      if (run->C <= 384) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ85, ser_sweep_kernel<384, 2, false>, run->C, run->smem_sweep));
-      run->variant = (occ85 >= occ64 && occ85 > 0) ? 1 : 0;
-      if (const char *v = getenv("SER_SWEEP_VARIANT")) run->variant = (atoi(v) == 1 && run->C <= 384) ? 1 : 0;
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ64, SWEEP_SMALL[manycd][0], run->C, run->sweep_smem));
+      if (fits85) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ85, SWEEP_SMALL[manycd][1], run->C, run->sweep_smem));
+      int variant = (occ85 >= occ64 && occ85 > 0) ? 1 : 0;
+      if (const char *v = getenv("SER_SWEEP_VARIANT")) variant = (atoi(v) == 1 && fits85) ? 1 : 0;
+      run->sweep_fn = SWEEP_SMALL[manycd][variant];
+      run->sweep_block = run->C;
     }
   }
-  if (run->big && !cfg->manycd && getenv("SER_BIG_MODE") && !strcmp(getenv("SER_BIG_MODE"), "cluster")) {
-    /* Cluster path (opt-in, SER_BIG_MODE=cluster): the chain's bit columns sharded over the shared memory of R CTAs
-     * (ser_sweep_kernel_cluster.cuh).  It removes the HBM re-streaming of the slot path, but on the 1024 x 4096 matrix it
-     * needs R = 8, and the per-proposal latency chain, replicated in 8 CTAs, costs more than the DRAM round trips it saves
-     * (measured 93 k vs 160 k sweeps/s, profiles/r02): the slot path stays the default.
-     * R = the smallest cluster whose CTAs hold their share of the columns + prefix tables and an item buffer of at least
-     * max(M, N + 1, 4096) items (M: the per-taxon terms of the exact sums are gathered there); SER_CLUSTER_R forces it. */
-    int force_r = 0;
-    if (const char *v = getenv("SER_CLUSTER_R")) force_r = atoi(v);
-    for (int R = 1; R <= SER_CL_MAXR && !run->cl_mode; R <<= 1) {
-      if (force_r && R != force_r) continue;
-      if (R > 1 && M < 2 * R) continue;
-      const int Mc = (M + R - 1) / R, gcap = std::min(Mc, 256);
-      const size_t fixed = cl_layout(nullptr, nullptr, N, run->W, Mc, 0, gcap);
-      const long long want = std::max(std::max(M, N + 1), 4096);
-      long long icap = ((long long)SER_SMEM_DYN_MAX - (long long)fixed - 64) / 10 / 32 * 32; /* val 8 + pos 2 bytes per item */
-      if (icap < want) continue;
-      /* per-rank item numbering, item tables and column groups */
-      std::vector<int> cl_off(M, 0), grp_all;
-      std::vector<uint32_t> item_all;
-      long long max_items = 0;
-      for (int r = 0; r < R; r++) {
-        kp.cl_item_base[r] = (int)item_all.size();
-        kp.cl_grp_base[r] = (int)grp_all.size() / 2;
-        const int nloc = (M - r + R - 1) / R;
-        std::vector<int> loff(nloc + 1, 0);
-        for (int lc = 0; lc < nloc; lc++) {
-          const int gc = lc * R + r;
-          cl_off[gc] = loff[lc];
-          loff[lc + 1] = loff[lc] + ones[gc] + 1;
-          for (int kk = 0; kk <= ones[gc]; kk++) item_all.push_back(((uint32_t)lc << 16) | (uint32_t)kk);
-        }
-        max_items = std::max<long long>(max_items, loff[nloc]);
-        const long long cap = std::min<long long>(icap, ((long long)loff[nloc] + 31) / 32 * 32);
-        int c0 = 0;
-        while (c0 < nloc) {
-          int c1 = c0;
-          while (c1 < nloc && c1 - c0 < gcap && loff[c1 + 1] - loff[c0] <= cap) c1++;
-          if (c1 == c0) { c1 = c0 + 1; } /* cannot happen: icap >= N + 1 >= one column */
-          grp_all.push_back(c0); grp_all.push_back(loff[c0]);
-          c0 = c1;
-        }
-        grp_all.push_back(nloc); grp_all.push_back(loff[nloc]);
-      }
-      kp.cl_item_base[R] = (int)item_all.size();
-      kp.cl_grp_base[R] = (int)grp_all.size() / 2;
-      icap = std::min<long long>(icap, std::max<long long>(want, (max_items + 31) / 32 * 32));
-      kp.cl_R = R; kp.cl_Mc = Mc; kp.cl_icap = (int)icap; kp.cl_gcap = gcap;
-      run->smem_cl = cl_layout(nullptr, nullptr, N, run->W, Mc, (int)icap, gcap);
-      /* how many clusters the device holds at once */
-      cudaLaunchConfig_t lc;
-      memset(&lc, 0, sizeof(lc));
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = R; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      lc.gridDim = dim3(R * 64, 1, 1); lc.blockDim = dim3(run->big_threads, 1, 1); lc.dynamicSmemBytes = run->smem_cl;
-      lc.attrs = at; lc.numAttrs = 1;
-      int n_cl = 0;
-      if (cudaOccupancyMaxActiveClusters(&n_cl, ser_sweep_kernel_cl, &lc) != cudaSuccess || n_cl < 1) { cudaGetLastError(); continue; }
-      if (const char *v = getenv("SER_CLUSTERS")) n_cl = std::max(1, std::min(n_cl, atoi(v)));
-      run->cl_clusters = std::max(1, std::min(cfg->n_chains, n_cl));
-      CUDA_TRY(POOL_ALLOC(&run->d_cl_off, (size_t)M * sizeof(int)));
-      CUDA_TRY(POOL_ALLOC(&run->d_cl_item, item_all.size() * sizeof(uint32_t)));
-      CUDA_TRY(POOL_ALLOC(&run->d_cl_grp, grp_all.size() * sizeof(int)));
-      CUDA_TRY(cudaMemcpyAsync(run->d_cl_off, cl_off.data(), (size_t)M * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-      CUDA_TRY(cudaMemcpyAsync(run->d_cl_item, item_all.data(), item_all.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, run->stream));
-      CUDA_TRY(cudaMemcpyAsync(run->d_cl_grp, grp_all.data(), grp_all.size() * sizeof(int), cudaMemcpyHostToDevice, run->stream));
-      CUDA_TRY(cudaStreamSynchronize(run->stream));
-      kp.cl_off = run->d_cl_off; kp.cl_item = run->d_cl_item; kp.cl_grp = run->d_cl_grp;
-      run->cl_mode = 1; run->cl_R = R;
-    }
-    if (!run->cl_mode && getenv("SER_BIG_MODE") && !strcmp(getenv("SER_BIG_MODE"), "cluster")) {
-      ser_set_error("ser_run_create: the shape does not fit the shared memory of a cluster of up to %d CTAs", SER_CL_MAXR);
-      return SER_E_ARG;
-    }
-  }
-  if (run->big && !run->cl_mode) {
+  if (run->big) {
     /* column groups of the Gibbs phase: as many items as the shared-memory budget holds
      * (SER_BIG_SMEM_KB, default 220), at most 1024 columns, never splitting a column */
     int budget_kb = 220;
@@ -586,21 +498,24 @@ static int run_create_impl(const ser_dataset *ds, const ser_run_config *cfg, ser
     CUDA_TRY(cudaMemcpyAsync(run->d_bgrp, bgrp.data(), bgrp.size() * sizeof(int), cudaMemcpyHostToDevice, run->stream));
     CUDA_TRY(cudaStreamSynchronize(run->stream));
     kp.bgrp = run->d_bgrp;
-    run->smem_big = big_layout(nullptr, nullptr, N, M, (int)icap, gcap, cfg->manycd, run->big_warp ? 32 * (run->big_threads / 32) : gcap);
-    if (run->smem_big > SER_SMEM_DYN_MAX) { ser_set_error("ser_run_create: shape needs %zu B of shared memory per chain", run->smem_big); return SER_E_ARG; }
-    int per_sm = 1, n_sm = 1;
-    if (cfg->manycd) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel_big<true, false>, run->big_threads, run->smem_big));
-    else CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel_big<false, false>, run->big_threads, run->smem_big));
-    CUDA_TRY(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, cfg->device));
-    run->big_slots = std::max(1, std::min(cfg->n_chains, per_sm * n_sm));
+    run->sweep_smem = big_layout(nullptr, nullptr, N, M, (int)icap, gcap, cfg->manycd, run->big_warp ? 32 * (run->big_threads / 32) : gcap);
+    if (run->sweep_smem > SER_SMEM_DYN_MAX) { ser_set_error("ser_run_create: shape needs %zu B of shared memory per chain", run->sweep_smem); return SER_E_ARG; }
+    run->sweep_fn = SWEEP_BIG[run->big_warp][manycd];
+    run->sweep_block = run->big_threads;
+  }
+  kp.n_chains = cfg->n_chains;
+  int per_sm = 1, n_sm = 1;
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, run->sweep_fn, run->sweep_block, run->sweep_smem));
+  CUDA_TRY(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, cfg->device));
+  run->sweep_slots = std::max(1, per_sm * n_sm);
+  if (run->big) { /* one global scratch slot per resident CTA */
+    run->sweep_slots = std::min(cfg->n_chains, run->sweep_slots);
     kp.Cs = ((M + 1) + 31) / 32 * 32;
-    const size_t sl = (size_t)run->big_slots;
+    const size_t sl = (size_t)run->sweep_slots;
     CUDA_TRY(POOL_ALLOC(&run->d_gV, sl * run->W * kp.Cs * sizeof(uint32_t)));
     CUDA_TRY(POOL_ALLOC(&run->d_gpre, sl * ((run->W >> SER_BIG_G) + 1) * kp.Cs * sizeof(uint16_t)));
     kp.gV = run->d_gV; kp.gpre = run->d_gpre;
-  }
-  kp.n_chains = cfg->n_chains;
-  if (!run->big) {
+  } else {
     /* Units of the Gibbs phase: a column with many items is served by 2, 4, .. 32 adjacent lanes.  Columns are sorted by
      * occurrence count and every column group starts its own round at lane 0, so inside a group the lane counts are
      * non-increasing and every lane group is aligned inside its warp.  T = items per lane aimed at, chosen per group:
@@ -641,16 +556,7 @@ static int run_create_impl(const ser_dataset *ds, const ser_run_config *cfg, ser
     CUDA_TRY(cudaMemcpyAsync(run->d_unit_tab, units.data(), units.size() * sizeof(uint2), cudaMemcpyHostToDevice, run->stream));
     CUDA_TRY(cudaStreamSynchronize(run->stream));
     kp.unit_tab = run->d_unit_tab;
-  }
-  if (!run->big) { /* persistent work-queue grid: bit columns carried between work items, queue head, per-chain progress */
-    int per_sm = 1, n_sm = 1;
-    const size_t smem = cfg->manycd ? run->smem_many : run->smem_sweep;
-    if (cfg->manycd && run->variant_many) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel<384, 2, true>, run->C, smem));
-    else if (cfg->manycd) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel<1024, 1, true>, run->C, smem));
-    else if (run->variant == 1) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel<384, 2, false>, run->C, smem));
-    else CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ser_sweep_kernel<1024, 1, false>, run->C, smem));
-    CUDA_TRY(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, cfg->device));
-    run->sweep_slots = std::max(1, per_sm * n_sm);
+    /* persistent work-queue grid: bit columns carried between work items, queue head, per-chain progress */
     if (const char *v = getenv("SER_SWEEP_SLOTS")) run->sweep_slots = std::max(1, atoi(v));
     CUDA_TRY(POOL_ALLOC(&run->d_V, nc * (size_t)run->W * run->C * sizeof(uint32_t)));
     CUDA_TRY(POOL_ALLOC(&run->d_queue, sizeof(unsigned int)));
@@ -769,7 +675,7 @@ extern "C" void ser_run_destroy(ser_run *run)
   void *bufs[] = {run->d_Xs, run->d_hard, run->d_ones, run->d_off, run->d_order, run->d_item_col, run->d_ab, run->d_rpi,
                   run->d_scal, run->d_tape, run->d_tape_off, run->d_samp_a, run->d_samp_b, run->d_samp_pi, run->d_samp_cdl,
                   run->d_scratch_i, run->d_bad, run->d_cd4, run->d_samp_cd_all, run->d_gV, run->d_gpre, run->d_bgrp, run->d_bbat,
-                  run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites, run->d_cl_off, run->d_cl_item, run->d_cl_grp,
+                  run->d_V, run->d_queue, run->d_done, run->d_e_all, run->d_info, run->d_chosen, run->d_counts, run->d_unit_tab, run->d_hbits, run->d_col_sites,
                   run->d_chain_ids, run->d_acc};
   for (void *b : bufs) if (b) cudaFreeAsync(b, run->stream);
   if (run->stream) cudaStreamSynchronize(run->stream);
@@ -871,47 +777,21 @@ static int launch_sweeps(ser_run *run, int burn_calls, int sample_calls)
     ev0 = (*run->sweep_ev)[run->sweep_ev_used]; ev1 = (*run->sweep_ev)[run->sweep_ev_used + 1];
     run->sweep_ev_used += 2;
   }
-  if (run->big && run->cl_mode) {
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = run->cl_R; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    lc.gridDim = dim3(run->cl_clusters * run->cl_R, 1, 1); lc.blockDim = dim3(run->big_threads, 1, 1);
-    lc.dynamicSmemBytes = run->smem_cl; lc.stream = run->stream; lc.attrs = at; lc.numAttrs = 1;
-    if (rec) CUDA_TRY(cudaEventRecord(ev0, run->stream));
-    CUDA_TRY(cudaLaunchKernelEx(&lc, ser_sweep_kernel_cl, kp));
-    if (rec) CUDA_TRY(cudaEventRecord(ev1, run->stream));
-    return SER_OK;
+  int grid = run->sweep_slots; /* large shapes: one CTA per scratch slot, the chains strided over them */
+  if (!run->big) {
+    const long long work = (long long)run->cfg.n_chains * n_calls;
+    int chunk = (int)std::min<long long>(n_calls, std::max<long long>(1, work / (32ll * run->sweep_slots)));
+    if (const char *v = getenv("SER_CHUNK_CALLS")) chunk = std::max(1, std::min(n_calls, atoi(v)));
+    const int per_chain = (n_calls + chunk - 1) / chunk;
+    kp.chunk_calls = chunk;
+    kp.n_items = (unsigned int)run->cfg.n_chains * (unsigned int)per_chain;
+    kp.chunk_base = run->chunks_done;
+    run->chunks_done += (unsigned int)per_chain;
+    grid = (int)std::min<long long>((long long)kp.n_items, run->sweep_slots);
+    CUDA_TRY(cudaMemsetAsync(run->d_queue, 0, sizeof(unsigned int), run->stream));
   }
-  if (run->big) {
-    if (rec) CUDA_TRY(cudaEventRecord(ev0, run->stream));
-    if (run->big_warp) {
-      if (run->cfg.manycd) ser_sweep_kernel_big<true, true><<<run->big_slots, run->big_threads, run->smem_big, run->stream>>>(kp);
-      else ser_sweep_kernel_big<false, true><<<run->big_slots, run->big_threads, run->smem_big, run->stream>>>(kp);
-    } else {
-      if (run->cfg.manycd) ser_sweep_kernel_big<true, false><<<run->big_slots, run->big_threads, run->smem_big, run->stream>>>(kp);
-      else ser_sweep_kernel_big<false, false><<<run->big_slots, run->big_threads, run->smem_big, run->stream>>>(kp);
-    }
-    CUDA_TRY(cudaGetLastError());
-    if (rec) CUDA_TRY(cudaEventRecord(ev1, run->stream));
-    return SER_OK;
-  }
-  const long long work = (long long)run->cfg.n_chains * n_calls;
-  int chunk = (int)std::min<long long>(n_calls, std::max<long long>(1, work / (32ll * run->sweep_slots)));
-  if (const char *v = getenv("SER_CHUNK_CALLS")) chunk = std::max(1, std::min(n_calls, atoi(v)));
-  const int per_chain = (n_calls + chunk - 1) / chunk;
-  kp.chunk_calls = chunk;
-  kp.n_items = (unsigned int)run->cfg.n_chains * (unsigned int)per_chain;
-  kp.chunk_base = run->chunks_done;
-  run->chunks_done += (unsigned int)per_chain;
-  const int grid = (int)std::min<long long>((long long)kp.n_items, run->sweep_slots);
-  CUDA_TRY(cudaMemsetAsync(run->d_queue, 0, sizeof(unsigned int), run->stream));
   if (rec) CUDA_TRY(cudaEventRecord(ev0, run->stream));
-  if (run->cfg.manycd && run->variant_many) ser_sweep_kernel<384, 2, true><<<grid, run->C, run->smem_many, run->stream>>>(kp);
-  else if (run->cfg.manycd) ser_sweep_kernel<1024, 1, true><<<grid, run->C, run->smem_many, run->stream>>>(kp);
-  else if (run->variant == 1) ser_sweep_kernel<384, 2, false><<<grid, run->C, run->smem_sweep, run->stream>>>(kp);
-  else ser_sweep_kernel<1024, 1, false><<<grid, run->C, run->smem_sweep, run->stream>>>(kp);
+  run->sweep_fn<<<grid, run->sweep_block, run->sweep_smem, run->stream>>>(kp);
   CUDA_TRY(cudaGetLastError());
   if (rec) CUDA_TRY(cudaEventRecord(ev1, run->stream));
   return SER_OK;
@@ -1104,7 +984,7 @@ extern "C" int ser_run_kernel_launches(const ser_run *run, int64_t *n)
 extern "C" int ser_run_kernel_path(const ser_run *run, int32_t *path)
 {
   if (!run || !path) return SER_E_ARG;
-  *path = !run->big ? 0 : run->cl_mode ? 3 : run->big_warp ? 2 : 1;
+  *path = !run->big ? 0 : run->big_warp ? 2 : 1;
   return SER_OK;
 }
 

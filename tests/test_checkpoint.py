@@ -115,8 +115,7 @@ def test_cli_checkpoint_flags_need_a_checkpoint_file(S):
 
 # ----------------------------------------------------------------------------- GPU
 PATHS = {"default": {}, "big_groups": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "0"},
-         "big_warp": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "1"},
-         "cluster": {"SER_FORCE_BIG": "256", "SER_BIG_MODE": "cluster", "SER_CLUSTER_R": "2"}, "manycd": {}}
+         "big_warp": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "1"}, "manycd": {}}
 
 
 def _advance(run, done, n, burn):

@@ -1098,41 +1098,6 @@ def test_cli_multi_gpu_and_index_check(S, tmp_path):
         assert (tmp_path / "po1.csv").read_bytes() == (tmp_path / ("po%d.csv" % G)).read_bytes()
 
 
-# ----------------------------------------------------------------------------- round 2: the cluster variant of the large-shape kernel
-@pytest.mark.parametrize("R", ["1", "2", "4", "8"])
-def test_cluster_path_replay_bit_exact(S, oracle_mod, monkeypatch, R):
-    """SER_BIG_MODE=cluster: one chain per cluster of R CTAs, the bit columns sharded over their shared memory
-    (ser_sweep_kernel_cluster.cuh); the deltas of a proposal are summed through DSMEM + one cluster barrier"""
-    monkeypatch.setenv("SER_FORCE_BIG", "256")
-    monkeypatch.setenv("SER_BIG_MODE", "cluster")
-    monkeypatch.setenv("SER_CLUSTER_R", R)
-    for name, burn, samp in (("g10s10", 8, 8), ("g2s2", 2, 2)):
-        X, hard = load_hex_dataset(name)
-        _replay_case(S, oracle_mod, X, hard, [5, 6, 7], burn, samp)
-    rng = np.random.default_rng(7)
-    for shape in EDGE_SHAPES[3::3]:
-        if shape[1] >= 2 * int(R):
-            X, hard = random_dataset(rng, *shape)
-            _replay_case(S, oracle_mod, X, hard, [1, 2], 6, 6)
-
-
-def test_cluster_path_config5_and_many_chains(S, oracle_mod, monkeypatch):
-    """the 1024 x 4096 matrix through clusters of 8 CTAs: replay vs the oracle, and more chains than clusters"""
-    monkeypatch.setenv("SER_BIG_MODE", "cluster")
-    X, hard = S.Dataset.synthetic(1024, 4096, 16).arrays()
-    _replay_case(S, oracle_mod, X, hard, [42], 1, 1)
-    monkeypatch.setenv("SER_FORCE_BIG", "1024")
-    monkeypatch.setenv("SER_CLUSTER_R", "4")
-    Xs, hs = load_hex_dataset("g10s10")
-    run = S.Run(S.Dataset.from_bits(Xs, hs), 300, seed=3, store=S.STORE_PI, max_samples=2).init().advance_both(2, 2).sync()
-    assert run.check() == 0
-    monkeypatch.delenv("SER_FORCE_BIG"); monkeypatch.delenv("SER_BIG_MODE"); monkeypatch.delenv("SER_CLUSTER_R")
-    ref = S.Run(S.Dataset.from_bits(Xs, hs), 300, seed=3, store=S.STORE_PI, max_samples=2).init().advance_both(2, 2).sync()
-    assert run.chain_stats()["e_negloglik"].tobytes() == ref.chain_stats()["e_negloglik"].tobytes()
-    for i in (0, 37, 299):
-        assert np.array_equal(run.fetch_samples(i, full=False)["pi"], ref.fetch_samples(i, full=False)["pi"])
-
-
 # ----------------------------------------------------------------------------- round 2: per-taxon c, d for large shapes
 @pytest.mark.parametrize("threads", ["64", "1024"])
 def test_manycd_big_path_replay_bit_exact(S, oracle_mod, monkeypatch, threads):

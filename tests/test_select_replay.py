@@ -53,8 +53,7 @@ def _same_state(x, y, what):
 
 
 PATHS = {"default": {}, "big_groups": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "0"},
-         "big_warp": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "1"},
-         "cluster": {"SER_FORCE_BIG": "256", "SER_BIG_MODE": "cluster", "SER_CLUSTER_R": "2"}, "manycd": {}}
+         "big_warp": {"SER_FORCE_BIG": "256", "SER_BIG_WARP": "1"}, "manycd": {}}
 
 
 @pytest.mark.gpu
