@@ -485,12 +485,14 @@ __global__ void __launch_bounds__(1024, 1) ser_diag_kernel(const uint16_t *samp_
         P = fmin(P, pprev);
         pprev = P; psum += P; lags += 2;
       }
-      if (k0 + 33 >= L) on = false;
+      if (k0 + 33 >= L || !(g0 >= DBL_MIN)) on = false;
     }
   }
   if (lane == 0 && qw >= qlo && qw < qhi) {
     double *o = stats + ((size_t)c * Q + qw) * 4;
-    const bool defined = s_on[w] != 0;
+    /* gamma_0 below DBL_MIN (a spread under ~1e-154, e.g. exp(c) at c ~ -745): the centred products underflow and rho_k means
+     * nothing, so the ESS is undefined as for a constant quantity, not the floor that rho = NaN would give */
+    const bool defined = s_on[w] != 0 && g0 >= DBL_MIN;
     o[2] = defined ? T / fmax(-1.0 + 2.0 * psum, 1.0 / log10((double)T)) : NaN;
     o[3] = defined ? (double)lags : 0.0;
   }

@@ -17,6 +17,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
+#include <cfloat>
 #include <climits>
 #include <cstring>
 #include <vector>

@@ -95,7 +95,8 @@ def test_summary_kernels_are_built_for_sm100a_without_stack_or_spills(S):
     out = subprocess.run([exe, "-res-usage", S.LIB_PATH], check=True, capture_output=True, text=True).stdout
     assert "sm_100a" in out
     names = ("ser_po_kernel", "ser_posterior_kernel", "ser_alive_kernel", "ser_pos_hist_kernel", "ser_range_hist_kernel",
-             "ser_po_acc_out_kernel", "ser_posterior_acc_out_kernel", "ser_alive_acc_out_kernel", "ser_hist_acc_out_kernel")
+             "ser_po_acc_out_kernel", "ser_posterior_acc_out_kernel", "ser_alive_acc_out_kernel", "ser_hist_acc_out_kernel",
+             "ser_diag_kernel")
     lines = out.splitlines()
     for name in names:
         idx = [i for i, ln in enumerate(lines) if "Function" in ln and name in ln]
