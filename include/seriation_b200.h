@@ -210,6 +210,24 @@ int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t 
  * SER_E_ARG when the chains' T differ or T < 4. */
 int ser_split_rhat(const double *halves, const int32_t *n_samples, int32_t k, int32_t Q, double *rhat);
 
+/* Rank-normalised split-R-hat, bulk-ESS and tail-ESS pooled over the chosen chains (Vehtari et al. 2021; DESIGN.md section 3.9).
+ * The quantities and `what` are those of ser_run_diagnostics.  Draws: each chosen chain (GLOBAL ids, any order; they are sorted) holds
+ * T = min(n_samples, max_samples) stored samples, the same T for all, n = floor(T/2); its first n and its last n samples are two
+ * sequences (the middle sample of an odd T is in neither), 2c and 2c + 1 for the c-th id in ascending order: m = 2k sequences, S = m n
+ * draws per quantity.  out [3+N][SER_RDIAG_FIELDS] doubles (host memory; rows `what` does not request are left untouched):
+ *   rhat_bulk = R-hat of z, the draws rank-normalised over all S (average ranks r of equal doubles, z = Phi^-1((r - 3/8) / (S + 1/4)));
+ *   rhat_fold = R-hat of the rank-normalised |x - median|; ess_bulk = ESS of z; ess_mean = ESS of x; ess_q05 / ess_q95 = ESS of the
+ *   indicators 1{x <= q05} / 1{x <= q95}; q05, q95 = numpy.quantile(draws, 0.05 / 0.95) ('linear'), bit for bit.
+ * R-hat = sqrt(((n-1)/n W + B/n) / W) over the m sequences (W = mean of their variances, B/n = variance of their means); +inf when
+ * W = 0 < B (every sequence constant, not all at one level), NaN when W = B = 0.  ESS = Stan's multi-chain estimator (ArviZ's _ess):
+ * Geyer's initial positive and monotone sequence on the pooled autocorrelations; NaN for a series whose S values are all equal.  The
+ * rank-normalised R-hat is max(rhat_bulk, rhat_fold), the tail-ESS min(ess_q05, ess_q95).  The same chains and stored samples give the
+ * same bits on any run that holds them (full, subset, sharded or resumed).  Every check runs before `out` is written:
+ * SER_E_ARG   k < 1, a NULL pointer, what not in 1..3, a chosen id that is negative, repeated or not held by this run (no CUDA call);
+ * SER_E_STATE a store below what `what` needs, an accumulating run, a run not initialised, chosen chains whose T differ, T < 4. */
+#define SER_RDIAG_FIELDS 8 /* rhat_bulk, rhat_fold, ess_bulk, ess_mean, ess_q05, ess_q95, q05, q95 */
+int ser_run_rank_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, double *out);
+
 /* alive[c][j][m] = #{t : a_t(m) <= j <= b_t(m)} over the stored samples of the chosen chains owned by
  * this run (same slab convention as above; int32 [k][N][M], host memory; needs SER_STORE_FULL).
  * The counts behind plot_taxa_occurence_probability_matrix, plot_false_taxa_occurence_probability

@@ -20,6 +20,7 @@ MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
 ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE = 1, 2, 4, 8, 16, 32
 DIAG_SCALARS, DIAG_SITES = 1, 2
+RDIAG_FIELDS = ("rhat_bulk", "rhat_fold", "ess_bulk", "ess_mean", "ess_q05", "ess_q95", "q05", "q95")
 
 _i32p, _dp, _u8p = C.POINTER(C.c_int32), C.POINTER(C.c_double), C.POINTER(C.c_uint8)
 _i64p, _u64p = C.POINTER(C.c_int64), C.POINTER(C.c_uint64)
@@ -82,6 +83,7 @@ SYMBOLS = [
     ("ser_run_posterior_sums", C.c_int, [_vp, _i32p, C.c_int32, _i64p, _i32p, _i32p, _i32p, _i32p]),
     ("ser_run_diagnostics", C.c_int, [_vp, _i32p, C.c_int32, C.c_int32, C.c_int32, _dp, _dp, _i32p]),
     ("ser_split_rhat", C.c_int, [_dp, _i32p, C.c_int32, C.c_int32, _dp]),
+    ("ser_run_rank_diagnostics", C.c_int, [_vp, _i32p, C.c_int32, C.c_int32, _dp]),
     ("ser_run_marginals", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p]),
     ("ser_hist_quantiles", C.c_int, [_i32p, C.c_int32, C.c_int32, _dp, C.c_int32, _i32p]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
@@ -413,6 +415,20 @@ class Run:
         rhat = split_rhat(halves[held], n[held]) if held.any() and np.all(n[held] == n[held][0]) else None
         return dict(mean=stats[..., 0], var=stats[..., 1], ess=stats[..., 2], lags=stats[..., 3], halves=halves, n_samples=n, rhat=rhat)
 
+    def rank_diagnostics(self, chosen, scalars: bool = True, sites: bool = True) -> dict:
+        """rank-normalised split-R-hat, bulk- and tail-ESS pooled over the chosen chains (global ids, all held by this run, the same
+        number of stored samples each) (ser_run_rank_diagnostics): arrays of length Q = 3 + N (-loglik, exp(c), exp(d), then pi of
+        every site) ``rhat_bulk``, ``rhat_fold``, ``rhat`` (their maximum), ``ess_bulk``, ``ess_tail`` (min of ``ess_q05`` and
+        ``ess_q95``), ``ess_mean``, ``ess_q05``, ``ess_q95``, ``q05``, ``q95``.  Rows that were not requested are NaN."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        out = np.full((3 + self.N, len(RDIAG_FIELDS)), np.nan)
+        what = (DIAG_SCALARS if scalars else 0) | (DIAG_SITES if sites else 0)
+        _check(lib().ser_run_rank_diagnostics(self._h, _p(chosen, C.c_int32), len(chosen), what, _p(out, C.c_double)))
+        res = {name: out[:, i].copy() for i, name in enumerate(RDIAG_FIELDS)}
+        res["rhat"] = np.maximum(res["rhat_bulk"], res["rhat_fold"])
+        res["ess_tail"] = np.minimum(res["ess_q05"], res["ess_q95"])
+        return res
+
     def marginals(self, chosen, ranges: bool = False, positions: bool = True) -> dict:
         """histograms of the chosen chains (global ids) over their samples (ser_run_marginals): ``pos`` [k][N][N] = #{t: pi_t(i) = p},
         and with ``ranges`` ``a`` / ``b`` [k][M][N+1] = #{t: a_t(m) = j}; ``n_samples`` [k] = T.  Slabs the run does not fill stay 0
@@ -723,6 +739,13 @@ def diagnostics(batch: ChainBatch, chains, max_lag: int = 0) -> dict:
     full sample store (their rows stay NaN otherwise).  A batch from replay_chosen(..., window=0) keeps it."""
     run = batch.run
     return run.diagnostics(np.asarray(chains, dtype=np.int32), scalars=run.cfg.store >= STORE_FULL, max_lag=max_lag)
+
+
+def rank_diagnostics(batch: ChainBatch, chains) -> dict:
+    """Run.rank_diagnostics pooled over the chosen chains of a batch: every site's pi, and -loglik, exp(c), exp(d) when the batch
+    keeps the full sample store (their rows stay NaN otherwise).  A batch from replay_chosen(..., window=0) keeps it."""
+    run = batch.run
+    return run.rank_diagnostics(np.asarray(chains, dtype=np.int32), scalars=run.cfg.store >= STORE_FULL)
 
 
 def _marginal_summary(hist, probs):

@@ -17,7 +17,8 @@
  * sharded over the GPUs of the box -- ser_multi_*):
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
- *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--marginals PREFIX]
+ *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--rank-diagnostics FILE]
+ *        [--marginals PREFIX]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
@@ -31,6 +32,10 @@
  * --diagnostics FILE (with --select) re-simulates the chosen chains alone keeping every sample (SER_STORE_FULL, bit-identical to
  * their first run, which is checked), writes per-quantity split-R-hat and effective sample sizes to FILE and prints one summary
  * line; under --replay-selected --po the same run supplies the pair-order counts.
+ * --rank-diagnostics FILE (with --select) does the same replay (one replay serves both flags) and writes the rank-normalised R-hat,
+ * bulk- and tail-ESS pooled over the chosen chains (ser_run_rank_diagnostics) to FILE
+ * "quantity,rhat,rhat_bulk,rhat_fold,ess_bulk,ess_tail,ess_mean,q05,q95", with one summary line: the largest R-hat, the smallest
+ * bulk- and tail-ESS, and how many quantities have R-hat > 1.01 or a bulk- or tail-ESS below 100 per chain.
  * --marginals PREFIX (with --select) re-simulates the chosen chains alone through a window of W samples (--window, default 64) while
  * their position and a / b histograms accumulate (bit-identical to their first run, which is checked), pools the counts over the
  * chains and writes PREFIX.sites.csv "site,hard,mean,q025,median,q975,mode,p_mode" (file order, 0-based positions) and
@@ -65,17 +70,62 @@ static void usage(const char *argv0)
           "                  (save every chain to FILE at the end and every C calls; --resume continues FILE's run; --stop-after C\n"
           "                   advances at most C calls, saves and exits)\n"
           "              [--diagnostics FILE]   (with --select: split-R-hat and ESS of the chosen chains to FILE)\n"
+          "              [--rank-diagnostics FILE]   (with --select: rank-normalised R-hat, bulk- and tail-ESS pooled over the\n"
+          "                                           chosen chains to FILE)\n"
           "              [--marginals PREFIX]   (with --select: position and a / b credible intervals of the chosen chains to\n"
           "                                      PREFIX.sites.csv and PREFIX.taxa.csv; the replay uses --window W)\n",
           argv0, argv0, argv0);
   exit(1);
 }
 
-/* --diagnostics: the chosen chains re-simulated alone with every sample kept (bit-identical to their first run, whose E[-logL]
- * per global id - first is e[]; any difference exits 1), their split-R-hat and ESS written to `path` as CSV and summarised in one
- * line.  `counts` (NULL: not wanted) receives their pair-order counts from the same run. */
+static const char *quantity_name(int q, char *buf, size_t len)
+{
+  if (q < 3) return q == 0 ? "-logL" : q == 1 ? "c" : "d";
+  snprintf(buf, len, "site_%d", q - 3);
+  return buf;
+}
+
+/* NaN when either is NaN, as numpy.maximum / numpy.minimum */
+static double max_nan(double a, double b) { return isnan(a) || isnan(b) ? NAN : a > b ? a : b; }
+static double min_nan(double a, double b) { return isnan(a) || isnan(b) ? NAN : a < b ? a : b; }
+
+/* --rank-diagnostics: the pooled rank-normalised diagnostics of the chosen chains of `sub` to `path` and one summary line */
+static void write_rank_diagnostics(ser_run *sub, const int32_t *chosen, int32_t k, int32_t N, const char *path)
+{
+  const int Q = 3 + N;
+  double *out = (double *)malloc(sizeof(double) * (size_t)Q * SER_RDIAG_FIELDS);
+  double r_max = NAN, bulk_min = NAN, tail_min = NAN;
+  int q, q_r = -1, q_b = -1, q_t = -1, flagged = 0;
+  char b1[32], b2[32], b3[32];
+  FILE *f;
+  if (!out) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  if (ser_run_rank_diagnostics(sub, chosen, k, SER_DIAG_SCALARS | SER_DIAG_SITES, out)) die("ser_run_rank_diagnostics");
+  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  fprintf(f, "quantity,rhat,rhat_bulk,rhat_fold,ess_bulk,ess_tail,ess_mean,q05,q95\n");
+  for (q = 0; q < Q; q++) {
+    const double *o = out + (size_t)q * SER_RDIAG_FIELDS;
+    const double rhat = max_nan(o[0], o[1]), tail = min_nan(o[4], o[5]);
+    fprintf(f, "%s,%.17g,%.17g,%.17g,%.17g,%.17g,%.17g,%.17g,%.17g\n", quantity_name(q, b1, sizeof(b1)), rhat, o[0], o[1], o[2], tail, o[3],
+            o[6], o[7]);
+    if (!isnan(rhat) && (q_r < 0 || rhat > r_max)) { r_max = rhat; q_r = q; }
+    if (!isnan(o[2]) && (q_b < 0 || o[2] < bulk_min)) { bulk_min = o[2]; q_b = q; }
+    if (!isnan(tail) && (q_t < 0 || tail < tail_min)) { tail_min = tail; q_t = q; }
+    flagged += rhat > 1.01 || o[2] < 100.0 * k || tail < 100.0 * k;
+  }
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  printf("rank diagnostics: %d chains  R-hat max %.4f (%s)  bulk-ESS min %.1f (%s)  tail-ESS min %.1f (%s)  "
+         "%d of %d quantities with R-hat > 1.01 or ESS < %d\n", k, r_max, q_r < 0 ? "none" : quantity_name(q_r, b1, sizeof(b1)), bulk_min,
+         q_b < 0 ? "none" : quantity_name(q_b, b2, sizeof(b2)), tail_min, q_t < 0 ? "none" : quantity_name(q_t, b3, sizeof(b3)), flagged, Q,
+         100 * k);
+  free(out);
+}
+
+/* --diagnostics / --rank-diagnostics: the chosen chains re-simulated alone with every sample kept (bit-identical to their first run,
+ * whose E[-logL] per global id - first is e[]; any difference exits 1); their split-R-hat and ESS written to `path` as CSV and
+ * summarised in one line, and their rank-normalised diagnostics to `rank_path` (either may be NULL).  `counts` (NULL: not wanted)
+ * receives their pair-order counts from the same run. */
 static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
-                               int burn, int samples, int32_t *counts, const char *path)
+                               int burn, int samples, int32_t *counts, const char *path, const char *rank_path)
 {
   ser_run_config c2 = *cfg;
   ser_run *sub = NULL;
@@ -107,6 +157,12 @@ static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg,
       exit(1);
     }
   if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
+  if (rank_path) write_rank_diagnostics(sub, chosen, k, N, rank_path);
+  if (!path) {
+    ser_run_destroy(sub);
+    free(e2); free(stats); free(halves); free(rhat); free(n);
+    return;
+  }
   if (ser_run_diagnostics(sub, chosen, k, SER_DIAG_SCALARS | SER_DIAG_SITES, 0, stats, halves, n)) die("ser_run_diagnostics");
   if (ser_split_rhat(halves, n, k, Q, rhat)) die("ser_split_rhat");
   ser_run_destroy(sub);
@@ -263,7 +319,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
-  const char *diag_path = NULL, *marg_prefix = NULL;
+  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -298,6 +354,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--window")) window = atoi(v);
       else if (!strcmp(a, "--checkpoint")) ckpt_path = v;
       else if (!strcmp(a, "--diagnostics")) diag_path = v;
+      else if (!strcmp(a, "--rank-diagnostics")) rdiag_path = v;
       else if (!strcmp(a, "--marginals")) marg_prefix = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
@@ -306,7 +363,7 @@ int main(int argc, char **argv)
     }
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
-    if (diag_path && select_k < 1) usage(argv[0]);
+    if ((diag_path || rdiag_path) && select_k < 1) usage(argv[0]);
     if (marg_prefix && (select_k < 1 || window < 1)) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
@@ -438,7 +495,7 @@ int main(int argc, char **argv)
         /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0 && !diag_path && !marg_prefix) {
+        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix) {
           ser_run_config c2 = cfg;
           ser_run *sub = NULL;
           c2.n_chains = nchosen;
@@ -459,10 +516,11 @@ int main(int argc, char **argv)
         for (i = 0; i < nchosen; i++) { sc += ec[chosen[i] - first]; sdd += ed[chosen[i] - first]; }
         printf("E[c] %.6f  E[d] %.6f over the chosen chains\n", sc / nchosen, sdd / nchosen);
       }
-      if (diag_path && nchosen > 0)
-        replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path);
+      if ((diag_path || rdiag_path) && nchosen > 0)
+        replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path, rdiag_path);
       if (marg_prefix && nchosen > 0)
-        replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window, (replay_selected && !diag_path) ? counts : NULL,
+        replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window,
+                         (replay_selected && !diag_path && !rdiag_path) ? counts : NULL,
                          marg_prefix);
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);

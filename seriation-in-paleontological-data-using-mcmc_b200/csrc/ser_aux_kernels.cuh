@@ -364,6 +364,30 @@ __device__ __forceinline__ double diag_value(const uint16_t *pi, const double *c
   return exp(cdl[(size_t)t * 3 + q - 1]);
 }
 
+/* One staged chunk of the lag sums over traces of length len (1024 threads): row j of sA holds val(j, t) for t = t0 .. t0 + 63 and
+ * row j of sB for t = t0 + k0 .. t0 + k0 + 95, zero where t >= len or the warp of quantity j has stopped (act[j] == 0).  val(j, t)
+ * returns the centred value.  Every thread of the block calls it, between barriers. */
+template <class Val>
+__device__ __forceinline__ void stage_lag_chunk(double *sA, double *sB, const int *act, int t0, int k0, int len, Val val)
+{
+  for (int e = threadIdx.x; e < 32 * SER_DIAG_TC; e += 1024) {
+    const int t = t0 + (e >> 5), j = e & 31;
+    sA[j * SER_DIAG_SA + (e >> 5)] = (act[j] && t < len) ? val(j, t) : 0.0;
+  }
+  for (int e = threadIdx.x; e < 32 * (SER_DIAG_TC + 32); e += 1024) {
+    const int t = t0 + k0 + (e >> 5), j = e & 31;
+    sB[j * SER_DIAG_SB + (e >> 5)] = (act[j] && t < len) ? val(j, t) : 0.0;
+  }
+}
+
+/* warp w's lane l adds the products of its quantity's staged chunk at lag k0 + l, for the chunk's first nt samples, in t order */
+__device__ __forceinline__ double lag_chunk_dot(const double *sA, const double *sB, int w, int lane, int nt, double acc)
+{
+  const double *a = sA + w * SER_DIAG_SA, *b = sB + w * SER_DIAG_SB + lane;
+  for (int t = 0; t < nt; t++) acc = fma(a[t], b[t], acc);
+  return acc;
+}
+
 /* stats [k][3+N][4] = mean, var, ess, lags; halves [k][3+N][4] = mean1, var1, mean2, var2 for quantities [qlo, qhi); n_out[c] = T */
 __global__ void __launch_bounds__(1024, 1) ser_diag_kernel(const uint16_t *samp_pi, const double *samp_cdl, const ChainScalars *scal, int N,
                                                            int max_samples, const int *chosen, int chain_offset, int n_local, const int *ids,
@@ -460,20 +484,9 @@ __global__ void __launch_bounds__(1024, 1) ser_diag_kernel(const uint16_t *samp_
     const int span = T - k0;
     for (int t0 = 0; t0 < span; t0 += SER_DIAG_TC) {
       __syncthreads();
-      for (int e = threadIdx.x; e < 32 * SER_DIAG_TC; e += 1024) {
-        const int t = t0 + (e >> 5), j = e & 31;
-        sA[j * SER_DIAG_SA + (e >> 5)] = (s_act[j] && t < T) ? diag_value(pi, cdl, N, q0 + j, t) - s_mean[j] : 0.0;
-      }
-      for (int e = threadIdx.x; e < 32 * (SER_DIAG_TC + 32); e += 1024) {
-        const int t = t0 + k0 + (e >> 5), j = e & 31;
-        sB[j * SER_DIAG_SB + (e >> 5)] = (s_act[j] && t < T) ? diag_value(pi, cdl, N, q0 + j, t) - s_mean[j] : 0.0;
-      }
+      stage_lag_chunk(sA, sB, s_act, t0, k0, T, [&](int j, int t) { return diag_value(pi, cdl, N, q0 + j, t) - s_mean[j]; });
       __syncthreads();
-      if (on) {
-        const double *a = sA + w * SER_DIAG_SA, *b = sB + w * SER_DIAG_SB + lane;
-        const int nt = min(SER_DIAG_TC, span - t0);
-        for (int t = 0; t < nt; t++) acc = fma(a[t], b[t], acc);
-      }
+      if (on) acc = lag_chunk_dot(sA, sB, w, lane, min(SER_DIAG_TC, span - t0), acc);
     }
     if (on) { /* Geyer's initial monotone sequence over this block's 16 pairs; every lane follows it, so `on` stays warp-uniform */
       if (k0 == 0) g0 = __shfl_sync(0xffffffffu, acc, 0) / T;
@@ -548,6 +561,263 @@ __global__ void ser_range_hist_kernel(const uint16_t *samp_a, const uint16_t *sa
   if (local < 0) return;
   const uint16_t *x = (blockIdx.z ? samp_b : samp_a) + (size_t)local * max_samples * M;
   hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, out + blockIdx.x * stride, use_smem ? s_hist : nullptr, add);
+}
+
+/* ------------------------------------------------------------------ rank-normalised diagnostics (ser_run_rank_diagnostics, DESIGN.md 3.9)
+ * The draws pool the chosen chains, ascending global id: sequence j is the first (j even) or the last (j odd) n = T/2 stored samples
+ * of chosen chain j/2, draw (j, t) its row t or T - n + t (the middle row of an odd T is in neither), S = m n draws over m = 2k
+ * sequences.  Series s of quantity q: 0 = z (the rank-normalised draws), 1 = z of the folded draws |x - median|, 2 = x,
+ * 3 / 4 = 1{x <= q05} / 1{x <= q95}.  Sites get z from per-site tables built from the pooled position histogram; the three scalars
+ * from two device sorts each.  No sum depends on the grid. */
+struct RankSeq {
+  const int *loc; /* local chain of each chosen chain, ascending global id */
+  int T, n, m, max_samples;
+};
+
+__device__ __forceinline__ size_t rank_row(const RankSeq &r, int j, int t)
+{
+  return (size_t)r.loc[j >> 1] * r.max_samples + ((j & 1) ? r.T - r.n + t : t);
+}
+
+/* numpy's _lerp (numpy.quantile, method 'linear'), with no contraction */
+__device__ __forceinline__ double np_lerp(double a, double b, double t)
+{
+  const double d = __dsub_rn(b, a);
+  return t < 0.5 ? __dadd_rn(a, __dmul_rn(d, t)) : __dsub_rn(b, __dmul_rn(d, __dsub_rn(1.0, t)));
+}
+
+/* q05, q95 (numpy.quantile) and the median (numpy.median, S even) of S draws whose 0-based order statistic i is xs(i) */
+template <class X>
+__device__ void rank_quantiles(X xs, int S, double out[3])
+{
+  const double p[2] = {0.05, 0.95};
+  for (int u = 0; u < 2; u++) {
+    const double h = __dmul_rn((double)(S - 1), p[u]), j = floor(h);
+    out[u] = np_lerp(xs((int)j), xs(min((int)j + 1, S - 1)), __dsub_rn(h, j));
+  }
+  out[2] = __dmul_rn(__dadd_rn(xs(S / 2 - 1), xs(S / 2)), 0.5);
+}
+
+/* z = Phi^-1((r - 3/8) / (S + 1/4)) of a value whose `ties` equal draws sit at the 0-based sorted positions [below, below + ties) */
+__device__ __forceinline__ double rank_z(long long below, long long ties, int S)
+{
+  const double r = (double)below + (double)(ties + 1) * 0.5;
+  return normcdfinv((r - 0.375) / ((double)S + 0.25));
+}
+
+/* the pooled position histogram hist [N][N] of the split rows: hist_tile over the m sequences in order (the first stores, the others add) */
+__global__ void ser_rank_hist_kernel(const uint16_t *samp_pi, int N, RankSeq r, int use_smem, int *hist)
+{
+  extern __shared__ int s_hist[];
+  for (int j = 0; j < r.m; j++)
+    hist_tile(samp_pi + rank_row(r, j, 0) * N, N, N, N, r.n, blockIdx.x * blockDim.x, hist, use_smem ? s_hist : nullptr, j > 0);
+}
+
+/* dst[p] = sum_{v < p} get(v) for p <= len (dst[len] = the total), in integers; every thread of the block calls it */
+template <class Get>
+__device__ void block_scan_counts(Get get, int len, int *dst, int *part)
+{
+  const int per = (len + blockDim.x - 1) / blockDim.x, lo = min(len, (int)threadIdx.x * per), hi = min(len, lo + per);
+  int s = 0;
+  for (int p = lo; p < hi; p++) s += get(p);
+  part[threadIdx.x] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int a = 0;
+    for (int u = 0; u < (int)blockDim.x; u++) { const int v = part[u]; part[u] = a; a += v; }
+    dst[len] = a;
+  }
+  __syncthreads();
+  s = part[threadIdx.x];
+  for (int p = lo; p < hi; p++) { dst[p] = s; s += get(p); }
+  __syncthreads();
+}
+
+/* Site i = blockIdx.x from its row of the pooled histogram: z[i][p] and z_fold[i][p] of every position p held by a draw (0 elsewhere),
+ * qs[3 + i] = q05, q95, median and out[3 + i][6..7] = q05, q95.  The folded value |p - med| is shared by p = med -/+ s (med an
+ * integer) or floor(med) - s and floor(med) + 1 + s (med a half-integer): fold index s counts both, and the ranks of the folded draws
+ * follow from the running counts over s. */
+__global__ void __launch_bounds__(256) ser_rank_table_kernel(const int *hist, int N, int S, double *zt, double *zft, double *qs, double *out)
+{
+  __shared__ int s_h[SER_MAX_SITES], s_c[SER_MAX_SITES + 1], s_f[SER_MAX_SITES + 1], s_part[256];
+  __shared__ double s_q[3];
+  const int i = blockIdx.x;
+  for (int p = threadIdx.x; p < N; p += blockDim.x) s_h[p] = hist[(size_t)i * N + p];
+  __syncthreads();
+  block_scan_counts([&](int p) { return s_h[p]; }, N, s_c, s_part);
+  if (threadIdx.x == 0) {
+    double v[3];
+    rank_quantiles([&](int j) { /* the position holding order statistic j: the smallest p with s_c[p + 1] > j */
+      int lo = 0, hi = N - 1;
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (s_c[mid + 1] > j) hi = mid; else lo = mid + 1; }
+      return (double)lo;
+    }, S, v);
+    for (int u = 0; u < 3; u++) { s_q[u] = v[u]; qs[(size_t)(3 + i) * 3 + u] = v[u]; }
+    out[(size_t)(3 + i) * 8 + 6] = v[0]; out[(size_t)(3 + i) * 8 + 7] = v[1];
+  }
+  __syncthreads();
+  const double med = s_q[2];
+  const int m0 = (int)floor(med), half = med != (double)m0;
+  auto fold_count = [&](int s) {
+    const int lo = m0 - s, hi = half ? m0 + 1 + s : m0 + s;
+    return (lo >= 0 ? s_h[lo] : 0) + (hi != lo && hi < N ? s_h[hi] : 0);
+  };
+  block_scan_counts(fold_count, N, s_f, s_part);
+  for (int p = threadIdx.x; p < N; p += blockDim.x) {
+    const int h = s_h[p], s = p <= m0 ? m0 - p : p - m0 - half;
+    zt[(size_t)i * N + p] = h ? rank_z(s_c[p], h, S) : 0.0;
+    zft[(size_t)i * N + p] = h ? rank_z(s_f[s], fold_count(s), S) : 0.0;
+  }
+}
+
+/* keys[q][s] = x of draw s = j n + t of scalar q = blockIdx.y (fold: |x - median_q|), vals[q][s] = s */
+__global__ void ser_rank_gather_kernel(const double *samp_cdl, RankSeq r, const double *qs, int fold, double *keys, int *vals)
+{
+  const int q = blockIdx.y, S = r.m * r.n;
+  for (int s = blockIdx.x * blockDim.x + threadIdx.x; s < S; s += gridDim.x * blockDim.x) {
+    const int j = s / r.n, t = s - j * r.n;
+    const double x = diag_value(nullptr, samp_cdl + rank_row(r, j, t) * 3, 0, q, 0);
+    keys[(size_t)q * S + s] = fold ? fabs(__dsub_rn(x, qs[q * 3 + 2])) : x;
+    vals[(size_t)q * S + s] = s;
+  }
+}
+
+/* From the sorted keys of scalar q = blockIdx.y: z[q][draw] of every draw from its average rank (ties = equal doubles, found by binary
+ * search), and unless fold, qs[q] = q05, q95, median and out[q][6..7] = q05, q95 */
+__global__ void ser_rank_scalar_kernel(const double *keys, const int *vals, int S, int fold, double *z, double *qs, double *out)
+{
+  const int q = blockIdx.y;
+  const double *k = keys + (size_t)q * S;
+  for (int s = blockIdx.x * blockDim.x + threadIdx.x; s < S; s += gridDim.x * blockDim.x) {
+    const double x = k[s];
+    int lo = 0, hi = s; /* first index whose key equals x */
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (k[mid] < x) lo = mid + 1; else hi = mid; }
+    const int a = lo;
+    lo = s + 1; hi = S; /* one past the last */
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (k[mid] > x) hi = mid; else lo = mid + 1; }
+    z[(size_t)q * S + vals[(size_t)q * S + s]] = rank_z(a, lo - a, S);
+  }
+  if (!fold && blockIdx.x == 0 && threadIdx.x == 0) {
+    double v[3];
+    rank_quantiles([&](int j) { return k[j]; }, S, v);
+    for (int u = 0; u < 3; u++) qs[q * 3 + u] = v[u];
+    out[q * 8 + 6] = v[0]; out[q * 8 + 7] = v[1];
+  }
+}
+
+/* What the series of a quantity read: the store, the site tables z / z_fold [N][N], the scalar traces z / z_fold [3][S] (draw order) and
+ * qs [3 + N][3] = q05, q95, median */
+struct RankSrc {
+  const uint16_t *pi;
+  const double *cdl, *zt, *zft, *zs, *zfs, *qs;
+  int N;
+};
+
+__device__ __forceinline__ double rank_value(const RankSrc &s, const RankSeq &r, int series, int q, int j, int t)
+{
+  const size_t row = rank_row(r, j, t);
+  if (series < 2) {
+    if (q < 3) return (series ? s.zfs : s.zs)[(size_t)q * r.m * r.n + (size_t)j * r.n + t];
+    return (series ? s.zft : s.zt)[(size_t)(q - 3) * s.N + s.pi[row * s.N + q - 3]];
+  }
+  const double x = q < 3 ? diag_value(nullptr, s.cdl + row * 3, s.N, q, 0) : (double)s.pi[row * s.N + q - 3];
+  return series == 2 ? x : (x <= s.qs[q * 3 + series - 3] ? 1.0 : 0.0);
+}
+
+/* R-hat and ESS of series blockIdx.y over the m sequences, one block of 32 warps per 32 consecutive quantities.  Pass 1: lane = quantity,
+ * warp w takes sequences w, w + 32, ..., each summed in t order: its mean (its value when constant) and variance (divisor n - 1; 0 when
+ * constant) go to seq [5][3+N][m][2].  Warp 0 then pools them in sequence order: W, B/n, R-hat (series 0, 1 into out[q][0..1]) and
+ * var+.  Pass 2 (not for series 1): warp w owns quantity q0 + w, lane l sums lag k0 + l over sequence j = 0 .. m-1, then t, about each
+ * sequence's own mean, staged as in ser_diag_kernel; after each 32-lag block the warp walks Stan's loop on rho(k0 .. k0 + 31) and stops
+ * where the loop stops.  ESS goes to out[q][2..5] (series 0, 2, 3, 4). */
+__global__ void __launch_bounds__(1024, 1) ser_rank_ess_kernel(RankSrc src, RankSeq r, int qlo, int qhi, double *seq, double *out)
+{
+  __shared__ double sbuf[32 * (SER_DIAG_SA + SER_DIAG_SB)];
+  __shared__ double s_W[32], s_varp[32], s_cm[32];
+  __shared__ int s_on[32], s_act[32];
+  const int series = blockIdx.y, lane = threadIdx.x & 31, w = threadIdx.x >> 5, Q = 3 + src.N, m = r.m, n = r.n;
+  const int q0 = (qlo / 32 + blockIdx.x) * 32, q = q0 + lane, field = series == 0 ? 2 : series + 1;
+  const bool valid = q >= qlo && q < qhi;
+  const double NaN = __longlong_as_double(0x7ff8000000000000LL);
+  if (valid)
+    for (int j = w; j < m; j += 32) {
+      double s = 0.0, lo = INFINITY, hi = -INFINITY;
+      for (int t = 0; t < n; t++) {
+        const double x = rank_value(src, r, series, q, j, t);
+        s += x; lo = fmin(lo, x); hi = fmax(hi, x);
+      }
+      const double mu = lo == hi ? lo : s / n;
+      double v = 0.0;
+      if (lo != hi)
+        for (int t = 0; t < n; t++) { const double d = rank_value(src, r, series, q, j, t) - mu; v += d * d; }
+      double *o = seq + (((size_t)series * Q + q) * m + j) * 2;
+      o[0] = mu; o[1] = v / (n - 1);
+    }
+  __syncthreads();
+  if (w == 0) {
+    double W = 0.0, M = 0.0, Bn = 0.0, mlo = INFINITY, mhi = -INFINITY;
+    const double *o = seq + ((size_t)series * Q + q) * m * 2;
+    if (valid) {
+      for (int j = 0; j < m; j++) { W += o[2 * j + 1]; M += o[2 * j]; mlo = fmin(mlo, o[2 * j]); mhi = fmax(mhi, o[2 * j]); }
+      W /= m;
+      if (mlo != mhi) { /* equal sequence means: B = 0 exactly, not the residue of their mean */
+        const double mbar = M / m;
+        for (int j = 0; j < m; j++) { const double d = o[2 * j] - mbar; Bn += d * d; }
+        Bn /= m - 1;
+      }
+    }
+    const double varp = W * (n - 1.0) / n + Bn;
+    if (valid && series < 2) out[(size_t)q * 8 + series] = W > 0.0 ? sqrt(((n - 1.0) / n * W + Bn) / W) : Bn > 0.0 ? INFINITY : NaN;
+    if (valid && series != 1 && !(varp > 0.0)) out[(size_t)q * 8 + field] = NaN; /* every draw equal */
+    s_W[lane] = W; s_varp[lane] = varp;
+    s_on[lane] = valid && series != 1 && varp > 0.0;
+  }
+  __syncthreads();
+
+  /* Stan's loop, kept warp-uniform: (pe, po) is the last pair read (rho(t-1), rho(t)), stored when pe + po >= 0; reading the next pair
+   * commits it, monotonised against the previous committed pair, into psum */
+  const int qw = q0 + w;
+  bool on = s_on[w] != 0;
+  const double Wq = s_W[w], varp = s_varp[w], mn = (double)m * n;
+  double pe = 1.0, po = 0.0, psum = 0.0, pprev = 0.0;
+  bool stored = true, first = true;
+  int t = 1;
+  double *sA = sbuf, *sB = sbuf + 32 * SER_DIAG_SA;
+  for (int k0 = 0;; k0 += 32) {
+    if (lane == 0) s_act[w] = on;
+    if (!__syncthreads_or(on)) break;
+    double acc = 0.0;
+    const int span = n - k0;
+    for (int j = 0; j < m; j++) {
+      if (threadIdx.x < 32) /* read by the staging after the barrier below; the previous staging is behind the last barrier */
+        s_cm[threadIdx.x] = s_act[threadIdx.x] ? seq[(((size_t)series * Q + q0 + threadIdx.x) * m + j) * 2] : 0.0;
+      for (int t0 = 0; t0 < span; t0 += SER_DIAG_TC) {
+        __syncthreads();
+        stage_lag_chunk(sA, sB, s_act, t0, k0, n, [&](int jq, int tt) { return rank_value(src, r, series, q0 + jq, j, tt) - s_cm[jq]; });
+        __syncthreads();
+        if (on) acc = lag_chunk_dot(sA, sB, w, lane, min(SER_DIAG_TC, span - t0), acc);
+      }
+    }
+    if (on) {
+      const double rho = 1.0 - (Wq - acc / mn) / varp; /* rho(k0 + lane) */
+      if (k0 == 0) po = __shfl_sync(0xffffffffu, rho, 1);
+      for (;;) {
+        if (!(t < n - 3 && pe + po > 0.0)) { on = false; break; }
+        if (t + 1 >= k0 + 32) break; /* the next pair is in the next lag block */
+        const double e = __shfl_sync(0xffffffffu, rho, t + 1 - k0), o = __shfl_sync(0xffffffffu, rho, t + 2 - k0);
+        double P = pe + po;
+        if (!first && P > pprev) P = pprev;
+        first = false; psum += P; pprev = P;
+        pe = e; po = o; stored = e + o >= 0.0;
+        t += 2;
+      }
+    }
+  }
+  if (lane == 0 && s_on[w]) {
+    const double last = (pe > 0.0 || stored) ? pe : 0.0; /* rho[max_t + 1] */
+    const double tau = fmax(-1.0 + 2.0 * psum + last, 1.0 / log10(mn));
+    out[(size_t)qw * 8 + field] = mn / tau;
+  }
 }
 
 /* ------------------------------------------------------------------ streaming accumulators (ser_run_accumulate)

@@ -12,6 +12,7 @@
  * Reference: /root/reference/C_Implementation/mcmc.c (line numbers next to each device function).
  */
 #include <cuda_runtime.h>
+#include <cub/device/device_radix_sort.cuh>
 
 #include <cstdarg>
 #include <cstdio>
@@ -1458,6 +1459,108 @@ extern "C" int ser_run_diagnostics(ser_run *run, const int32_t *chosen, int32_t 
   };
   const int rc = body();
   void *tmp[] = {d_ch, d_n, d_stats, d_halves};
+  for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
+  return rc;
+}
+
+extern "C" int ser_run_rank_diagnostics(ser_run *run, const int32_t *chosen, int32_t k, int32_t what, double *out)
+{
+  if (!run || !chosen || !out || k < 1 || what < 1 || what > 3) {
+    ser_set_error("ser_run_rank_diagnostics: bad argument (k = %d, what = %d)", k, what);
+    return SER_E_ARG;
+  }
+  std::vector<int> ids(chosen, chosen + k), loc(k);
+  std::sort(ids.begin(), ids.end()); /* the sequences' order, whatever the order of `chosen` */
+  for (int c = 0; c < k; c++) {
+    if (ids[c] < 0 || (c > 0 && ids[c] == ids[c - 1]) || (loc[c] = ser_run_local_chain(run, ids[c])) < 0) {
+      ser_set_error("ser_run_rank_diagnostics: chosen chain %d is %s", ids[c],
+                    ids[c] < 0 ? "negative" : (c > 0 && ids[c] == ids[c - 1]) ? "repeated" : "not held by this run");
+      return SER_E_ARG;
+    }
+  }
+  if (!run->initialized) { ser_set_error("ser_run_rank_diagnostics: run not initialised"); return SER_E_STATE; }
+  if (run->acc_what) { ser_set_error("ser_run_rank_diagnostics: the store of an accumulating run is a transient window"); return SER_E_STATE; }
+  if ((what & SER_DIAG_SCALARS) && run->cfg.store < SER_STORE_FULL) {
+    ser_set_error("ser_run_rank_diagnostics: -loglik, exp(c), exp(d) need SER_STORE_FULL");
+    return SER_E_STATE;
+  }
+  if ((what & SER_DIAG_SITES) && run->cfg.store < SER_STORE_PI) { ser_set_error("ser_run_rank_diagnostics: pi needs SER_STORE_PI"); return SER_E_STATE; }
+  if (set_device(run)) return SER_E_CUDA;
+  std::vector<int> ns(k);
+  for (int c = 0; c < k; c++)
+    CUDA_TRY(cudaMemcpyAsync(&ns[c], &run->d_scal[loc[c]].n_samples, sizeof(int), cudaMemcpyDeviceToHost, run->stream));
+  CUDA_TRY(cudaStreamSynchronize(run->stream));
+  const int T = std::min(ns[0], run->cfg.max_samples);
+  for (int c = 0; c < k; c++) {
+    const int Tc = std::min(ns[c], run->cfg.max_samples);
+    if (Tc != T) {
+      ser_set_error("ser_run_rank_diagnostics: chains %d and %d hold different numbers of samples (%d vs %d)", ids[0], ids[c], T, Tc);
+      return SER_E_STATE;
+    }
+  }
+  if (T < 4) { ser_set_error("ser_run_rank_diagnostics: the chains hold %d stored samples (at least 4 are needed)", T); return SER_E_STATE; }
+
+  const int N = run->N, Q = 3 + N, m = 2 * k, n = T / 2, S = m * n;
+  const int qlo = (what & SER_DIAG_SCALARS) ? 0 : 3, qhi = (what & SER_DIAG_SITES) ? Q : 3;
+  const bool sites = what & SER_DIAG_SITES, scalars = what & SER_DIAG_SCALARS;
+  int *d_loc = nullptr, *d_hist = nullptr, *d_vals = nullptr;
+  double *d_out = nullptr, *d_seq = nullptr, *d_qs = nullptr, *d_zt = nullptr, *d_zs = nullptr, *d_keys = nullptr;
+  void *d_cub = nullptr;
+  auto body = [&]() -> int {
+    const size_t NN = (size_t)N * N, S3 = (size_t)3 * S;
+    CUDA_TRY(POOL_ALLOC(&d_loc, k * sizeof(int)));
+    CUDA_TRY(POOL_ALLOC(&d_out, (size_t)Q * 8 * sizeof(double)));
+    CUDA_TRY(POOL_ALLOC(&d_seq, (size_t)5 * Q * m * 2 * sizeof(double)));
+    CUDA_TRY(POOL_ALLOC(&d_qs, (size_t)Q * 3 * sizeof(double)));
+    CUDA_TRY(cudaMemcpyAsync(d_loc, loc.data(), k * sizeof(int), cudaMemcpyHostToDevice, run->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_out, out, (size_t)Q * 8 * sizeof(double), cudaMemcpyHostToDevice, run->stream));
+    const RankSeq rs = {d_loc, T, n, m, run->cfg.max_samples};
+    RankSrc src = {run->d_samp_pi, run->d_samp_cdl, nullptr, nullptr, nullptr, nullptr, d_qs, N};
+    if (sites) { /* the pooled histogram, then z, z_fold, q05, q95 and the median of every site */
+      CUDA_TRY(POOL_ALLOC(&d_hist, NN * sizeof(int)));
+      CUDA_TRY(POOL_ALLOC(&d_zt, 2 * NN * sizeof(double)));
+      src.zt = d_zt; src.zft = d_zt + NN;
+      HistShape hs;
+      CUDA_TRY(hist_shape((const void *)ser_rank_hist_kernel, N, &hs));
+      mark_launch(run);
+      ser_rank_hist_kernel<<<(N + hs.threads - 1) / hs.threads, hs.threads, hs.smem, run->stream>>>(run->d_samp_pi, N, rs, hs.smem > 0, d_hist);
+      CUDA_TRY(cudaGetLastError());
+      mark_launch(run);
+      ser_rank_table_kernel<<<N, 256, 0, run->stream>>>(d_hist, N, S, d_zt, d_zt + NN, d_qs, d_out);
+      CUDA_TRY(cudaGetLastError());
+    }
+    if (scalars) { /* per scalar: sort the draws, rank them (and take the quantiles and median); then the same for the folded draws */
+      CUDA_TRY(POOL_ALLOC(&d_keys, 2 * S3 * sizeof(double)));
+      CUDA_TRY(POOL_ALLOC(&d_vals, 2 * S3 * sizeof(int)));
+      CUDA_TRY(POOL_ALLOC(&d_zs, 2 * S3 * sizeof(double)));
+      src.zs = d_zs; src.zfs = d_zs + S3;
+      size_t cub_bytes = 0;
+      CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, d_keys, d_keys + S3, d_vals, d_vals + S3, S, 0, 64, run->stream));
+      CUDA_TRY(POOL_ALLOC(&d_cub, cub_bytes));
+      const int blocks = std::min((S + 255) / 256, 1024);
+      for (int fold = 0; fold < 2; fold++) {
+        mark_launch(run);
+        ser_rank_gather_kernel<<<dim3(blocks, 3), 256, 0, run->stream>>>(run->d_samp_cdl, rs, d_qs, fold, d_keys, d_vals);
+        CUDA_TRY(cudaGetLastError());
+        for (int q = 0; q < 3; q++) {
+          size_t bytes = cub_bytes;
+          CUDA_TRY(cub::DeviceRadixSort::SortPairs(d_cub, bytes, d_keys + q * (size_t)S, d_keys + S3 + q * (size_t)S, d_vals + q * (size_t)S,
+                                                   d_vals + S3 + q * (size_t)S, S, 0, 64, run->stream));
+        }
+        mark_launch(run);
+        ser_rank_scalar_kernel<<<dim3(blocks, 3), 256, 0, run->stream>>>(d_keys + S3, d_vals + S3, S, fold, d_zs + fold * S3, d_qs, d_out);
+        CUDA_TRY(cudaGetLastError());
+      }
+    }
+    mark_launch(run);
+    ser_rank_ess_kernel<<<dim3((qhi - 1) / 32 - qlo / 32 + 1, 5), 1024, 0, run->stream>>>(src, rs, qlo, qhi, d_seq, d_out);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(out, d_out, (size_t)Q * 8 * sizeof(double), cudaMemcpyDeviceToHost, run->stream));
+    CUDA_TRY(cudaStreamSynchronize(run->stream));
+    return SER_OK;
+  };
+  const int rc = body();
+  void *tmp[] = {d_loc, d_hist, d_vals, d_out, d_seq, d_qs, d_zt, d_zs, d_keys, d_cub};
   for (void *t : tmp) if (t) cudaFreeAsync(t, run->stream);
   return rc;
 }
