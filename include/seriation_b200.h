@@ -251,6 +251,23 @@ int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k, int32_t *p
  * SER_E_ARG: rows < 1, bins < 1, n_probs < 1, a NULL pointer, or a probability outside (0, 1] (NaN included). */
 int ser_hist_quantiles(const int32_t *hist, int32_t rows, int32_t bins, const double *probs, int32_t n_probs, int32_t *out);
 
+/* Taxon pair relations (DESIGN.md section 3.10).  For chosen chain c over its T samples t, taxa m, n in file order, ranges half-open
+ * (taxon m is alive at a_t(m) <= pos < b_t(m), a <= b <= N):
+ *   first[c][m][n]    = #{t : a_t(m) < a_t(n)}                              m originated strictly before n (FAD order)
+ *   last[c][m][n]     = #{t : b_t(m) < b_t(n)}                              m went extinct strictly before n (LAD order)
+ *   precedes[c][m][n] = #{t : b_t(m) <= a_t(n)}                             m's range ends before n's begins (superposition)
+ *   coexist[c][m][n]  = #{t : max(a_t(m), a_t(n)) < min(b_t(m), b_t(n))}    the two ranges share at least one position
+ * No special case on the diagonal: first[m][m] = last[m][m] = 0, precedes[m][m] = #{t : a = b} (empty ranges), coexist[m][m] =
+ * #{t : a < b}.  Exact identities: first[m][n] + first[n][m] + #{t : a_t(m) = a_t(n)} = T (last alike); coexist is symmetric;
+ * coexist[m][n] + precedes[m][n] + precedes[n][m] = T when neither range is empty in any sample.
+ * Counts add over windows, chains and devices.  Chosen ids are GLOBAL; -1 or a chain this run does not hold leaves its slabs untouched
+ * and n_samples[c] = 0; a held chain's slabs are written in full.  Host memory: each output [k][M][M] int32, any of the four may be
+ * NULL but not all.  Needs SER_STORE_FULL.  On an accumulating run (SER_ACC_TAXA) T counts every sample taken since accumulation began.
+ * Checked before any CUDA call: SER_E_ARG for k < 1, a NULL chosen or n_samples, or all four outputs NULL; SER_E_STATE for a store
+ * below SER_STORE_FULL, an accumulating run without SER_ACC_TAXA, or a run not initialised. */
+int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t k, int32_t *first, int32_t *last, int32_t *precedes,
+                        int32_t *coexist, int32_t *n_samples);
+
 /* CORR_MN (Docs/Report.pdf Table 1; SURVEY section 8f #3): Pearson correlation of the posterior mean
  * position E[pi(site)] over the stored samples of the chosen chains owned by this run with the MN age
  * of the site read from the .sites file (ser_dataset_read_names): the mean over the stored samples of
@@ -269,15 +286,17 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
 #define SER_ACC_ALIVE 8 /* alive difference slab        [N][M]      (needs SER_STORE_FULL)                  */
 #define SER_ACC_POS 16  /* position histograms          [N][N]      (ser_run_marginals' pos)                */
 #define SER_ACC_RANGE 32 /* a and b histograms          [2][M][N+1] (needs SER_STORE_FULL)                  */
+#define SER_ACC_TAXA 128 /* taxon pair relations       [4][M][M]   (ser_run_taxon_pairs; needs SER_STORE_FULL); 64 is not a flag */
 /* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
  * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
  * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),
- * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals and ser_run_site_age_corr then return totals over EVERY sample taken since
- * (T = the chain's sample count), with the usual global ids and slab convention; ser_run_fetch_samples /
+ * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals, ser_run_taxon_pairs and ser_run_site_age_corr then return totals over
+ * EVERY sample taken since (T = the chain's sample count), with the usual global ids and slab convention; ser_run_fetch_samples /
  * ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does ser_run_cross_chain_async.
  * Call it before the first sampling call (ser_run_init zeroes the accumulators).  Errors: SER_E_STATE on a run that has
  * already sampled, on a store below what the flags need, or a second time; SER_E_ARG for max_samples < 1; SER_E_CUDA with
- * the byte count when an accumulator does not fit (per chain at 2048 x 8192: the alive slab is 64 MB, the a / b histograms 134 MB). */
+ * the byte count when an accumulator does not fit (per chain at 2048 x 8192: the alive slab is 64 MB, the a / b histograms 134 MB,
+ * the taxon pair relations 1 GiB; 256 MB at 1024 x 4096). */
 int ser_run_accumulate(ser_run *run, int32_t what);
 
 /* ---------------------------------------------------------------- cross-chain step, one call

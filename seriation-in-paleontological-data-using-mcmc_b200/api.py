@@ -18,7 +18,8 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
-ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE = 1, 2, 4, 8, 16, 32
+ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE, ACC_TAXA = 1, 2, 4, 8, 16, 32, 128
+TAXON_PAIRS = ("first", "last", "precedes", "coexist")
 DIAG_SCALARS, DIAG_SITES = 1, 2
 RDIAG_FIELDS = ("rhat_bulk", "rhat_fold", "ess_bulk", "ess_mean", "ess_q05", "ess_q95", "q05", "q95")
 
@@ -86,6 +87,7 @@ SYMBOLS = [
     ("ser_run_rank_diagnostics", C.c_int, [_vp, _i32p, C.c_int32, C.c_int32, _dp]),
     ("ser_run_marginals", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p]),
     ("ser_hist_quantiles", C.c_int, [_i32p, C.c_int32, C.c_int32, _dp, C.c_int32, _i32p]),
+    ("ser_run_taxon_pairs", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p, _i32p]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
     ("ser_write_labelled_files", C.c_int, [_vp, C.c_int32, _vp, C.c_char_p]),
     ("ser_microbench", C.c_int, [C.c_int32, _dp]),
@@ -240,12 +242,12 @@ class Run:
             _check(lib().ser_run_create_chains(ds._h, C.byref(self.cfg), _p(ids, C.c_int32), ids.size, C.byref(h)))
         self._h = h
 
-    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False):
+    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False, taxon_pairs=False):
         """from now on the sample store is a window of max_samples rows and the summaries sum over every sample taken
         afterwards (ser_run_accumulate); call before the first sampling call.  ``positions`` / ``ranges`` accumulate the
-        histograms of marginals()"""
+        histograms of marginals(), ``taxon_pairs`` the counts of taxon_pairs()"""
         what = (ACC_PO if po else 0) | (ACC_SUMS if sums else 0) | (ACC_AB if ab else 0) | (ACC_ALIVE if alive else 0)
-        what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0)
+        what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0) | (ACC_TAXA if taxon_pairs else 0)
         _check(lib().ser_run_accumulate(self._h, what))
         return self
 
@@ -442,6 +444,21 @@ class Run:
         _check(lib().ser_run_marginals(self._h, _p(chosen, C.c_int32), k, _p(pos, C.c_int32), _p(a, C.c_int32), _p(b, C.c_int32),
                                        _p(n, C.c_int32)))
         return dict(pos=pos, a=a, b=b, n_samples=n)
+
+    def taxon_pairs(self, chosen, first: bool = True, last: bool = True, precedes: bool = True, coexist: bool = True) -> dict:
+        """taxon pair relations of the chosen chains (global ids) over their samples (ser_run_taxon_pairs), each [k][M][M] int32 (None
+        when not requested): ``first`` = #{t: a_t(m) < a_t(n)}, ``last`` = #{t: b_t(m) < b_t(n)}, ``precedes`` = #{t: b_t(m) <= a_t(n)},
+        ``coexist`` = #{t: max(a_t(m), a_t(n)) < min(b_t(m), b_t(n))}; ``n_samples`` [k] = T.  Slabs the run does not fill stay 0
+        (n_samples 0)."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        k, M = len(chosen), self.M
+        want = dict(first=first, last=last, precedes=precedes, coexist=coexist)
+        out = {key: (np.zeros((k, M, M), np.int32) if want[key] else None) for key in TAXON_PAIRS}
+        n = np.zeros(k, np.int32)
+        _check(lib().ser_run_taxon_pairs(self._h, _p(chosen, C.c_int32), k, *(_p(out[key], C.c_int32) for key in TAXON_PAIRS),
+                                         _p(n, C.c_int32)))
+        out["n_samples"] = n
+        return out
 
     def po_counts_device(self, chosen_ptr: int, k: int, counts_ptr: int):
         _check(lib().ser_run_po_counts_device(self._h, chosen_ptr, k, counts_ptr))
@@ -699,23 +716,24 @@ def choose_chains(batch: ChainBatch, chains_selected: int):
 
 
 def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, marginals: bool = False,
-                  device=None) -> ChainBatch:
+                  taxon_pairs: bool = False, device=None) -> ChainBatch:
     """The second phase of select-then-replay: re-simulate the chosen chains of a batch (typically one run with
     ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
     ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
     run's, so compute_pair_order_matrix, compute_exp_* and the probability maps work on it unchanged.  ``with_ab``
     also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  ``window=0`` keeps every
     sample instead (``STORE_FULL``, no accumulators): the summaries take the one-shot path and ``diagnostics`` works on
-    the result.  ``marginals`` also accumulates the position and a/b histograms of marginals() (the window then keeps a and b).
+    the result.  ``marginals`` also accumulates the position and a/b histograms of marginals(), and ``taxon_pairs`` the counts of
+    taxon_pairs() (either makes the window keep a and b).
     Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
     ids = np.ascontiguousarray(chains, dtype=np.int32)
     keep_all = window == 0
     run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
-              store=STORE_FULL if (with_ab or keep_all or marginals) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
+              store=STORE_FULL if (with_ab or keep_all or marginals or taxon_pairs) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
               device=batch.run.cfg.device if device is None else device, chain_ids=ids)
     run.init()
     if not keep_all:
-        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals)
+        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals, taxon_pairs=taxon_pairs)
     run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
     want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
     if want.tobytes() != got.tobytes():
@@ -769,6 +787,20 @@ def marginals(batch: ChainBatch, chains, probs=(0.025, 0.5, 0.975)) -> dict:
                 a=_marginal_summary(pooled["a"], probs) if ranges else None,
                 b=_marginal_summary(pooled["b"], probs) if ranges else None,
                 counts=pooled, n_samples=int(m["n_samples"].sum()), probs=tuple(probs))
+
+
+def taxon_pairs(batch: ChainBatch, chains) -> dict:
+    """Taxon pair relations pooled over the chosen chains by summing their counts (int64): the probability matrices [M][M] (taxa in file
+    order) ``first`` = P(m originated strictly before n), ``last`` = P(m went extinct strictly before n), ``precedes`` = P(m's range ends
+    before n's begins) and ``coexist`` = P(the two ranges share a position), each the pooled count over the pooled sample count;
+    ``counts`` holds the pooled counts and ``n_samples`` the pooled sample count.  Needs a batch that keeps a and b: the full sample
+    store, or replay_chosen(..., taxon_pairs=True)."""
+    tp = batch.run.taxon_pairs(np.asarray(chains, dtype=np.int32))
+    counts = {key: tp[key].sum(axis=0, dtype=np.int64) for key in TAXON_PAIRS}
+    n = int(tp["n_samples"].sum(dtype=np.int64))
+    out = {key: counts[key] / n for key in TAXON_PAIRS}
+    out.update(counts=counts, n_samples=n)
+    return out
 
 
 def compute_exp_cd(batch: ChainBatch, chains, chains_selected: int, faithful: bool = True):

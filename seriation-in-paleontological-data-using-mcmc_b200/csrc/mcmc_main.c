@@ -18,7 +18,7 @@
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
  *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--rank-diagnostics FILE]
- *        [--marginals PREFIX]
+ *        [--marginals PREFIX] [--taxon-pairs PREFIX]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
@@ -41,6 +41,10 @@
  * chains and writes PREFIX.sites.csv "site,hard,mean,q025,median,q975,mode,p_mode" (file order, 0-based positions) and
  * PREFIX.taxa.csv "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975", and prints one summary line; under
  * --replay-selected --po (without --diagnostics) the same run supplies the pair-order counts, so the chains are replayed once.
+ * --taxon-pairs PREFIX (with --select) accumulates the taxon pair relations of the chosen chains (ser_run_taxon_pairs) through the same
+ * replay (one replay serves it and --marginals), pools the counts over the chains and writes PREFIX.first.csv, PREFIX.last.csv,
+ * PREFIX.precedes.csv and PREFIX.coexist.csv: dense M x M probability matrices (row m, column n, taxa in file order; po.csv's format) of
+ * P(a_m < a_n), P(b_m < b_n), P(b_m <= a_n) and P(the ranges of m and n share a position), and prints one summary line.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -73,7 +77,9 @@ static void usage(const char *argv0)
           "              [--rank-diagnostics FILE]   (with --select: rank-normalised R-hat, bulk- and tail-ESS pooled over the\n"
           "                                           chosen chains to FILE)\n"
           "              [--marginals PREFIX]   (with --select: position and a / b credible intervals of the chosen chains to\n"
-          "                                      PREFIX.sites.csv and PREFIX.taxa.csv; the replay uses --window W)\n",
+          "                                      PREFIX.sites.csv and PREFIX.taxa.csv; the replay uses --window W)\n"
+          "              [--taxon-pairs PREFIX]   (with --select: first / last appearance order, superposition and coexistence\n"
+          "                                        of every pair of taxa to PREFIX.{first,last,precedes,coexist}.csv; --window W)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -231,12 +237,41 @@ static double median_width(const struct marginal *m, int32_t n, double *w)
   return n % 2 ? w[n / 2] : 0.5 * (w[n / 2 - 1] + w[n / 2]);
 }
 
-/* --marginals: the chosen chains re-simulated alone through a window of W samples while their position and a / b histograms accumulate
- * (bit-identical to their first run, whose E[-logL] per global id - first is e[]; any difference exits 1), the counts pooled over the
- * chains, PREFIX.sites.csv and PREFIX.taxa.csv written and one summary line printed.  `counts` (NULL: not wanted) receives their
- * pair-order counts from the same run. */
+/* --taxon-pairs: the four [k][M][M] count slabs of ser_run_taxon_pairs pooled over the k chains (tot samples) to PREFIX.<name>.csv as
+ * probability matrices, and one summary line */
+static void write_taxon_pairs(int32_t *const tp[4], int32_t k, int32_t M, int32_t tot, const char *prefix)
+{
+  static const char *names[4] = {"first", "last", "precedes", "coexist"};
+  const size_t MM = (size_t)M * M;
+  long long hi = 0, lo = 0;
+  char path[4096];
+  int q, c;
+  size_t j;
+  FILE *f;
+  for (q = 0; q < 4; q++) {
+    snprintf(path, sizeof(path), "%s.%s.csv", prefix, names[q]);
+    if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+    for (j = 0; j < MM; j++) {
+      int64_t sum = 0;
+      double p;
+      for (c = 0; c < k; c++) sum += tp[q][c * MM + j];
+      p = (double)sum / (double)tot;
+      fprintf(f, "%.6f%c", p, (j + 1) % (size_t)M ? ',' : '\n');
+      if (q == 3 && j / M < j % M) { hi += p >= 0.95; lo += p <= 0.05; }
+    }
+    if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  }
+  printf("taxon pairs: %d chains  %d samples  of %lld pairs of taxa %lld coexist with P >= 0.95 and %lld with P <= 0.05\n", k, tot,
+         (long long)M * (M - 1) / 2, hi, lo);
+}
+
+/* --marginals / --taxon-pairs: the chosen chains re-simulated alone through a window of W samples while their position and a / b
+ * histograms (prefix) and their taxon pair relations (pairs_prefix) accumulate (either prefix may be NULL; bit-identical to their first
+ * run, whose E[-logL] per global id - first is e[]; any difference exits 1), the counts pooled over the chains, PREFIX.sites.csv and
+ * PREFIX.taxa.csv or the four taxon pair matrices written, and one summary line printed for each.  `counts` (NULL: not wanted) receives
+ * their pair-order counts from the same run. */
 static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
-                             int burn, int samples, int window, int32_t *counts, const char *prefix)
+                             int burn, int samples, int window, int32_t *counts, const char *prefix, const char *pairs_prefix)
 {
   ser_run_config c2 = *cfg;
   ser_run *sub = NULL;
@@ -258,7 +293,9 @@ static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, c
   c2.store = SER_STORE_FULL;
   c2.max_samples = window;
   if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
-  if (ser_run_init(sub) || ser_run_accumulate(sub, SER_ACC_POS | SER_ACC_RANGE | (counts ? SER_ACC_PO : 0))) die("ser_run_accumulate");
+  if (ser_run_init(sub) || ser_run_accumulate(sub, (prefix ? SER_ACC_POS | SER_ACC_RANGE : 0) | (pairs_prefix ? SER_ACC_TAXA : 0) |
+                                                     (counts ? SER_ACC_PO : 0)))
+    die("ser_run_accumulate");
   if (ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
   if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
   for (i = 0; i < k; i++)
@@ -268,8 +305,24 @@ static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, c
       exit(1);
     }
   if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
+  if (pairs_prefix) {
+    const size_t MM = (size_t)M * M;
+    int32_t *tp[4];
+    for (c = 0; c < 4; c++)
+      if (!(tp[c] = (int32_t *)malloc(sizeof(int32_t) * k * MM))) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+    if (ser_run_taxon_pairs(sub, chosen, k, tp[0], tp[1], tp[2], tp[3], n)) die("ser_run_taxon_pairs");
+    for (tot = 0, c = 0; c < k; c++) tot += n[c];
+    write_taxon_pairs(tp, k, M, tot, pairs_prefix);
+    for (c = 0; c < 4; c++) free(tp[c]);
+  }
+  if (!prefix) {
+    ser_run_destroy(sub);
+    free(pos); free(ah); free(bh); free(n); free(e2); free(w); free(ms); free(ma); free(mb); free(hard);
+    return;
+  }
   if (ser_run_marginals(sub, chosen, k, pos, ah, bh, n)) die("ser_run_marginals");
   ser_run_destroy(sub);
+  tot = 0;
   for (c = 1; c < k; c++) { /* pool the chains' counts into chain 0's slabs */
     for (j = 0; j < NN; j++) pos[j] += pos[c * NN + j];
     for (j = 0; j < MB; j++) { ah[j] += ah[c * MB + j]; bh[j] += bh[c * MB + j]; }
@@ -319,7 +372,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
-  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL;
+  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL, *pairs_prefix = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -356,6 +409,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--diagnostics")) diag_path = v;
       else if (!strcmp(a, "--rank-diagnostics")) rdiag_path = v;
       else if (!strcmp(a, "--marginals")) marg_prefix = v;
+      else if (!strcmp(a, "--taxon-pairs")) pairs_prefix = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
@@ -364,7 +418,7 @@ int main(int argc, char **argv)
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
     if ((diag_path || rdiag_path) && select_k < 1) usage(argv[0]);
-    if (marg_prefix && (select_k < 1 || window < 1)) usage(argv[0]);
+    if ((marg_prefix || pairs_prefix) && (select_k < 1 || window < 1)) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
@@ -495,7 +549,7 @@ int main(int argc, char **argv)
         /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix) {
+        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix && !pairs_prefix) {
           ser_run_config c2 = cfg;
           ser_run *sub = NULL;
           c2.n_chains = nchosen;
@@ -518,10 +572,10 @@ int main(int argc, char **argv)
       }
       if ((diag_path || rdiag_path) && nchosen > 0)
         replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path, rdiag_path);
-      if (marg_prefix && nchosen > 0)
+      if ((marg_prefix || pairs_prefix) && nchosen > 0)
         replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window,
                          (replay_selected && !diag_path && !rdiag_path) ? counts : NULL,
-                         marg_prefix);
+                         marg_prefix, pairs_prefix);
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);
         FILE *f;

@@ -347,6 +347,64 @@ __global__ void ser_alive_kernel(const uint16_t *samp_a, const uint16_t *samp_b,
   for (int j = 0; j < N; j++) { acc += col[(size_t)j * M]; col[(size_t)j * M] = acc; }
 }
 
+/* taxon pair relations (ser_run_taxon_pairs, DESIGN.md 3.10), one 32 x 32 tile of (m, n) per block, slab blockIdx.z of each output
+ * that is not nullptr: first = #{t : a_m < a_n}, last = #{t : b_m < b_n}, precedes = #{t : b_m <= a_n}, coexist = #{t : max(a_m, a_n) <
+ * min(b_m, b_n)}.  The tile's 64 taxa are staged 32 samples at a time as (a | b << 16) words from coalesced rows of the a and b stores;
+ * thread (tx, ty) owns n = n0 + tx and the four rows m = m0 + 4 ty + r, read as one 16-byte word (a broadcast within the warp).  Its 16
+ * counters stay in registers over all T rows: no atomics, so the counts do not depend on the launch shape.  All four are counted
+ * whatever is requested: every caller in the project asks for all four, and a one-output variant would be a second kernel (DESIGN.md
+ * 3.10). */
+__global__ void __launch_bounds__(256) ser_taxon_pair_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const ChainScalars *scal, int M,
+                                                             int max_samples, SumSel sel, int *first, int *last, int *precedes, int *coexist,
+                                                             size_t stride, int add)
+{
+  __shared__ __align__(16) uint32_t sm[SER_PO_TS][32], sn[SER_PO_TS][32];
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.z, blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0, &T);
+  if (local < 0) return;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5, m0 = blockIdx.y * 32, n0 = blockIdx.x * 32;
+  const uint16_t *A = samp_a + (size_t)local * max_samples * M, *B = samp_b + (size_t)local * max_samples * M;
+  int cf[4] = {0, 0, 0, 0}, cl[4] = {0, 0, 0, 0}, cp[4] = {0, 0, 0, 0}, cc[4] = {0, 0, 0, 0};
+  for (int t0 = 0; t0 < T; t0 += SER_PO_TS) {
+    const int nt = min(SER_PO_TS, T - t0);
+    __syncthreads();
+    for (int q = threadIdx.x; q < nt * 32; q += 256) {
+      const int t = q >> 5, x = q & 31;
+      const size_t row = (size_t)(t0 + t) * M;
+      sm[t][x] = m0 + x < M ? (uint32_t)A[row + m0 + x] | (uint32_t)B[row + m0 + x] << 16 : 0u;
+      sn[t][x] = n0 + x < M ? (uint32_t)A[row + n0 + x] | (uint32_t)B[row + n0 + x] << 16 : 0u;
+    }
+    __syncthreads();
+    for (int t = 0; t < nt; t++) {
+      const uint32_t wn = sn[t][tx];
+      const int an = (int)(wn & 0xffffu), bn = (int)(wn >> 16);
+      const uint4 w4 = *reinterpret_cast<const uint4 *>(&sm[t][4 * ty]);
+      const uint32_t wm[4] = {w4.x, w4.y, w4.z, w4.w};
+#pragma unroll
+      for (int r = 0; r < 4; r++) {
+        const int am = (int)(wm[r] & 0xffffu), bm = (int)(wm[r] >> 16);
+        cf[r] += am < an;
+        cl[r] += bm < bn;
+        cp[r] += bm <= an;
+        cc[r] += max(am, an) < min(bm, bn);
+      }
+    }
+  }
+  const int n = n0 + tx;
+  if (n >= M) return;
+  int *const outs[4] = {first, last, precedes, coexist};
+#pragma unroll
+  for (int r = 0; r < 4; r++) {
+    const int m = m0 + 4 * ty + r;
+    if (m >= M) continue;
+    const size_t e = (size_t)blockIdx.z * stride + (size_t)m * M + n;
+    const int v[4] = {cf[r], cl[r], cp[r], cc[r]};
+#pragma unroll
+    for (int q = 0; q < 4; q++)
+      if (outs[q]) outs[q][e] = add ? outs[q][e] + v[q] : v[q];
+  }
+}
+
 /* ------------------------------------------------------------------ convergence diagnostics (ser_run_diagnostics, DESIGN.md 3.7)
  * Quantity q of a chain's stored sample t: 0 = -loglik, 1 = exp(c), 2 = exp(d) (samp_cdl; taxon 0's c, d on a manycd run),
  * 3 + i = pi_t(i), the position of site i.  One block of 32 warps per (chosen chain, 32 consecutive quantities).  The moments
@@ -825,14 +883,15 @@ __global__ void __launch_bounds__(1024, 1) ser_rank_ess_kernel(RankSrc src, Rank
  * the summary kernels above add the window's rows of EVERY local chain into that chain's accumulator record; the getters turn the
  * records into what the one-shot kernels compute from a store that holds all samples, with the kernels below. */
 
-#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE)
+#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE | SER_ACC_TAXA)
 
 /* One local chain's accumulator record: int32 offsets of the parts the flags `what` select, in this order, and the record's length.
  * The run holds [n_local][ints]; a checkpoint record holds the same ints in the same order.
  *   po [N][N] (SER_ACC_PO; diagonal 0), pi [N] (SER_ACC_SUMS or SER_ACC_AB), asum [M], bsum [M] (SER_ACC_AB),
- *   alive [N][M] (SER_ACC_ALIVE; the difference slab), pos [N][N] (SER_ACC_POS), range [2][M][N+1] (SER_ACC_RANGE; a, then b) */
+ *   alive [N][M] (SER_ACC_ALIVE; the difference slab), pos [N][N] (SER_ACC_POS), range [2][M][N+1] (SER_ACC_RANGE; a, then b),
+ *   taxa [4][M][M] (SER_ACC_TAXA; first, last, precedes, coexist) */
 struct AccLayout {
-  size_t po, pi, asum, bsum, alive, pos, range, ints;
+  size_t po, pi, asum, bsum, alive, pos, range, taxa, ints;
 };
 __host__ __device__ inline AccLayout acc_layout(int N, int M, int what)
 {
@@ -846,6 +905,7 @@ __host__ __device__ inline AccLayout acc_layout(int N, int M, int what)
   L.alive = o; o += (what & SER_ACC_ALIVE) ? n * m : 0;
   L.pos = o; o += (what & SER_ACC_POS) ? n * n : 0;
   L.range = o; o += (what & SER_ACC_RANGE) ? 2 * m * (n + 1) : 0;
+  L.taxa = o; o += (what & SER_ACC_TAXA) ? 4 * m * m : 0;
   L.ints = o;
   return L;
 }

@@ -649,7 +649,7 @@ extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
   if (what < 1 || (what & ~SER_ACC_ALL)) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
   if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
   if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
-  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE)) ? SER_STORE_FULL : SER_STORE_PI;
+  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE | SER_ACC_TAXA)) ? SER_STORE_FULL : SER_STORE_PI;
   if (run->cfg.store < need) {
     ser_set_error("ser_run_accumulate: these summaries need %s", need == SER_STORE_FULL ? "SER_STORE_FULL (a, b samples)" : "SER_STORE_PI or more");
     return SER_E_STATE;
@@ -884,6 +884,18 @@ static int launch_range_hist(ser_run *run, const SumSel &sel, int k, int *a_hist
   return SER_OK;
 }
 
+/* taxa [4] = first, last, precedes, coexist slabs (any may be nullptr), slab z at taxa[q] + z * stride */
+static int launch_taxon_pairs(ser_run *run, const SumSel &sel, int k, int *const taxa[4], size_t stride, int add)
+{
+  const int M = run->M;
+  mark_launch(run);
+  ser_taxon_pair_kernel<<<dim3((M + 31) / 32, (M + 31) / 32, k), 256, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_scal, M,
+                                                                                         run->cfg.max_samples, sel, taxa[0], taxa[1],
+                                                                                         taxa[2], taxa[3], stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
 /* rows [0, w) of every chain's window added into its accumulator record (ser_run_accumulate), on the run's stream */
 static int accumulate_window(ser_run *run, int w)
 {
@@ -900,6 +912,11 @@ static int accumulate_window(ser_run *run, int w)
   if (!rc && (what & SER_ACC_ALIVE)) rc = launch_alive(run, sel, nc, acc + L.alive, L.ints, 1);
   if (!rc && (what & SER_ACC_POS)) rc = launch_pos_hist(run, sel, nc, acc + L.pos, L.ints, 1);
   if (!rc && (what & SER_ACC_RANGE)) rc = launch_range_hist(run, sel, nc, acc + L.range, acc + L.range + (size_t)run->M * (run->N + 1), L.ints, 1);
+  if (!rc && (what & SER_ACC_TAXA)) {
+    const size_t mm = (size_t)run->M * run->M;
+    int *const taxa[4] = {acc + L.taxa, acc + L.taxa + mm, acc + L.taxa + 2 * mm, acc + L.taxa + 3 * mm};
+    rc = launch_taxon_pairs(run, sel, nc, taxa, L.ints, 1);
+  }
   return rc;
 }
 
@@ -1406,6 +1423,45 @@ extern "C" int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k,
   });
   if (rc != SER_OK) return rc;
   for (int c = 0; c < k; c++) n_samples[c] = n_out[c] < 0 ? 0 : n_out[c];
+  return SER_OK;
+}
+
+extern "C" int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t k, int32_t *first, int32_t *last, int32_t *precedes,
+                                   int32_t *coexist, int32_t *n_samples)
+{
+  if (!run || !chosen || !n_samples || k < 1 || (!first && !last && !precedes && !coexist)) {
+    ser_set_error("ser_run_taxon_pairs: bad argument (k = %d; chosen, n_samples and at least one of first, last, precedes, coexist are needed)", k);
+    return SER_E_ARG;
+  }
+  if (!run->initialized) { ser_set_error("ser_run_taxon_pairs: run not initialised"); return SER_E_STATE; }
+  if (run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_taxon_pairs: needs SER_STORE_FULL (a, b samples)"); return SER_E_STATE; }
+  if (run->acc_what && !(run->acc_what & SER_ACC_TAXA)) { ser_set_error("ser_run_taxon_pairs: the run accumulates without SER_ACC_TAXA"); return SER_E_STATE; }
+  if (set_device(run)) return SER_E_CUDA;
+  const int M = run->M;
+  const size_t cells = (size_t)M * M;
+  GetterOut f = {first, cells * sizeof(int), nullptr}, l = {last, cells * sizeof(int), nullptr};
+  GetterOut p = {precedes, cells * sizeof(int), nullptr}, c = {coexist, cells * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&f, &l, &p, &c}, [&](const int *d_ch, int *d_n) -> int {
+    if (!run->acc_what) {
+      int *const taxa[4] = {(int *)f.dev, (int *)l.dev, (int *)p.dev, (int *)c.dev};
+      return launch_taxon_pairs(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, taxa, cells, 0);
+    }
+    /* the record's four parts in order: (first, last), then (precedes, coexist), each pair one copy-out launch */
+    const AccLayout L = acc_layout(run->N, M, run->acc_what);
+    const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
+    GetterOut *pairs[2][2] = {{&f, &l}, {&p, &c}};
+    for (int h = 0; h < 2; h++) {
+      if (!pairs[h][0]->dev && !pairs[h][1]->dev) continue;
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.taxa + 2 * h * cells, L.ints, cells, run->d_scal, sel,
+                                                                        (int *)pairs[h][0]->dev, (int *)pairs[h][1]->dev);
+      CUDA_TRY(cudaGetLastError());
+    }
+    return SER_OK;
+  });
+  if (rc != SER_OK) return rc;
+  for (int q = 0; q < k; q++) n_samples[q] = n_out[q] < 0 ? 0 : n_out[q];
   return SER_OK;
 }
 
