@@ -25,6 +25,7 @@
  *   ser_run_posterior_sums    compute_exp_ages / compute_exp_pi / compute_exp_a
  *                                                       script.py:129-152, :230-276
  *   ser_run_alive_counts      plot_taxa_occurence_probability_matrix / plot_false_*  script.py:306-448
+ *   ser_run_cd_marginals      per-taxon (manycd) or scalar posterior of the error rates c, d: exp sums and histograms
  *   ser_run_site_age_corr     CORR_MN of Docs/Report.pdf Table 1 (E[pi] against the .sites MN ages)
  *   run_all_chains' Pool(8) over 100 processes (script.py:48-67) is replaced by
  *   n_chains in ser_run_config: one persistent launch over all chains of a GPU, and by
@@ -268,6 +269,31 @@ int ser_hist_quantiles(const int32_t *hist, int32_t rows, int32_t bins, const do
 int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t k, int32_t *first, int32_t *last, int32_t *precedes,
                         int32_t *coexist, int32_t *n_samples);
 
+/* Bounds of the error model's log-probabilities: the sampler keeps c (a false one, a recorded occurrence outside the taxon's range)
+ * in [SER_MINC, SER_MAXC] = [log .001, log .1] and d (a false zero, a missed occurrence inside it) in [SER_MIND, SER_MAXD] =
+ * [log .2, log .8].  They are also the edges of the histograms of ser_run_cd_marginals. */
+#define SER_MINC (-6.9077552789821368)
+#define SER_MAXC (-2.3025850929940455)
+#define SER_MIND (-1.6094379124341003)
+#define SER_MAXD (-0.22314355131420971)
+#define SER_CD_BINS 256
+
+/* Posterior of the error rates c, d (DESIGN.md section 3.11).  Rows: R = M on a manycd run (taxa in file order, each taxon's own
+ * c_m, d_m), R = 1 on a scalar run.  For chosen chain c and row r over its T samples t:
+ *   c_sum[c][r]     = sum_t exp(c_t(r)), a sequential fold in sample order from 0.0 with the sweep kernels' exp and rounding, so on
+ *                     a run whose samples all fit the store c_sum[c][0] / T equals ser_run_chain_stats' e_c bit for bit (d_sum: e_d)
+ *   c_hist[c][r][j] = #{t : bin(c_t(r)) = j}, j in [0, SER_CD_BINS), bins uniform on the stored log value over [SER_MINC, SER_MAXC]:
+ *                     bin(x) = min(B - 1, floor((x - lo) * s)) with s = B / (hi - lo) in double, each step rounded to nearest;
+ *                     x <= lo or NaN -> 0, x >= hi -> B - 1.  d_sum / d_hist alike over [SER_MIND, SER_MAXD].
+ * Every histogram row sums to T.  Counts and sums add over windows, chains and devices.  Chosen ids are GLOBAL; -1 or a chain this
+ * run does not hold leaves its slabs untouched and n_samples[c] = 0; a held chain's slabs are written in full.  Host memory: sums
+ * [k][R] double, histograms [k][R][SER_CD_BINS] int32; any of the four may be NULL but not all.  Needs SER_STORE_FULL.  On an
+ * accumulating run (SER_ACC_CD) T counts every sample taken since accumulation began, and the sums continue the same fold.
+ * Checked before any CUDA call: SER_E_ARG for k < 1, a NULL chosen or n_samples, or all four outputs NULL; SER_E_STATE for a store
+ * below SER_STORE_FULL, an accumulating run without SER_ACC_CD, or a run not initialised. */
+int ser_run_cd_marginals(ser_run *run, const int32_t *chosen, int32_t k, double *c_sum, double *d_sum, int32_t *c_hist, int32_t *d_hist,
+                         int32_t *n_samples);
+
 /* CORR_MN (Docs/Report.pdf Table 1; SURVEY section 8f #3): Pearson correlation of the posterior mean
  * position E[pi(site)] over the stored samples of the chosen chains owned by this run with the MN age
  * of the site read from the .sites file (ser_dataset_read_names): the mean over the stored samples of
@@ -287,12 +313,15 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
 #define SER_ACC_POS 16  /* position histograms          [N][N]      (ser_run_marginals' pos)                */
 #define SER_ACC_RANGE 32 /* a and b histograms          [2][M][N+1] (needs SER_STORE_FULL)                  */
 #define SER_ACC_TAXA 128 /* taxon pair relations       [4][M][M]   (ser_run_taxon_pairs; needs SER_STORE_FULL); 64 is not a flag */
+#define SER_ACC_CD 512  /* error-rate marginals         f64 [2][R], then [2][R][SER_CD_BINS] (ser_run_cd_marginals; needs SER_STORE_FULL;
+                           the part and the record's length padded to an even number of int32 words, so the doubles are aligned); 256 is not a flag */
 /* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
  * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
  * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),
- * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals, ser_run_taxon_pairs and ser_run_site_age_corr then return totals over
- * EVERY sample taken since (T = the chain's sample count), with the usual global ids and slab convention; ser_run_fetch_samples /
- * ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does ser_run_cross_chain_async.
+ * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals, ser_run_taxon_pairs, ser_run_cd_marginals and ser_run_site_age_corr
+ * then return totals over EVERY sample taken since (T = the chain's sample count), with the usual global ids and slab convention;
+ * ser_run_fetch_samples / ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does
+ * ser_run_cross_chain_async.
  * Call it before the first sampling call (ser_run_init zeroes the accumulators).  Errors: SER_E_STATE on a run that has
  * already sampled, on a store below what the flags need, or a second time; SER_E_ARG for max_samples < 1; SER_E_CUDA with
  * the byte count when an accumulator does not fit (per chain at 2048 x 8192: the alive slab is 64 MB, the a / b histograms 134 MB,

@@ -18,8 +18,13 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
-ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE, ACC_TAXA = 1, 2, 4, 8, 16, 32, 128
+ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE, ACC_TAXA, ACC_CD = 1, 2, 4, 8, 16, 32, 128, 512
 TAXON_PAIRS = ("first", "last", "precedes", "coexist")
+# the sampler's bounds of the log error rates (SER_MINC ... SER_MAXD): c in [log .001, log .1], d in [log .2, log .8]; the histograms of
+# cd_marginals() have CD_BINS uniform bins on the log value between them
+MINC, MAXC, MIND, MAXD = -6.9077552789821368, -2.3025850929940455, -1.6094379124341003, -0.22314355131420971
+CD_BOUNDS = dict(c=(MINC, MAXC), d=(MIND, MAXD))
+CD_BINS = 256
 DIAG_SCALARS, DIAG_SITES = 1, 2
 RDIAG_FIELDS = ("rhat_bulk", "rhat_fold", "ess_bulk", "ess_mean", "ess_q05", "ess_q95", "q05", "q95")
 
@@ -88,6 +93,7 @@ SYMBOLS = [
     ("ser_run_marginals", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p]),
     ("ser_hist_quantiles", C.c_int, [_i32p, C.c_int32, C.c_int32, _dp, C.c_int32, _i32p]),
     ("ser_run_taxon_pairs", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p, _i32p]),
+    ("ser_run_cd_marginals", C.c_int, [_vp, _i32p, C.c_int32, _dp, _dp, _i32p, _i32p, _i32p]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
     ("ser_write_labelled_files", C.c_int, [_vp, C.c_int32, _vp, C.c_char_p]),
     ("ser_microbench", C.c_int, [C.c_int32, _dp]),
@@ -242,12 +248,12 @@ class Run:
             _check(lib().ser_run_create_chains(ds._h, C.byref(self.cfg), _p(ids, C.c_int32), ids.size, C.byref(h)))
         self._h = h
 
-    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False, taxon_pairs=False):
+    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False, taxon_pairs=False, cd=False):
         """from now on the sample store is a window of max_samples rows and the summaries sum over every sample taken
         afterwards (ser_run_accumulate); call before the first sampling call.  ``positions`` / ``ranges`` accumulate the
-        histograms of marginals(), ``taxon_pairs`` the counts of taxon_pairs()"""
+        histograms of marginals(), ``taxon_pairs`` the counts of taxon_pairs(), ``cd`` the sums and histograms of cd_marginals()"""
         what = (ACC_PO if po else 0) | (ACC_SUMS if sums else 0) | (ACC_AB if ab else 0) | (ACC_ALIVE if alive else 0)
-        what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0) | (ACC_TAXA if taxon_pairs else 0)
+        what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0) | (ACC_TAXA if taxon_pairs else 0) | (ACC_CD if cd else 0)
         _check(lib().ser_run_accumulate(self._h, what))
         return self
 
@@ -459,6 +465,20 @@ class Run:
                                          _p(n, C.c_int32)))
         out["n_samples"] = n
         return out
+
+    def cd_marginals(self, chosen) -> dict:
+        """posterior of the error rates of the chosen chains (global ids) over their samples (ser_run_cd_marginals), R rows (every taxon
+        in file order on a manycd run, one row otherwise): ``c_sum`` / ``d_sum`` [k][R] = sum_t exp(c_t) / exp(d_t) in sample order,
+        ``c_hist`` / ``d_hist`` [k][R][CD_BINS] int32 = the samples' bins on the log value over CD_BOUNDS; ``n_samples`` [k] = T.  Slabs
+        the run does not fill stay 0 (n_samples 0)."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        k, R = len(chosen), self.M if self.manycd else 1
+        c_sum, d_sum = np.zeros((k, R)), np.zeros((k, R))
+        c_hist, d_hist = np.zeros((k, R, CD_BINS), np.int32), np.zeros((k, R, CD_BINS), np.int32)
+        n = np.zeros(k, np.int32)
+        _check(lib().ser_run_cd_marginals(self._h, _p(chosen, C.c_int32), k, _p(c_sum, C.c_double), _p(d_sum, C.c_double),
+                                          _p(c_hist, C.c_int32), _p(d_hist, C.c_int32), _p(n, C.c_int32)))
+        return dict(c_sum=c_sum, d_sum=d_sum, c_hist=c_hist, d_hist=d_hist, n_samples=n)
 
     def po_counts_device(self, chosen_ptr: int, k: int, counts_ptr: int):
         _check(lib().ser_run_po_counts_device(self._h, chosen_ptr, k, counts_ptr))
@@ -716,24 +736,25 @@ def choose_chains(batch: ChainBatch, chains_selected: int):
 
 
 def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, marginals: bool = False,
-                  taxon_pairs: bool = False, device=None) -> ChainBatch:
+                  taxon_pairs: bool = False, cd: bool = False, device=None) -> ChainBatch:
     """The second phase of select-then-replay: re-simulate the chosen chains of a batch (typically one run with
     ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
     ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
     run's, so compute_pair_order_matrix, compute_exp_* and the probability maps work on it unchanged.  ``with_ab``
     also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  ``window=0`` keeps every
     sample instead (``STORE_FULL``, no accumulators): the summaries take the one-shot path and ``diagnostics`` works on
-    the result.  ``marginals`` also accumulates the position and a/b histograms of marginals(), and ``taxon_pairs`` the counts of
-    taxon_pairs() (either makes the window keep a and b).
+    the result.  ``marginals`` also accumulates the position and a/b histograms of marginals(), ``taxon_pairs`` the counts of
+    taxon_pairs() and ``cd`` the sums and histograms of cd_marginals() (each makes the window keep a, b, c and d).
     Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
     ids = np.ascontiguousarray(chains, dtype=np.int32)
     keep_all = window == 0
     run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
-              store=STORE_FULL if (with_ab or keep_all or marginals or taxon_pairs) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
+              store=STORE_FULL if (with_ab or keep_all or marginals or taxon_pairs or cd) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
               device=batch.run.cfg.device if device is None else device, chain_ids=ids)
     run.init()
     if not keep_all:
-        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals, taxon_pairs=taxon_pairs)
+        run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals, taxon_pairs=taxon_pairs,
+                       cd=cd)
     run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
     want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
     if want.tobytes() != got.tobytes():
@@ -800,6 +821,33 @@ def taxon_pairs(batch: ChainBatch, chains) -> dict:
     n = int(tp["n_samples"].sum(dtype=np.int64))
     out = {key: counts[key] / n for key in TAXON_PAIRS}
     out.update(counts=counts, n_samples=n)
+    return out
+
+
+def cd_bin_edges(name: str) -> np.ndarray:
+    """the CD_BINS + 1 edges of the histograms of ``name`` ("c" or "d") on the log scale: lo + j (hi - lo) / CD_BINS"""
+    lo, hi = CD_BOUNDS[name]
+    return lo + np.arange(CD_BINS + 1) * ((hi - lo) / CD_BINS)
+
+
+def cd_marginals(batch: ChainBatch, chains, probs=(0.025, 0.5, 0.975)) -> dict:
+    """Posterior of the error rates pooled over the chosen chains by summing their sums and counts.  Per row (every taxon in file order
+    on a manycd run, one row otherwise), for ``c`` and for ``d``: ``mean`` = the posterior mean of exp(.) (a probability), the
+    ``quantiles`` [R][len(probs)] as hist_quantiles bins with their edges as probabilities ``lower`` / ``upper`` (exp of the bin's log
+    edges), ``mode`` (bin) and ``p_mode``, and the pooled ``counts`` [R][CD_BINS] (int64) and ``sum``.  ``n_samples`` is the pooled
+    sample count.  Needs a batch that keeps c and d: the full sample store, or replay_chosen(..., cd=True)."""
+    m = batch.run.cd_marginals(np.asarray(chains, dtype=np.int32))
+    n = int(m["n_samples"].sum(dtype=np.int64))
+    out = dict(n_samples=n, probs=tuple(probs))
+    for name in ("c", "d"):
+        counts, total = m[name + "_hist"].sum(axis=0, dtype=np.int64), np.zeros(len(m[name + "_sum"][0]))
+        for chain_sum in m[name + "_sum"]:   # chain by chain, in the order of `chains`
+            total = total + chain_sum
+        q = hist_quantiles(counts, probs)
+        edges = np.exp(cd_bin_edges(name))
+        mode = counts.argmax(axis=1)
+        out[name] = dict(mean=total / n, quantiles=q, lower=edges[q], upper=edges[q + 1], mode=mode,
+                         p_mode=counts[np.arange(len(counts)), mode] / n, counts=counts, sum=total)
     return out
 
 

@@ -18,7 +18,7 @@
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
  *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--rank-diagnostics FILE]
- *        [--marginals PREFIX] [--taxon-pairs PREFIX]
+ *        [--marginals PREFIX] [--taxon-pairs PREFIX] [--cd-marginals FILE]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
  * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
@@ -45,6 +45,12 @@
  * replay (one replay serves it and --marginals), pools the counts over the chains and writes PREFIX.first.csv, PREFIX.last.csv,
  * PREFIX.precedes.csv and PREFIX.coexist.csv: dense M x M probability matrices (row m, column n, taxa in file order; po.csv's format) of
  * P(a_m < a_n), P(b_m < b_n), P(b_m <= a_n) and P(the ranges of m and n share a position), and prints one summary line.
+ * --cd-marginals FILE (with --select) accumulates the error-rate marginals of the chosen chains (ser_run_cd_marginals) through the same
+ * replay (one replay serves it, --marginals and --taxon-pairs), pools them over the chains and writes FILE
+ * "taxon,c_mean,c_q025,c_median,c_q975,d_mean,d_q025,d_median,d_q975": one row per taxon (file order) on a --manycd 1 run, one row
+ * "all" otherwise; the means are the posterior means of the probabilities exp(c), exp(d), q025 is the lower edge of the 2.5 % quantile's
+ * bin, q975 the upper edge of the 97.5 % quantile's bin and the median the log-midpoint of its bin, all as probabilities.  It prints one
+ * summary line: the rows with the highest mean d (most missed occurrences) and the highest mean c (most spurious ones).
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -79,7 +85,9 @@ static void usage(const char *argv0)
           "              [--marginals PREFIX]   (with --select: position and a / b credible intervals of the chosen chains to\n"
           "                                      PREFIX.sites.csv and PREFIX.taxa.csv; the replay uses --window W)\n"
           "              [--taxon-pairs PREFIX]   (with --select: first / last appearance order, superposition and coexistence\n"
-          "                                        of every pair of taxa to PREFIX.{first,last,precedes,coexist}.csv; --window W)\n",
+          "                                        of every pair of taxa to PREFIX.{first,last,precedes,coexist}.csv; --window W)\n"
+          "              [--cd-marginals FILE]   (with --select: posterior means and credible intervals of the error rates c, d\n"
+          "                                       per taxon (--manycd 1) or of the scalar pair to FILE; --window W)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -265,13 +273,72 @@ static void write_taxon_pairs(int32_t *const tp[4], int32_t k, int32_t M, int32_
          (long long)M * (M - 1) / 2, hi, lo);
 }
 
-/* --marginals / --taxon-pairs: the chosen chains re-simulated alone through a window of W samples while their position and a / b
- * histograms (prefix) and their taxon pair relations (pairs_prefix) accumulate (either prefix may be NULL; bit-identical to their first
+/* --cd-marginals: the error-rate marginals of the chosen chains of `sub` pooled over the chains (sums chain by chain in the order of
+ * `chosen`) to `path`, and one summary line */
+static void write_cd_marginals(ser_run *sub, const int32_t *chosen, int32_t k, int32_t R, const char *path)
+{
+  static const double probs[3] = {0.025, 0.5, 0.975};
+  const double lo[2] = {SER_MINC, SER_MIND}, hi[2] = {SER_MAXC, SER_MAXD};
+  const size_t RB = (size_t)R * SER_CD_BINS;
+  double *sum[2], *mean[2], best[2] = {-1.0, -1.0};
+  int32_t *hist[2], *q[2], *n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k), tot = 0, arg[2] = {0, 0}, h, c, r, i;
+  size_t j;
+  char name[2][32];
+  FILE *f;
+  for (h = 0; h < 2; h++) {
+    sum[h] = (double *)malloc(sizeof(double) * (size_t)k * R);
+    mean[h] = (double *)malloc(sizeof(double) * (size_t)R);
+    hist[h] = (int32_t *)malloc(sizeof(int32_t) * k * RB);
+    q[h] = (int32_t *)malloc(sizeof(int32_t) * (size_t)R * 3);
+    if (!sum[h] || !mean[h] || !hist[h] || !q[h]) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  }
+  if (!n) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  if (ser_run_cd_marginals(sub, chosen, k, sum[0], sum[1], hist[0], hist[1], n)) die("ser_run_cd_marginals");
+  for (c = 0; c < k; c++) tot += n[c];
+  for (h = 0; h < 2; h++) {
+    for (r = 0; r < R; r++) {
+      double s = 0.0;
+      for (c = 0; c < k; c++) s += sum[h][(size_t)c * R + r];
+      mean[h][r] = s / (double)tot;
+      if (mean[h][r] > best[h]) { best[h] = mean[h][r]; arg[h] = r; }
+    }
+    for (c = 1; c < k; c++) /* pool the chains' counts into chain 0's slab */
+      for (j = 0; j < RB; j++) hist[h][j] += hist[h][c * RB + j];
+    if (ser_hist_quantiles(hist[h], R, SER_CD_BINS, probs, 3, q[h])) die("ser_hist_quantiles");
+  }
+  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  fprintf(f, "taxon,c_mean,c_q025,c_median,c_q975,d_mean,d_q025,d_median,d_q975\n");
+  for (r = 0; r < R; r++) {
+    if (R > 1) fprintf(f, "%d", r);
+    else fprintf(f, "all");
+    for (h = 0; h < 2; h++) {
+      const double w = (hi[h] - lo[h]) / SER_CD_BINS;
+      const int32_t *qr = q[h] + (size_t)r * 3;
+      fprintf(f, ",%.6g,%.6g,%.6g,%.6g", mean[h][r], exp(lo[h] + qr[0] * w), exp(0.5 * ((lo[h] + qr[1] * w) + (lo[h] + (qr[1] + 1) * w))),
+              exp(lo[h] + (qr[2] + 1) * w));
+    }
+    fprintf(f, "\n");
+  }
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  for (i = 0; i < 2; i++) {
+    if (R > 1) snprintf(name[i], sizeof(name[i]), "taxon %d", arg[1 - i]);
+    else snprintf(name[i], sizeof(name[i]), "all");
+  }
+  printf("cd marginals: %d chains  %d samples  highest mean d %.6g (%s)  highest mean c %.6g (%s)\n", k, tot, best[1], name[0], best[0],
+         name[1]);
+  for (h = 0; h < 2; h++) { free(sum[h]); free(mean[h]); free(hist[h]); free(q[h]); }
+  free(n);
+}
+
+/* --marginals / --taxon-pairs / --cd-marginals: the chosen chains re-simulated alone through a window of W samples while their position and a / b
+ * histograms (prefix), their taxon pair relations (pairs_prefix) and their error-rate marginals (cd_path) accumulate (any of the three
+ * may be NULL; bit-identical to their first
  * run, whose E[-logL] per global id - first is e[]; any difference exits 1), the counts pooled over the chains, PREFIX.sites.csv and
  * PREFIX.taxa.csv or the four taxon pair matrices written, and one summary line printed for each.  `counts` (NULL: not wanted) receives
  * their pair-order counts from the same run. */
 static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
-                             int burn, int samples, int window, int32_t *counts, const char *prefix, const char *pairs_prefix)
+                             int burn, int samples, int window, int32_t *counts, const char *prefix, const char *pairs_prefix,
+                             const char *cd_path)
 {
   ser_run_config c2 = *cfg;
   ser_run *sub = NULL;
@@ -294,7 +361,7 @@ static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, c
   c2.max_samples = window;
   if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
   if (ser_run_init(sub) || ser_run_accumulate(sub, (prefix ? SER_ACC_POS | SER_ACC_RANGE : 0) | (pairs_prefix ? SER_ACC_TAXA : 0) |
-                                                     (counts ? SER_ACC_PO : 0)))
+                                                     (cd_path ? SER_ACC_CD : 0) | (counts ? SER_ACC_PO : 0)))
     die("ser_run_accumulate");
   if (ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
   if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
@@ -315,6 +382,7 @@ static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, c
     write_taxon_pairs(tp, k, M, tot, pairs_prefix);
     for (c = 0; c < 4; c++) free(tp[c]);
   }
+  if (cd_path) write_cd_marginals(sub, chosen, k, cfg->manycd ? M : 1, cd_path);
   if (!prefix) {
     ser_run_destroy(sub);
     free(pos); free(ah); free(bh); free(n); free(e2); free(w); free(ms); free(ma); free(mb); free(hard);
@@ -372,7 +440,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
-  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL, *pairs_prefix = NULL;
+  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL, *pairs_prefix = NULL, *cd_path = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -410,6 +478,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--rank-diagnostics")) rdiag_path = v;
       else if (!strcmp(a, "--marginals")) marg_prefix = v;
       else if (!strcmp(a, "--taxon-pairs")) pairs_prefix = v;
+      else if (!strcmp(a, "--cd-marginals")) cd_path = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
@@ -418,7 +487,7 @@ int main(int argc, char **argv)
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
     if ((diag_path || rdiag_path) && select_k < 1) usage(argv[0]);
-    if ((marg_prefix || pairs_prefix) && (select_k < 1 || window < 1)) usage(argv[0]);
+    if ((marg_prefix || pairs_prefix || cd_path) && (select_k < 1 || window < 1)) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
@@ -549,7 +618,7 @@ int main(int argc, char **argv)
         /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix && !pairs_prefix) {
+        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix && !pairs_prefix && !cd_path) {
           ser_run_config c2 = cfg;
           ser_run *sub = NULL;
           c2.n_chains = nchosen;
@@ -572,10 +641,10 @@ int main(int argc, char **argv)
       }
       if ((diag_path || rdiag_path) && nchosen > 0)
         replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path, rdiag_path);
-      if ((marg_prefix || pairs_prefix) && nchosen > 0)
+      if ((marg_prefix || pairs_prefix || cd_path) && nchosen > 0)
         replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window,
                          (replay_selected && !diag_path && !rdiag_path) ? counts : NULL,
-                         marg_prefix, pairs_prefix);
+                         marg_prefix, pairs_prefix, cd_path);
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);
         FILE *f;

@@ -405,6 +405,70 @@ __global__ void __launch_bounds__(256) ser_taxon_pair_kernel(const uint16_t *sam
   }
 }
 
+/* Error-rate marginals (ser_run_cd_marginals, DESIGN.md 3.11).  Sample t of a chain holds the R rows' c at cd[t * rs + r] and their d
+ * at cd[t * rs + d_off + r]: samp_cd_all (rs = 2M, d_off = M) on a manycd run, samp_cdl (rs = 3, d_off = 1, R = 1) on a scalar one.
+ * Bin of x on [lo, hi] with s = SER_CD_BINS / (hi - lo): floor((x - lo) * s) rounded step by step, clamped to the bins; x <= lo and
+ * NaN give bin 0. */
+#define SER_CD_ROWS 32
+#define SER_CD_PITCH (SER_CD_BINS + 1) /* a padded shared row: lanes counting the same bin hit 32 different banks */
+#define SER_CD_SMEM (2 * SER_CD_ROWS * SER_CD_PITCH * sizeof(int))
+__device__ __forceinline__ int cd_bin(double x, double lo, double s)
+{
+  const double y = __dmul_rn(__dsub_rn(x, lo), s);
+  return y >= (double)(SER_CD_BINS - 1) ? SER_CD_BINS - 1 : y > 0.0 ? (int)y : 0;
+}
+
+/* One block per (32 rows, chosen chain blockIdx.y); lane = row, so a sample's 32 values are one coalesced load.  Warp 0 folds the
+ * rows' exp sums, c_sum / d_sum [R] at slab stride sum_stride: each lane one row, sequentially over t from the stored sum (add) or 0.0,
+ * with the sweep kernels' exp and SER_ADD, so the sum is theirs bit for bit.  The other warps stride over the samples and count the
+ * rows' c and d bins with shared-memory atomics (integer counts: the same in any order); the block's rows are contiguous in a
+ * [R][SER_CD_BINS] slab at stride hist_stride and go out with plain stores.  Both are computed whatever is requested; a nullptr output
+ * is not written. */
+__global__ void __launch_bounds__(256) ser_cd_hist_kernel(const double *cd, size_t rs, int d_off, int R, const ChainScalars *scal,
+                                                          int max_samples, SumSel sel, double *c_sum, double *d_sum, size_t sum_stride,
+                                                          int *c_hist, int *d_hist, size_t hist_stride, int add)
+{
+  extern __shared__ int s_cd[]; /* [2][SER_CD_ROWS][SER_CD_PITCH]: c, then d */
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.y, blockIdx.x == 0 && threadIdx.x == 0, &T);
+  if (local < 0) return;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int r0 = blockIdx.x * SER_CD_ROWS, n = min(SER_CD_ROWS, R - r0), r = r0 + lane;
+  const double *x = cd + (size_t)local * max_samples * rs + r;
+  for (int e = threadIdx.x; e < 2 * SER_CD_ROWS * SER_CD_PITCH; e += blockDim.x) s_cd[e] = 0;
+  __syncthreads();
+  if (lane < n) {
+    if (warp == 0) {
+      const size_t e = (size_t)blockIdx.y * sum_stride + r;
+      double sc = add && c_sum ? c_sum[e] : 0.0, sd = add && d_sum ? d_sum[e] : 0.0;
+      for (int t = 0; t < T; t++) {
+        sc = SER_ADD(sc, exp(x[(size_t)t * rs]));
+        sd = SER_ADD(sd, exp(x[(size_t)t * rs + d_off]));
+      }
+      if (c_sum) c_sum[e] = sc;
+      if (d_sum) d_sum[e] = sd;
+    } else {
+      const double sc = (double)SER_CD_BINS / (SER_MAXC - SER_MINC), sd = (double)SER_CD_BINS / (SER_MAXD - SER_MIND);
+      int *hc = s_cd + lane * SER_CD_PITCH, *hd = hc + SER_CD_ROWS * SER_CD_PITCH;
+      for (int t = warp - 1; t < T; t += nw - 1) {
+        atomicAdd(&hc[cd_bin(x[(size_t)t * rs], SER_MINC, sc)], 1);
+        atomicAdd(&hd[cd_bin(x[(size_t)t * rs + d_off], SER_MIND, sd)], 1);
+      }
+    }
+  }
+  __syncthreads();
+  int *const outs[2] = {c_hist, d_hist};
+  for (int h = 0; h < 2; h++) {
+    if (!outs[h]) continue;
+    int *dst = outs[h] + (size_t)blockIdx.y * hist_stride + (size_t)r0 * SER_CD_BINS;
+    const int *src = s_cd + h * SER_CD_ROWS * SER_CD_PITCH;
+    for (int e = threadIdx.x; e < n * SER_CD_BINS; e += blockDim.x) {
+      const int v = src[(e / SER_CD_BINS) * SER_CD_PITCH + e % SER_CD_BINS];
+      dst[e] = add ? dst[e] + v : v;
+    }
+  }
+}
+
 /* ------------------------------------------------------------------ convergence diagnostics (ser_run_diagnostics, DESIGN.md 3.7)
  * Quantity q of a chain's stored sample t: 0 = -loglik, 1 = exp(c), 2 = exp(d) (samp_cdl; taxon 0's c, d on a manycd run),
  * 3 + i = pi_t(i), the position of site i.  One block of 32 warps per (chosen chain, 32 consecutive quantities).  The moments
@@ -883,20 +947,23 @@ __global__ void __launch_bounds__(1024, 1) ser_rank_ess_kernel(RankSrc src, Rank
  * the summary kernels above add the window's rows of EVERY local chain into that chain's accumulator record; the getters turn the
  * records into what the one-shot kernels compute from a store that holds all samples, with the kernels below. */
 
-#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE | SER_ACC_TAXA)
+#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD)
 
 /* One local chain's accumulator record: int32 offsets of the parts the flags `what` select, in this order, and the record's length.
  * The run holds [n_local][ints]; a checkpoint record holds the same ints in the same order.
  *   po [N][N] (SER_ACC_PO; diagonal 0), pi [N] (SER_ACC_SUMS or SER_ACC_AB), asum [M], bsum [M] (SER_ACC_AB),
  *   alive [N][M] (SER_ACC_ALIVE; the difference slab), pos [N][N] (SER_ACC_POS), range [2][M][N+1] (SER_ACC_RANGE; a, then b),
- *   taxa [4][M][M] (SER_ACC_TAXA; first, last, precedes, coexist) */
+ *   taxa [4][M][M] (SER_ACC_TAXA; first, last, precedes, coexist),
+ *   cd: f64 c_sum, d_sum [R] as pairs of int32 words, then c_hist, d_hist [R][SER_CD_BINS] (SER_ACC_CD; R = M on a manycd run, else 1).
+ * Under SER_ACC_CD alone the part's start and the record's length are rounded up to an even number of words, so every double is
+ * 8-byte aligned in the run's records; records without the flag keep their length, and checkpoint files their bytes. */
 struct AccLayout {
-  size_t po, pi, asum, bsum, alive, pos, range, taxa, ints;
+  size_t po, pi, asum, bsum, alive, pos, range, taxa, cd, ints;
 };
-__host__ __device__ inline AccLayout acc_layout(int N, int M, int what)
+__host__ __device__ inline AccLayout acc_layout(int N, int M, int manycd, int what)
 {
   AccLayout L;
-  const size_t n = N, m = M;
+  const size_t n = N, m = M, cdr = manycd ? M : 1;
   size_t o = 0;
   L.po = o; o += (what & SER_ACC_PO) ? n * n : 0;
   L.pi = o; o += (what & (SER_ACC_SUMS | SER_ACC_AB)) ? n : 0;
@@ -906,6 +973,8 @@ __host__ __device__ inline AccLayout acc_layout(int N, int M, int what)
   L.pos = o; o += (what & SER_ACC_POS) ? n * n : 0;
   L.range = o; o += (what & SER_ACC_RANGE) ? 2 * m * (n + 1) : 0;
   L.taxa = o; o += (what & SER_ACC_TAXA) ? 4 * m * m : 0;
+  if (what & SER_ACC_CD) o += o & 1;
+  L.cd = o; o += (what & SER_ACC_CD) ? 4 * cdr + 2 * cdr * SER_CD_BINS : 0;
   L.ints = o;
   return L;
 }

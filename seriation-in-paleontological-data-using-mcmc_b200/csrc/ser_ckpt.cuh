@@ -125,7 +125,7 @@ __host__ __device__ inline CkptLayout ckpt_layout(int N, int M, int manycd, int 
   L.cd = o; o += manycd ? 8 * 4 * m : 0;
   L.cdl = o; o += full ? 8 * 3 * r : 0;
   L.cd_all = o; o += (full && manycd) ? 8 * 2 * m * r : 0;
-  L.acc = o; o += 4 * (long long)acc_layout(N, M, acc).ints;
+  L.acc = o; o += 4 * (long long)acc_layout(N, M, manycd, acc).ints;
   L.rpi = o; o += 2 * n;
   L.ab = o; o += 4 * m;
   L.spi = o; o += store >= SER_STORE_PI ? 2 * n * r : 0;

@@ -26,11 +26,6 @@
 #include "ser_chain_core.h"
 #include "ser_internal.h"
 
-#define SER_MINC (-6.9077552789821368)
-#define SER_MAXC (-2.3025850929940455)
-#define SER_MIND (-1.6094379124341003)
-#define SER_MAXD (-0.22314355131420971)
-
 #define SER_PI_DRAWS 72 /* >= 4 + 5*13 = 69 draws a sweep's pi part can consume */
 #define SER_MAX_WARPS 32
 #define SER_MAX_GROUPS 8 /* column groups the item weights of a Gibbs step are evaluated in */
@@ -634,7 +629,8 @@ extern "C" int ser_run_create_chains(const ser_dataset *ds, const ser_run_config
   return SER_OK;
 }
 
-static size_t acc_bytes(const ser_run *run) { return (size_t)run->cfg.n_chains * acc_layout(run->N, run->M, run->acc_what).ints * sizeof(int); }
+static AccLayout run_acc_layout(const ser_run *run) { return acc_layout(run->N, run->M, run->cfg.manycd, run->acc_what); }
+static size_t acc_bytes(const ser_run *run) { return (size_t)run->cfg.n_chains * run_acc_layout(run).ints * sizeof(int); }
 
 /* zero the accumulators of an accumulating run (start of ser_run_init) */
 static int acc_zero(ser_run *run)
@@ -649,7 +645,7 @@ extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
   if (what < 1 || (what & ~SER_ACC_ALL)) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
   if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
   if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
-  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE | SER_ACC_TAXA)) ? SER_STORE_FULL : SER_STORE_PI;
+  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD)) ? SER_STORE_FULL : SER_STORE_PI;
   if (run->cfg.store < need) {
     ser_set_error("ser_run_accumulate: these summaries need %s", need == SER_STORE_FULL ? "SER_STORE_FULL (a, b samples)" : "SER_STORE_PI or more");
     return SER_E_STATE;
@@ -896,11 +892,29 @@ static int launch_taxon_pairs(ser_run *run, const SumSel &sel, int k, int *const
   return SER_OK;
 }
 
+/* rows of the error-rate marginals: every taxon on a manycd run, the one scalar c, d otherwise */
+static int cd_rows(const ser_run *run) { return run->cfg.manycd ? run->M : 1; }
+
+/* c_sum / d_sum [R] slabs at sum_stride doubles, c_hist / d_hist [R][SER_CD_BINS] at hist_stride ints (any may be nullptr) */
+static int launch_cd_hist(ser_run *run, const SumSel &sel, int k, double *c_sum, double *d_sum, size_t sum_stride, int *c_hist, int *d_hist,
+                          size_t hist_stride, int add)
+{
+  const int R = cd_rows(run), M = run->M;
+  const bool many = run->cfg.manycd;
+  CUDA_TRY(cudaFuncSetAttribute((const void *)ser_cd_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SER_CD_SMEM));
+  mark_launch(run);
+  ser_cd_hist_kernel<<<dim3((R + SER_CD_ROWS - 1) / SER_CD_ROWS, k), 256, SER_CD_SMEM, run->stream>>>(
+      many ? run->d_samp_cd_all : run->d_samp_cdl, many ? 2 * (size_t)M : 3, many ? M : 1, R, run->d_scal, run->cfg.max_samples, sel, c_sum,
+      d_sum, sum_stride, c_hist, d_hist, hist_stride, add);
+  CUDA_TRY(cudaGetLastError());
+  return SER_OK;
+}
+
 /* rows [0, w) of every chain's window added into its accumulator record (ser_run_accumulate), on the run's stream */
 static int accumulate_window(ser_run *run, int w)
 {
   const int what = run->acc_what, nc = run->cfg.n_chains;
-  const AccLayout L = acc_layout(run->N, run->M, what);
+  const AccLayout L = run_acc_layout(run);
   const SumSel sel = {nullptr, 0, 0, nullptr, run->kp.sample_base, w, nullptr};
   int *acc = run->d_acc;
   int rc = SER_OK;
@@ -916,6 +930,11 @@ static int accumulate_window(ser_run *run, int w)
     const size_t mm = (size_t)run->M * run->M;
     int *const taxa[4] = {acc + L.taxa, acc + L.taxa + mm, acc + L.taxa + 2 * mm, acc + L.taxa + 3 * mm};
     rc = launch_taxon_pairs(run, sel, nc, taxa, L.ints, 1);
+  }
+  if (!rc && (what & SER_ACC_CD)) {
+    const size_t R = cd_rows(run);
+    double *sums = (double *)(acc + L.cd); /* L.cd and L.ints are even: 8-byte aligned */
+    rc = launch_cd_hist(run, sel, nc, sums, sums + R, L.ints / 2, acc + L.cd + 4 * R, acc + L.cd + 4 * R + R * SER_CD_BINS, L.ints, 1);
   }
   return rc;
 }
@@ -1246,7 +1265,7 @@ static int po_counts_to(ser_run *run, const int32_t *d_chosen, int k, int32_t *d
                      (size_t)run->N * run->N, 0);
   if (!(run->acc_what & SER_ACC_PO)) { ser_set_error("ser_run_po_counts: the run accumulates without SER_ACC_PO"); return SER_E_STATE; }
   const int N = run->N, nb = (int)std::min<long long>(((long long)N * N + 255) / 256, 1024);
-  const AccLayout L = acc_layout(N, run->M, run->acc_what);
+  const AccLayout L = run_acc_layout(run);
   mark_launch(run);
   ser_po_acc_out_kernel<<<dim3(nb, k), 256, 0, run->stream>>>(run->d_acc + L.po, L.ints, run->d_scal, N,
                                                               sel_chosen(run, d_chosen, run->cfg.chain_offset, INT_MAX, d_n), d_counts);
@@ -1342,7 +1361,7 @@ extern "C" int ser_run_posterior_sums(ser_run *run, const int32_t *chosen, int32
     if (!run->acc_what)
       return launch_posterior(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, (int *)pi.dev, N,
                               (int *)a.dev, (int *)b.dev, M, (long long *)corr.dev, 0);
-    const AccLayout L = acc_layout(N, M, run->acc_what);
+    const AccLayout L = run_acc_layout(run);
     mark_launch(run);
     ser_posterior_acc_out_kernel<<<k, 256, 0, run->stream>>>(run->d_acc + L.pi, run->d_acc + L.asum, run->d_acc + L.bsum, L.ints, run->d_scal,
                                                              N, M, sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n),
@@ -1366,7 +1385,7 @@ extern "C" int ser_run_alive_counts(ser_run *run, const int32_t *chosen, int32_t
   const int rc = run_getter(run, chosen, k, n_out, {&out}, [&](const int *d_ch, int *d_n) -> int {
     if (!run->acc_what)
       return launch_alive(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, (int *)out.dev, (size_t)N * M, 0);
-    const AccLayout L = acc_layout(N, M, run->acc_what);
+    const AccLayout L = run_acc_layout(run);
     mark_launch(run);
     ser_alive_acc_out_kernel<<<dim3(k, (M + 127) / 128), 128, 0, run->stream>>>(run->d_acc + L.alive, L.ints, run->d_scal, N, M,
                                                                                  sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n),
@@ -1406,7 +1425,7 @@ extern "C" int ser_run_marginals(ser_run *run, const int32_t *chosen, int32_t k,
       if (!rc && ranges) rc = launch_range_hist(run, sel, k, (int *)a.dev, (int *)b.dev, range_cells, 0);
       return rc;
     }
-    const AccLayout L = acc_layout(N, M, run->acc_what);
+    const AccLayout L = run_acc_layout(run);
     const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
     if (pos) {
       mark_launch(run);
@@ -1448,7 +1467,7 @@ extern "C" int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t 
       return launch_taxon_pairs(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, taxa, cells, 0);
     }
     /* the record's four parts in order: (first, last), then (precedes, coexist), each pair one copy-out launch */
-    const AccLayout L = acc_layout(run->N, M, run->acc_what);
+    const AccLayout L = run_acc_layout(run);
     const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
     GetterOut *pairs[2][2] = {{&f, &l}, {&p, &c}};
     for (int h = 0; h < 2; h++) {
@@ -1456,6 +1475,47 @@ extern "C" int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t 
       mark_launch(run);
       ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.taxa + 2 * h * cells, L.ints, cells, run->d_scal, sel,
                                                                         (int *)pairs[h][0]->dev, (int *)pairs[h][1]->dev);
+      CUDA_TRY(cudaGetLastError());
+    }
+    return SER_OK;
+  });
+  if (rc != SER_OK) return rc;
+  for (int q = 0; q < k; q++) n_samples[q] = n_out[q] < 0 ? 0 : n_out[q];
+  return SER_OK;
+}
+
+extern "C" int ser_run_cd_marginals(ser_run *run, const int32_t *chosen, int32_t k, double *c_sum, double *d_sum, int32_t *c_hist,
+                                    int32_t *d_hist, int32_t *n_samples)
+{
+  if (!run || !chosen || !n_samples || k < 1 || (!c_sum && !d_sum && !c_hist && !d_hist)) {
+    ser_set_error("ser_run_cd_marginals: bad argument (k = %d; chosen, n_samples and at least one of c_sum, d_sum, c_hist, d_hist are needed)", k);
+    return SER_E_ARG;
+  }
+  if (!run->initialized) { ser_set_error("ser_run_cd_marginals: run not initialised"); return SER_E_STATE; }
+  if (run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_cd_marginals: needs SER_STORE_FULL (c, d samples)"); return SER_E_STATE; }
+  if (run->acc_what && !(run->acc_what & SER_ACC_CD)) { ser_set_error("ser_run_cd_marginals: the run accumulates without SER_ACC_CD"); return SER_E_STATE; }
+  if (set_device(run)) return SER_E_CUDA;
+  const size_t R = cd_rows(run), cells = R * SER_CD_BINS;
+  GetterOut cs = {c_sum, R * sizeof(double), nullptr}, ds = {d_sum, R * sizeof(double), nullptr};
+  GetterOut ch = {c_hist, cells * sizeof(int), nullptr}, dh = {d_hist, cells * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&cs, &ds, &ch, &dh}, [&](const int *d_ch, int *d_n) -> int {
+    if (!run->acc_what)
+      return launch_cd_hist(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, (double *)cs.dev,
+                            (double *)ds.dev, R, (int *)ch.dev, (int *)dh.dev, cells, 0);
+    /* the record's part: the two sums (each double two int32 words, copied as such), then the two histograms */
+    const AccLayout L = run_acc_layout(run);
+    const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
+    if (cs.dev || ds.dev) {
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3((unsigned)std::min<size_t>((2 * R + 255) / 256, 256), k, 2), 256, 0, run->stream>>>(
+          run->d_acc + L.cd, L.ints, 2 * R, run->d_scal, sel, (int *)cs.dev, (int *)ds.dev);
+      CUDA_TRY(cudaGetLastError());
+    }
+    if (ch.dev || dh.dev) {
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.cd + 4 * R, L.ints, cells, run->d_scal, sel,
+                                                                        (int *)ch.dev, (int *)dh.dev);
       CUDA_TRY(cudaGetLastError());
     }
     return SER_OK;
