@@ -20,33 +20,32 @@
  *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--rank-diagnostics FILE]
  *        [--marginals PREFIX] [--taxon-pairs PREFIX] [--cd-marginals FILE]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
- * Chains/ files), the K chosen chains are re-simulated alone on --device (ser_run_create_chains, bit-identical) while
- * their pair-order counts accumulate through a window of W samples (ser_run_accumulate, default 64): the same output
- * lines and po.csv as the one-shot step, with device memory for K chains' window instead of every chain's history.
+ * Chains/ files) and the pair-order counts of the K chosen chains come from their replay: the same output lines and po.csv
+ * as the one-shot step, with device memory for K chains' window instead of every chain's history.
+ * Every --select output (po.csv under --replay-selected, and the outputs of the five flags below) comes from one replay of the chosen
+ * chains, alone on --device (ser_run_create_chains), which exits 1 unless each reproduces its first run's E[-logL] bit for
+ * bit.  That replay keeps every sample (SER_STORE_FULL) when --diagnostics or --rank-diagnostics is given, and otherwise
+ * runs through a window of W samples (--window, default 64) while what the outputs read accumulates (ser_run_accumulate);
+ * the summaries are the same bits from either store.
  * --checkpoint FILE writes every chain's state to FILE at the end of the sweeps (ser_multi_save_checkpoint), and every C calls
  * with --checkpoint-every C (the advance runs in segments of at most C calls; splitting a launch changes no chain).  --resume
  * loads FILE when it exists in place of the random start and runs the calls of the --burn B --samples S schedule that are left
  * (it refuses a file that has advanced past B + S calls, or whose sample count is not max(0, calls - B)).  --stop-after C
  * advances at most C calls in this invocation, writes FILE and exits 0 with one line saying where it stopped, before any
  * summary or Chains/ file: a long run split into slices gives the same output as the run done in one piece.
- * --diagnostics FILE (with --select) re-simulates the chosen chains alone keeping every sample (SER_STORE_FULL, bit-identical to
- * their first run, which is checked), writes per-quantity split-R-hat and effective sample sizes to FILE and prints one summary
- * line; under --replay-selected --po the same run supplies the pair-order counts.
- * --rank-diagnostics FILE (with --select) does the same replay (one replay serves both flags) and writes the rank-normalised R-hat,
- * bulk- and tail-ESS pooled over the chosen chains (ser_run_rank_diagnostics) to FILE
- * "quantity,rhat,rhat_bulk,rhat_fold,ess_bulk,ess_tail,ess_mean,q05,q95", with one summary line: the largest R-hat, the smallest
- * bulk- and tail-ESS, and how many quantities have R-hat > 1.01 or a bulk- or tail-ESS below 100 per chain.
- * --marginals PREFIX (with --select) re-simulates the chosen chains alone through a window of W samples (--window, default 64) while
- * their position and a / b histograms accumulate (bit-identical to their first run, which is checked), pools the counts over the
- * chains and writes PREFIX.sites.csv "site,hard,mean,q025,median,q975,mode,p_mode" (file order, 0-based positions) and
- * PREFIX.taxa.csv "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975", and prints one summary line; under
- * --replay-selected --po (without --diagnostics) the same run supplies the pair-order counts, so the chains are replayed once.
- * --taxon-pairs PREFIX (with --select) accumulates the taxon pair relations of the chosen chains (ser_run_taxon_pairs) through the same
- * replay (one replay serves it and --marginals), pools the counts over the chains and writes PREFIX.first.csv, PREFIX.last.csv,
- * PREFIX.precedes.csv and PREFIX.coexist.csv: dense M x M probability matrices (row m, column n, taxa in file order; po.csv's format) of
- * P(a_m < a_n), P(b_m < b_n), P(b_m <= a_n) and P(the ranges of m and n share a position), and prints one summary line.
- * --cd-marginals FILE (with --select) accumulates the error-rate marginals of the chosen chains (ser_run_cd_marginals) through the same
- * replay (one replay serves it, --marginals and --taxon-pairs), pools them over the chains and writes FILE
+ * --diagnostics FILE (with --select) writes the per-quantity split-R-hat and effective sample sizes of the chosen chains to FILE and
+ * prints one summary line.
+ * --rank-diagnostics FILE (with --select) writes the rank-normalised R-hat, bulk- and tail-ESS pooled over the chosen chains
+ * (ser_run_rank_diagnostics) to FILE "quantity,rhat,rhat_bulk,rhat_fold,ess_bulk,ess_tail,ess_mean,q05,q95", with one summary line:
+ * the largest R-hat, the smallest bulk- and tail-ESS, and how many quantities have R-hat > 1.01 or a bulk- or tail-ESS below 100 per chain.
+ * --marginals PREFIX (with --select) pools the position and a / b histograms of the chosen chains and writes PREFIX.sites.csv
+ * "site,hard,mean,q025,median,q975,mode,p_mode" (file order, 0-based positions) and PREFIX.taxa.csv
+ * "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975", and prints one summary line.
+ * --taxon-pairs PREFIX (with --select) pools the taxon pair relations of the chosen chains (ser_run_taxon_pairs) and writes
+ * PREFIX.first.csv, PREFIX.last.csv, PREFIX.precedes.csv and PREFIX.coexist.csv: dense M x M probability matrices (row m, column n,
+ * taxa in file order; po.csv's format) of P(a_m < a_n), P(b_m < b_n), P(b_m <= a_n) and P(the ranges of m and n share a position), and
+ * prints one summary line.
+ * --cd-marginals FILE (with --select) pools the error-rate marginals of the chosen chains (ser_run_cd_marginals) and writes FILE
  * "taxon,c_mean,c_q025,c_median,c_q975,d_mean,d_q025,d_median,d_q975": one row per taxon (file order) on a --manycd 1 run, one row
  * "all" otherwise; the means are the posterior means of the probabilities exp(c), exp(d), q025 is the lower edge of the 2.5 % quantile's
  * bin, q975 the upper edge of the 97.5 % quantile's bin and the median the log-midpoint of its bin, all as probabilities.  It prints one
@@ -66,6 +65,25 @@ static void die(const char *what)
 {
   fprintf(stderr, "mcmc: %s: %s\n", what, ser_last_error());
   exit(1);
+}
+
+static void *xmalloc(size_t bytes)
+{
+  void *p = malloc(bytes);
+  if (!p) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+  return p;
+}
+
+static FILE *open_out(const char *path)
+{
+  FILE *f = fopen(path, "w");
+  if (!f) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  return f;
+}
+
+static void close_out(FILE *f, const char *path)
+{
+  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
 }
 
 static void usage(const char *argv0)
@@ -107,14 +125,13 @@ static double min_nan(double a, double b) { return isnan(a) || isnan(b) ? NAN : 
 static void write_rank_diagnostics(ser_run *sub, const int32_t *chosen, int32_t k, int32_t N, const char *path)
 {
   const int Q = 3 + N;
-  double *out = (double *)malloc(sizeof(double) * (size_t)Q * SER_RDIAG_FIELDS);
+  double *out = xmalloc(sizeof(double) * (size_t)Q * SER_RDIAG_FIELDS);
   double r_max = NAN, bulk_min = NAN, tail_min = NAN;
   int q, q_r = -1, q_b = -1, q_t = -1, flagged = 0;
   char b1[32], b2[32], b3[32];
   FILE *f;
-  if (!out) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
   if (ser_run_rank_diagnostics(sub, chosen, k, SER_DIAG_SCALARS | SER_DIAG_SITES, out)) die("ser_run_rank_diagnostics");
-  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  f = open_out(path);
   fprintf(f, "quantity,rhat,rhat_bulk,rhat_fold,ess_bulk,ess_tail,ess_mean,q05,q95\n");
   for (q = 0; q < Q; q++) {
     const double *o = out + (size_t)q * SER_RDIAG_FIELDS;
@@ -126,7 +143,7 @@ static void write_rank_diagnostics(ser_run *sub, const int32_t *chosen, int32_t 
     if (!isnan(tail) && (q_t < 0 || tail < tail_min)) { tail_min = tail; q_t = q; }
     flagged += rhat > 1.01 || o[2] < 100.0 * k || tail < 100.0 * k;
   }
-  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  close_out(f, path);
   printf("rank diagnostics: %d chains  R-hat max %.4f (%s)  bulk-ESS min %.1f (%s)  tail-ESS min %.1f (%s)  "
          "%d of %d quantities with R-hat > 1.01 or ESS < %d\n", k, r_max, q_r < 0 ? "none" : quantity_name(q_r, b1, sizeof(b1)), bulk_min,
          q_b < 0 ? "none" : quantity_name(q_b, b2, sizeof(b2)), tail_min, q_t < 0 ? "none" : quantity_name(q_t, b3, sizeof(b3)), flagged, Q,
@@ -134,53 +151,20 @@ static void write_rank_diagnostics(ser_run *sub, const int32_t *chosen, int32_t 
   free(out);
 }
 
-/* --diagnostics / --rank-diagnostics: the chosen chains re-simulated alone with every sample kept (bit-identical to their first run,
- * whose E[-logL] per global id - first is e[]; any difference exits 1); their split-R-hat and ESS written to `path` as CSV and
- * summarised in one line, and their rank-normalised diagnostics to `rank_path` (either may be NULL).  `counts` (NULL: not wanted)
- * receives their pair-order counts from the same run. */
-static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
-                               int burn, int samples, int32_t *counts, const char *path, const char *rank_path)
+/* --diagnostics: the split-R-hat and ESS of the chosen chains of `sub` to `path` as CSV, and one summary line */
+static void write_diagnostics(ser_run *sub, const int32_t *chosen, int32_t k, int32_t N, const char *path)
 {
-  ser_run_config c2 = *cfg;
-  ser_run *sub = NULL;
-  int32_t N, M, nh, ns = 0, i, q, c;
-  double *e2, *stats, *halves, *rhat;
-  int32_t *n;
-  FILE *f;
-  int s_max = -1, s_min = -1, constant = 0;
-  double r_max = NAN, ess_min_site = NAN, ess_min[3];
-  ser_dataset_dims(ds, &N, &M, &nh);
   const int Q = 3 + N;
-  c2.n_chains = k;
-  c2.chain_offset = 0;
-  c2.store = SER_STORE_FULL;
-  c2.max_samples = samples;
-  e2 = (double *)malloc(sizeof(double) * (size_t)k);
-  stats = (double *)malloc(sizeof(double) * (size_t)k * Q * 4);
-  halves = (double *)malloc(sizeof(double) * (size_t)k * Q * 4);
-  rhat = (double *)malloc(sizeof(double) * (size_t)Q);
-  n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k);
-  if (!e2 || !stats || !halves || !rhat || !n) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
-  if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
-  if (ser_run_init(sub) || ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
-  if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
-  for (i = 0; i < k; i++)
-    if (memcmp(&e2[i], &e[chosen[i] - first], sizeof(double))) {
-      fprintf(stderr, "mcmc: the replayed chain %d does not reproduce its first run (E[-logL] %.17g vs %.17g)\n", chosen[i], e2[i],
-              e[chosen[i] - first]);
-      exit(1);
-    }
-  if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
-  if (rank_path) write_rank_diagnostics(sub, chosen, k, N, rank_path);
-  if (!path) {
-    ser_run_destroy(sub);
-    free(e2); free(stats); free(halves); free(rhat); free(n);
-    return;
-  }
+  double *stats = xmalloc(sizeof(double) * (size_t)k * Q * 4), *halves = xmalloc(sizeof(double) * (size_t)k * Q * 4);
+  double *rhat = xmalloc(sizeof(double) * (size_t)Q);
+  int32_t *n = xmalloc(sizeof(int32_t) * (size_t)k);
+  int q, c, s_max = -1, s_min = -1, constant = 0;
+  double r_max = NAN, ess_min_site = NAN, ess_min[3];
+  char name[32];
+  FILE *f;
   if (ser_run_diagnostics(sub, chosen, k, SER_DIAG_SCALARS | SER_DIAG_SITES, 0, stats, halves, n)) die("ser_run_diagnostics");
   if (ser_split_rhat(halves, n, k, Q, rhat)) die("ser_split_rhat");
-  ser_run_destroy(sub);
-  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  f = open_out(path);
   fprintf(f, "quantity,mean,rhat,ess_min,ess_sum\n");
   for (q = 0; q < Q; q++) {
     double mean = 0.0, emin = NAN, esum = NAN;
@@ -192,9 +176,7 @@ static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg,
       esum = isnan(esum) ? st[2] : esum + st[2];
     }
     mean /= k;
-    if (q < 3) fprintf(f, "%s,", q == 0 ? "-logL" : q == 1 ? "c" : "d");
-    else fprintf(f, "site_%d,", q - 3);
-    fprintf(f, "%.17g,%.17g,%.17g,%.17g\n", mean, rhat[q], emin, esum);
+    fprintf(f, "%s,%.17g,%.17g,%.17g,%.17g\n", quantity_name(q, name, sizeof(name)), mean, rhat[q], emin, esum);
     if (q < 3) ess_min[q] = emin;
     else {
       if (isnan(emin)) constant++; /* constant in every chosen chain */
@@ -202,11 +184,11 @@ static void replay_diagnostics(const ser_dataset *ds, const ser_run_config *cfg,
       if (!isnan(emin) && (s_min < 0 || emin < ess_min_site)) { ess_min_site = emin; s_min = q - 3; }
     }
   }
-  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  close_out(f, path);
   for (q = 0; q < 3; q++) constant += isnan(ess_min[q]);
   printf("diagnostics: R-hat -logL %.4f  c %.4f  d %.4f  sites max %.4f (site %d)  ESS -logL min %.1f  sites min %.1f (site %d)  "
          "constant %d\n", rhat[0], rhat[1], rhat[2], r_max, s_max, ess_min[0], ess_min_site, s_min, constant);
-  free(e2); free(stats); free(halves); free(rhat); free(n);
+  free(stats); free(halves); free(rhat); free(n);
 }
 
 /* mean, 2.5 / 50 / 97.5 % quantiles, mode and P(mode) of one row of pooled counts */
@@ -245,20 +227,24 @@ static double median_width(const struct marginal *m, int32_t n, double *w)
   return n % 2 ? w[n / 2] : 0.5 * (w[n / 2 - 1] + w[n / 2]);
 }
 
-/* --taxon-pairs: the four [k][M][M] count slabs of ser_run_taxon_pairs pooled over the k chains (tot samples) to PREFIX.<name>.csv as
- * probability matrices, and one summary line */
-static void write_taxon_pairs(int32_t *const tp[4], int32_t k, int32_t M, int32_t tot, const char *prefix)
+/* --taxon-pairs: the taxon pair relations of the chosen chains of `sub` pooled over the chains to PREFIX.<name>.csv as probability
+ * matrices, and one summary line */
+static void write_taxon_pairs(ser_run *sub, const int32_t *chosen, int32_t k, int32_t M, const char *prefix)
 {
   static const char *names[4] = {"first", "last", "precedes", "coexist"};
   const size_t MM = (size_t)M * M;
+  int32_t *tp[4], *n = xmalloc(sizeof(int32_t) * (size_t)k), tot = 0;
   long long hi = 0, lo = 0;
   char path[4096];
   int q, c;
   size_t j;
   FILE *f;
+  for (q = 0; q < 4; q++) tp[q] = xmalloc(sizeof(int32_t) * k * MM);
+  if (ser_run_taxon_pairs(sub, chosen, k, tp[0], tp[1], tp[2], tp[3], n)) die("ser_run_taxon_pairs");
+  for (c = 0; c < k; c++) tot += n[c];
   for (q = 0; q < 4; q++) {
     snprintf(path, sizeof(path), "%s.%s.csv", prefix, names[q]);
-    if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+    f = open_out(path);
     for (j = 0; j < MM; j++) {
       int64_t sum = 0;
       double p;
@@ -267,10 +253,12 @@ static void write_taxon_pairs(int32_t *const tp[4], int32_t k, int32_t M, int32_
       fprintf(f, "%.6f%c", p, (j + 1) % (size_t)M ? ',' : '\n');
       if (q == 3 && j / M < j % M) { hi += p >= 0.95; lo += p <= 0.05; }
     }
-    if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+    close_out(f, path);
   }
   printf("taxon pairs: %d chains  %d samples  of %lld pairs of taxa %lld coexist with P >= 0.95 and %lld with P <= 0.05\n", k, tot,
          (long long)M * (M - 1) / 2, hi, lo);
+  for (q = 0; q < 4; q++) free(tp[q]);
+  free(n);
 }
 
 /* --cd-marginals: the error-rate marginals of the chosen chains of `sub` pooled over the chains (sums chain by chain in the order of
@@ -281,18 +269,16 @@ static void write_cd_marginals(ser_run *sub, const int32_t *chosen, int32_t k, i
   const double lo[2] = {SER_MINC, SER_MIND}, hi[2] = {SER_MAXC, SER_MAXD};
   const size_t RB = (size_t)R * SER_CD_BINS;
   double *sum[2], *mean[2], best[2] = {-1.0, -1.0};
-  int32_t *hist[2], *q[2], *n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k), tot = 0, arg[2] = {0, 0}, h, c, r, i;
+  int32_t *hist[2], *q[2], *n = xmalloc(sizeof(int32_t) * (size_t)k), tot = 0, arg[2] = {0, 0}, h, c, r, i;
   size_t j;
   char name[2][32];
   FILE *f;
   for (h = 0; h < 2; h++) {
-    sum[h] = (double *)malloc(sizeof(double) * (size_t)k * R);
-    mean[h] = (double *)malloc(sizeof(double) * (size_t)R);
-    hist[h] = (int32_t *)malloc(sizeof(int32_t) * k * RB);
-    q[h] = (int32_t *)malloc(sizeof(int32_t) * (size_t)R * 3);
-    if (!sum[h] || !mean[h] || !hist[h] || !q[h]) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
+    sum[h] = xmalloc(sizeof(double) * (size_t)k * R);
+    mean[h] = xmalloc(sizeof(double) * (size_t)R);
+    hist[h] = xmalloc(sizeof(int32_t) * k * RB);
+    q[h] = xmalloc(sizeof(int32_t) * (size_t)R * 3);
   }
-  if (!n) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
   if (ser_run_cd_marginals(sub, chosen, k, sum[0], sum[1], hist[0], hist[1], n)) die("ser_run_cd_marginals");
   for (c = 0; c < k; c++) tot += n[c];
   for (h = 0; h < 2; h++) {
@@ -306,7 +292,7 @@ static void write_cd_marginals(ser_run *sub, const int32_t *chosen, int32_t k, i
       for (j = 0; j < RB; j++) hist[h][j] += hist[h][c * RB + j];
     if (ser_hist_quantiles(hist[h], R, SER_CD_BINS, probs, 3, q[h])) die("ser_hist_quantiles");
   }
-  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  f = open_out(path);
   fprintf(f, "taxon,c_mean,c_q025,c_median,c_q975,d_mean,d_q025,d_median,d_q975\n");
   for (r = 0; r < R; r++) {
     if (R > 1) fprintf(f, "%d", r);
@@ -319,7 +305,7 @@ static void write_cd_marginals(ser_run *sub, const int32_t *chosen, int32_t k, i
     }
     fprintf(f, "\n");
   }
-  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  close_out(f, path);
   for (i = 0; i < 2; i++) {
     if (R > 1) snprintf(name[i], sizeof(name[i]), "taxon %d", arg[1 - i]);
     else snprintf(name[i], sizeof(name[i]), "all");
@@ -330,67 +316,23 @@ static void write_cd_marginals(ser_run *sub, const int32_t *chosen, int32_t k, i
   free(n);
 }
 
-/* --marginals / --taxon-pairs / --cd-marginals: the chosen chains re-simulated alone through a window of W samples while their position and a / b
- * histograms (prefix), their taxon pair relations (pairs_prefix) and their error-rate marginals (cd_path) accumulate (any of the three
- * may be NULL; bit-identical to their first
- * run, whose E[-logL] per global id - first is e[]; any difference exits 1), the counts pooled over the chains, PREFIX.sites.csv and
- * PREFIX.taxa.csv or the four taxon pair matrices written, and one summary line printed for each.  `counts` (NULL: not wanted) receives
- * their pair-order counts from the same run. */
-static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
-                             int burn, int samples, int window, int32_t *counts, const char *prefix, const char *pairs_prefix,
-                             const char *cd_path)
+/* --marginals: the position and a / b histograms of the chosen chains of `sub` pooled over the chains to PREFIX.sites.csv and
+ * PREFIX.taxa.csv, and one summary line */
+static void write_marginals(ser_run *sub, const ser_dataset *ds, const int32_t *chosen, int32_t k, const char *prefix)
 {
-  ser_run_config c2 = *cfg;
-  ser_run *sub = NULL;
-  int32_t N, M, nh, ns = 0, i, c, tot = 0;
+  int32_t N, M, nh, i, c, tot = 0;
   size_t j;
   char path[4096];
   FILE *f;
   ser_dataset_dims(ds, &N, &M, &nh);
   const size_t NN = (size_t)N * N, MB = (size_t)M * (N + 1);
-  int32_t *pos = (int32_t *)malloc(sizeof(int32_t) * k * NN), *ah = (int32_t *)malloc(sizeof(int32_t) * k * MB);
-  int32_t *bh = (int32_t *)malloc(sizeof(int32_t) * k * MB), *n = (int32_t *)malloc(sizeof(int32_t) * (size_t)k);
-  double *e2 = (double *)malloc(sizeof(double) * (size_t)k), *w = (double *)malloc(sizeof(double) * (size_t)(N > M ? N : M));
-  struct marginal *ms = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)N);
-  struct marginal *ma = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)M), *mb = (struct marginal *)malloc(sizeof(struct marginal) * (size_t)M);
-  uint8_t *hard = (uint8_t *)malloc((size_t)N);
-  if (!pos || !ah || !bh || !n || !e2 || !w || !ms || !ma || !mb || !hard) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
-  c2.n_chains = k;
-  c2.chain_offset = 0;
-  c2.store = SER_STORE_FULL;
-  c2.max_samples = window;
-  if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
-  if (ser_run_init(sub) || ser_run_accumulate(sub, (prefix ? SER_ACC_POS | SER_ACC_RANGE : 0) | (pairs_prefix ? SER_ACC_TAXA : 0) |
-                                                     (cd_path ? SER_ACC_CD : 0) | (counts ? SER_ACC_PO : 0)))
-    die("ser_run_accumulate");
-  if (ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
-  if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
-  for (i = 0; i < k; i++)
-    if (memcmp(&e2[i], &e[chosen[i] - first], sizeof(double))) {
-      fprintf(stderr, "mcmc: the replayed chain %d does not reproduce its first run (E[-logL] %.17g vs %.17g)\n", chosen[i], e2[i],
-              e[chosen[i] - first]);
-      exit(1);
-    }
-  if (counts && ser_run_po_counts(sub, chosen, k, counts)) die("ser_run_po_counts");
-  if (pairs_prefix) {
-    const size_t MM = (size_t)M * M;
-    int32_t *tp[4];
-    for (c = 0; c < 4; c++)
-      if (!(tp[c] = (int32_t *)malloc(sizeof(int32_t) * k * MM))) { fprintf(stderr, "mcmc: out of memory\n"); exit(1); }
-    if (ser_run_taxon_pairs(sub, chosen, k, tp[0], tp[1], tp[2], tp[3], n)) die("ser_run_taxon_pairs");
-    for (tot = 0, c = 0; c < k; c++) tot += n[c];
-    write_taxon_pairs(tp, k, M, tot, pairs_prefix);
-    for (c = 0; c < 4; c++) free(tp[c]);
-  }
-  if (cd_path) write_cd_marginals(sub, chosen, k, cfg->manycd ? M : 1, cd_path);
-  if (!prefix) {
-    ser_run_destroy(sub);
-    free(pos); free(ah); free(bh); free(n); free(e2); free(w); free(ms); free(ma); free(mb); free(hard);
-    return;
-  }
+  int32_t *pos = xmalloc(sizeof(int32_t) * k * NN), *ah = xmalloc(sizeof(int32_t) * k * MB), *bh = xmalloc(sizeof(int32_t) * k * MB);
+  int32_t *n = xmalloc(sizeof(int32_t) * (size_t)k);
+  double *w = xmalloc(sizeof(double) * (size_t)(N > M ? N : M));
+  struct marginal *ms = xmalloc(sizeof(struct marginal) * (size_t)N);
+  struct marginal *ma = xmalloc(sizeof(struct marginal) * (size_t)M), *mb = xmalloc(sizeof(struct marginal) * (size_t)M);
+  uint8_t *hard = xmalloc((size_t)N);
   if (ser_run_marginals(sub, chosen, k, pos, ah, bh, n)) die("ser_run_marginals");
-  ser_run_destroy(sub);
-  tot = 0;
   for (c = 1; c < k; c++) { /* pool the chains' counts into chain 0's slabs */
     for (j = 0; j < NN; j++) pos[j] += pos[c * NN + j];
     for (j = 0; j < MB; j++) { ah[j] += ah[c * MB + j]; bh[j] += bh[c * MB + j]; }
@@ -400,21 +342,51 @@ static void replay_marginals(const ser_dataset *ds, const ser_run_config *cfg, c
   for (i = 0; i < M; i++) { summarise(ah + (size_t)i * (N + 1), N + 1, &ma[i]); summarise(bh + (size_t)i * (N + 1), N + 1, &mb[i]); }
   ser_dataset_get(ds, NULL, hard);
   snprintf(path, sizeof(path), "%s.sites.csv", prefix);
-  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  f = open_out(path);
   fprintf(f, "site,hard,mean,q025,median,q975,mode,p_mode\n");
   for (i = 0; i < N; i++)
     fprintf(f, "%d,%d,%.6f,%d,%d,%d,%d,%.6f\n", i, hard[i] != 0, ms[i].mean, ms[i].q[0], ms[i].q[1], ms[i].q[2], ms[i].mode, ms[i].p_mode);
-  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  close_out(f, path);
   snprintf(path, sizeof(path), "%s.taxa.csv", prefix);
-  if (!(f = fopen(path, "w"))) { fprintf(stderr, "mcmc: cannot open %s\n", path); exit(1); }
+  f = open_out(path);
   fprintf(f, "taxon,a_mean,a_q025,a_median,a_q975,b_mean,b_q025,b_median,b_q975\n");
   for (i = 0; i < M; i++)
     fprintf(f, "%d,%.6f,%d,%d,%d,%.6f,%d,%d,%d\n", i, ma[i].mean, ma[i].q[0], ma[i].q[1], ma[i].q[2], mb[i].mean, mb[i].q[0], mb[i].q[1],
             mb[i].q[2]);
-  if (fclose(f)) { fprintf(stderr, "mcmc: cannot write %s\n", path); exit(1); }
+  close_out(f, path);
   printf("marginals: %d chains  %d samples  median width of the 95%% intervals: sites %.1f  a %.1f  b %.1f positions\n", k, tot,
          median_width(ms, N, w), median_width(ma, M, w), median_width(mb, M, w));
-  free(pos); free(ah); free(bh); free(n); free(e2); free(w); free(ms); free(ma); free(mb); free(hard);
+  free(pos); free(ah); free(bh); free(n); free(w); free(ms); free(ma); free(mb); free(hard);
+}
+
+/* The chosen chains re-simulated alone, once for every --select output: bit-identical to their first run, whose E[-logL] per global
+ * id - first is e[] (any difference exits 1).  acc = 0 keeps every sample (SER_STORE_FULL, max_samples = samples), so every getter
+ * reads the store; otherwise the SER_ACC_* parts in acc accumulate through a window of W samples, in SER_STORE_PI when acc is
+ * SER_ACC_PO alone (pair order reads pi only) and SER_STORE_FULL else.  The caller destroys the run. */
+static ser_run *replay_chosen(const ser_dataset *ds, const ser_run_config *cfg, const int32_t *chosen, int32_t k, const double *e, int first,
+                              int burn, int samples, int window, int acc)
+{
+  ser_run_config c2 = *cfg;
+  ser_run *sub = NULL;
+  double *e2 = xmalloc(sizeof(double) * (size_t)k);
+  int32_t ns = 0, i;
+  c2.n_chains = k;
+  c2.chain_offset = 0;
+  c2.store = acc == SER_ACC_PO ? SER_STORE_PI : SER_STORE_FULL;
+  c2.max_samples = acc ? window : samples;
+  if (ser_run_create_chains(ds, &c2, chosen, k, &sub)) die("ser_run_create_chains");
+  if (ser_run_init(sub)) die("ser_run_init");
+  if (acc && ser_run_accumulate(sub, acc)) die("ser_run_accumulate");
+  if (ser_run_advance_both(sub, burn, samples) || ser_run_sync(sub)) die("replay of the chosen chains");
+  if (ser_run_chain_stats(sub, e2, NULL, NULL, &ns)) die("ser_run_chain_stats");
+  for (i = 0; i < k; i++)
+    if (memcmp(&e2[i], &e[chosen[i] - first], sizeof(double))) {
+      fprintf(stderr, "mcmc: the replayed chain %d does not reproduce its first run (E[-logL] %.17g vs %.17g)\n", chosen[i], e2[i],
+              e[chosen[i] - first]);
+      exit(1);
+    }
+  free(e2);
+  return sub;
 }
 
 static double *read_tape(const char *path, uint64_t *len)
@@ -615,21 +587,9 @@ int main(int argc, char **argv)
         /* E[-logL] -> selection -> pair-order counts in one step on the device(s) (script.py:70-99, :155-189) */
         if (ser_multi_cross_chain(multi, select_k, chosen, &nchosen, &mn, &sd, counts)) die("ser_multi_cross_chain");
       } else {
-        /* selection on the host, then the chosen chains again, alone, with the pair-order counts accumulating */
+        /* selection on the host; the chosen chains' pair-order counts come from their replay below */
         if (ser_select_chains(e, n_chains, select_k, chosen, &nchosen, &mn, &sd)) die("ser_select_chains");
         for (i = 0; i < nchosen; i++) chosen[i] += first; /* index in e -> global id */
-        if (counts && nchosen > 0 && !diag_path && !rdiag_path && !marg_prefix && !pairs_prefix && !cd_path) {
-          ser_run_config c2 = cfg;
-          ser_run *sub = NULL;
-          c2.n_chains = nchosen;
-          c2.chain_offset = 0;
-          c2.store = SER_STORE_PI;
-          c2.max_samples = window;
-          if (ser_run_create_chains(ds, &c2, chosen, nchosen, &sub)) die("ser_run_create_chains");
-          if (ser_run_init(sub) || ser_run_accumulate(sub, SER_ACC_PO)) die("ser_run_accumulate");
-          if (ser_run_advance_both(sub, burn, samples) || ser_run_po_counts(sub, chosen, nchosen, counts)) die("replay of the chosen chains");
-          ser_run_destroy(sub);
-        }
       }
       printf("selection: min E[-logL] %.6f  sigma %.6f  chosen", mn, sd);
       for (i = 0; i < nchosen; i++) printf(" %d", chosen[i]);
@@ -639,12 +599,20 @@ int main(int argc, char **argv)
         for (i = 0; i < nchosen; i++) { sc += ec[chosen[i] - first]; sdd += ed[chosen[i] - first]; }
         printf("E[c] %.6f  E[d] %.6f over the chosen chains\n", sc / nchosen, sdd / nchosen);
       }
-      if ((diag_path || rdiag_path) && nchosen > 0)
-        replay_diagnostics(ds, &cfg, chosen, nchosen, e, first, burn, samples, replay_selected ? counts : NULL, diag_path, rdiag_path);
-      if ((marg_prefix || pairs_prefix || cd_path) && nchosen > 0)
-        replay_marginals(ds, &cfg, chosen, nchosen, e, first, burn, samples, window,
-                         (replay_selected && !diag_path && !rdiag_path) ? counts : NULL,
-                         marg_prefix, pairs_prefix, cd_path);
+      if (nchosen > 0 && (diag_path || rdiag_path || marg_prefix || pairs_prefix || cd_path || (replay_selected && po_path))) {
+        /* one replay for every output: every sample kept for the diagnostics, else a window accumulating what the outputs read */
+        const int acc = (diag_path || rdiag_path) ? 0
+                        : (replay_selected && po_path ? SER_ACC_PO : 0) | (marg_prefix ? SER_ACC_POS | SER_ACC_RANGE : 0) |
+                          (pairs_prefix ? SER_ACC_TAXA : 0) | (cd_path ? SER_ACC_CD : 0);
+        ser_run *sub = replay_chosen(ds, &cfg, chosen, nchosen, e, first, burn, samples, window, acc);
+        if (replay_selected && po_path && ser_run_po_counts(sub, chosen, nchosen, counts)) die("ser_run_po_counts");
+        if (rdiag_path) write_rank_diagnostics(sub, chosen, nchosen, N, rdiag_path);
+        if (diag_path) write_diagnostics(sub, chosen, nchosen, N, diag_path);
+        if (pairs_prefix) write_taxon_pairs(sub, chosen, nchosen, M, pairs_prefix);
+        if (cd_path) write_cd_marginals(sub, chosen, nchosen, manycd ? M : 1, cd_path);
+        if (marg_prefix) write_marginals(sub, ds, chosen, nchosen, marg_prefix);
+        ser_run_destroy(sub);
+      }
       if (po_path && nchosen > 0) {
         double *po = (double *)malloc(sizeof(double) * (size_t)N * N);
         FILE *f;
