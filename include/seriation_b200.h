@@ -26,6 +26,7 @@
  *                                                       script.py:129-152, :230-276
  *   ser_run_alive_counts      plot_taxa_occurence_probability_matrix / plot_false_*  script.py:306-448
  *   ser_run_cd_marginals      per-taxon (manycd) or scalar posterior of the error rates c, d: exp sums and histograms
+ *   ser_run_diversity         diversity curves: posterior of range-through richness, originations and extinctions per position and site
  *   ser_run_site_age_corr     CORR_MN of Docs/Report.pdf Table 1 (E[pi] against the .sites MN ages)
  *   run_all_chains' Pool(8) over 100 processes (script.py:48-67) is replaced by
  *   n_chains in ser_run_config: one persistent launch over all chains of a GPU, and by
@@ -294,6 +295,31 @@ int ser_run_taxon_pairs(ser_run *run, const int32_t *chosen, int32_t k, int32_t 
 int ser_run_cd_marginals(ser_run *run, const int32_t *chosen, int32_t k, double *c_sum, double *d_sum, int32_t *c_hist, int32_t *d_hist,
                          int32_t *n_samples);
 
+/* Diversity curves (DESIGN.md section 3.12).  Ranges are half-open: taxon m is alive at positions a_t(m) <= p < b_t(m), 0 <= a <= b <= N.
+ * For chosen chain c over its T samples t, positions p in [0, N), sites i in file order, taxa counted over every m:
+ *   D_t(p) = #{m : a_t(m) <= p < b_t(m)}       richness at position p (range-through)
+ *   O_t(p) = #{m : a_t(m) = p < b_t(m)}        originations: non-empty ranges whose first position is p
+ *   E_t(p) = #{m : a_t(m) < b_t(m) = p + 1}    extinctions: non-empty ranges whose last position is p
+ *   richness[c][p][v]      = #{t : D_t(p) = v}
+ *   originations[c][p][v]  = #{t : O_t(p) = v}
+ *   extinctions[c][p][v]   = #{t : E_t(p) = v}
+ *   site_richness[c][i][v] = #{t : D_t(pi_t(i)) = v}   richness at the position site i holds in sample t
+ * Each output is int32 [k][N][M + 1], v in [0, M]; every row sums to T.  Empty ranges (a = b) count nowhere.  The ends are not special:
+ * every taxon alive at position 0 originates there and every taxon alive at N - 1 goes extinct there (an edge effect of the sequence's
+ * ends, not an event).  Exact integer identities, with S_X(p) = sum_v v * X[c][p][v]:
+ *   sum_i site_richness[c][i][v] == sum_p richness[c][p][v] for every v                     (pi_t is a permutation)
+ *   S_richness(p)     == sum_m alive[c][p][m] - sum_m b_hist[c][m][p]                        (ser_run_alive_counts, ser_run_marginals)
+ *   S_originations(p) == sum_m a_hist[c][m][p] - z[p]
+ *   S_extinctions(p)  == sum_m b_hist[c][m][p + 1] - z[p + 1],   z[q] = #{(t, m) : a_t(m) = b_t(m) = q}
+ *   S_richness(p)     == S_richness(p - 1) + S_originations(p) - S_extinctions(p - 1),   S_richness(-1) = 0
+ * Counts add over windows, chains and devices.  Chosen ids are GLOBAL; -1 or a chain this run does not hold leaves its slabs untouched
+ * and n_samples[c] = 0; a held chain's slabs are written in full.  Host memory: any of the four outputs may be NULL but not all.  Needs
+ * SER_STORE_FULL.  On an accumulating run (SER_ACC_DIV) T counts every sample taken since accumulation began.
+ * Checked before any CUDA call: SER_E_ARG for k < 1, a NULL chosen or n_samples, or all four outputs NULL; SER_E_STATE for a store
+ * below SER_STORE_FULL, an accumulating run without SER_ACC_DIV, or a run not initialised. */
+int ser_run_diversity(ser_run *run, const int32_t *chosen, int32_t k, int32_t *richness, int32_t *originations, int32_t *extinctions,
+                      int32_t *site_richness, int32_t *n_samples);
+
 /* CORR_MN (Docs/Report.pdf Table 1; SURVEY section 8f #3): Pearson correlation of the posterior mean
  * position E[pi(site)] over the stored samples of the chosen chains owned by this run with the MN age
  * of the site read from the .sites file (ser_dataset_read_names): the mean over the stored samples of
@@ -315,17 +341,18 @@ int ser_run_site_age_corr(ser_run *run, const ser_dataset *ds, const int32_t *ch
 #define SER_ACC_TAXA 128 /* taxon pair relations       [4][M][M]   (ser_run_taxon_pairs; needs SER_STORE_FULL); 64 is not a flag */
 #define SER_ACC_CD 512  /* error-rate marginals         f64 [2][R], then [2][R][SER_CD_BINS] (ser_run_cd_marginals; needs SER_STORE_FULL;
                            the part and the record's length padded to an even number of int32 words, so the doubles are aligned); 256 is not a flag */
+#define SER_ACC_DIV 2048 /* diversity curves            [4][N][M+1] (ser_run_diversity; needs SER_STORE_FULL); 1024 is not a flag */
 /* From this call on the sample store is a window of cfg->max_samples rows per chain: ser_run_advance / _advance_both split
  * their sampling calls into sweep launches of at most max_samples calls and, after each, add the window's rows of every
  * local chain into the accumulators on the run's stream (no host synchronisation).  ser_run_po_counts(_device),
- * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals, ser_run_taxon_pairs, ser_run_cd_marginals and ser_run_site_age_corr
- * then return totals over EVERY sample taken since (T = the chain's sample count), with the usual global ids and slab convention;
+ * ser_run_posterior_sums, ser_run_alive_counts, ser_run_marginals, ser_run_taxon_pairs, ser_run_cd_marginals, ser_run_diversity and
+ * ser_run_site_age_corr then return totals over EVERY sample taken since (T = the chain's sample count), with the usual global ids and slab convention;
  * ser_run_fetch_samples / ser_run_fetch_cd_samples return SER_E_STATE (the window is transient), and so does
  * ser_run_cross_chain_async.
  * Call it before the first sampling call (ser_run_init zeroes the accumulators).  Errors: SER_E_STATE on a run that has
  * already sampled, on a store below what the flags need, or a second time; SER_E_ARG for max_samples < 1; SER_E_CUDA with
  * the byte count when an accumulator does not fit (per chain at 2048 x 8192: the alive slab is 64 MB, the a / b histograms 134 MB,
- * the taxon pair relations 1 GiB; 256 MB at 1024 x 4096). */
+ * the taxon pair relations 1 GiB, the diversity curves 268 MB; 256 MB and 67 MB at 1024 x 4096). */
 int ser_run_accumulate(ser_run *run, int32_t what);
 
 /* ---------------------------------------------------------------- cross-chain step, one call

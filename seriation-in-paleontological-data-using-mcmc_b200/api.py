@@ -18,8 +18,9 @@ LIB_PATH = os.environ.get("SERIATION_B200_LIB") or os.path.join(HERE, "libseriat
 
 MODE_FREE, MODE_REPLAY = 0, 1
 STORE_NONE, STORE_PI, STORE_FULL = 0, 1, 2
-ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE, ACC_TAXA, ACC_CD = 1, 2, 4, 8, 16, 32, 128, 512
+ACC_PO, ACC_SUMS, ACC_AB, ACC_ALIVE, ACC_POS, ACC_RANGE, ACC_TAXA, ACC_CD, ACC_DIV = 1, 2, 4, 8, 16, 32, 128, 512, 2048
 TAXON_PAIRS = ("first", "last", "precedes", "coexist")
+DIVERSITY = ("richness", "originations", "extinctions", "site_richness")
 # the sampler's bounds of the log error rates (SER_MINC ... SER_MAXD): c in [log .001, log .1], d in [log .2, log .8]; the histograms of
 # cd_marginals() have CD_BINS uniform bins on the log value between them
 MINC, MAXC, MIND, MAXD = -6.9077552789821368, -2.3025850929940455, -1.6094379124341003, -0.22314355131420971
@@ -94,6 +95,7 @@ SYMBOLS = [
     ("ser_hist_quantiles", C.c_int, [_i32p, C.c_int32, C.c_int32, _dp, C.c_int32, _i32p]),
     ("ser_run_taxon_pairs", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p, _i32p]),
     ("ser_run_cd_marginals", C.c_int, [_vp, _i32p, C.c_int32, _dp, _dp, _i32p, _i32p, _i32p]),
+    ("ser_run_diversity", C.c_int, [_vp, _i32p, C.c_int32, _i32p, _i32p, _i32p, _i32p, _i32p]),
     ("ser_write_chain_files", C.c_int, [_vp, C.c_int32, C.c_char_p]),
     ("ser_write_labelled_files", C.c_int, [_vp, C.c_int32, _vp, C.c_char_p]),
     ("ser_microbench", C.c_int, [C.c_int32, _dp]),
@@ -248,12 +250,15 @@ class Run:
             _check(lib().ser_run_create_chains(ds._h, C.byref(self.cfg), _p(ids, C.c_int32), ids.size, C.byref(h)))
         self._h = h
 
-    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False, taxon_pairs=False, cd=False):
+    def accumulate(self, po=True, sums=True, ab=False, alive=False, positions=False, ranges=False, taxon_pairs=False, cd=False,
+                   diversity=False):
         """from now on the sample store is a window of max_samples rows and the summaries sum over every sample taken
         afterwards (ser_run_accumulate); call before the first sampling call.  ``positions`` / ``ranges`` accumulate the
-        histograms of marginals(), ``taxon_pairs`` the counts of taxon_pairs(), ``cd`` the sums and histograms of cd_marginals()"""
+        histograms of marginals(), ``taxon_pairs`` the counts of taxon_pairs(), ``cd`` the sums and histograms of cd_marginals(),
+        ``diversity`` the histograms of diversity()"""
         what = (ACC_PO if po else 0) | (ACC_SUMS if sums else 0) | (ACC_AB if ab else 0) | (ACC_ALIVE if alive else 0)
         what |= (ACC_POS if positions else 0) | (ACC_RANGE if ranges else 0) | (ACC_TAXA if taxon_pairs else 0) | (ACC_CD if cd else 0)
+        what |= ACC_DIV if diversity else 0
         _check(lib().ser_run_accumulate(self._h, what))
         return self
 
@@ -479,6 +484,21 @@ class Run:
         _check(lib().ser_run_cd_marginals(self._h, _p(chosen, C.c_int32), k, _p(c_sum, C.c_double), _p(d_sum, C.c_double),
                                           _p(c_hist, C.c_int32), _p(d_hist, C.c_int32), _p(n, C.c_int32)))
         return dict(c_sum=c_sum, d_sum=d_sum, c_hist=c_hist, d_hist=d_hist, n_samples=n)
+
+    def diversity(self, chosen, richness: bool = True, originations: bool = True, extinctions: bool = True, sites: bool = True) -> dict:
+        """diversity curves of the chosen chains (global ids) over their samples (ser_run_diversity), each [k][N][M+1] int32 (None when
+        not requested): ``richness`` [c][p][v] = #{t: D_t(p) = v} with D_t(p) = #{m: a_t(m) <= p < b_t(m)}, ``originations`` (ranges
+        starting at p) and ``extinctions`` (ranges whose last position is p) alike, ``site_richness`` [c][i][v] = #{t: D_t(pi_t(i)) = v}
+        for site i in file order; ``n_samples`` [k] = T.  Slabs the run does not fill stay 0 (n_samples 0)."""
+        chosen = np.ascontiguousarray(chosen, dtype=np.int32)
+        k, N, M = len(chosen), self.N, self.M
+        want = dict(richness=richness, originations=originations, extinctions=extinctions, site_richness=sites)
+        out = {key: (np.zeros((k, N, M + 1), np.int32) if want[key] else None) for key in DIVERSITY}
+        n = np.zeros(k, np.int32)
+        _check(lib().ser_run_diversity(self._h, _p(chosen, C.c_int32), k, *(_p(out[key], C.c_int32) for key in DIVERSITY),
+                                       _p(n, C.c_int32)))
+        out["n_samples"] = n
+        return out
 
     def po_counts_device(self, chosen_ptr: int, k: int, counts_ptr: int):
         _check(lib().ser_run_po_counts_device(self._h, chosen_ptr, k, counts_ptr))
@@ -736,7 +756,7 @@ def choose_chains(batch: ChainBatch, chains_selected: int):
 
 
 def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool = False, marginals: bool = False,
-                  taxon_pairs: bool = False, cd: bool = False, device=None) -> ChainBatch:
+                  taxon_pairs: bool = False, cd: bool = False, diversity: bool = False, device=None) -> ChainBatch:
     """The second phase of select-then-replay: re-simulate the chosen chains of a batch (typically one run with
     ``store=STORE_NONE``, which holds no sample history) alone, bit for bit, while their summaries accumulate through a
     ``window``-row sample store.  The returned batch's ``run`` is that subset run and its ``stats()`` are the first
@@ -744,17 +764,19 @@ def replay_chosen(batch: ChainBatch, chains, *, window: int = 64, with_ab: bool 
     also accumulates the a/b sums and alive counts (compute_exp_a and the maps need them).  ``window=0`` keeps every
     sample instead (``STORE_FULL``, no accumulators): the summaries take the one-shot path and ``diagnostics`` works on
     the result.  ``marginals`` also accumulates the position and a/b histograms of marginals(), ``taxon_pairs`` the counts of
-    taxon_pairs() and ``cd`` the sums and histograms of cd_marginals() (each makes the window keep a, b, c and d).
+    taxon_pairs(), ``cd`` the sums and histograms of cd_marginals() and ``diversity`` the histograms of diversity() (each makes
+    the window keep a, b, c and d).
     Raises SeriationError when a replayed chain's E[-logL] differs from its first run in any bit."""
     ids = np.ascontiguousarray(chains, dtype=np.int32)
     keep_all = window == 0
     run = Run(batch.run.ds, ids.size, seed=batch.seed, sweeps_per_call=batch.sweeps_per_call, manycd=batch.manycd,
-              store=STORE_FULL if (with_ab or keep_all or marginals or taxon_pairs or cd) else STORE_PI, max_samples=batch.sample_calls if keep_all else window,
+              store=STORE_FULL if (with_ab or keep_all or marginals or taxon_pairs or cd or diversity) else STORE_PI,
+              max_samples=batch.sample_calls if keep_all else window,
               device=batch.run.cfg.device if device is None else device, chain_ids=ids)
     run.init()
     if not keep_all:
         run.accumulate(po=True, sums=True, ab=with_ab, alive=with_ab, positions=marginals, ranges=marginals, taxon_pairs=taxon_pairs,
-                       cd=cd)
+                       cd=cd, diversity=diversity)
     run.advance(batch.burn_calls, False).advance(batch.sample_calls, True).sync()
     want, got = batch.stats()["e_negloglik"][ids], run.chain_stats()["e_negloglik"]
     if want.tobytes() != got.tobytes():
@@ -848,6 +870,19 @@ def cd_marginals(batch: ChainBatch, chains, probs=(0.025, 0.5, 0.975)) -> dict:
         mode = counts.argmax(axis=1)
         out[name] = dict(mean=total / n, quantiles=q, lower=edges[q], upper=edges[q + 1], mode=mode,
                          p_mode=counts[np.arange(len(counts)), mode] / n, counts=counts, sum=total)
+    return out
+
+
+def diversity(batch: ChainBatch, chains, probs=(0.025, 0.5, 0.975)) -> dict:
+    """Diversity curves pooled over the chosen chains by summing their counts: for each of ``richness``, ``originations``,
+    ``extinctions`` (per position) and ``site_richness`` (per site, file order) the ``mean``, ``quantiles`` [N][len(probs)]
+    (hist_quantiles: the bins are the counts of taxa themselves), ``mode`` and ``p_mode`` of every row; ``counts`` holds the pooled
+    histograms [N][M+1] and ``n_samples`` the pooled sample count.  Needs a batch that keeps a, b and pi: the full sample store, or
+    replay_chosen(..., diversity=True)."""
+    d = batch.run.diversity(np.asarray(chains, dtype=np.int32))
+    counts = {key: d[key].sum(axis=0, dtype=np.int64).astype(np.int32) for key in DIVERSITY}
+    out = {key: _marginal_summary(counts[key], probs) for key in DIVERSITY}
+    out.update(counts=counts, n_samples=int(d["n_samples"].sum(dtype=np.int64)), probs=tuple(probs))
     return out
 
 

@@ -18,11 +18,11 @@
  *   mcmc --chains N [--gpus G] [--first I] [--burn B] [--samples S] [--seed X] [--dataset file]
  *        [--chains-dir DIR] [--select K] [--po file.csv] [--device D] [--manycd 0|1] [--replay-selected --window W]
  *        [--checkpoint FILE [--checkpoint-every C] [--resume] [--stop-after C]] [--diagnostics FILE] [--rank-diagnostics FILE]
- *        [--marginals PREFIX] [--taxon-pairs PREFIX] [--cd-marginals FILE]
+ *        [--marginals PREFIX] [--taxon-pairs PREFIX] [--cd-marginals FILE] [--diversity PREFIX]
  * --replay-selected (with --select) runs select-then-replay: the chains keep no sample history (SER_STORE_NONE, so no
  * Chains/ files) and the pair-order counts of the K chosen chains come from their replay: the same output lines and po.csv
  * as the one-shot step, with device memory for K chains' window instead of every chain's history.
- * Every --select output (po.csv under --replay-selected, and the outputs of the five flags below) comes from one replay of the chosen
+ * Every --select output (po.csv under --replay-selected, and the outputs of the six flags below) comes from one replay of the chosen
  * chains, alone on --device (ser_run_create_chains), which exits 1 unless each reproduces its first run's E[-logL] bit for
  * bit.  That replay keeps every sample (SER_STORE_FULL) when --diagnostics or --rank-diagnostics is given, and otherwise
  * runs through a window of W samples (--window, default 64) while what the outputs read accumulates (ser_run_accumulate);
@@ -50,6 +50,11 @@
  * "all" otherwise; the means are the posterior means of the probabilities exp(c), exp(d), q025 is the lower edge of the 2.5 % quantile's
  * bin, q975 the upper edge of the 97.5 % quantile's bin and the median the log-midpoint of its bin, all as probabilities.  It prints one
  * summary line: the rows with the highest mean d (most missed occurrences) and the highest mean c (most spurious ones).
+ * --diversity PREFIX (with --select) pools the diversity curves of the chosen chains (ser_run_diversity) and writes PREFIX.positions.csv
+ * "position,rich_mean,rich_q025,rich_median,rich_q975,orig_mean,orig_q025,orig_median,orig_q975,ext_mean,ext_q025,ext_median,ext_q975"
+ * (range-through richness, originations and extinctions at every position of the sequence) and PREFIX.sites.csv
+ * "site,hard,rich_mean,rich_q025,rich_median,rich_q975" (the richness at the position each site holds; file order, 0-based), the
+ * quantiles as numbers of taxa, and prints one summary line: the peak mean richness, its position and its 95 % interval.
  * Replay mode: SER_TAPE_IN=<file of raw doubles> mcmc <idx> < dataset.txt
  */
 #include <errno.h>
@@ -105,7 +110,9 @@ static void usage(const char *argv0)
           "              [--taxon-pairs PREFIX]   (with --select: first / last appearance order, superposition and coexistence\n"
           "                                        of every pair of taxa to PREFIX.{first,last,precedes,coexist}.csv; --window W)\n"
           "              [--cd-marginals FILE]   (with --select: posterior means and credible intervals of the error rates c, d\n"
-          "                                       per taxon (--manycd 1) or of the scalar pair to FILE; --window W)\n",
+          "                                       per taxon (--manycd 1) or of the scalar pair to FILE; --window W)\n"
+          "              [--diversity PREFIX]   (with --select: richness, originations and extinctions per position and richness\n"
+          "                                      per site of the chosen chains to PREFIX.positions.csv and PREFIX.sites.csv; --window W)\n",
           argv0, argv0, argv0);
   exit(1);
 }
@@ -359,6 +366,53 @@ static void write_marginals(ser_run *sub, const ser_dataset *ds, const int32_t *
   free(pos); free(ah); free(bh); free(n); free(w); free(ms); free(ma); free(mb); free(hard);
 }
 
+/* --diversity: the diversity curves of the chosen chains of `sub` pooled over the chains to PREFIX.positions.csv and PREFIX.sites.csv,
+ * and one summary line */
+static void write_diversity(ser_run *sub, const ser_dataset *ds, const int32_t *chosen, int32_t k, const char *prefix)
+{
+  int32_t N, M, nh, i, c, q, tot = 0, peak = 0;
+  size_t j;
+  char path[4096];
+  FILE *f;
+  ser_dataset_dims(ds, &N, &M, &nh);
+  const size_t cells = (size_t)N * (M + 1);
+  int32_t *h[4], *n = xmalloc(sizeof(int32_t) * (size_t)k);
+  struct marginal *m[4];
+  uint8_t *hard = xmalloc((size_t)N);
+  for (q = 0; q < 4; q++) {
+    h[q] = xmalloc(sizeof(int32_t) * k * cells);
+    m[q] = xmalloc(sizeof(struct marginal) * (size_t)N);
+  }
+  if (ser_run_diversity(sub, chosen, k, h[0], h[1], h[2], h[3], n)) die("ser_run_diversity");
+  for (c = 0; c < k; c++) tot += n[c];
+  for (q = 0; q < 4; q++) {
+    for (c = 1; c < k; c++) /* pool the chains' counts into chain 0's slab */
+      for (j = 0; j < cells; j++) h[q][j] += h[q][c * cells + j];
+    for (i = 0; i < N; i++) summarise(h[q] + (size_t)i * (M + 1), M + 1, &m[q][i]);
+  }
+  snprintf(path, sizeof(path), "%s.positions.csv", prefix);
+  f = open_out(path);
+  fprintf(f, "position,rich_mean,rich_q025,rich_median,rich_q975,orig_mean,orig_q025,orig_median,orig_q975,ext_mean,ext_q025,ext_median,"
+             "ext_q975\n");
+  for (i = 0; i < N; i++) {
+    fprintf(f, "%d", i);
+    for (q = 0; q < 3; q++) fprintf(f, ",%.6f,%d,%d,%d", m[q][i].mean, m[q][i].q[0], m[q][i].q[1], m[q][i].q[2]);
+    fprintf(f, "\n");
+    if (m[0][i].mean > m[0][peak].mean) peak = i;
+  }
+  close_out(f, path);
+  ser_dataset_get(ds, NULL, hard);
+  snprintf(path, sizeof(path), "%s.sites.csv", prefix);
+  f = open_out(path);
+  fprintf(f, "site,hard,rich_mean,rich_q025,rich_median,rich_q975\n");
+  for (i = 0; i < N; i++) fprintf(f, "%d,%d,%.6f,%d,%d,%d\n", i, hard[i] != 0, m[3][i].mean, m[3][i].q[0], m[3][i].q[1], m[3][i].q[2]);
+  close_out(f, path);
+  printf("diversity: %d chains  %d samples  peak mean richness %.6f taxa at position %d (95%% interval %d-%d)\n", k, tot, m[0][peak].mean,
+         peak, m[0][peak].q[0], m[0][peak].q[2]);
+  for (q = 0; q < 4; q++) { free(h[q]); free(m[q]); }
+  free(n); free(hard);
+}
+
 /* The chosen chains re-simulated alone, once for every --select output: bit-identical to their first run, whose E[-logL] per global
  * id - first is e[] (any difference exits 1).  acc = 0 keeps every sample (SER_STORE_FULL, max_samples = samples), so every getter
  * reads the store; otherwise the SER_ACC_* parts in acc accumulate through a window of W samples, in SER_STORE_PI when acc is
@@ -412,7 +466,7 @@ int main(int argc, char **argv)
   int64_t done = 0, total;
   unsigned long seed = 0;
   const char *dataset = NULL, *chains_dir = "Chains", *po_path = NULL, *tape_path = getenv("SER_TAPE_IN"), *ckpt_path = NULL;
-  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL, *pairs_prefix = NULL, *cd_path = NULL;
+  const char *diag_path = NULL, *marg_prefix = NULL, *rdiag_path = NULL, *pairs_prefix = NULL, *cd_path = NULL, *div_prefix = NULL;
   const char *env_seed = getenv("GSL_RNG_SEED");
   ser_dataset *ds = NULL;
   ser_run *run = NULL;   /* single-chain replay */
@@ -451,6 +505,7 @@ int main(int argc, char **argv)
       else if (!strcmp(a, "--marginals")) marg_prefix = v;
       else if (!strcmp(a, "--taxon-pairs")) pairs_prefix = v;
       else if (!strcmp(a, "--cd-marginals")) cd_path = v;
+      else if (!strcmp(a, "--diversity")) div_prefix = v;
       else if (!strcmp(a, "--checkpoint-every")) { if ((ckpt_every = atoi(v)) < 1) usage(argv[0]); }
       else if (!strcmp(a, "--stop-after")) { if ((stop_after = atoi(v)) < 0) usage(argv[0]); }
       else usage(argv[0]);
@@ -459,7 +514,7 @@ int main(int argc, char **argv)
     if (n_chains < 1 || burn < 0 || samples < 0 || gpus < 1 || gpus > 8 || n_chains < gpus) usage(argv[0]);
     if (replay_selected && (select_k < 1 || window < 1)) usage(argv[0]);
     if ((diag_path || rdiag_path) && select_k < 1) usage(argv[0]);
-    if ((marg_prefix || pairs_prefix || cd_path) && (select_k < 1 || window < 1)) usage(argv[0]);
+    if ((marg_prefix || pairs_prefix || cd_path || div_prefix) && (select_k < 1 || window < 1)) usage(argv[0]);
     if (!ckpt_path && (ckpt_every || stop_after >= 0 || resume)) usage(argv[0]); /* these act on the --checkpoint file */
   } else if (argc == 2) {
     char *end = NULL;
@@ -599,11 +654,11 @@ int main(int argc, char **argv)
         for (i = 0; i < nchosen; i++) { sc += ec[chosen[i] - first]; sdd += ed[chosen[i] - first]; }
         printf("E[c] %.6f  E[d] %.6f over the chosen chains\n", sc / nchosen, sdd / nchosen);
       }
-      if (nchosen > 0 && (diag_path || rdiag_path || marg_prefix || pairs_prefix || cd_path || (replay_selected && po_path))) {
+      if (nchosen > 0 && (diag_path || rdiag_path || marg_prefix || pairs_prefix || cd_path || div_prefix || (replay_selected && po_path))) {
         /* one replay for every output: every sample kept for the diagnostics, else a window accumulating what the outputs read */
         const int acc = (diag_path || rdiag_path) ? 0
                         : (replay_selected && po_path ? SER_ACC_PO : 0) | (marg_prefix ? SER_ACC_POS | SER_ACC_RANGE : 0) |
-                          (pairs_prefix ? SER_ACC_TAXA : 0) | (cd_path ? SER_ACC_CD : 0);
+                          (pairs_prefix ? SER_ACC_TAXA : 0) | (cd_path ? SER_ACC_CD : 0) | (div_prefix ? SER_ACC_DIV : 0);
         ser_run *sub = replay_chosen(ds, &cfg, chosen, nchosen, e, first, burn, samples, window, acc);
         if (replay_selected && po_path && ser_run_po_counts(sub, chosen, nchosen, counts)) die("ser_run_po_counts");
         if (rdiag_path) write_rank_diagnostics(sub, chosen, nchosen, N, rdiag_path);
@@ -611,6 +666,7 @@ int main(int argc, char **argv)
         if (pairs_prefix) write_taxon_pairs(sub, chosen, nchosen, M, pairs_prefix);
         if (cd_path) write_cd_marginals(sub, chosen, nchosen, manycd ? M : 1, cd_path);
         if (marg_prefix) write_marginals(sub, ds, chosen, nchosen, marg_prefix);
+        if (div_prefix) write_diversity(sub, ds, chosen, nchosen, div_prefix);
         ser_run_destroy(sub);
       }
       if (po_path && nchosen > 0) {

@@ -685,6 +685,81 @@ __global__ void ser_range_hist_kernel(const uint16_t *samp_a, const uint16_t *sa
   hist_tile(x, M, M, N + 1, T, blockIdx.y * blockDim.x, out + blockIdx.x * stride, use_smem ? s_hist : nullptr, add);
 }
 
+/* ------------------------------------------------------------------ diversity curves (ser_run_diversity, DESIGN.md 3.12)
+ * Two stages over a pass of `rows` sample rows [t0, t0 + rows) of every chain (SER_DIV_CHUNK at most, so the scratch stays bounded):
+ * stage 1 turns each sample row into its curves, u16 rows of scratch [k][rows][4][N] (D richness, O originations, E extinctions, then
+ * D at the position of each site); stage 2 histograms every position's or site's column of them with hist_tile, bins = M + 1. */
+#define SER_DIV_CHUNK 1024
+#define SER_DIV_THREADS 256
+
+/* Stage 1, one block per (row t0 + blockIdx.x, chain blockIdx.y).  The non-empty ranges' starts (at a) and stops (at b) are counted in
+ * shared memory with integer atomics (the same in any order); D(p) = sum_{q <= p} (starts[q] - stops[q]) is a block scan taken
+ * SER_DIV_THREADS positions at a time, O(p) = starts[p], E(p) = stops[p + 1]; the site row gathers D(pi_t(i)). */
+__global__ void __launch_bounds__(SER_DIV_THREADS) ser_div_curve_kernel(const uint16_t *samp_a, const uint16_t *samp_b, const uint16_t *samp_pi,
+                                                                        const ChainScalars *scal, int N, int M, int max_samples, SumSel sel,
+                                                                        int t0, uint16_t *scratch)
+{
+  __shared__ int s_st[SER_MAX_SITES + 1], s_en[SER_MAX_SITES + 1], s_warp[SER_DIV_THREADS / 32];
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.y, false, &T), t = t0 + blockIdx.x;
+  if (local < 0 || t >= T) return;
+  for (int p = threadIdx.x; p <= N; p += blockDim.x) { s_st[p] = 0; s_en[p] = 0; }
+  __syncthreads();
+  const size_t row = (size_t)local * max_samples + t;
+  const uint16_t *A = samp_a + row * M, *B = samp_b + row * M;
+  for (int m = threadIdx.x; m < M; m += blockDim.x) {
+    const int a = A[m], b = B[m];
+    if (a < b) { atomicAdd(&s_st[a], 1); atomicAdd(&s_en[b], 1); }
+  }
+  __syncthreads();
+  uint16_t *out = scratch + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 4 * N;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int carry = 0;
+  for (int p0 = 0; p0 < N; p0 += blockDim.x) {
+    const int p = p0 + threadIdx.x;
+    const int o = p < N ? s_st[p] : 0, e = p < N ? s_en[p + 1] : 0;
+    int v = p < N ? o - s_en[p] : 0;
+    for (int d = 1; d < 32; d <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, v, d);
+      if (lane >= d) v += y;
+    }
+    if (lane == 31) s_warp[warp] = v;
+    __syncthreads();
+    int before = carry;
+    for (int w = 0; w < nw; w++) {
+      const int s = s_warp[w];
+      carry += s;
+      if (w < warp) before += s;
+    }
+    if (p < N) { /* only this thread reads s_st[p]: it becomes D(p) */
+      const int D = before + v;
+      s_st[p] = D;
+      out[p] = (uint16_t)D;
+      out[N + p] = (uint16_t)o;
+      out[2 * N + p] = (uint16_t)e;
+    }
+    __syncthreads();
+  }
+  const uint16_t *P = samp_pi + row * N;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) out[3 * N + i] = (uint16_t)s_st[P[i]];
+}
+
+/* Stage 2: output blockIdx.z (richness, originations, extinctions, site richness; nullptr: not wanted) of chain blockIdx.x, its rows
+ * [blockIdx.y * blockDim.x, +blockDim.x) of [N][M + 1], over the pass's rows of that chain; add = 0 stores the slab, add = 1 adds. */
+__global__ void ser_div_hist_kernel(const uint16_t *scratch, const ChainScalars *scal, int N, int M, SumSel sel, int t0, int rows, int use_smem,
+                                    int *rich, int *orig, int *ext, int *site, size_t stride, int add)
+{
+  extern __shared__ int s_hist[];
+  int *out = blockIdx.z == 0 ? rich : blockIdx.z == 1 ? orig : blockIdx.z == 2 ? ext : site;
+  if (!out) return;
+  int T;
+  const int local = sel_chain(sel, scal, blockIdx.x, blockIdx.y == 0 && threadIdx.x == 0, &T);
+  if (local < 0) return;
+  const int n = min(max(T - t0, 0), rows);
+  hist_tile(scratch + (size_t)blockIdx.x * rows * 4 * N + (size_t)blockIdx.z * N, 4 * N, N, M + 1, n, blockIdx.y * blockDim.x,
+            out + blockIdx.x * stride, use_smem ? s_hist : nullptr, add);
+}
+
 /* ------------------------------------------------------------------ rank-normalised diagnostics (ser_run_rank_diagnostics, DESIGN.md 3.9)
  * The draws pool the chosen chains, ascending global id: sequence j is the first (j even) or the last (j odd) n = T/2 stored samples
  * of chosen chain j/2, draw (j, t) its row t or T - n + t (the middle row of an odd T is in neither), S = m n draws over m = 2k
@@ -947,18 +1022,20 @@ __global__ void __launch_bounds__(1024, 1) ser_rank_ess_kernel(RankSrc src, Rank
  * the summary kernels above add the window's rows of EVERY local chain into that chain's accumulator record; the getters turn the
  * records into what the one-shot kernels compute from a store that holds all samples, with the kernels below. */
 
-#define SER_ACC_ALL (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD)
+#define SER_ACC_ALL \
+  (SER_ACC_PO | SER_ACC_SUMS | SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_POS | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD | SER_ACC_DIV)
 
 /* One local chain's accumulator record: int32 offsets of the parts the flags `what` select, in this order, and the record's length.
  * The run holds [n_local][ints]; a checkpoint record holds the same ints in the same order.
  *   po [N][N] (SER_ACC_PO; diagonal 0), pi [N] (SER_ACC_SUMS or SER_ACC_AB), asum [M], bsum [M] (SER_ACC_AB),
  *   alive [N][M] (SER_ACC_ALIVE; the difference slab), pos [N][N] (SER_ACC_POS), range [2][M][N+1] (SER_ACC_RANGE; a, then b),
  *   taxa [4][M][M] (SER_ACC_TAXA; first, last, precedes, coexist),
- *   cd: f64 c_sum, d_sum [R] as pairs of int32 words, then c_hist, d_hist [R][SER_CD_BINS] (SER_ACC_CD; R = M on a manycd run, else 1).
+ *   cd: f64 c_sum, d_sum [R] as pairs of int32 words, then c_hist, d_hist [R][SER_CD_BINS] (SER_ACC_CD; R = M on a manycd run, else 1),
+ *   div [4][N][M+1] (SER_ACC_DIV; richness, originations, extinctions, site richness: an even length, so the alignment below holds).
  * Under SER_ACC_CD alone the part's start and the record's length are rounded up to an even number of words, so every double is
  * 8-byte aligned in the run's records; records without the flag keep their length, and checkpoint files their bytes. */
 struct AccLayout {
-  size_t po, pi, asum, bsum, alive, pos, range, taxa, cd, ints;
+  size_t po, pi, asum, bsum, alive, pos, range, taxa, cd, div, ints;
 };
 __host__ __device__ inline AccLayout acc_layout(int N, int M, int manycd, int what)
 {
@@ -975,6 +1052,7 @@ __host__ __device__ inline AccLayout acc_layout(int N, int M, int manycd, int wh
   L.taxa = o; o += (what & SER_ACC_TAXA) ? 4 * m * m : 0;
   if (what & SER_ACC_CD) o += o & 1;
   L.cd = o; o += (what & SER_ACC_CD) ? 4 * cdr + 2 * cdr * SER_CD_BINS : 0;
+  L.div = o; o += (what & SER_ACC_DIV) ? 4 * n * (m + 1) : 0;
   L.ints = o;
   return L;
 }

@@ -645,7 +645,7 @@ extern "C" int ser_run_accumulate(ser_run *run, int32_t what)
   if (what < 1 || (what & ~SER_ACC_ALL)) { ser_set_error("ser_run_accumulate: bad flags %d", what); return SER_E_ARG; }
   if (run->acc_what) { ser_set_error("ser_run_accumulate: the run already accumulates"); return SER_E_STATE; }
   if (run->sampled) { ser_set_error("ser_run_accumulate: the run has already taken samples; call it before the first sampling call"); return SER_E_STATE; }
-  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD)) ? SER_STORE_FULL : SER_STORE_PI;
+  const int need = (what & (SER_ACC_AB | SER_ACC_ALIVE | SER_ACC_RANGE | SER_ACC_TAXA | SER_ACC_CD | SER_ACC_DIV)) ? SER_STORE_FULL : SER_STORE_PI;
   if (run->cfg.store < need) {
     ser_set_error("ser_run_accumulate: these summaries need %s", need == SER_STORE_FULL ? "SER_STORE_FULL (a, b samples)" : "SER_STORE_PI or more");
     return SER_E_STATE;
@@ -910,6 +910,39 @@ static int launch_cd_hist(ser_run *run, const SumSel &sel, int k, double *c_sum,
   return SER_OK;
 }
 
+/* diversity curves of at most rows_max rows of each chain into slabs z at out[q] + z * stride (richness, originations, extinctions, site
+ * richness; any may be nullptr): passes of SER_DIV_CHUNK rows through a scratch buffer of 8 N bytes per chain and row, the first pass
+ * with `add`, the others adding */
+static int launch_diversity(ser_run *run, const SumSel &sel, int k, int rows_max, int *const out[4], size_t stride, int add)
+{
+  const int N = run->N, M = run->M, chunk = std::max(1, std::min(rows_max, SER_DIV_CHUNK));
+  uint16_t *scratch = nullptr;
+  auto passes = [&]() -> int {
+    HistShape hs;
+    CUDA_TRY(hist_shape((const void *)ser_div_hist_kernel, M + 1, &hs));
+    CUDA_TRY(POOL_ALLOC(&scratch, (size_t)k * chunk * 4 * N * sizeof(uint16_t)));
+    int t0 = 0;
+    do {
+      const int rows = std::min(chunk, rows_max - t0);
+      if (rows > 0) {
+        mark_launch(run);
+        ser_div_curve_kernel<<<dim3(rows, k), SER_DIV_THREADS, 0, run->stream>>>(run->d_samp_a, run->d_samp_b, run->d_samp_pi, run->d_scal, N,
+                                                                                 M, run->cfg.max_samples, sel, t0, scratch);
+        CUDA_TRY(cudaGetLastError());
+      }
+      mark_launch(run);
+      ser_div_hist_kernel<<<dim3(k, (N + hs.threads - 1) / hs.threads, 4), hs.threads, hs.smem, run->stream>>>(
+          scratch, run->d_scal, N, M, sel, t0, std::max(rows, 0), hs.smem > 0, out[0], out[1], out[2], out[3], stride, t0 > 0 || add);
+      CUDA_TRY(cudaGetLastError());
+      t0 += chunk;
+    } while (t0 < rows_max);
+    return SER_OK;
+  };
+  const int rc = passes();
+  if (scratch) cudaFreeAsync(scratch, run->stream);
+  return rc;
+}
+
 /* rows [0, w) of every chain's window added into its accumulator record (ser_run_accumulate), on the run's stream */
 static int accumulate_window(ser_run *run, int w)
 {
@@ -935,6 +968,11 @@ static int accumulate_window(ser_run *run, int w)
     const size_t R = cd_rows(run);
     double *sums = (double *)(acc + L.cd); /* L.cd and L.ints are even: 8-byte aligned */
     rc = launch_cd_hist(run, sel, nc, sums, sums + R, L.ints / 2, acc + L.cd + 4 * R, acc + L.cd + 4 * R + R * SER_CD_BINS, L.ints, 1);
+  }
+  if (!rc && (what & SER_ACC_DIV)) {
+    const size_t cells = (size_t)run->N * (run->M + 1);
+    int *const div[4] = {acc + L.div, acc + L.div + cells, acc + L.div + 2 * cells, acc + L.div + 3 * cells};
+    rc = launch_diversity(run, sel, nc, w, div, L.ints, 1);
   }
   return rc;
 }
@@ -1516,6 +1554,50 @@ extern "C" int ser_run_cd_marginals(ser_run *run, const int32_t *chosen, int32_t
       mark_launch(run);
       ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.cd + 4 * R, L.ints, cells, run->d_scal, sel,
                                                                         (int *)ch.dev, (int *)dh.dev);
+      CUDA_TRY(cudaGetLastError());
+    }
+    return SER_OK;
+  });
+  if (rc != SER_OK) return rc;
+  for (int q = 0; q < k; q++) n_samples[q] = n_out[q] < 0 ? 0 : n_out[q];
+  return SER_OK;
+}
+
+extern "C" int ser_run_diversity(ser_run *run, const int32_t *chosen, int32_t k, int32_t *richness, int32_t *originations,
+                                 int32_t *extinctions, int32_t *site_richness, int32_t *n_samples)
+{
+  if (!run || !chosen || !n_samples || k < 1 || (!richness && !originations && !extinctions && !site_richness)) {
+    ser_set_error("ser_run_diversity: bad argument (k = %d; chosen, n_samples and at least one of richness, originations, extinctions, "
+                  "site_richness are needed)", k);
+    return SER_E_ARG;
+  }
+  if (!run->initialized) { ser_set_error("ser_run_diversity: run not initialised"); return SER_E_STATE; }
+  if (run->cfg.store < SER_STORE_FULL) { ser_set_error("ser_run_diversity: needs SER_STORE_FULL (a, b and pi samples)"); return SER_E_STATE; }
+  if (run->acc_what && !(run->acc_what & SER_ACC_DIV)) { ser_set_error("ser_run_diversity: the run accumulates without SER_ACC_DIV"); return SER_E_STATE; }
+  if (set_device(run)) return SER_E_CUDA;
+  const size_t cells = (size_t)run->N * (run->M + 1);
+  GetterOut r = {richness, cells * sizeof(int), nullptr}, o = {originations, cells * sizeof(int), nullptr};
+  GetterOut e = {extinctions, cells * sizeof(int), nullptr}, st = {site_richness, cells * sizeof(int), nullptr};
+  std::vector<int> n_out;
+  const int rc = run_getter(run, chosen, k, n_out, {&r, &o, &e, &st}, [&](const int *d_ch, int *d_n) -> int {
+    int *const out[4] = {(int *)r.dev, (int *)o.dev, (int *)e.dev, (int *)st.dev};
+    if (!run->acc_what) {
+      /* the passes cover the longest store of the run's chains */
+      std::vector<ChainScalars> sc(run->cfg.n_chains);
+      CUDA_TRY(cudaMemcpyAsync(sc.data(), run->d_scal, sc.size() * sizeof(ChainScalars), cudaMemcpyDeviceToHost, run->stream));
+      CUDA_TRY(cudaStreamSynchronize(run->stream));
+      int rows = 0;
+      for (const ChainScalars &c : sc) rows = std::max(rows, std::min(c.n_samples, run->cfg.max_samples));
+      return launch_diversity(run, sel_chosen(run, d_ch, run->cfg.chain_offset, run->cfg.max_samples, d_n), k, rows, out, cells, 0);
+    }
+    /* the record's four parts in order, each pair one copy-out launch */
+    const AccLayout L = run_acc_layout(run);
+    const SumSel sel = sel_chosen(run, d_ch, run->cfg.chain_offset, INT_MAX, d_n);
+    for (int h = 0; h < 2; h++) {
+      if (!out[2 * h] && !out[2 * h + 1]) continue;
+      mark_launch(run);
+      ser_hist_acc_out_kernel<<<dim3(256, k, 2), 256, 0, run->stream>>>(run->d_acc + L.div + 2 * h * cells, L.ints, cells, run->d_scal, sel,
+                                                                        out[2 * h], out[2 * h + 1]);
       CUDA_TRY(cudaGetLastError());
     }
     return SER_OK;
